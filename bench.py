@@ -29,6 +29,12 @@ candidates (40 distinct device-resident sets, 4.8 GB), so that 20 steps time > 0
 
 `--impl reference` times that CPU port alone, all host threads, on the same workload; it never loads
 libcoverage_cuda (synth.py is imported by file path).
+
+`--dump-outputs DIR` writes what the last device-resident launch of the last timed step returned (rank 0):
+obj.npy and count.npy (float64) and feasible.npy (float32), one row per candidate.  The candidates come from
+the seeded device generator, so the same arguments give the same inputs on every run and two builds can be
+compared output for output.  Above 64 MB in all a fixed, seeded sample of the rows is written, with their
+row numbers in index.npy.
 """
 from __future__ import annotations
 
@@ -352,16 +358,40 @@ def device_resident(c, eng, wl, B, launches, steps, warmup, n_sets, seed0, sampl
         n_launch = eng.launch_count() - launches0
     kernel_ms = (ms1 - ms0) / max(l1 - l0, 1)
     key = kernel_key(eng.last_launch())
+    # every launch writes the same output buffers: they hold the last launch of the last step
     obj = np.empty(B)
     cnt = np.empty(B, dtype=np.int64)
+    fe = np.empty(B, dtype=np.uint8)
     eng.memcpy_d2h(obj, d_obj)
     eng.memcpy_d2h(cnt, d_cnt)
+    eng.memcpy_d2h(fe, d_fe)
     eng.sync()
     for p in dX + [d_obj, d_cnt, d_fe]:
         eng.device_free(p)
     dev_ms, kernel_ms = max_over_ranks(c, [dev_ms, kernel_ms])
     return dict(dev_ms=dev_ms, kernel_ms=kernel_ms, launches=int(n_launch), key=key, wall=(t_wall0, t_wall1),
-                count_sum=int(cnt.sum()), obj_finite=bool(np.isfinite(obj).all()))
+                count_sum=int(cnt.sum()), obj_finite=bool(np.isfinite(obj).all()),
+                outputs={"obj": obj, "count": cnt, "feasible": fe})
+
+
+DUMP_LIMIT_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir: str, outputs: dict, seed: int = 0):
+    """obj / count as float64 and feasible as float32, <name>.npy each (see the module docstring)."""
+    arrays = {"obj": outputs["obj"].astype(np.float64), "count": outputs["count"].astype(np.float64),
+              "feasible": outputs["feasible"].astype(np.float32)}
+    n = len(arrays["obj"])
+    row_bytes = sum(a.itemsize for a in arrays.values())
+    budget = DUMP_LIMIT_BYTES - 4096  # room for the .npy headers
+    if n * row_bytes > budget:
+        keep = budget // (row_bytes + 8)  # + 8: index.npy
+        idx = np.sort(np.random.default_rng(seed).choice(n, keep, replace=False))
+        arrays = {k: a[idx] for k, a in arrays.items()}
+        arrays["index"] = idx.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 def h2d_ceiling(c, eng, nbytes=120_000_000, reps=12, sets=4, d2h_bytes=0):
@@ -609,6 +639,7 @@ def c1_poll(c, cov, synth, steps=200):
 
 
 def main():
+    sys.dont_write_bytecode = True  # the tree may be read-only: leave no __pycache__ behind in it
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--steps", type=int, default=20)
@@ -622,6 +653,7 @@ def main():
     ap.add_argument("--no-extra", action="store_true", help="skip the C3 / C4 / C1 sub-runs")
     ap.add_argument("--no-e2e", action="store_true", help="device-resident measurement only (profiling)")
     ap.add_argument("--cpu-seconds", type=float, default=20.0)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed launch's outputs to DIR/<name>.npy")
     args = ap.parse_args()
     wl = dict(WORKLOADS[args.workload])
     named = args.batch in (0, wl["batch"]) and args.kernel == "auto"
@@ -664,6 +696,8 @@ def main():
     sampler = ClockSampler(c.local) if c.rank == 0 else None
     m = device_resident(c, eng, wl, B, L, args.steps, args.warmup, L, seed0=1 + c.rank, sampler=sampler)
     clocks = sampler.stop(*m["wall"]) if c.rank == 0 else None
+    if args.dump_outputs and c.rank == 0:
+        dump_outputs(args.dump_outputs, m["outputs"])
 
     # ---- host-facing ----
     e = None

@@ -955,15 +955,18 @@ def test_device_path_misaligned_and_odd_batches(cov, orc, engine):
         engine.device_free(d_obj)
 
 
-def test_bench_line_contract(cov):
-    """bench.py runs end to end on one GPU and prints ONE JSON line with the contract's keys."""
+def test_bench_line_contract(cov, tmp_path):
+    """bench.py runs end to end on one GPU and prints ONE JSON line with the contract's keys; --dump-outputs writes
+    the last timed launch's outputs."""
     import json
     import os
     import subprocess
     import sys
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    dump = str(tmp_path / "dump")
     r = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--steps", "2", "--warmup", "3", "--batch", "50000",
-                        "--launches", "3", "--cpu-seconds", "0.5"], capture_output=True, text=True, timeout=280, cwd=root)
+                        "--launches", "3", "--cpu-seconds", "0.5", "--dump-outputs", dump],
+                       capture_output=True, text=True, timeout=280, cwd=root)
     assert r.returncode == 0, r.stderr[-2000:]
     lines = [l for l in r.stdout.strip().splitlines() if l.startswith("{")]
     assert len(lines) == 1
@@ -989,6 +992,11 @@ def test_bench_line_contract(cov):
         assert ex[k]["roofline"]["bound"] == "issue" and 0 < ex[k]["roofline"]["frac"] < 1.0, ex[k]["roofline"]
         assert ex[k]["kernel"].startswith("span_cta_kernel<") and ex[k]["value"] > 0
     assert ex["C1"]["poll_latency_us"] > 0 and ex["C1"]["mads_solve_ms"] > 0
+    out = {f[:-4]: np.load(os.path.join(dump, f)) for f in os.listdir(dump)}
+    assert set(out) == {"obj", "count", "feasible"} and all(len(a) == 50000 for a in out.values())
+    assert out["obj"].dtype == np.float64 and out["count"].dtype == np.float64 and out["feasible"].dtype == np.float32
+    assert out["count"].sum() == d["check"]["count_sum_last_launch"] and np.isfinite(out["obj"]).all()
+    assert set(np.unique(out["feasible"])) <= {0.0, 1.0}
 
 
 def test_reference_arm_does_not_load_the_product_library():

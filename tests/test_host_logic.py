@@ -124,6 +124,45 @@ def test_bench_issue_roofline_helpers(tmp_path, monkeypatch):
     assert len(bench.source_sha()) == 16 and bench.source_sha() == bench.source_sha()
 
 
+def test_bench_dump_outputs(tmp_path):
+    """bench.py --dump-outputs: obj / count as float64 and feasible as float32, one row per candidate; above 64 MB in
+    all, the same seeded sample of rows on every run, with their row numbers in index.npy."""
+    import importlib.util
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    spec = importlib.util.spec_from_file_location("bench_under_test", os.path.join(root, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    rng = np.random.default_rng(3)
+
+    def outputs(n):
+        return {"obj": rng.normal(size=n), "count": rng.integers(0, 1 << 16, n),
+                "feasible": rng.integers(0, 2, n).astype(np.uint8)}
+
+    def load(d):
+        return {f[:-4]: np.load(os.path.join(d, f)) for f in sorted(os.listdir(d))}
+
+    small = outputs(1000)
+    bench.dump_outputs(str(tmp_path / "small"), small)
+    got = load(tmp_path / "small")
+    assert set(got) == {"obj", "count", "feasible"}
+    assert got["obj"].dtype == np.float64 and got["count"].dtype == np.float64 and got["feasible"].dtype == np.float32
+    for k in got:
+        assert np.array_equal(got[k], small[k]), k
+
+    n = bench.DUMP_LIMIT_BYTES // 20 + 12345  # 20 bytes per row once widened: just over the limit
+    big = outputs(n)
+    bench.dump_outputs(str(tmp_path / "a"), big)
+    bench.dump_outputs(str(tmp_path / "b"), big)
+    a, b = load(tmp_path / "a"), load(tmp_path / "b")
+    assert set(a) == {"obj", "count", "feasible", "index"} and all(np.array_equal(a[k], b[k]) for k in a)
+    assert sum(os.path.getsize(os.path.join(tmp_path, "a", f)) for f in os.listdir(tmp_path / "a")) <= bench.DUMP_LIMIT_BYTES
+    idx = a["index"].astype(np.int64)
+    assert np.array_equal(idx.astype(np.float64), a["index"]) and np.all(np.diff(idx) > 0) and idx[-1] < n
+    assert len(idx) > n // 2
+    for k in ("obj", "count", "feasible"):
+        assert np.array_equal(a[k], big[k][idx]), k
+
+
 def test_pack_candidates_is_lossless_or_refuses(cov):
     """Mesh indices for cov_eval_batch_packed: what the device computes from them, (double)q * granularity, must be the
     caller's Float64 candidates bit for bit -- pack_candidates checks exactly that and refuses anything else."""
