@@ -35,7 +35,8 @@ extern "C" {
 #endif
 
 #define COV_ABI_VERSION 3 /* 2: COV_OPT_PROGRESSIVE_INDEX, COV_KERNEL_ORDERED, cov_get_class_weights, cov_eval_batch_best;
-                             3: cov_eval_batch_packed (COV_PACK_*) */
+                             3: cov_eval_batch_packed (COV_PACK_*); later, with no existing symbol changed:
+                                cov_mads_solve_batch */
 
 #if defined(__GNUC__)
 #define COV_API __attribute__((visibility("default")))
@@ -244,6 +245,29 @@ COV_API int cov_eval_batch_packed(cov_handle *h, const void *Q, int32_t pack, do
  * polling, one launch per poll set. stats (nullable): iterations, evaluations, batches, successes. */
 COV_API int cov_mads_solve(cov_handle *h, const double *x0, int64_t n_iter, double granularity, uint64_t seed,
                            double *x_out, double *obj_out, int64_t *stats);
+
+/* S independent MADS solves on the device, one kernel launch for all of them (multi-start: MADS is a local method).
+ * Each CTA owns one solve from its first evaluation to its result; the host uploads the starts once, downloads the
+ * results once and synchronises once.  X0, X_out: S x 3N in the candidate layout; obj_out (nullable): S values;
+ * stats (nullable): S x 4 values [iterations, evaluations, successes, converged] -- converged = 1 when the solve
+ * stopped because the mesh could not refine any further, 0 when it reached n_iter.  S == 0 does nothing.
+ * Settings and results as cov_mads_solve: the constraints of cov_set_params as extreme barrier, one granularity on
+ * every variable (0: continuous), X_out[k] = the feasible incumbent if one was found, else X0[k], obj_out[k] = its
+ * barrier value (+Inf when no feasible point was found).  The loop is cov_mads_solve's in the same FP64 operations,
+ * with two differences:
+ *  - directions: solve k uses Philox4x32-10 keyed by (low, high 32 bits of seed + k mod 2^64).  At iteration t
+ *    (0-based), variable i takes the 12 words of the blocks with counter (t low 32, t high 32, i, g), g = 0, 1, 2,
+ *    summed as a uint64 s; v_i = s * 2^-32 - 6.0 (an Irwin-Hall(12) normal, mean 0, variance 1, exact in binary64);
+ *    v /= sqrt(sum of v_i^2 summed in index order).  Powers of ten and the initial mesh are computed by the host's
+ *    libm, so every iterate can be replayed on a host;
+ *  - no cache and no duplicate removal: every kept poll point is evaluated (the winner, the first strict minimum in
+ *    generation order -- sign + for columns 0..n-1, then sign -, is the same); evaluations counts them and x0.
+ * Limits: N <= 64 (384 poll points per iteration) and a grid whose framebuffer (ny x stride words) fits one warp's
+ * share of shared memory, else COV_ERR_LIMIT.  COV_OPT_FORCE_EXACT is honoured, COV_OPT_KERNEL does not apply
+ * (stores with area_exact == 0 use the list-order sum, as every evaluation does).  cov_launch_count counts the
+ * launch; cov_last_launch and the kernel timers are left unchanged. */
+COV_API int cov_mads_solve_batch(cov_handle *h, const double *X0, int64_t S, int64_t n_iter, double granularity,
+                                 uint64_t seed, double *X_out, double *obj_out, int64_t *stats);
 
 /* Covered-cell mask of ONE candidate: nx*ny bytes, 1 where the cell is inside some disc (whether
  * or not it holds entries). Lets the host replay an ordered Float64 sum over a weighted list. */

@@ -55,6 +55,15 @@ class AreaMaxObjective:
         res, eng = self._engine()
         return eng.mads_solve
 
+    def native_batch_solver(self, constraints):
+        """A callable (X0, n_iter, granularity, seed) -> (X, objectives, stats) running cov_mads_solve_batch (S solves
+        in one launch, solve k seeded seed + k) with these extreme constraints fused, or None when a constraint cannot
+        be fused."""
+        if self.fuse(constraints):
+            return None
+        res, eng = self._engine()
+        return eng.mads_solve_batch
+
     def _engine(self):
         res = self._resident()
         eng = res.sync()

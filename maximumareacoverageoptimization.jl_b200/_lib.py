@@ -77,6 +77,7 @@ SIGNATURES = {
     "cov_argmin": (_i, [_vp, _vp, _i64, C.c_int32, _pd, _pi64]),
     "cov_union_area_batch": (_i, [_vp, _vp, _i64, _i64, _vp]),
     "cov_mads_solve": (_i, [_vp, _vp, _i64, _d, C.c_uint64, _vp, _pd, _pi64]),
+    "cov_mads_solve_batch": (_i, [_vp, _vp, _i64, _i64, _d, C.c_uint64, _vp, _vp, _vp]),
     "cov_covered_mask": (_i, [_vp, _vp, _vp]),
     "cov_sync": (_i, [_vp]),
     "cov_stream": (_vp, [_vp]),

@@ -172,6 +172,7 @@ struct cov_handle {
     // evaluation window (device) and staging (pinned host)
     DevBuf dX, d_obj, d_count, d_feas, d_clscnt, d_prog;
     DevBuf d_raw[2]; // packed slices as they arrive (cov_eval_batch_packed), widened into dX
+    DevBuf mads_in, mads_out; // cov_mads_solve_batch: starts, initial meshes, powers of ten / results
     void *h_in[2] = {nullptr, nullptr};
     size_t h_in_cap = 0;
     void *h_out = nullptr;
@@ -423,7 +424,7 @@ extern "C" void cov_destroy(cov_handle *h)
     DevBuf *bufs[] = {&h->mult, &h->cls, &h->planes, &h->planes_q, &h->params, &h->counter, &h->stats, &h->xyT,
                       &h->small_in, &h->argmin_obj, &h->argmin_idx, &h->removed, &h->overflow, &h->dX,
                       &h->d_obj, &h->d_count, &h->d_feas, &h->d_clscnt, &h->d_prog, &h->fire[0], &h->fire[1], &h->fire_p,
-                      &h->backup, &h->ent_cell, &h->ent_cls, &h->d_raw[0], &h->d_raw[1]};
+                      &h->backup, &h->ent_cell, &h->ent_cls, &h->d_raw[0], &h->d_raw[1], &h->mads_in, &h->mads_out};
     for (DevBuf *b : bufs)
         if (b->p) cudaFree(b->p);
     for (int k = 0; k < 2; ++k)
@@ -1217,6 +1218,17 @@ extern "C" int cov_set_params(cov_handle *h, int64_t N, const double *r_max, dou
 // ------------------------------------------------------------------------------------------
 // evaluation
 // ------------------------------------------------------------------------------------------
+// A fresh zeroed slot of the counter ring (the work dispenser of one launch on the main stream).
+static int take_counter(cov_handle *h, unsigned long long **counter)
+{
+    if (h->counter_next >= kCounterSlots) { // ring used up: zero it again (stream-ordered after its last user)
+        CK(cudaMemsetAsync(h->counter.p, 0, kCounterSlots * sizeof(unsigned long long), h->stream));
+        h->counter_next = 0;
+    }
+    *counter = (unsigned long long *)h->counter.p + h->counter_next++;
+    return COV_OK;
+}
+
 static int launch_on_main(cov_handle *h, const double *dX, int64_t B, const EvalOut &out, bool timed)
 {
     h->cfg.ordered = h->area_exact ? 0 : 1; // non-dyadic weights: the sum is replayed in list order
@@ -1227,13 +1239,9 @@ static int launch_on_main(cov_handle *h, const double *dX, int64_t B, const Eval
         e1 = get_event(h);
         CK(cudaEventRecord(e0, h->stream));
     }
-    if (h->counter_next >= kCounterSlots) { // ring used up: zero it again (stream-ordered after its last user)
-        CK(cudaMemsetAsync(h->counter.p, 0, kCounterSlots * sizeof(unsigned long long), h->stream));
-        h->counter_next = 0;
-    }
-    cudaError_t e = launch_eval(h->g, h->o, h->cfg, dX, (long long)B, out,
-                                (unsigned long long *)h->counter.p + h->counter_next++,
-                                h->stream, &h->last_info);
+    unsigned long long *counter = nullptr;
+    OK(take_counter(h, &counter));
+    cudaError_t e = launch_eval(h->g, h->o, h->cfg, dX, (long long)B, out, counter, h->stream, &h->last_info);
     if (e != cudaSuccess) {
         if (timed) {
             h->ev_pool.push_back(e0);
@@ -1760,6 +1768,14 @@ struct MeshVar {
     double a;
     int b, b0;
 };
+// initial poll size: about |x0_i| / 10 (at least 1), on the {1, 2, 5} x 10^b ladder
+MeshVar initial_mesh(double x0, double g)
+{
+    const double target = std::max(std::max(std::fabs(x0) / 10.0, 1.0), g);
+    const int b = (int)std::floor(std::log10(target));
+    const double mant = target / std::pow(10.0, b);
+    return {mant < 2 ? 1.0 : (mant < 5 ? 2.0 : 5.0), b, b};
+}
 } // namespace
 
 extern "C" int cov_mads_solve(cov_handle *h, const double *x0, int64_t n_iter, double granularity, uint64_t seed,
@@ -1811,12 +1827,7 @@ extern "C" int cov_mads_solve(cov_handle *h, const double *x0, int64_t n_iter, d
     double fx = f[0];
     bool feasible_found = std::isfinite(fx);
     std::vector<MeshVar> mesh((size_t)n);
-    for (int i = 0; i < n; ++i) { // initial poll size: about |x0_i| / 10 (at least 1), on the {1, 2, 5} x 10^b ladder
-        const double target = std::max(std::max(std::fabs(x[i]) / 10.0, 1.0), g);
-        const int b = (int)std::floor(std::log10(target));
-        const double mant = target / std::pow(10.0, b);
-        mesh[i] = {mant < 2 ? 1.0 : (mant < 5 ? 2.0 : 5.0), b, b};
-    }
+    for (int i = 0; i < n; ++i) mesh[i] = initial_mesh(x[i], g);
     Rng rng{seed * 0x9E3779B97F4A7C15ull + 0x1234567ull};
     std::vector<double> v((size_t)n), H((size_t)n * n), delta((size_t)n), rho((size_t)n);
     for (int64_t it = 0; it < n_iter; ++it) {
@@ -1906,6 +1917,73 @@ extern "C" int cov_mads_solve(cov_handle *h, const double *x0, int64_t n_iter, d
         stats[2] = batches;
         stats[3] = successes;
     }
+    return COV_OK;
+}
+
+// S solves of the same loop on the device, one launch for all of them (cov_mads.cu).  The host contributes what
+// must carry its libm's bits: the initial mesh of every start and the table of powers of ten.
+extern "C" int cov_mads_solve_batch(cov_handle *h, const double *X0, int64_t S, int64_t n_iter, double granularity,
+                                    uint64_t seed, double *X_out, double *obj_out, int64_t *stats)
+{
+    if (!h) return fail(nullptr, COV_ERR_INVALID, "NULL handle");
+    DeviceGuard dg(h->device);
+    OK(check_ready(h, "cov_mads_solve_batch"));
+    if (S < 0 || n_iter < 0 || !(granularity >= 0) || (S > 0 && (!X0 || !X_out)))
+        return fail(h, COV_ERR_INVALID, "cov_mads_solve_batch: bad arguments");
+    if (S == 0) return COV_OK;
+    const int N = h->o.N, n = 3 * N;
+    int warps = 0, smem = 0, planes_smem = 0;
+    if (N > kMadsMaxUavs)
+        return fail(h, COV_ERR_LIMIT, "cov_mads_solve_batch: N = " + std::to_string(N) + " exceeds the " +
+                                          std::to_string(kMadsMaxUavs) + " UAVs of the solver's launch plan");
+    if (!mads_plan(h->g, N, h->cfg, &warps, &smem, &planes_smem))
+        return fail(h, COV_ERR_LIMIT, "cov_mads_solve_batch: one warp's framebuffer of the " + std::to_string(h->g.nx) +
+                                          " x " + std::to_string(h->g.ny) + " grid does not fit the " +
+                                          std::to_string(h->cfg.max_smem_optin) + " bytes of shared memory per CTA");
+    if (!h->area_exact) OK(entries_on_device(h)); // non-dyadic weights: the list-order sum
+    // in: [pow10: 801 doubles | X0: S n doubles | a0: S n doubles | b0: S n ints]; out: [X_out | obj | stats]
+    constexpr int kPow = 1 - 2 * kMadsPow10Min;
+    const size_t sn = (size_t)S * n;
+    const size_t o_x = (size_t)kPow * 8, o_a = o_x + sn * 8, o_b = o_a + sn * 8, in_bytes = o_b + sn * 4;
+    const size_t o_obj = sn * 8, o_st = o_obj + (size_t)S * 8, out_bytes = o_st + (size_t)S * 4 * 8;
+    std::vector<unsigned char> hin(in_bytes), hout(out_bytes);
+    double *p10 = (double *)hin.data(), *ha = (double *)(hin.data() + o_a);
+    int *hb = (int *)(hin.data() + o_b);
+    for (int b = kMadsPow10Min; b <= -kMadsPow10Min; ++b) p10[b - kMadsPow10Min] = std::pow(10.0, b);
+    memcpy(hin.data() + o_x, X0, sn * 8);
+    for (size_t q = 0; q < sn; ++q) {
+        const MeshVar m = initial_mesh(X0[q], granularity);
+        ha[q] = m.a;
+        hb[q] = m.b;
+    }
+    OK(ensure(h, h->mads_in, in_bytes));
+    OK(ensure(h, h->mads_out, out_bytes));
+    unsigned char *din = (unsigned char *)h->mads_in.p, *dout = (unsigned char *)h->mads_out.p;
+    CK(cudaMemcpyAsync(din, hin.data(), in_bytes, cudaMemcpyHostToDevice, h->stream));
+    MadsArgs a{};
+    a.pow10 = (const double *)din;
+    a.X0 = (const double *)(din + o_x);
+    a.a0 = (const double *)(din + o_a);
+    a.b0 = (const int *)(din + o_b);
+    a.X_out = (double *)dout;
+    a.obj_out = (double *)(dout + o_obj);
+    a.stats = (long long *)(dout + o_st);
+    a.S = S;
+    a.n_iter = n_iter;
+    a.granularity = granularity;
+    a.seed = seed;
+    a.force_exact = h->cfg.force_exact;
+    a.ordered = h->area_exact ? 0 : 1;
+    unsigned long long *counter = nullptr;
+    OK(take_counter(h, &counter));
+    cudaError_t e = launch_mads(h->g, h->o, h->cfg, a, counter, h->stream);
+    if (e != cudaSuccess) return fail_cuda(h, e, "cov_mads_solve_batch: kernel launch");
+    h->launches += 1;
+    CK(cudaMemcpyAsync(hout.data(), dout, out_bytes, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    memcpy(X_out, hout.data(), sn * 8);
+    if (obj_out) memcpy(obj_out, hout.data() + o_obj, (size_t)S * 8);
+    if (stats) memcpy(stats, hout.data() + o_st, (size_t)S * 4 * 8);
     return COV_OK;
 }
 

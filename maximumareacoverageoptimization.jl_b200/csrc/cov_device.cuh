@@ -126,6 +126,30 @@ __device__ __forceinline__ double radicand(double px, double py, double cx, doub
     const double ddy = __dsub_rn(py, cy);
     return __dadd_rn(__dmul_rn(ddx, ddx), __dmul_rn(ddy, ddy));
 }
+
+// Philox4x32-10 (Salmon et al., SC'11): counter (c0..c3), key (k0, k1) -> 4 words.  The stream of the candidate
+// generator, the fire automaton and the device MADS solver's directions; synth._philox restates it in NumPy.
+__device__ __forceinline__ void philox4x32_10(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3, uint32_t k0,
+                                              uint32_t k1, uint32_t out[4])
+{
+    const uint32_t M0 = 0xD2511F53u, M1 = 0xCD9E8D57u, W0 = 0x9E3779B9u, W1 = 0xBB67AE85u;
+#pragma unroll
+    for (int r = 0; r < 10; ++r) {
+        const uint32_t hi0 = __umulhi(M0, c0), lo0 = M0 * c0;
+        const uint32_t hi1 = __umulhi(M1, c2), lo1 = M1 * c2;
+        const uint32_t n0 = hi1 ^ c1 ^ k0, n1 = lo1, n2 = hi0 ^ c3 ^ k1, n3 = lo0;
+        c0 = n0;
+        c1 = n1;
+        c2 = n2;
+        c3 = n3;
+        k0 += W0;
+        k1 += W1;
+    }
+    out[0] = c0;
+    out[1] = c1;
+    out[2] = c2;
+    out[3] = c3;
+}
 #endif
 
 } // namespace cov

@@ -387,28 +387,8 @@ cudaError_t launch_argmin(const double *obj, const unsigned char *feasible, long
 }
 
 // ---- synthetic candidates on the device: Philox4x32-10, counter = (index lo, index hi, uav, draw),
-//      key = (seed lo, seed hi). The host reproduces the same stream (synth.py). ----
-__device__ __forceinline__ void philox4x32_10(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3, uint32_t k0,
-                                              uint32_t k1, uint32_t out[4])
-{
-    const uint32_t M0 = 0xD2511F53u, M1 = 0xCD9E8D57u, W0 = 0x9E3779B9u, W1 = 0xBB67AE85u;
-#pragma unroll
-    for (int r = 0; r < 10; ++r) {
-        const uint32_t hi0 = __umulhi(M0, c0), lo0 = M0 * c0;
-        const uint32_t hi1 = __umulhi(M1, c2), lo1 = M1 * c2;
-        const uint32_t n0 = hi1 ^ c1 ^ k0, n1 = lo1, n2 = hi0 ^ c3 ^ k1, n3 = lo0;
-        c0 = n0;
-        c1 = n1;
-        c2 = n2;
-        c3 = n3;
-        k0 += W0;
-        k1 += W1;
-    }
-    out[0] = c0;
-    out[1] = c1;
-    out[2] = c2;
-    out[3] = c3;
-}
+//      key = (seed lo, seed hi). The host reproduces the same stream (synth.py); philox4x32_10 is in
+//      cov_device.cuh. ----
 __device__ __forceinline__ double u01_53(uint32_t a, uint32_t b)
 {
     // 53 random bits -> [0, 1)

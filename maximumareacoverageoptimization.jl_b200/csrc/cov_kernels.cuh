@@ -46,6 +46,29 @@ cudaError_t launch_span_cta(const GridDesc &g, const ObjParams &o, const LaunchC
                             long long B, const EvalOut &out, unsigned long long *counter, cudaStream_t stream,
                             LaunchInfo *info);
 
+// ---- the device MADS solver (cov_mads.cu): S independent solves, one persistent CTA per solve at a time ----
+constexpr int kMadsMaxUavs = 64;    // N of the launch plan (2 * 3N = 384 poll points per iteration)
+constexpr int kMadsPow10Min = -400; // pow10 holds 10^b for b in [kMadsPow10Min, -kMadsPow10Min]; clamped outside
+struct MadsArgs {
+    const double *X0;        // S x n start points (n = 3N)
+    const double *a0;        // S x n initial poll-size mantissas (1, 2 or 5)
+    const int *b0;           // S x n initial poll-size exponents
+    const double *pow10;     // 10^b as the host's libm computes it, b = kMadsPow10Min .. -kMadsPow10Min
+    double *X_out;           // S x n
+    double *obj_out;         // S
+    long long *stats;        // S x 4: iterations, evaluations, successes, converged
+    long long S, n_iter;
+    double granularity;
+    unsigned long long seed; // solve k uses the Philox key seed + k
+    int force_exact;
+    int ordered;             // 1: the list-order Float64 sum (cov_grid_info.area_exact == 0)
+};
+// Shared-memory plan of the solver for this store and swarm size: warps per CTA and dynamic bytes; false when
+// not even one warp's framebuffer fits (or N > kMadsMaxUavs).
+bool mads_plan(const GridDesc &g, int N, const LaunchCfg &cfg, int *warps, int *smem, int *planes_smem);
+cudaError_t launch_mads(const GridDesc &g, const ObjParams &o, const LaunchCfg &cfg, const MadsArgs &a,
+                        unsigned long long *counter, cudaStream_t stream);
+
 // ---- cell-store kernels (cov_grid_kernels.cu) ----
 // stats[0] = entries, stats[1] = cells, stats[2 + k] = OR of the multiplicities of class k
 cudaError_t launch_grid_stats(const unsigned char *mult, const unsigned char *cls, long long ncell,

@@ -1,0 +1,375 @@
+// cov_mads.cu -- the device-resident multi-start MADS solver of libcoverage_cuda (sm_100a): S independent solves
+// in ONE launch (cov_mads_solve_batch).
+//
+// Persistent CTAs take solves from an atomic dispenser; a CTA runs one solve from its first evaluation to its
+// result, then takes the next.  No CTA talks to another.  Per iteration of a solve:
+//   1. warp 0 draws the Householder vector v (Irwin-Hall(12) normals from Philox, see coverage_cuda.h) and
+//      normalises it; every thread sets the mesh and poll sizes of its variables;
+//   2. __syncthreads;
+//   3. warp w builds poll points k = w, w + W, ... (column k mod n of I - 2 v v^T, scaled, rounded onto the mesh,
+//      sign + for k < n, - after) into its own stage and applies cov_mads_solve's drop rules;
+//   4. the warp evaluates every kept point (candidate_prologue, then the row spans of make_sdisc / fast_span /
+//      slow_item painted into the warp's framebuffer, or the list-order loop for non-dyadic weights) and stores
+//      the barrier value f[k] (NaN marks a dropped point);
+//   5. __syncthreads;
+//   6. thread 0 picks the first strict minimum in generation order; the incumbent is re-built from its index
+//      (the same arithmetic, so the same bits) and the mesh enlarged, or the mesh refined / the solve stopped.
+// Everything is cov_mads_solve's loop (cov_api.cu) in the same FP64 operations and order, so a host model can
+// replay every iterate bit for bit; only the direction stream and the absence of a cache differ.
+#include <cuda_runtime.h>
+#include <algorithm>
+#include <cstdint>
+#include "cov_device.cuh"
+#include "cov_kernel_common.cuh"
+#include "cov_candidate.cuh"
+#include "cov_span_common.cuh"
+#include "cov_kernels.cuh"
+
+namespace cov {
+
+constexpr int kMadsThreads = 256; // 8 warps: 30 poll points of a 5-UAV swarm are 4 rounds of one point per warp
+constexpr int kMadsCtas = 2;      // co-resident CTAs per SM the register budget is compiled for
+
+// Shared memory of a CTA: [planes (optional)] [solve state] [W x per-warp] [mbarrier]
+__host__ __device__ inline int mads_state_bytes(int n) { return round_up(7 * n * 8 + 2 * n * 4, 16) + 64; }
+__host__ __device__ inline int mads_fb_bytes(const GridDesc &g, int N)
+{
+    const int fb = round_up(g.ny * g.stride * 4, 16), ts = round_up(N * 8, 16);
+    return fb > ts ? fb : ts; // the list-order path keeps the N thresholds there instead
+}
+__host__ __device__ inline int mads_warp_bytes(const GridDesc &g, int N)
+{
+    return round_up(3 * N * 8, 16) + N * 32 + round_up(N * 4, 16) + mads_fb_bytes(g, N);
+}
+
+struct MadsShared {
+    double fx, nrm;
+    unsigned long long solve;
+    int kb, feasible_found;
+};
+
+__device__ __forceinline__ double max_host(double a, double b) { return (a < b) ? b : a; } // std::max
+
+__device__ __forceinline__ double pow10_of(const MadsArgs &a, int b)
+{
+    b = b < kMadsPow10Min ? kMadsPow10Min : (b > -kMadsPow10Min ? -kMadsPow10Min : b);
+    return __ldg(a.pow10 + (b - kMadsPow10Min));
+}
+
+// v_i = (sum of the 12 words of the blocks (t lo, t hi, i, 0..2)) * 2^-32 - 6: exact in binary64
+__device__ __forceinline__ double irwin_hall(uint32_t k0, uint32_t k1, unsigned long long t, int i)
+{
+    unsigned long long s = 0;
+#pragma unroll
+    for (uint32_t q = 0; q < 3; ++q) {
+        uint32_t r[4];
+        philox4x32_10((uint32_t)t, (uint32_t)(t >> 32), (uint32_t)i, q, k0, k1, r);
+        s += (unsigned long long)r[0] + r[1] + r[2] + r[3];
+    }
+    return __dsub_rn(__dmul_rn((double)s, 2.3283064365386962890625e-10), 6.0);
+}
+
+// Poll point kk (column kk mod n, sign + for kk < n) of cov_mads_solve, built by one warp into dst (which may be x
+// itself).  Returns whether cov_mads_solve keeps it: some rounded direction component is non-zero and the snapped
+// point differs from x.
+__device__ __forceinline__ bool poll_point(int kk, int n, const double *x, const double *v, const double *rho,
+                                           const double *delta, double gran, double *dst)
+{
+    const uint32_t lane = lane_id();
+    const bool neg = kk >= n;
+    const int j = neg ? kk - n : kk;
+    const double sgn = neg ? -1.0 : 1.0;
+    const double vj = v[j];
+    double hmax = 0.0; // a maximum of non-NaN values (NaN components never win std::max), so any order gives it
+    for (int i = lane; i < n; i += 32) {
+        const double H = __dsub_rn(i == j ? 1.0 : 0.0, __dmul_rn(__dmul_rn(2.0, v[i]), vj));
+        hmax = max_host(hmax, fabs(H));
+    }
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) hmax = max_host(hmax, __shfl_xor_sync(0xffffffffu, hmax, off));
+    bool any = false, moved = false;
+    for (int i = lane; i < n; i += 32) {
+        const double H = __dsub_rn(i == j ? 1.0 : 0.0, __dmul_rn(__dmul_rn(2.0, v[i]), vj));
+        const double d = rint(__ddiv_rn(__dmul_rn(rho[i], H), hmax));
+        any |= d != 0.0;
+        const double xi = x[i];
+        double p = __dadd_rn(xi, __dmul_rn(__dmul_rn(sgn, d), delta[i]));
+        if (gran > 0) p = __dmul_rn(rint(__ddiv_rn(p, gran)), gran);
+        moved |= p != xi;
+        dst[i] = p;
+    }
+    return __any_sync(0xffffffffu, any) && __any_sync(0xffffffffu, moved);
+}
+
+// The objective with the extreme barrier for the candidate in `stage`, by one warp: +Inf where a fused constraint
+// fails (its coverage is never counted) or the objective is NaN.  fb: the warp's framebuffer, all-zero on entry and
+// on return (the list-order path keeps the thresholds there instead and never paints it).
+template <bool MULTI, bool PLANES_SMEM>
+__device__ double mads_eval(const GridDesc &g, const ObjParams &o, const double *stage, SDisc *sd, int *pre,
+                            uint32_t *fb, const uint32_t *planes, int force_exact, int ordered)
+{
+    const int N = o.N;
+    const uint32_t lane = lane_id();
+    const CandScalars cs = candidate_prologue<false>(g, o, stage, nullptr, false);
+    if (!cs.feasible) return __longlong_as_double(0x7ff0000000000000ll);
+    double obj;
+    long long cls[kMaxClasses];
+    if (ordered) {
+        double *Ts = reinterpret_cast<double *>(fb);
+        for (int c = lane; c < N; c += 32) Ts[c] = threshold(stage[2 * N + c]);
+        __syncwarp();
+        const double area = ordered_area(g, N, stage, Ts, cls);
+        __syncwarp();
+        obj = __dadd_rn(-area, __dmul_rn(cs.violation, o.penalty_scale));
+    } else {
+        for (int c = lane; c < N; c += 32) make_sdisc(g, stage[c], stage[N + c], stage[2 * N + c], sd[c]);
+        __syncwarp();
+        // (disc, row) items flattened over the lanes: inclusive prefix of the discs' row counts, and the rows the
+        // framebuffer has to be cleared on afterwards
+        int total = 0, rmin = g.ny + 1, rmax = 0;
+        if (lane == 0) {
+            for (int c = 0; c < N; ++c) {
+                const int r0 = (int)(sd[c].rows & 0xffffu), r1 = (int)(sd[c].rows >> 16);
+                if (r1 >= r0) {
+                    total += r1 - r0 + 1;
+                    rmin = min(rmin, r0);
+                    rmax = max(rmax, r1);
+                }
+                pre[c] = total;
+            }
+        }
+        total = __shfl_sync(0xffffffffu, total, 0);
+        rmin = __shfl_sync(0xffffffffu, rmin, 0);
+        rmax = __shfl_sync(0xffffffffu, rmax, 0);
+        __syncwarp();
+        uint32_t cnt[MULTI ? kMaxClasses : 1];
+#pragma unroll
+        for (int k = 0; k < (MULTI ? kMaxClasses : 1); ++k) cnt[k] = 0;
+        const FbLayout fl{g.stride, 0};
+        for (int tb = 0; tb < total; tb += 32) {
+            const int t = tb + (int)lane;
+            const bool has = t < total;
+            int c = 0;
+            if (has)
+                while (pre[c] <= t) ++c;
+            const SDisc d = sd[c];
+            const int j = has ? (int)(d.rows & 0xffffu) + t - (c ? pre[c - 1] : 0) : 1;
+            int lo, hi;
+            int st = fast_span(g, d, j, force_exact, lo, hi);
+            if (!has) st = kEmpty;
+            if (st == kSlow) {
+                slow_item(g, stage, N, c, j, (d.flags & 1u) || force_exact, lo, hi);
+                if (lo <= hi) st = kSpan;
+                else {
+                    st = kEmpty;
+                    lo = hi = 1;
+                }
+            }
+            // every disc goes through the framebuffer: a lane counts only the bits it was first to set
+            paint_span<MULTI, PLANES_SMEM>(g, fb, planes, j, lo, hi, st == kSpan, true, cnt, 1, fl);
+        }
+        __syncwarp();
+        if (rmax >= rmin)
+            for (int w = (rmin - 1) * g.stride + (int)lane; w < rmax * g.stride; w += 32) fb[w] = 0u;
+        __syncwarp();
+#pragma unroll
+        for (int k = 0; k < kMaxClasses; ++k)
+            cls[k] = k < (MULTI ? kMaxClasses : 1) ? (long long)__reduce_add_sync(0xffffffffu, cnt[MULTI ? k : 0]) : 0;
+        obj = assemble_objective(g, o, cls, cs.violation);
+    }
+    return (obj == obj) ? obj : __longlong_as_double(0x7ff0000000000000ll);
+}
+
+template <bool MULTI, bool PLANES_SMEM, int THREADS, int CTAS>
+__global__ void __launch_bounds__(THREADS, CTAS)
+mads_kernel(const __grid_constant__ GridDesc g, const __grid_constant__ ObjParams o, const __grid_constant__ MadsArgs a,
+            unsigned long long *counter)
+{
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    const int W = blockDim.x >> 5;
+    const int warp = threadIdx.x >> 5;
+    const uint32_t lane = lane_id();
+    const int N = o.N, n = 3 * N;
+    const int planes_bytes = PLANES_SMEM ? g.n_planes * g.plane_words * 4 : 0;
+    const int warp_bytes = mads_warp_bytes(g, N);
+    uint32_t *planes_s = reinterpret_cast<uint32_t *>(smem_raw);
+    unsigned char *sbase = smem_raw + planes_bytes;
+    double *x = reinterpret_cast<double *>(sbase);
+    double *v = x + n, *rho = v + n, *delta = rho + n, *am = delta + n, *f = am + n; // f: 2n
+    int *bm = reinterpret_cast<int *>(f + 2 * n), *bz = bm + n;
+    MadsShared *sh = reinterpret_cast<MadsShared *>(sbase + round_up(7 * n * 8 + 2 * n * 4, 16));
+    unsigned char *wbase = sbase + mads_state_bytes(n) + (size_t)warp * warp_bytes;
+    double *stage = reinterpret_cast<double *>(wbase);
+    SDisc *sd = reinterpret_cast<SDisc *>(wbase + round_up(3 * N * 8, 16));
+    int *pre = reinterpret_cast<int *>(wbase + round_up(3 * N * 8, 16) + N * 32);
+    uint32_t *fb = reinterpret_cast<uint32_t *>(wbase + round_up(3 * N * 8, 16) + N * 32 + round_up(N * 4, 16));
+    uint64_t *bar = reinterpret_cast<uint64_t *>(sbase + mads_state_bytes(n) + (size_t)W * warp_bytes);
+
+    if (PLANES_SMEM) stage_planes(g, planes_s, bar, planes_bytes); // TMA bulk copy, once per CTA (syncs)
+    const uint32_t *planes = PLANES_SMEM ? planes_s : g.planes;
+    for (int t = lane; t < mads_fb_bytes(g, N) / 16; t += 32) reinterpret_cast<uint4 *>(fb)[t] = make_uint4(0, 0, 0, 0);
+    __syncwarp();
+    const double gran = a.granularity;
+    const int tid = threadIdx.x, nthr = blockDim.x;
+
+    for (;;) {
+        if (tid == 0) sh->solve = atomicAdd(counter, 1ull);
+        __syncthreads();
+        const unsigned long long k = sh->solve;
+        if ((long long)k >= a.S) break;
+        const double *x0 = a.X0 + (long long)k * n;
+        for (int i = tid; i < n; i += nthr) {
+            x[i] = x0[i];
+            am[i] = a.a0[(long long)k * n + i];
+            bm[i] = bz[i] = a.b0[(long long)k * n + i];
+        }
+        __syncthreads();
+        if (warp == 0) {
+            const double f0 = mads_eval<MULTI, PLANES_SMEM>(g, o, x, sd, pre, fb, planes, a.force_exact, a.ordered);
+            if (lane == 0) {
+                sh->fx = f0;
+                sh->feasible_found = isfinite(f0) ? 1 : 0;
+            }
+        }
+        long long iterations = 0, evaluations = 1, successes = 0; // kept by thread 0
+        int converged = 0;
+        const unsigned long long key = a.seed + k;
+        for (long long it = 0; it < a.n_iter; ++it) {
+            ++iterations;
+            for (int i = tid; i < n; i += nthr) {
+                const double Delta = max_host(__dmul_rn(am[i], pow10_of(a, bm[i])), gran);
+                const int e = bm[i] - abs(bm[i] - bz[i]);
+                delta[i] = max_host(pow10_of(a, e), gran);
+                rho[i] = max_host(rint(__ddiv_rn(Delta, delta[i])), 1.0);
+            }
+            if (warp == 0) {
+                for (int i = lane; i < n; i += 32) v[i] = irwin_hall((uint32_t)key, (uint32_t)(key >> 32), it, i);
+                __syncwarp();
+                if (lane == 0) {
+                    double s = 0.0;
+                    for (int i = 0; i < n; ++i) s = __dadd_rn(s, __dmul_rn(v[i], v[i]));
+                    sh->nrm = __dsqrt_rn(s);
+                }
+                __syncwarp();
+                const double nrm = sh->nrm;
+                for (int i = lane; i < n; i += 32) v[i] = __ddiv_rn(v[i], nrm);
+            }
+            __syncthreads();
+            for (int kk = warp; kk < 2 * n; kk += W) {
+                const bool keep = poll_point(kk, n, x, v, rho, delta, gran, stage);
+                __syncwarp();
+                double fk = __longlong_as_double(0x7ff8000000000000ll); // dropped
+                if (keep) fk = mads_eval<MULTI, PLANES_SMEM>(g, o, stage, sd, pre, fb, planes, a.force_exact, a.ordered);
+                if (lane == 0) f[kk] = fk;
+                __syncwarp();
+            }
+            __syncthreads();
+            if (tid == 0) {
+                double best = __longlong_as_double(0x7ff0000000000000ll);
+                int kb = -1;
+                for (int kk = 0; kk < 2 * n; ++kk) {
+                    const double fk = f[kk];
+                    if (fk != fk) continue;
+                    ++evaluations;
+                    if (fk < best) {
+                        best = fk;
+                        kb = kk;
+                    }
+                }
+                const bool success = kb >= 0 && (best < sh->fx || (!sh->feasible_found && isfinite(best)));
+                sh->kb = success ? kb : -1;
+                if (success) {
+                    sh->fx = best;
+                    sh->feasible_found = 1;
+                    ++successes;
+                }
+            }
+            __syncthreads();
+            const int kb = sh->kb;
+            if (kb >= 0) {
+                if (warp == 0) poll_point(kb, n, x, v, rho, delta, gran, x); // the winner, re-built in place
+                for (int i = tid; i < n; i += nthr) { // enlarge
+                    if (am[i] == 1.0) am[i] = 2.0;
+                    else if (am[i] == 2.0) am[i] = 5.0;
+                    else {
+                        am[i] = 1.0;
+                        ++bm[i];
+                    }
+                }
+                __syncthreads(); // x, rho and delta are read by the rebuild and rewritten by the next iteration
+            } else { // refine; stop when every poll size sits at its granularity
+                bool moved = false;
+                for (int i = tid; i < n; i += nthr) {
+                    if (gran > 0 && __dmul_rn(am[i], pow10_of(a, bm[i])) <= gran) continue;
+                    if (am[i] == 1.0) {
+                        am[i] = 5.0;
+                        --bm[i];
+                    } else if (am[i] == 2.0) am[i] = 1.0;
+                    else am[i] = 2.0;
+                    moved = true;
+                }
+                if (!__syncthreads_or(moved)) {
+                    converged = 1;
+                    break;
+                }
+            }
+        }
+        __syncthreads();
+        const bool found = sh->feasible_found != 0;
+        for (int i = tid; i < n; i += nthr) a.X_out[(long long)k * n + i] = found ? x[i] : x0[i];
+        if (tid == 0) {
+            a.obj_out[k] = sh->fx;
+            long long *st = a.stats + 4 * (long long)k;
+            st[0] = iterations;
+            st[1] = evaluations;
+            st[2] = successes;
+            st[3] = converged;
+        }
+        __syncthreads(); // the state and the dispenser slot are rewritten by the next solve
+    }
+}
+
+bool mads_plan(const GridDesc &g, int N, const LaunchCfg &cfg, int *warps, int *smem, int *planes_smem)
+{
+    if (N < 1 || N > kMadsMaxUavs) return false;
+    const int planes_bytes = g.n_planes * g.plane_words * 4;
+    const int fixed = mads_state_bytes(3 * N) + 16, per_warp = mads_warp_bytes(g, N);
+    int w = kMadsThreads / 32;
+    while (w > 1 && fixed + w * per_warp > cfg.max_smem_optin) w /= 2;
+    if (fixed + w * per_warp > cfg.max_smem_optin) return false;
+    const bool ps = planes_bytes + fixed + w * per_warp <= cfg.max_smem_optin;
+    *warps = w;
+    *smem = (ps ? planes_bytes : 0) + fixed + w * per_warp;
+    *planes_smem = ps;
+    return true;
+}
+
+template <bool M, bool P>
+static cudaError_t launch_mads_variant(const GridDesc &g, const ObjParams &o, const LaunchCfg &cfg, const MadsArgs &a,
+                                       unsigned long long *counter, cudaStream_t stream, int warps, int smem)
+{
+    auto kern = mads_kernel<M, P, kMadsThreads, kMadsCtas>;
+    cudaError_t err = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+    if (err != cudaSuccess) return err;
+    int per_sm = 0;
+    err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, warps * 32, smem);
+    if (err != cudaSuccess) return err;
+    const int grid = (int)std::min<long long>(a.S, (long long)cfg.num_sms * std::max(per_sm, 1));
+    kern<<<grid, warps * 32, smem, stream>>>(g, o, a, counter);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_mads(const GridDesc &g, const ObjParams &o, const LaunchCfg &cfg, const MadsArgs &a,
+                        unsigned long long *counter, cudaStream_t stream)
+{
+    if (a.S <= 0) return cudaSuccess;
+    int warps = 0, smem = 0, ps = 0;
+    if (!mads_plan(g, o.N, cfg, &warps, &smem, &ps)) return cudaErrorInvalidConfiguration;
+    const bool multi = !(g.n_planes == 1 && g.n_classes == 1 && g.plane_mult[0] == 1);
+    if (multi) return ps ? launch_mads_variant<true, true>(g, o, cfg, a, counter, stream, warps, smem)
+                         : launch_mads_variant<true, false>(g, o, cfg, a, counter, stream, warps, smem);
+    return ps ? launch_mads_variant<false, true>(g, o, cfg, a, counter, stream, warps, smem)
+              : launch_mads_variant<false, false>(g, o, cfg, a, counter, stream, warps, smem);
+}
+
+} // namespace cov

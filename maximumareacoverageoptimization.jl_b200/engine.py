@@ -318,6 +318,24 @@ class CoverageEngine:
                                        _ptr(out), C.byref(obj), st))
         return out, obj.value, {"iterations": st[0], "evaluations": st[1], "batches": st[2], "successes": st[3]}
 
+    def mads_solve_batch(self, X0, n_iter: int = 100, granularity: float = 1.0, seed: int = 0):
+        """S independent MADS solves in one launch on the device (cov_mads_solve_batch): solve k starts at X0[k] and
+        draws its directions from the Philox key seed + k.  Returns (X S x 3N, objectives S, stats) with stats a dict
+        of per-solve int64 arrays: iterations, evaluations, successes, converged."""
+        X0 = _f64(X0)
+        if X0.ndim == 1:
+            X0 = X0.reshape(1, -1)
+        if self.N is None or X0.ndim != 2 or X0.shape[1] != 3 * self.N:
+            raise ValueError("X0 must be (S, 3N) with the N given to set_params")
+        S = X0.shape[0]
+        X = np.empty_like(X0)
+        obj = np.empty(S, dtype=np.float64)
+        st = np.empty((S, 4), dtype=np.int64)
+        self._check(lib.cov_mads_solve_batch(self._h, _ptr(X0), S, int(n_iter), float(granularity),
+                                             int(seed) & (2**64 - 1), _ptr(X), _ptr(obj), _ptr(st)))
+        names = ("iterations", "evaluations", "successes", "converged")
+        return X, obj, {name: st[:, q].copy() for q, name in enumerate(names)}
+
     def argmin(self, X, barrier: bool = True):
         X = _f64(X)
         if X.ndim == 1:

@@ -269,6 +269,23 @@ function mads_solve(h::Handle, x0::Vector{Float64}; N_iter = 100, granularity = 
 end
 
 """
+    mads_solve_batch(h, X0; N_iter = 100, granularity = 1.0, seed = 0)
+
+S independent MADS solves in one launch on the device (`cov_mads_solve_batch`), one start per column of `X0`
+(3N x S); solve k (1-based) draws its directions from the Philox key `seed + k - 1`. Returns
+`(X_out, objectives, stats, runtime_seconds)`: `X_out` 3N x S, `stats` 4 x S with rows iterations, evaluations,
+successes, converged.
+"""
+function mads_solve_batch(h::Handle, X0::Matrix{Float64}; N_iter = 100, granularity = 1.0, seed = 0)
+    S = size(X0, 2)
+    out = similar(X0); obj = zeros(Float64, S); stats = zeros(Int64, 4, S)
+    t = @elapsed GC.@preserve X0 out obj stats check(h, ccall((:cov_mads_solve_batch, LIB), Cint,
+        (Ptr{Cvoid}, Ptr{Float64}, Int64, Int64, Float64, UInt64, Ptr{Float64}, Ptr{Float64}, Ptr{Int64}),
+        h.ptr, X0, S, N_iter, granularity, seed, out, obj, stats))
+    return out, obj, stats, t
+end
+
+"""
     createObjective(cells, N, r_max; handle = Handle())
 
 Same signature and value as the reference's `TDM_STATIC_opt.createObjective` (src/TDM_STATIC_opt.jl:82):

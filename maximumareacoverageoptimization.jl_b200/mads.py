@@ -239,7 +239,8 @@ def optimize(input, obj, cons_ext, cons_prog, N_iter, granularity=1.0, seed=None
     return result, runtime
 
 
-def optimize_multistart(inputs, obj, cons_ext, cons_prog, N_iter, granularity=1.0, seed=None, return_stats=False):
+def optimize_multistart(inputs, obj, cons_ext, cons_prog, N_iter, granularity=1.0, seed=None, return_stats=False,
+                        native=False):
     """S independent MADS solves from the rows of `inputs` (S x n), with the settings of `optimize`, advanced in
     LOCKSTEP: at every iteration the poll sets of all the solves still running are concatenated and evaluated in ONE
     `obj.batch` call (S x 2n trial points per launch instead of 2n -- SURVEY.md 8f-1's multi-start swarms: a 30-point
@@ -248,13 +249,31 @@ def optimize_multistart(inputs, obj, cons_ext, cons_prog, N_iter, granularity=1.
     native=False)`; lockstep changes how the work is batched, not what is computed.
     Returns (results S x n, objectives S, runtime) -- results[k] is solve k's feasible incumbent, else its start;
     objectives[k] is +inf where solve k never found a feasible point.  With return_stats=True also a dict of counters
-    (iterations = lockstep iterations, batches = obj.batch calls, per_solve_iterations, best = argmin of objectives)."""
+    (iterations = lockstep iterations, batches = obj.batch calls, per_solve_iterations, best = argmin of objectives).
+
+    native=True runs all S solves on the device in ONE launch (cov_mads_solve_batch: the same algorithm and settings,
+    solve k seeded seed + k, directions from the library's own Philox stream instead of NumPy's, so the iterates differ
+    from native=False); stats["batches"] is 1.  It needs an objective made by createObjective, constraints that all
+    fuse and a scalar granularity, and raises ValueError otherwise."""
     t_start = time.perf_counter()
     X0 = np.ascontiguousarray(inputs, dtype=np.float64)
     if X0.ndim != 2 or not len(X0):
         raise ValueError("inputs must be S x n with S >= 1")
     S, n = X0.shape
     flat = _flatten_constraints(cons_ext)
+    if native:
+        solver = obj.native_batch_solver(flat) if hasattr(obj, "native_batch_solver") else None
+        if solver is None or not np.isscalar(granularity):
+            raise ValueError("native multistart needs an objective from createObjective, constraints that all fuse and "
+                             "a scalar granularity")
+        results, objectives, st = solver(X0, int(N_iter), float(granularity), 0 if seed is None else int(seed))
+        runtime = time.perf_counter() - t_start
+        if return_stats:
+            stats = {"iterations": int(st["iterations"].max()), "evaluations": int(st["evaluations"].sum()),
+                     "batches": 1, "cache_hits": 0, "successes": int(st["successes"].sum()),
+                     "per_solve_iterations": st["iterations"].tolist(), "best": int(np.argmin(objectives))}
+            return results, objectives, runtime, stats
+        return results, objectives, runtime
     host_cons = obj.fuse(flat) if hasattr(obj, "fuse") else flat
     stats = {"iterations": 0, "evaluations": 0, "batches": 0, "cache_hits": 0, "successes": 0}
     evaluate = _barrier_evaluator(obj, host_cons, stats, {})
