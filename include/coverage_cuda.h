@@ -312,7 +312,7 @@ typedef struct cov_launch_info {
     int32_t chunk;          /* small-swarm kernel: candidates per work unit; CTA kernel: co-resident CTAs per SM the
                                instantiation is compiled for (3 or 4); else 0 */
     int32_t max_warps;      /* small-swarm kernel: warps per CTA the instantiation allows (20 or 24); else 0 */
-    int32_t plane_mode;     /* CTA kernel: COV_OPT_PLANE_MODE it resolved to (0, 1, 2); else -1 */
+    int32_t plane_mode;     /* CTA kernel: COV_OPT_PLANE_MODE it resolved to (0 to 4); else -1 */
 } cov_launch_info;
 COV_API int cov_last_launch(const cov_handle *h, cov_launch_info *out);
 /* Running totals over every coverage-kernel launch of this handle: summed device time (CUDA

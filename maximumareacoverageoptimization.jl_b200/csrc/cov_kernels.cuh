@@ -14,7 +14,8 @@ struct LaunchCfg {
     int force_exact;
     int num_sms;
     int max_smem_optin;  // bytes
-    int plane_mode;      // CTA kernel: -1 auto, 0 lazy global, 1 early global, 2 staged per band (TMA), 3 sweep
+    int plane_mode;      // CTA kernel: -1 auto, 0 lazy global, 1 early global, 2 staged per band (TMA), 3 sweep with
+                         // a staged plane band, 4 sweep with the plane read through L2
     int ordered;         // 1: the store's area depends on the order of the Float64 additions -> ordered kernel
 };
 
@@ -25,7 +26,7 @@ struct LaunchInfo {
     int multi;      // 1: several planes / classes / multiplicities
     int chunk;      // small-swarm kernel: candidates per unit (CHUNK); else 0
     int max_warps;  // small-swarm kernel: MAXW of the instantiation (20 or 24); else 0
-    int plane_mode; // CTA kernel: 0 lazy, 1 early, 2 staged (PLANES); else -1
+    int plane_mode; // CTA kernel: 0 lazy, 1 early, 2 staged, 3 sweep, 4 sweep through L2 (PLANES); else -1
 };
 
 // Coverage objective over B candidates (device pointers). counter: one ZEROED unsigned long long

@@ -424,7 +424,10 @@ bool span_small_applies(const GridDesc &g, int N, const LaunchCfg &cfg, long lon
     for (int chunk : {32, 16}) {
         const int per = small_warp_bytes(g, N, chunk);
         int w = (cfg.max_smem_optin - planes_bytes - small_param_bytes(N) - 16) / per;
-        w = std::min(w, 24); // the 24-warp instantiation (launch_small_variant picks 20 or 24 by this count)
+        // the 24-warp instantiation (launch_small_variant picks 20 or 24 by this count) -- except 32-candidate
+        // units of 6 to 8 UAVs: >= 11 392 bytes per warp, so 21 warps would take more than the 227 KB a CTA can
+        // have on sm_100, and that instantiation is not built
+        w = std::min(w, (chunk == 32 && N > 5) ? 20 : 24);
         if (cfg.warps_per_cta > 0) w = std::min(w, cfg.warps_per_cta);
         // prefer the 32-candidate chunk unless the 16-candidate one buys >= 25 % more warps
         if (w >= 4 && (best_w == 0 || w * 4 >= best_w * 5)) {
@@ -502,8 +505,8 @@ cudaError_t launch_span_small(const GridDesc &g, const ObjParams &o, const Launc
         if (o.N <= 5)                                                                                            \
             return warps > 20 ? launch_small_variant<M, C, 24, true>(COV_SMALL_ARGS)                             \
                               : launch_small_variant<M, C, 20, true>(COV_SMALL_ARGS);                            \
-        return warps > 20 ? launch_small_variant<M, C, 24, false>(COV_SMALL_ARGS)                                \
-                          : launch_small_variant<M, C, 20, false>(COV_SMALL_ARGS)
+        return warps > 20 && C != 32 ? launch_small_variant<M, C, C == 32 ? 20 : 24, false>(COV_SMALL_ARGS)      \
+                                     : launch_small_variant<M, C, 20, false>(COV_SMALL_ARGS)
     if (multi) {
         switch (chunk) {
             COV_SMALL_CASE(true, 32);

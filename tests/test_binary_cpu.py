@@ -44,7 +44,7 @@ def test_only_sm100a_code():
 def test_objective_kernels_fit_their_launch_plans(usage):
     small = {k: v for k, v in usage.items() if "span_small_kernel" in k}
     cta = {k: v for k, v in usage.items() if "span_cta_kernel" in k}
-    assert len(small) == 32 and len(cta) >= 8
+    assert len(small) == 30 and len(cta) >= 8  # 2 x 4 x 2 x 2, less <*, 32, 24, false> (tests/test_launch_matrix.py)
     for k, v in {**small, **cta, **{k: v for k, v in usage.items() if re.search(r"brute_kernel|exact_kernel|ordered_kernel", k)}}.items():
         assert v["LOCAL"] == 0, (k, v)          # no local-memory arrays (the stack frame is the FP64 slow path's call)
         assert v["STACK"] <= 128, (k, v)
