@@ -106,7 +106,15 @@ COV_API int cov_get_option(const cov_handle *h, int option, int64_t *value);
 
 /* ---- the cell store (replaces CellFunctions.Cells.points_of_interest as the kernel's input;
  *      src/CellFunctions.jl:5-16, producers src/AreaCoverageCalculation.jl:11-21,
- *      src/CellFunctions.jl:20-79) ----------------------------------------------------------- */
+ *      src/CellFunctions.jl:20-79) -----------------------------------------------------------
+ * The store also stands for a point LIST, whose order decides the Float64 area when the weights are not
+ * dyadic (cov_grid_info.area_exact == 0, COV_KERNEL_ORDERED):
+ *  - cov_set_points: the order given;
+ *  - cov_set_grid_bits, cov_set_grid_cells, cov_set_grid_full, cov_fire_init and cov_fire_step: createPOI's order
+ *    (i outer, j inner, src/AreaCoverageCalculation.jl:14-15), the entries of a cell next to each other (these
+ *    stores hold one weight class, or several given per cell by cov_set_grid_cells);
+ *  - cov_add_points: the new entries after all the others, in the order given (push!, src/CellFunctions.jl:74);
+ *  - cov_remove_covered: the remaining entries keep their order (src/CellFunctions.jl:81-108). */
 
 /* 1 bit per cell, every set cell is one list entry of weight `weight`.
  * bits: ny rows of ceil(nx/32) uint32 words; bit b of word w of row j-1 is cell i = 32*w + b + 1. */
@@ -133,8 +141,9 @@ COV_API int cov_set_grid_full(cov_handle *h, int64_t nx, int64_t ny, double dx, 
 
 /* Append list entries (update_POI, src/CellFunctions.jl:59-79): same rules as cov_set_points,
  * multiplicities add up. Limits of the store (also of cov_set_points): at most 4 distinct weights (weight classes),
- * one weight per cell, at most 255 entries per cell (COV_ERR_LIMIT / COV_ERR_INVALID otherwise). A failing append
- * leaves the store exactly as it was. */
+ * one weight per cell, at most 255 entries per cell, at most 8 bit planes (the set bits of the multiplicities of
+ * each class, summed over the classes) (COV_ERR_LIMIT / COV_ERR_INVALID otherwise). A failing append leaves the
+ * store exactly as it was. */
 COV_API int cov_add_points(cov_handle *h, const double *pts5, int64_t P);
 
 typedef struct cov_grid_info {
@@ -168,7 +177,9 @@ COV_API int cov_remove_covered(cov_handle *h, const double *xyR, int64_t N, int6
  * neighbour, `wind_speed*cos(wind_direction - atan(2-b, 2-a))*prob_spread > u`, u from
  * Philox4x32-10 keyed by seed with counter (cell, step, neighbour); every success pushes one list
  * entry (append != 0: straight into the device-resident store; multiplicities add up like the
- * duplicates of FirePoints.xlsx). n_pushed (nullable) = entries pushed by this step. */
+ * duplicates of FirePoints.xlsx). n_pushed (nullable) = entries pushed by this step. The pushed entries weigh
+ * dx*dy, so the store must hold a single weight class of weight dx*dy (else COV_ERR_STATE, nothing changes); with one
+ * class the order of the entries does not change the area. */
 COV_API int cov_fire_init(cov_handle *h, int64_t nx, int64_t ny, double dx, double dy, const uint8_t *state,
                           int32_t push_initial);
 COV_API int cov_fire_step(cov_handle *h, double wind_speed, double wind_direction, double prob_spread,

@@ -149,6 +149,7 @@ struct cov_handle {
     // ent_known: the host mirror follows the order cov_set_points / cov_add_points gave (removals pending in
     // ent_removed_pending are applied lazily: every entry of a covered cell goes, the others keep their order);
     // otherwise the order is createPOI's (i outer, j inner, duplicates together), built from the cell store on demand.
+    // The first cov_add_points on such a store builds the mirror in that order and appends to it.
     std::vector<int> ent_cell_h;
     std::vector<unsigned char> ent_cls_h;
     bool ent_known = false, ent_removed_pending = false, ent_dev_valid = false;
@@ -708,30 +709,34 @@ static int entries_apply_removals(cov_handle *h)
     h->ent_dev_valid = false;
     return COV_OK;
 }
+// The host list of a store that no list was ever given for (bit grid, cell bytes, createPOI, automaton), built from
+// the cell store as it is now: createPOI's order, i outer and j inner (src/AreaCoverageCalculation.jl:14-15), the
+// entries of a cell together.
+static int entries_from_cells(cov_handle *h)
+{
+    const size_t ncell = (size_t)h->g.nx * h->g.ny;
+    std::vector<unsigned char> m(ncell), k(ncell);
+    CK(cudaMemcpyAsync(m.data(), h->mult.p, ncell, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaMemcpyAsync(k.data(), h->cls.p, ncell, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    h->ent_cell_h.clear();
+    h->ent_cls_h.clear();
+    for (int i = 0; i < h->g.nx; ++i)
+        for (int j = 0; j < h->g.ny; ++j) {
+            const size_t cell = (size_t)i + (size_t)h->g.nx * j;
+            for (unsigned r = 0; r < m[cell]; ++r) {
+                h->ent_cell_h.push_back((int)cell);
+                h->ent_cls_h.push_back((unsigned char)(k[cell] & (kMaxClasses - 1)));
+            }
+        }
+    return COV_OK;
+}
 // Make g.ent_cell / g.ent_cls / g.n_ent describe the current list on the device.
 static int entries_on_device(cov_handle *h)
 {
     if (h->ent_dev_valid) return COV_OK;
     OK(entries_apply_removals(h));
-    if (!h->ent_known) {
-        // no list was ever given (bit grid, cell bytes, createPOI, automaton): createPOI's order,
-        // i outer and j inner (src/AreaCoverageCalculation.jl:14-15), the entries of a cell together
-        const size_t ncell = (size_t)h->g.nx * h->g.ny;
-        std::vector<unsigned char> m(ncell), k(ncell);
-        CK(cudaMemcpyAsync(m.data(), h->mult.p, ncell, cudaMemcpyDeviceToHost, h->stream));
-        CK(cudaMemcpyAsync(k.data(), h->cls.p, ncell, cudaMemcpyDeviceToHost, h->stream));
-        CK(cudaStreamSynchronize(h->stream));
-        h->ent_cell_h.clear();
-        h->ent_cls_h.clear();
-        for (int i = 0; i < h->g.nx; ++i)
-            for (int j = 0; j < h->g.ny; ++j) {
-                const size_t cell = (size_t)i + (size_t)h->g.nx * j;
-                for (unsigned r = 0; r < m[cell]; ++r) {
-                    h->ent_cell_h.push_back((int)cell);
-                    h->ent_cls_h.push_back((unsigned char)(k[cell] & (kMaxClasses - 1)));
-                }
-            }
-    }
+    if (!h->ent_known) OK(entries_from_cells(h));
     const size_t P = h->ent_cell_h.size();
     if ((int64_t)P != h->n_entries)
         return fail(h, COV_ERR_STATE, "internal: the ordered point list disagrees with the cell store (" +
@@ -969,6 +974,12 @@ extern "C" int cov_add_points(cov_handle *h, const double *pts5, int64_t P)
         cw[0] = h->g.class_weight[0];
     }
     OK(entries_apply_removals(h)); // before new entries can land on cells that a removal emptied
+    if (!h->ent_known) {
+        // push! appends after every entry already in the list, whatever setter built it: fix the order of the
+        // store as it is (createPOI's) before the new entries land on its cells, and keep the list from here on
+        OK(entries_from_cells(h));
+        h->ent_known = true;
+    }
     OK(snapshot_cells(h));
     const int rc = upload_points(h, cell, pcls);
     if (rc != COV_OK) { // nothing was appended: the store, its planes and its counts stay as they were
@@ -977,12 +988,25 @@ extern "C" int cov_add_points(cov_handle *h, const double *pts5, int64_t P)
         h->err = msg;
         return rc;
     }
-    if (h->ent_known) { // push! appends at the end (src/CellFunctions.jl:74)
-        h->ent_cell_h.insert(h->ent_cell_h.end(), cell.begin(), cell.end());
-        h->ent_cls_h.insert(h->ent_cls_h.end(), pcls.begin(), pcls.end());
-    }
+    // push! appends at the end (src/CellFunctions.jl:74)
+    const size_t old_len = h->ent_cell_h.size();
+    const int old_classes = h->g.n_classes;
+    double old_cw[kMaxClasses];
+    for (int k = 0; k < kMaxClasses; ++k) old_cw[k] = h->g.class_weight[k];
+    h->ent_cell_h.insert(h->ent_cell_h.end(), cell.begin(), cell.end());
+    h->ent_cls_h.insert(h->ent_cls_h.end(), pcls.begin(), pcls.end());
     h->ent_dev_valid = false;
-    return rebuild_planes(h, n_classes, cw);
+    const int rc_planes = rebuild_planes(h, n_classes, cw);
+    if (rc_planes != COV_OK) { // more bit planes than the kernels sweep: put the store back as it was
+        const std::string msg = h->err;
+        restore_cells(h);
+        h->ent_cell_h.resize(old_len);
+        h->ent_cls_h.resize(old_len);
+        if (h->have_grid && rebuild_planes(h, old_classes, old_cw) != COV_OK) h->have_grid = false;
+        h->err = msg;
+        return rc_planes;
+    }
+    return COV_OK;
 }
 
 extern "C" int cov_get_grid_info(const cov_handle *h, cov_grid_info *info)
@@ -1117,6 +1141,9 @@ extern "C" int cov_fire_step(cov_handle *h, double wind_speed, double wind_direc
     if (step < 0 || step > 0xffffffffll) return fail(h, COV_ERR_INVALID, "cov_fire_step: step out of range");
     if (h->g.n_classes != 1)
         return fail(h, COV_ERR_STATE, "cov_fire_step: the cell store holds several weight classes");
+    if (h->g.class_weight[0] != h->g.dx * h->g.dy) // DynamicArea.jl:65: every pushed entry weighs dx*dy
+        return fail(h, COV_ERR_STATE, "cov_fire_step: the cell store's weight class is not dx*dy, the weight the "
+                                      "automaton pushes");
     // the probability of ignition from the neighbour at window index (a, b), a, b = 1..3, exactly as the
     // reference forms it: wind_speed * cos(wind_direction - atan(2-b, 2-a)) * prob_spread
     double *hp = (double *)h->h_small + 64;
@@ -1150,7 +1177,9 @@ extern "C" int cov_fire_step(cov_handle *h, double wind_speed, double wind_direc
     h->fire_cur = cur ^ 1;
     if (n_pushed) *n_pushed = (int64_t)*hr;
     if (!append || *hr == 0) return COV_OK;
-    entries_forget(h); // the automaton pushes in cell order; from here on the list order is createPOI's
+    // The automaton pushes in cell order; from here on the list order is createPOI's.  The store has one weight
+    // class, so every covered entry adds the same weight and the list-order sum is the same in any order.
+    entries_forget(h);
     double cw[kMaxClasses];
     for (int k = 0; k < kMaxClasses; ++k) cw[k] = h->g.class_weight[k];
     return rebuild_planes(h, 1, cw);
