@@ -220,8 +220,11 @@ COV_API int cov_eval_batch_device(cov_handle *h, const double *dX, int64_t B, do
 /* The scalar closure: AreaMaxObjective(x) for one candidate (src/TDM_STATIC_opt.jl:83-98). */
 COV_API int cov_eval_one(cov_handle *h, const double *x, double *obj);
 
-/* Poll winner: smallest objective and its 0-based index. barrier != 0: infeasible candidates
- * count as +Inf (extreme barrier); if none is feasible best_idx = -1, best_obj = +Inf. */
+/* Poll winner: smallest objective and its 0-based index; among equal objectives the smallest index wins (MADS's
+ * first strict minimum), however the candidates are split over threads, slices and devices. barrier != 0:
+ * infeasible candidates are skipped (extreme barrier); if none is feasible best_idx = -1, best_obj = +Inf. A
+ * feasible candidate whose objective is +Inf still counts: best_obj = +Inf with best_idx >= 0. The same rule holds
+ * for cov_eval_batch_best, cov_eval_batch_packed and cov_multi_argmin. */
 COV_API int cov_argmin(cov_handle *h, const double *X, int64_t B, int32_t barrier, double *best_obj,
                int64_t *best_idx);
 

@@ -627,8 +627,8 @@ __global__ void union_area_kernel(const double *__restrict__ X, long long B, int
 // circles j.  The covered angular intervals of circle i go to the warp's list in shared memory (warp-
 // aggregated appends); instead of sorting them, every interval END that no other interval covers opens an
 // exposed arc, which runs to the nearest interval START at or after it (plus the arc that starts at angle 0
-// when 0 is uncovered).  Among intervals with the same end the lowest list position speaks for all.  Same
-// formulas and tie rules as union_area_kernel; sums in a fixed order (deterministic).
+// when 0 is uncovered).  Among intervals with the same end the lowest list position speaks for all, and angle 0
+// speaks for every end at 0.  Same formulas and tie rules as union_area_kernel; sums in a fixed order (deterministic).
 constexpr int kUnionBigWarps = 4;
 __global__ void __launch_bounds__(kUnionBigWarps * 32)
 union_area_big_kernel(const double *__restrict__ X, long long B, int N, double *__restrict__ area)
@@ -698,7 +698,8 @@ union_area_big_kernel(const double *__restrict__ X, long long B, int N, double *
             double acc = 0.0;
             for (int p = lane - 1; p < n; p += 32) {
                 const double pos = p < 0 ? 0.0 : ib[p];
-                bool covered = !(pos < two_pi);
+                // an end at angle 0 (a zero-length interval there, when alpha rounds to 0) is angle 0's own candidate
+                bool covered = !(pos < two_pi) || (p >= 0 && pos == 0.0);
                 double nxt = two_pi;
                 for (int q = 0; q < n && !covered; ++q) {
                     const double aq = ia[q], bq = ib[q];
