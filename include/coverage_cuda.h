@@ -36,7 +36,8 @@ extern "C" {
 
 #define COV_ABI_VERSION 3 /* 2: COV_OPT_PROGRESSIVE_INDEX, COV_KERNEL_ORDERED, cov_get_class_weights, cov_eval_batch_best;
                              3: cov_eval_batch_packed (COV_PACK_*); later, with no existing symbol changed:
-                                cov_mads_solve_batch */
+                                cov_mads_solve_batch; cov_set_region, cov_eval_region_batch,
+                                cov_mads_solve_batch_region (the grid-free static objective) */
 
 #if defined(__GNUC__)
 #define COV_API __attribute__((visibility("default")))
@@ -293,6 +294,40 @@ COV_API int cov_covered_mask(cov_handle *h, const double *x, uint8_t *mask);
  *      an independent restatement to 1e-9 relative, far inside north_star's 1e-5). No grid is involved.
  *      N <= 1024 (one warp per candidate up to 64 discs, one CTA per candidate above). Host buffers, synchronous. */
 COV_API int cov_union_area_batch(cov_handle *h, const double *X, int64_t B, int64_t N, double *area);
+
+/* ---- grid-free static objective (SURVEY.md 8f-4, the continuous limit of the static environment): the exact area
+ *      A(x) = |(D_1 u ... u D_N) n Omega \ C| newly covered inside the domain, where Omega is the rectangle
+ *      [x_lo, x_hi] x [y_lo, y_hi] (createPOI's [0, nx dx] x [0, ny dy]) and C the union of the discs already covered
+ *      (what rmvCoveredPOI removed timestep after timestep).  As dx = dy -> 0 the grid objective's area term of the
+ *      static environment converges to A(x).  Computed in FP64 by boundary integration (Green's theorem, DESIGN.md 11);
+ *      no cell store is involved and the cell store is not touched: these calls need cov_set_region and
+ *      cov_set_params only, and every other entry point behaves as before.
+ *      Limits: N <= 64 discs per candidate, M <= 512 covered discs, and at most 2048 arcs of C's boundary inside
+ *      Omega (COV_ERR_LIMIT beyond them; 40 timesteps x 5 UAVs are 200 discs). ------------------------------------- */
+
+/* The domain rectangle and the discs already covered (the continuous rmvCoveredPOI).
+ * covered_xyR: M discs as [x_1..x_M, y_1..y_M, R_1..R_M] (NULL when M == 0); discs of radius <= 0 cover nothing.
+ * Replaces any earlier region; a failing call leaves the earlier region in place.  The arcs of C's boundary inside
+ * Omega are computed here, once, on the device.  COV_ERR_INVALID: non-finite values, x_hi <= x_lo, y_hi <= y_lo or
+ * M < 0. */
+COV_API int cov_set_region(cov_handle *h, double x_lo, double y_lo, double x_hi, double y_hi,
+                           const double *covered_xyR, int64_t M);
+
+/* obj[b] = -A(x_b) + penalty_scale * sum_i |R_i - r_max_i| (same FP64 assembly order as the grid objective);
+ * area[b] = A(x_b); feasible[b] as cov_eval_batch (the constraints of cov_set_params, fused). All nullable;
+ * best_obj / best_idx both NULL or both given: the poll winner with cov_argmin's rule (smallest index among ties,
+ * barrier != 0 skips infeasible candidates). Host buffers, synchronous. N <= 64.  A candidate's results have the same
+ * bits whatever the batch it is part of.  COV_ERR_STATE without a region or parameters.  cov_last_kernel_ms gives
+ * the device time of this call's evaluation kernel(s). */
+COV_API int cov_eval_region_batch(cov_handle *h, const double *X, int64_t B, double *obj, double *area,
+                                  uint8_t *feasible, int32_t barrier, double *best_obj, int64_t *best_idx);
+
+/* cov_mads_solve_batch (same arguments, loop, direction stream, drop rules, stats and results) with the region
+ * objective of cov_eval_region_batch as the function minimised, so every iterate can be replayed through
+ * cov_eval_region_batch. No cell store needed. N <= 64. */
+COV_API int cov_mads_solve_batch_region(cov_handle *h, const double *X0, int64_t S, int64_t n_iter,
+                                        double granularity, uint64_t seed, double *X_out, double *obj_out,
+                                        int64_t *stats);
 
 /* ---- streams, memory, timing (so hosts without a CUDA binding can keep data resident) ------ */
 COV_API int cov_sync(cov_handle *h);

@@ -6,6 +6,10 @@ points the UAVs already cover (`rmvCoveredPOI`), the r_max adjustment near the h
 rectangle, `create_cons3` from the previous positions, `createObjective`, `optimize`.  The
 trajectory side-stack (ALTRO / ORCA, :115-251) is out of scope: the UAVs are taken to reach the
 MADS targets, so the next step's `pre_optimized_circles_MADS` is the MADS output.
+
+objective="region" (static environment only) optimises the grid-free static objective instead
+(TDM_STATIC_opt.createRegionObjective): the domain is the cell lattice's rectangle, and where rmvCoveredPOI would
+remove the cells the previous swarm covers, its discs are appended to the covered set.
 """
 from __future__ import annotations
 
@@ -43,9 +47,15 @@ class SimulationParameters:
 
 
 def run_simulation(cells, starting_circles, cons_ext, cons_prog, N, r_max, params: SimulationParameters,
-                   Nt_sim: int | None = None):
-    """Returns (single_input_pb, single_output_pb, runtime_data_MADS, objective_pb)."""
+                   Nt_sim: int | None = None, objective: str = "grid", covered_pb: list | None = None):
+    """Returns (single_input_pb, single_output_pb, runtime_data_MADS, objective_pb).  objective: "grid" (the
+    reference's) or "region"; with "region", covered_pb (if given) receives the covered set (M x 3 rows x, y, R) each
+    timestep's objective was built on."""
     p = params
+    if objective not in ("grid", "region"):
+        raise ValueError("objective must be 'grid' or 'region'")
+    if objective == "region" and p.environment_type != "static":
+        raise ValueError("the region objective has no dynamic form: its points are not cells")
     t_half = math.tan(p.FOV / 2)
     single_input_pb, single_output_pb, runtime_data_MADS, objective_pb = [], [], [], []
     pre = np.ascontiguousarray(starting_circles if not hasattr(starting_circles[0], "x")
@@ -53,11 +63,20 @@ def run_simulation(cells, starting_circles, cons_ext, cons_prog, N, r_max, param
     r_max = np.ascontiguousarray(r_max, dtype=np.float64)
     d_lim = p.d_lim * np.ones(N)
     steps = p.Nt_sim if Nt_sim is None else Nt_sim
+    engine, covered = None, np.zeros((0, 3))
+    if objective == "region":
+        from .engine import CoverageEngine
+        pl = cells.points_of_interest
+        region = (0.0, 0.0, pl.nx * pl.dx, pl.ny * pl.dy)
+        engine = CoverageEngine(getattr(cells, "device", 0))
     for t in range(1, steps + 1):
         if p.environment_type == "dynamic":
             cells = CellFunctions.update_POI(cells, t)
         drone_locs = pre.copy()
-        cells = CellFunctions.rmvCoveredPOI(cells, drone_locs)
+        if objective == "region":
+            covered = np.vstack([covered, drone_locs.reshape(3, N).T])
+        else:
+            cells = CellFunctions.rmvCoveredPOI(cells, drone_locs)
         if t != 1:  # :65-76
             xl, xu, yl, yu = (np.asarray(v, dtype=np.float64) for v in (p.x_LB, p.x_UB, p.y_LB, p.y_UB))
             for i in range(N):
@@ -73,7 +92,12 @@ def run_simulation(cells, starting_circles, cons_ext, cons_prog, N, r_max, param
             single_input = single_output_pb[-1]
             if not cons1(single_input) or not cons3(single_input):
                 single_input = drone_locs
-        area_objective_func = TDM_STATIC_opt.createObjective(cells, N, r_max)
+        if objective == "region":
+            area_objective_func = TDM_STATIC_opt.createRegionObjective(region, covered, N, r_max, engine=engine)
+            if covered_pb is not None:
+                covered_pb.append(covered.copy())
+        else:
+            area_objective_func = TDM_STATIC_opt.createObjective(cells, N, r_max)
         out, runtime = TDM_STATIC_opt.optimize(single_input, area_objective_func, [cons_ext, cons3], cons_prog,
                                                p.N_iter, seed=None if p.seed is None else p.seed + t)
         runtime_data_MADS.append(runtime)
@@ -81,4 +105,6 @@ def run_simulation(cells, starting_circles, cons_ext, cons_prog, N, r_max, param
         single_output_pb.append(np.array(out))
         objective_pb.append(area_objective_func(out))
         pre = np.array(out)
+    if engine is not None:
+        engine.close()
     return single_input_pb, single_output_pb, runtime_data_MADS, objective_pb

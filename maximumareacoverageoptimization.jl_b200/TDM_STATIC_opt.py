@@ -106,6 +106,62 @@ def createObjective(cells, N, r_max) -> AreaMaxObjective:
     return AreaMaxObjective(cells, N, r_max)
 
 
+class RegionObjective(AreaMaxObjective):
+    """The grid-free static objective: -A(x) + 1e5 * sum_i abs(x[i+2N] - r_max[i]) with A(x) the exact area of
+    (union of the discs of x) n region \\ (union of the covered discs) -- the limit of AreaMaxObjective's value in the
+    static environment as the cells shrink (cov_eval_region_batch).  The same closure shape as AreaMaxObjective:
+    `__call__`, `.batch`, `.fuse`, `.native_batch_solver` (cov_mads_solve_batch_region); cov_mads_solve has no region
+    form, so `native_solver` is None and mads.optimize polls from Python."""
+
+    def __init__(self, region, covered, N: int, r_max, engine=None):
+        super().__init__(None, N, r_max)
+        self.region = tuple(float(v) for v in region)  # (x_lo, y_lo, x_hi, y_hi)
+        self.covered = np.array(np.zeros((0, 3)) if covered is None else covered, dtype=np.float64).reshape(-1, 3)
+        self._eng = engine
+        self._own_engine = engine is None
+
+    def _engine(self):
+        from .engine import CoverageEngine
+        if self._eng is None:
+            self._eng = CoverageEngine(0)
+        eng = self._eng
+        r = np.ascontiguousarray(self.r_max, dtype=np.float64).ravel()
+        key = (id(self), r.tobytes(), id(self._fused))
+        if eng.param_owner != key or eng.N != self.N:
+            eng.set_params(self.N, r, 1e5, **self._fused)
+            eng.set_region(*self.region, self.covered)  # the region is the objective's: set with its parameters
+            eng.param_owner = key
+        return None, eng
+
+    def native_solver(self, constraints):
+        return None
+
+    def native_batch_solver(self, constraints):
+        if self.fuse(constraints):
+            return None
+        return self._engine()[1].mads_solve_batch_region
+
+    def batch(self, X, want_feasible=False, granularity=1.0):
+        eng = self._engine()[1]
+        X = np.ascontiguousarray(X, dtype=np.float64).reshape(-1, 3 * self.N)
+        out = eng.eval_region_batch(X, want_area=False, want_feasible=want_feasible)
+        return (out["obj"], out["feasible"].astype(bool)) if want_feasible else out["obj"]
+
+    def __call__(self, x) -> float:
+        return float(self.batch(np.ravel(x))[0])
+
+    def close(self):
+        if self._own_engine and self._eng is not None:
+            self._eng.close()
+            self._eng = None
+
+
+def createRegionObjective(region, covered, N, r_max, engine=None) -> RegionObjective:
+    """The grid-free static objective on the domain region = (x_lo, y_lo, x_hi, y_hi) with the discs `covered`
+    (M x 3 rows x, y, R) already covered; engine: a CoverageEngine to run on (default: one of its own)."""
+    return RegionObjective(region, covered, N, r_max, engine)
+
+
 def optimize(input, obj, cons_ext, cons_prog, N_iter, **kw):
     """src/TDM_STATIC_opt.jl:118-222 -- see mads.optimize."""
     from .mads import optimize as _opt

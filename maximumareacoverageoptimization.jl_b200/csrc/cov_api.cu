@@ -22,6 +22,7 @@
 #include <vector>
 #include "cov_device.cuh"
 #include "cov_kernels.cuh"
+#include "cov_region.cuh"
 #include "../../include/coverage_cuda.h"
 
 using namespace cov;
@@ -159,6 +160,11 @@ struct cov_handle {
     bool have_params = false;
     ObjParams o{};
     DevBuf params; // 5N doubles: r_max, prev_x, prev_y, prev_z, cons3_G
+
+    // the grid-free static objective (cov_set_region): domain, covered discs, the arcs of their boundary
+    bool have_region = false;
+    RegionDesc region{};
+    DevBuf region_discs, region_arcs, region_count, d_area;
 
     LaunchCfg cfg{};
     int64_t chunk = 0;
@@ -425,7 +431,8 @@ extern "C" void cov_destroy(cov_handle *h)
     DevBuf *bufs[] = {&h->mult, &h->cls, &h->planes, &h->planes_q, &h->params, &h->counter, &h->stats, &h->xyT,
                       &h->small_in, &h->argmin_obj, &h->argmin_idx, &h->removed, &h->overflow, &h->dX,
                       &h->d_obj, &h->d_count, &h->d_feas, &h->d_clscnt, &h->d_prog, &h->fire[0], &h->fire[1], &h->fire_p,
-                      &h->backup, &h->ent_cell, &h->ent_cls, &h->d_raw[0], &h->d_raw[1], &h->mads_in, &h->mads_out};
+                      &h->backup, &h->ent_cell, &h->ent_cls, &h->d_raw[0], &h->d_raw[1], &h->mads_in, &h->mads_out,
+                      &h->region_discs, &h->region_arcs, &h->region_count, &h->d_area};
     for (DevBuf *b : bufs)
         if (b->p) cudaFree(b->p);
     for (int k = 0; k < 2; ++k)
@@ -1950,26 +1957,28 @@ extern "C" int cov_mads_solve(cov_handle *h, const double *x0, int64_t n_iter, d
 }
 
 // S solves of the same loop on the device, one launch for all of them (cov_mads.cu).  The host contributes what
-// must carry its libm's bits: the initial mesh of every start and the table of powers of ten.
-extern "C" int cov_mads_solve_batch(cov_handle *h, const double *X0, int64_t S, int64_t n_iter, double granularity,
-                                    uint64_t seed, double *X_out, double *obj_out, int64_t *stats)
+// must carry its libm's bits: the initial mesh of every start and the table of powers of ten.  region: the objective
+// of cov_eval_region_batch instead of the cell store's.
+static int mads_solve_batch(cov_handle *h, bool region, const double *X0, int64_t S, int64_t n_iter, double granularity,
+                            uint64_t seed, double *X_out, double *obj_out, int64_t *stats)
 {
-    if (!h) return fail(nullptr, COV_ERR_INVALID, "NULL handle");
-    DeviceGuard dg(h->device);
-    OK(check_ready(h, "cov_mads_solve_batch"));
+    const char *who = region ? "cov_mads_solve_batch_region" : "cov_mads_solve_batch";
     if (S < 0 || n_iter < 0 || !(granularity >= 0) || (S > 0 && (!X0 || !X_out)))
-        return fail(h, COV_ERR_INVALID, "cov_mads_solve_batch: bad arguments");
+        return fail(h, COV_ERR_INVALID, std::string(who) + ": bad arguments");
     if (S == 0) return COV_OK;
     const int N = h->o.N, n = 3 * N;
     int warps = 0, smem = 0, planes_smem = 0;
     if (N > kMadsMaxUavs)
-        return fail(h, COV_ERR_LIMIT, "cov_mads_solve_batch: N = " + std::to_string(N) + " exceeds the " +
+        return fail(h, COV_ERR_LIMIT, std::string(who) + ": N = " + std::to_string(N) + " exceeds the " +
                                           std::to_string(kMadsMaxUavs) + " UAVs of the solver's launch plan");
-    if (!mads_plan(h->g, N, h->cfg, &warps, &smem, &planes_smem))
-        return fail(h, COV_ERR_LIMIT, "cov_mads_solve_batch: one warp's framebuffer of the " + std::to_string(h->g.nx) +
-                                          " x " + std::to_string(h->g.ny) + " grid does not fit the " +
-                                          std::to_string(h->cfg.max_smem_optin) + " bytes of shared memory per CTA");
-    if (!h->area_exact) OK(entries_on_device(h)); // non-dyadic weights: the list-order sum
+    if (!region) {
+        if (!mads_plan(h->g, N, h->cfg, &warps, &smem, &planes_smem))
+            return fail(h, COV_ERR_LIMIT, std::string(who) + ": one warp's framebuffer of the " +
+                                              std::to_string(h->g.nx) + " x " + std::to_string(h->g.ny) +
+                                              " grid does not fit the " + std::to_string(h->cfg.max_smem_optin) +
+                                              " bytes of shared memory per CTA");
+        if (!h->area_exact) OK(entries_on_device(h)); // non-dyadic weights: the list-order sum
+    }
     // in: [pow10: 801 doubles | X0: S n doubles | a0: S n doubles | b0: S n ints]; out: [X_out | obj | stats]
     constexpr int kPow = 1 - 2 * kMadsPow10Min;
     const size_t sn = (size_t)S * n;
@@ -2005,8 +2014,9 @@ extern "C" int cov_mads_solve_batch(cov_handle *h, const double *X0, int64_t S, 
     a.ordered = h->area_exact ? 0 : 1;
     unsigned long long *counter = nullptr;
     OK(take_counter(h, &counter));
-    cudaError_t e = launch_mads(h->g, h->o, h->cfg, a, counter, h->stream);
-    if (e != cudaSuccess) return fail_cuda(h, e, "cov_mads_solve_batch: kernel launch");
+    cudaError_t e = region ? launch_mads_region(h->region, h->o, h->cfg, a, counter, h->stream)
+                           : launch_mads(h->g, h->o, h->cfg, a, counter, h->stream);
+    if (e != cudaSuccess) return fail_cuda(h, e, (std::string(who) + ": kernel launch").c_str());
     h->launches += 1;
     CK(cudaMemcpyAsync(hout.data(), dout, out_bytes, cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
@@ -2014,6 +2024,15 @@ extern "C" int cov_mads_solve_batch(cov_handle *h, const double *X0, int64_t S, 
     if (obj_out) memcpy(obj_out, hout.data() + o_obj, (size_t)S * 8);
     if (stats) memcpy(stats, hout.data() + o_st, (size_t)S * 4 * 8);
     return COV_OK;
+}
+
+extern "C" int cov_mads_solve_batch(cov_handle *h, const double *X0, int64_t S, int64_t n_iter, double granularity,
+                                    uint64_t seed, double *X_out, double *obj_out, int64_t *stats)
+{
+    if (!h) return fail(nullptr, COV_ERR_INVALID, "NULL handle");
+    DeviceGuard dg(h->device);
+    OK(check_ready(h, "cov_mads_solve_batch"));
+    return mads_solve_batch(h, false, X0, S, n_iter, granularity, seed, X_out, obj_out, stats);
 }
 
 extern "C" int cov_argmin(cov_handle *h, const double *X, int64_t B, int32_t barrier, double *best_obj,
@@ -2087,6 +2106,164 @@ extern "C" int cov_union_area_batch(cov_handle *h, const double *X, int64_t B, i
         CK(cudaStreamSynchronize(h->stream));
     }
     return COV_OK;
+}
+
+// ------------------------------------------------------------------------------------------
+// grid-free static objective: the region (domain and covered discs), its batch evaluation and device MADS
+// ------------------------------------------------------------------------------------------
+extern "C" int cov_set_region(cov_handle *h, double x_lo, double y_lo, double x_hi, double y_hi,
+                              const double *covered_xyR, int64_t M)
+{
+    if (!h) return fail(nullptr, COV_ERR_INVALID, "NULL handle");
+    DeviceGuard dg(h->device);
+    if (!(std::isfinite(x_lo) && std::isfinite(y_lo) && std::isfinite(x_hi) && std::isfinite(y_hi)) || !(x_hi > x_lo) ||
+        !(y_hi > y_lo))
+        return fail(h, COV_ERR_INVALID, "cov_set_region: the domain needs finite bounds with x_lo < x_hi, y_lo < y_hi");
+    if (M < 0 || (M > 0 && !covered_xyR)) return fail(h, COV_ERR_INVALID, "cov_set_region: bad covered discs");
+    if (M > kRegionMaxCovered)
+        return fail(h, COV_ERR_LIMIT, "cov_set_region: M = " + std::to_string(M) + " covered discs exceed the " +
+                                          std::to_string(kRegionMaxCovered) + " of the kernels' shared-memory plan");
+    std::vector<double> x, y, r; // discs of radius <= 0 cover nothing: dropped
+    for (int64_t m = 0; m < M; ++m) {
+        const double cx = covered_xyR[m], cy = covered_xyR[M + m], R = covered_xyR[2 * M + m];
+        if (!(std::isfinite(cx) && std::isfinite(cy) && std::isfinite(R)))
+            return fail(h, COV_ERR_INVALID, "cov_set_region: covered disc " + std::to_string(m) + " is not finite");
+        if (R > 0) {
+            x.push_back(cx);
+            y.push_back(cy);
+            r.push_back(R);
+        }
+    }
+    const int Mk = (int)r.size();
+    std::vector<double> discs(x);
+    discs.insert(discs.end(), y.begin(), y.end());
+    discs.insert(discs.end(), r.begin(), r.end());
+    // built in fresh buffers, swapped in on success: a failing call leaves the earlier region in place
+    DevBuf dd, da;
+    auto release = [&] {
+        if (dd.p) cudaFree(dd.p);
+        if (da.p) cudaFree(da.p);
+    };
+    int rc = ensure(h, dd, discs.size() * 8);
+    if (rc == COV_OK) rc = ensure(h, da, (size_t)kRegionMaxArcs * sizeof(RegionArc));
+    if (rc == COV_OK) rc = ensure(h, h->region_count, sizeof(int));
+    if (rc != COV_OK) {
+        release();
+        return rc;
+    }
+    RegionDesc rd{x_lo, y_lo, x_hi, y_hi, Mk, 0, (const double *)dd.p, (const RegionArc *)da.p};
+    int K = 0;
+    cudaError_t e = cudaSuccess;
+    if (Mk > 0) e = cudaMemcpyAsync(dd.p, discs.data(), discs.size() * 8, cudaMemcpyHostToDevice, h->stream);
+    if (e == cudaSuccess && Mk > 0) e = launch_region_arcs(rd, (RegionArc *)da.p, kRegionMaxArcs, (int *)h->region_count.p, h->stream);
+    if (e == cudaSuccess && Mk > 0) {
+        h->launches += 1;
+        e = cudaMemcpyAsync((int *)h->h_small + 96, h->region_count.p, sizeof(int), cudaMemcpyDeviceToHost, h->stream);
+    }
+    if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
+    if (e != cudaSuccess) {
+        release();
+        return fail_cuda(h, e, "cov_set_region");
+    }
+    if (Mk > 0) K = *((int *)h->h_small + 96);
+    if (K > kRegionMaxArcs) {
+        release();
+        return fail(h, COV_ERR_LIMIT, "cov_set_region: the covered discs' boundary has " + std::to_string(K) +
+                                          " arcs inside the domain, more than the " + std::to_string(kRegionMaxArcs) +
+                                          " of the kernels' shared-memory plan");
+    }
+    std::swap(h->region_discs, dd);
+    std::swap(h->region_arcs, da);
+    release(); // the earlier region's buffers
+    rd.K = K;
+    h->region = rd;
+    h->have_region = true;
+    return COV_OK;
+}
+
+static int check_region(cov_handle *h, const char *who)
+{
+    if (!h->have_region) return fail(h, COV_ERR_STATE, std::string(who) + ": no region set");
+    if (!h->have_params) return fail(h, COV_ERR_STATE, std::string(who) + ": no parameters set");
+    if (h->o.N > kRegionMaxUavs)
+        return fail(h, COV_ERR_LIMIT, std::string(who) + ": N = " + std::to_string(h->o.N) + " exceeds the " +
+                                          std::to_string(kRegionMaxUavs) + " discs of a candidate the kernels take");
+    return COV_OK;
+}
+
+extern "C" int cov_eval_region_batch(cov_handle *h, const double *X, int64_t B, double *obj, double *area,
+                                     uint8_t *feasible, int32_t barrier, double *best_obj, int64_t *best_idx)
+{
+    if (!h) return fail(nullptr, COV_ERR_INVALID, "NULL handle");
+    DeviceGuard dg(h->device);
+    OK(check_region(h, "cov_eval_region_batch"));
+    if (B < 0 || (B > 0 && !X) || (!best_obj != !best_idx))
+        return fail(h, COV_ERR_INVALID, "cov_eval_region_batch: bad arguments");
+    const bool want_best = best_obj != nullptr;
+    const int N = h->o.N;
+    const size_t row_bytes = (size_t)3 * N * 8;
+    const int64_t window = std::max<int64_t>(1, std::min<int64_t>(std::max<int64_t>(B, 1), (int64_t)((1ull << 30) / row_bytes)));
+    OK(ensure(h, h->dX, (size_t)window * row_bytes));
+    OK(ensure(h, h->d_obj, (size_t)window * 8));
+    OK(ensure(h, h->d_area, (size_t)window * 8));
+    OK(ensure(h, h->d_feas, (size_t)window));
+    double best = INFINITY;
+    int64_t bidx = -1;
+    recycle_spans(h);
+    for (int64_t w0 = 0; w0 < B; w0 += window) {
+        const int64_t wn = std::min(window, B - w0);
+        CK(cudaMemcpyAsync(h->dX.p, X + (size_t)w0 * 3 * N, (size_t)wn * row_bytes, cudaMemcpyHostToDevice, h->stream));
+        double *d_obj = (double *)h->d_obj.p, *d_area = (double *)h->d_area.p;
+        unsigned char *d_feas = (unsigned char *)h->d_feas.p;
+        cudaEvent_t e0 = get_event(h), e1 = get_event(h); // the kernel's device time, for cov_last_kernel_ms
+        CK(cudaEventRecord(e0, h->stream));
+        cudaError_t e = launch_region_eval(h->region, h->o, h->cfg, (const double *)h->dX.p, wn, d_obj, area ? d_area : nullptr,
+                                           d_feas, h->stream);
+        if (e != cudaSuccess) {
+            h->ev_pool.push_back(e0);
+            h->ev_pool.push_back(e1);
+            if (e != cudaErrorInvalidConfiguration) return fail_cuda(h, e, "cov_eval_region_batch: kernel launch");
+            (void)cudaGetLastError();
+            return fail(h, COV_ERR_LIMIT, "cov_eval_region_batch: the region does not fit the shared-memory plan");
+        }
+        CK(cudaEventRecord(e1, h->stream));
+        h->kernel_spans.emplace_back(e0, e1);
+        h->launches += 1;
+        if (want_best) {
+            CK(launch_argmin(d_obj, d_feas, wn, barrier, (double *)h->argmin_obj.p, (long long *)h->argmin_idx.p, 1024,
+                             h->stream));
+            h->launches += 2;
+            CK(cudaMemcpyAsync((double *)h->h_small + 40, h->argmin_obj.p, 8, cudaMemcpyDeviceToHost, h->stream));
+            CK(cudaMemcpyAsync((long long *)h->h_small + 41, h->argmin_idx.p, 8, cudaMemcpyDeviceToHost, h->stream));
+        }
+        if (obj) CK(cudaMemcpyAsync(obj + w0, d_obj, (size_t)wn * 8, cudaMemcpyDeviceToHost, h->stream));
+        if (area) CK(cudaMemcpyAsync(area + w0, d_area, (size_t)wn * 8, cudaMemcpyDeviceToHost, h->stream));
+        if (feasible) CK(cudaMemcpyAsync(feasible + w0, d_feas, (size_t)wn, cudaMemcpyDeviceToHost, h->stream));
+        CK(cudaStreamSynchronize(h->stream));
+        if (want_best) {
+            const double ho = *((double *)h->h_small + 40);
+            const long long hi = *((long long *)h->h_small + 41);
+            if (hi >= 0 && (bidx < 0 || ho < best)) { // ties keep the earlier window's index
+                best = ho;
+                bidx = w0 + hi;
+            }
+        }
+    }
+    if (want_best) {
+        *best_obj = bidx >= 0 ? best : INFINITY;
+        *best_idx = bidx;
+    }
+    return COV_OK;
+}
+
+extern "C" int cov_mads_solve_batch_region(cov_handle *h, const double *X0, int64_t S, int64_t n_iter,
+                                           double granularity, uint64_t seed, double *X_out, double *obj_out,
+                                           int64_t *stats)
+{
+    if (!h) return fail(nullptr, COV_ERR_INVALID, "NULL handle");
+    DeviceGuard dg(h->device);
+    OK(check_region(h, "cov_mads_solve_batch_region"));
+    return mads_solve_batch(h, true, X0, S, n_iter, granularity, seed, X_out, obj_out, stats);
 }
 
 // ------------------------------------------------------------------------------------------

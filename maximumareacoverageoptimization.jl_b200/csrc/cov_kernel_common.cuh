@@ -35,6 +35,12 @@ __device__ __forceinline__ void store_mirrors(const EvalOut &out, long long idx,
     }
 }
 
+// obj = -area + violation*scale (src/TDM_STATIC_opt.jl:89-97)
+__device__ __forceinline__ double objective_from_area(double area, double violation, const ObjParams &o)
+{
+    return __dadd_rn(-area, __dmul_rn(violation, o.penalty_scale));
+}
+
 // obj = -area + violation*scale, area from exact integer counts (see cov_grid_info.area_exact)
 __device__ __forceinline__ double assemble_objective(const GridDesc &g, const ObjParams &o,
                                                      const long long *class_cnt, double violation)
@@ -46,7 +52,7 @@ __device__ __forceinline__ double assemble_objective(const GridDesc &g, const Ob
         for (int k = 0; k < g.n_classes; ++k)
             area = __dadd_rn(area, __dmul_rn(g.class_weight[k], (double)class_cnt[k]));
     }
-    return __dadd_rn(-area, __dmul_rn(violation, o.penalty_scale));
+    return objective_from_area(area, violation, o);
 }
 
 // ------------------------------------------------------------------------------------------

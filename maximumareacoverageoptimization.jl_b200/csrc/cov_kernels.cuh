@@ -70,6 +70,18 @@ bool mads_plan(const GridDesc &g, int N, const LaunchCfg &cfg, int *warps, int *
 cudaError_t launch_mads(const GridDesc &g, const ObjParams &o, const LaunchCfg &cfg, const MadsArgs &a,
                         unsigned long long *counter, cudaStream_t stream);
 
+// ---- the grid-free static objective (cov_region.cu, cov_mads.cu; geometry and limits in cov_region.cuh) ----
+// The arcs of the covered set's boundary inside the domain (r.arcs / r.K unused): at most cap of them to out, the
+// count of all of them to *count (device).
+cudaError_t launch_region_arcs(const RegionDesc &r, RegionArc *out, int cap, int *count, cudaStream_t s);
+// obj / area / feasible (device, each nullable) of B candidates; cudaErrorInvalidConfiguration when N or the region
+// exceed the shared-memory plan.
+cudaError_t launch_region_eval(const RegionDesc &r, const ObjParams &o, const LaunchCfg &cfg, const double *dX,
+                               long long B, double *obj, double *area, unsigned char *feasible, cudaStream_t s);
+// cov_mads_solve_batch's solves with the region objective (a.force_exact and a.ordered unused).
+cudaError_t launch_mads_region(const RegionDesc &r, const ObjParams &o, const LaunchCfg &cfg, const MadsArgs &a,
+                               unsigned long long *counter, cudaStream_t stream);
+
 // ---- cell-store kernels (cov_grid_kernels.cu) ----
 // stats[0] = entries, stats[1] = cells, stats[2 + k] = OR of the multiplicities of class k
 cudaError_t launch_grid_stats(const unsigned char *mult, const unsigned char *cls, long long ncell,

@@ -16,6 +16,8 @@
 //      (the same arithmetic, so the same bits) and the mesh enlarged, or the mesh refined / the solve stopped.
 // Everything is cov_mads_solve's loop (cov_api.cu) in the same FP64 operations and order, so a host model can
 // replay every iterate bit for bit; only the direction stream and the absence of a cache differ.
+// region_solve_kernel (cov_mads_solve_batch_region) runs the same loop (mads_solves) with step 4 replaced by the
+// region objective of cov_region.cuh, the device function cov_eval_region_batch's kernel calls.
 #include <cuda_runtime.h>
 #include <algorithm>
 #include <cstdint>
@@ -24,6 +26,7 @@
 #include "cov_candidate.cuh"
 #include "cov_span_common.cuh"
 #include "cov_kernels.cuh"
+#include "cov_region.cuh"
 
 namespace cov {
 
@@ -180,35 +183,21 @@ __device__ double mads_eval(const GridDesc &g, const ObjParams &o, const double 
     return (obj == obj) ? obj : __longlong_as_double(0x7ff0000000000000ll);
 }
 
-template <bool MULTI, bool PLANES_SMEM, int THREADS, int CTAS>
-__global__ void __launch_bounds__(THREADS, CTAS)
-mads_kernel(const __grid_constant__ GridDesc g, const __grid_constant__ ObjParams o, const __grid_constant__ MadsArgs a,
-            unsigned long long *counter)
+// The solves of cov_mads_solve_batch from the dispenser `counter` until none is left, by the whole CTA: the loop
+// shared by mads_kernel (the grid objective) and region_solve_kernel (the region objective).  state: mads_state_bytes(n)
+// bytes of shared memory; stage: the calling warp's 3N doubles; eval(p): the barrier value of the point p (shared
+// memory) by the calling warp.
+template <class Eval>
+__device__ __forceinline__ void mads_solves(const MadsArgs &a, int n, unsigned char *state, double *stage,
+                                            unsigned long long *counter, const Eval &eval)
 {
-    extern __shared__ __align__(16) unsigned char smem_raw[];
     const int W = blockDim.x >> 5;
     const int warp = threadIdx.x >> 5;
     const uint32_t lane = lane_id();
-    const int N = o.N, n = 3 * N;
-    const int planes_bytes = PLANES_SMEM ? g.n_planes * g.plane_words * 4 : 0;
-    const int warp_bytes = mads_warp_bytes(g, N);
-    uint32_t *planes_s = reinterpret_cast<uint32_t *>(smem_raw);
-    unsigned char *sbase = smem_raw + planes_bytes;
-    double *x = reinterpret_cast<double *>(sbase);
+    double *x = reinterpret_cast<double *>(state);
     double *v = x + n, *rho = v + n, *delta = rho + n, *am = delta + n, *f = am + n; // f: 2n
     int *bm = reinterpret_cast<int *>(f + 2 * n), *bz = bm + n;
-    MadsShared *sh = reinterpret_cast<MadsShared *>(sbase + round_up(7 * n * 8 + 2 * n * 4, 16));
-    unsigned char *wbase = sbase + mads_state_bytes(n) + (size_t)warp * warp_bytes;
-    double *stage = reinterpret_cast<double *>(wbase);
-    SDisc *sd = reinterpret_cast<SDisc *>(wbase + round_up(3 * N * 8, 16));
-    int *pre = reinterpret_cast<int *>(wbase + round_up(3 * N * 8, 16) + N * 32);
-    uint32_t *fb = reinterpret_cast<uint32_t *>(wbase + round_up(3 * N * 8, 16) + N * 32 + round_up(N * 4, 16));
-    uint64_t *bar = reinterpret_cast<uint64_t *>(sbase + mads_state_bytes(n) + (size_t)W * warp_bytes);
-
-    if (PLANES_SMEM) stage_planes(g, planes_s, bar, planes_bytes); // TMA bulk copy, once per CTA (syncs)
-    const uint32_t *planes = PLANES_SMEM ? planes_s : g.planes;
-    for (int t = lane; t < mads_fb_bytes(g, N) / 16; t += 32) reinterpret_cast<uint4 *>(fb)[t] = make_uint4(0, 0, 0, 0);
-    __syncwarp();
+    MadsShared *sh = reinterpret_cast<MadsShared *>(state + round_up(7 * n * 8 + 2 * n * 4, 16));
     const double gran = a.granularity;
     const int tid = threadIdx.x, nthr = blockDim.x;
 
@@ -225,7 +214,7 @@ mads_kernel(const __grid_constant__ GridDesc g, const __grid_constant__ ObjParam
         }
         __syncthreads();
         if (warp == 0) {
-            const double f0 = mads_eval<MULTI, PLANES_SMEM>(g, o, x, sd, pre, fb, planes, a.force_exact, a.ordered);
+            const double f0 = eval(x);
             if (lane == 0) {
                 sh->fx = f0;
                 sh->feasible_found = isfinite(f0) ? 1 : 0;
@@ -259,7 +248,7 @@ mads_kernel(const __grid_constant__ GridDesc g, const __grid_constant__ ObjParam
                 const bool keep = poll_point(kk, n, x, v, rho, delta, gran, stage);
                 __syncwarp();
                 double fk = __longlong_as_double(0x7ff8000000000000ll); // dropped
-                if (keep) fk = mads_eval<MULTI, PLANES_SMEM>(g, o, stage, sd, pre, fb, planes, a.force_exact, a.ordered);
+                if (keep) fk = eval(stage);
                 if (lane == 0) f[kk] = fk;
                 __syncwarp();
             }
@@ -329,6 +318,36 @@ mads_kernel(const __grid_constant__ GridDesc g, const __grid_constant__ ObjParam
     }
 }
 
+template <bool MULTI, bool PLANES_SMEM, int THREADS, int CTAS>
+__global__ void __launch_bounds__(THREADS, CTAS)
+mads_kernel(const __grid_constant__ GridDesc g, const __grid_constant__ ObjParams o, const __grid_constant__ MadsArgs a,
+            unsigned long long *counter)
+{
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    const int W = blockDim.x >> 5;
+    const int warp = threadIdx.x >> 5;
+    const uint32_t lane = lane_id();
+    const int N = o.N, n = 3 * N;
+    const int planes_bytes = PLANES_SMEM ? g.n_planes * g.plane_words * 4 : 0;
+    const int warp_bytes = mads_warp_bytes(g, N);
+    uint32_t *planes_s = reinterpret_cast<uint32_t *>(smem_raw);
+    unsigned char *sbase = smem_raw + planes_bytes;
+    unsigned char *wbase = sbase + mads_state_bytes(n) + (size_t)warp * warp_bytes;
+    double *stage = reinterpret_cast<double *>(wbase);
+    SDisc *sd = reinterpret_cast<SDisc *>(wbase + round_up(3 * N * 8, 16));
+    int *pre = reinterpret_cast<int *>(wbase + round_up(3 * N * 8, 16) + N * 32);
+    uint32_t *fb = reinterpret_cast<uint32_t *>(wbase + round_up(3 * N * 8, 16) + N * 32 + round_up(N * 4, 16));
+    uint64_t *bar = reinterpret_cast<uint64_t *>(sbase + mads_state_bytes(n) + (size_t)W * warp_bytes);
+
+    if (PLANES_SMEM) stage_planes(g, planes_s, bar, planes_bytes); // TMA bulk copy, once per CTA (syncs)
+    const uint32_t *planes = PLANES_SMEM ? planes_s : g.planes;
+    for (int t = lane; t < mads_fb_bytes(g, N) / 16; t += 32) reinterpret_cast<uint4 *>(fb)[t] = make_uint4(0, 0, 0, 0);
+    __syncwarp();
+    mads_solves(a, n, sbase, stage, counter, [&](const double *p) {
+        return mads_eval<MULTI, PLANES_SMEM>(g, o, p, sd, pre, fb, planes, a.force_exact, a.ordered);
+    });
+}
+
 bool mads_plan(const GridDesc &g, int N, const LaunchCfg &cfg, int *warps, int *smem, int *planes_smem)
 {
     if (N < 1 || N > kMadsMaxUavs) return false;
@@ -370,6 +389,48 @@ cudaError_t launch_mads(const GridDesc &g, const ObjParams &o, const LaunchCfg &
                          : launch_mads_variant<true, false>(g, o, cfg, a, counter, stream, warps, smem);
     return ps ? launch_mads_variant<false, true>(g, o, cfg, a, counter, stream, warps, smem)
               : launch_mads_variant<false, false>(g, o, cfg, a, counter, stream, warps, smem);
+}
+
+// The solves of cov_mads_solve_batch with the region objective.  Shared memory: [solve state] [region] [W x (stage,
+// interval lists)].
+template <int THREADS, int CTAS>
+__global__ void __launch_bounds__(THREADS, CTAS)
+region_solve_kernel(const __grid_constant__ RegionDesc r, const __grid_constant__ ObjParams o,
+                    const __grid_constant__ MadsArgs a, unsigned long long *counter)
+{
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    const int N = o.N, n = 3 * N, warp = threadIdx.x >> 5;
+    unsigned char *rbase = smem_raw + mads_state_bytes(n);
+    const RegionView v = region_stage(r, rbase);
+    unsigned char *wbase = rbase + region_smem_bytes(r.M, r.K) + (size_t)warp * region_warp_bytes(N, r.M);
+    double *stage = reinterpret_cast<double *>(wbase);
+    double *ia = reinterpret_cast<double *>(wbase + round_up(3 * N * 8, 16)), *ib = ia + region_list_cap(N, r.M);
+    __syncthreads();
+    mads_solves(a, n, smem_raw, stage, counter, [&](const double *p) { // region_objective with the extreme barrier
+        const CandScalars cs = candidate_prologue<false>(GridDesc{}, o, p, nullptr, false);
+        if (!cs.feasible) return __longlong_as_double(0x7ff0000000000000ll);
+        const double obj = objective_from_area(region_area(v, p, N, ia, ib), cs.violation, o);
+        return (obj == obj) ? obj : __longlong_as_double(0x7ff0000000000000ll);
+    });
+}
+
+cudaError_t launch_mads_region(const RegionDesc &r, const ObjParams &o, const LaunchCfg &cfg, const MadsArgs &a,
+                               unsigned long long *counter, cudaStream_t stream)
+{
+    if (a.S <= 0) return cudaSuccess;
+    int warps = 0, smem = 0;
+    if (o.N > kRegionMaxUavs ||
+        !region_plan(o.N, r.M, r.K, mads_state_bytes(3 * o.N), cfg.max_smem_optin - 1024 /* the kernel's static shared memory */, &warps, &smem))
+        return cudaErrorInvalidConfiguration;
+    auto kern = region_solve_kernel<kRegionThreads, kRegionCtas>;
+    cudaError_t err = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+    if (err != cudaSuccess) return err;
+    int per_sm = 0;
+    err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, warps * 32, smem);
+    if (err != cudaSuccess) return err;
+    const int grid = (int)std::min<long long>(a.S, (long long)cfg.num_sms * std::max(per_sm, 1));
+    kern<<<grid, warps * 32, smem, stream>>>(r, o, a, counter);
+    return cudaGetLastError();
 }
 
 } // namespace cov

@@ -63,6 +63,19 @@ struct ObjParams {
     const double *cons3_G;  // device, N: sqrt(s) > d_lim[i]  <=>  s >= cons3_G[i]
 };
 
+// The grid-free static objective's region (cov_set_region): the domain rectangle and the covered discs C, with the
+// arcs of C's boundary that lie inside the domain (each a piece [a, b] of covered circle m, 0 <= a < b <= 2 pi).
+struct RegionArc {
+    double a, b;
+    int m, pad;
+};
+struct RegionDesc {
+    double x_lo, y_lo, x_hi, y_hi;
+    int M, K;               // covered discs (radius > 0), arcs
+    const double *discs;    // device: 3M doubles [x_1..x_M, y_1..y_M, R_1..R_M]
+    const RegionArc *arcs;  // device: K
+};
+
 struct EvalOut {
     double *obj;            // B
     long long *count;       // B or null

@@ -322,6 +322,13 @@ class CoverageEngine:
         """S independent MADS solves in one launch on the device (cov_mads_solve_batch): solve k starts at X0[k] and
         draws its directions from the Philox key seed + k.  Returns (X S x 3N, objectives S, stats) with stats a dict
         of per-solve int64 arrays: iterations, evaluations, successes, converged."""
+        return self._mads_batch(lib.cov_mads_solve_batch, X0, n_iter, granularity, seed)
+
+    def mads_solve_batch_region(self, X0, n_iter: int = 100, granularity: float = 1.0, seed: int = 0):
+        """mads_solve_batch on the grid-free static objective of eval_region_batch (cov_mads_solve_batch_region)."""
+        return self._mads_batch(lib.cov_mads_solve_batch_region, X0, n_iter, granularity, seed)
+
+    def _mads_batch(self, fn, X0, n_iter, granularity, seed):
         X0 = _f64(X0)
         if X0.ndim == 1:
             X0 = X0.reshape(1, -1)
@@ -331,10 +338,41 @@ class CoverageEngine:
         X = np.empty_like(X0)
         obj = np.empty(S, dtype=np.float64)
         st = np.empty((S, 4), dtype=np.int64)
-        self._check(lib.cov_mads_solve_batch(self._h, _ptr(X0), S, int(n_iter), float(granularity),
-                                             int(seed) & (2**64 - 1), _ptr(X), _ptr(obj), _ptr(st)))
+        self._check(fn(self._h, _ptr(X0), S, int(n_iter), float(granularity), int(seed) & (2**64 - 1), _ptr(X),
+                       _ptr(obj), _ptr(st)))
         names = ("iterations", "evaluations", "successes", "converged")
         return X, obj, {name: st[:, q].copy() for q, name in enumerate(names)}
+
+    # ---- grid-free static objective ----
+    def set_region(self, x_lo: float, y_lo: float, x_hi: float, y_hi: float, covered=None):
+        """The domain rectangle and the discs already covered (cov_set_region): covered is M x 3 rows (x, y, R), or
+        None for none."""
+        C3 = np.zeros((0, 3)) if covered is None else _f64(covered).reshape(-1, 3)
+        xyR = np.ascontiguousarray(C3.T).ravel()  # [x_1..x_M, y_1..y_M, R_1..R_M]
+        self._check(lib.cov_set_region(self._h, float(x_lo), float(y_lo), float(x_hi), float(y_hi),
+                                       _ptr(xyR) if len(C3) else None, len(C3)))
+
+    def eval_region_batch(self, X, want_area=True, want_feasible=True, best=False, barrier: bool = True):
+        """cov_eval_region_batch: dict(obj, area, feasible) for every row of X (B, 3N), with best=True also
+        res["best"] = (objective, index) of the poll winner."""
+        X = _f64(X)
+        if X.ndim == 1:
+            X = X.reshape(1, -1)
+        if self.N is None or X.shape[1] != 3 * self.N:
+            raise ValueError("X must be (B, 3N) with the N given to set_params")
+        B = X.shape[0]
+        res = {"obj": np.empty(B, dtype=np.float64)}
+        if want_area:
+            res["area"] = np.empty(B, dtype=np.float64)
+        if want_feasible:
+            res["feasible"] = np.empty(B, dtype=np.uint8)
+        bo, bi = C.c_double(), C.c_int64()
+        self._check(lib.cov_eval_region_batch(self._h, _ptr(X), B, _ptr(res["obj"]), _ptr(res.get("area")),
+                                              _ptr(res.get("feasible")), 1 if barrier else 0,
+                                              C.byref(bo) if best else None, C.byref(bi) if best else None))
+        if best:
+            res["best"] = (bo.value, bi.value)
+        return res
 
     def argmin(self, X, barrier: bool = True):
         X = _f64(X)

@@ -286,6 +286,40 @@ function mads_solve_batch(h::Handle, X0::Matrix{Float64}; N_iter = 100, granular
 end
 
 """
+    set_region!(h, x_lo, y_lo, x_hi, y_hi, covered)
+
+The grid-free static objective's region: the domain rectangle and the discs already covered, `covered` a 3 x M
+matrix with columns [x; y; R] (0 columns: nothing covered yet).
+"""
+function set_region!(h::Handle, x_lo, y_lo, x_hi, y_hi, covered::Matrix{Float64} = zeros(Float64, 3, 0))
+    M = size(covered, 2)
+    xyR = vec(permutedims(covered))  # [x_1..x_M; y_1..y_M; R_1..R_M]
+    GC.@preserve xyR check(h, ccall((:cov_set_region, LIB), Cint,
+        (Ptr{Cvoid}, Float64, Float64, Float64, Float64, Ptr{Float64}, Int64),
+        h.ptr, x_lo, y_lo, x_hi, y_hi, M == 0 ? C_NULL : pointer(xyR), M))
+end
+
+"Objective, newly covered area and feasibility of every column of `X` (3N x B) on the region (`set_region!`)."
+function objective_region_batch(h::Handle, X::Matrix{Float64})
+    B = size(X, 2)
+    obj = Vector{Float64}(undef, B); area = Vector{Float64}(undef, B); feasible = Vector{UInt8}(undef, B)
+    GC.@preserve X obj area feasible check(h, ccall((:cov_eval_region_batch, LIB), Cint,
+        (Ptr{Cvoid}, Ptr{Float64}, Int64, Ptr{Float64}, Ptr{Float64}, Ptr{UInt8}, Int32, Ptr{Float64}, Ptr{Int64}),
+        h.ptr, X, B, obj, area, feasible, 1, C_NULL, C_NULL))
+    return obj, area, feasible
+end
+
+"`mads_solve_batch` on the region objective of `objective_region_batch` (no cell store needed)."
+function mads_solve_batch_region(h::Handle, X0::Matrix{Float64}; N_iter = 100, granularity = 1.0, seed = 0)
+    S = size(X0, 2)
+    out = similar(X0); obj = zeros(Float64, S); stats = zeros(Int64, 4, S)
+    t = @elapsed GC.@preserve X0 out obj stats check(h, ccall((:cov_mads_solve_batch_region, LIB), Cint,
+        (Ptr{Cvoid}, Ptr{Float64}, Int64, Int64, Float64, UInt64, Ptr{Float64}, Ptr{Float64}, Ptr{Int64}),
+        h.ptr, X0, S, N_iter, granularity, seed, out, obj, stats))
+    return out, obj, stats, t
+end
+
+"""
     createObjective(cells, N, r_max; handle = Handle())
 
 Same signature and value as the reference's `TDM_STATIC_opt.createObjective` (src/TDM_STATIC_opt.jl:82):
