@@ -9,7 +9,7 @@ ORACLE    := oracle/libcoverage_oracle.so
 NVCCFLAGS := --threads 0 -gencode arch=compute_100a,code=sm_100a -O3 -std=c++17 -lineinfo --fmad=false \
              -Xcompiler -fPIC,-O2,-fno-fast-math,-ffp-contract=off,-fvisibility=hidden,-pthread -Xptxas -v $(EXTRA)
 SRCS      := $(CSRC)/cov_api.cu $(CSRC)/cov_kernels.cu $(CSRC)/cov_span_small.cu $(CSRC)/cov_span_cta.cu $(CSRC)/cov_grid_kernels.cu $(CSRC)/cov_mads.cu \
-             $(CSRC)/cov_region.cu
+             $(CSRC)/cov_region.cu $(CSRC)/cov_horizon.cu
 HDRS      := $(wildcard $(CSRC)/*.h $(CSRC)/*.cuh) include/coverage_cuda.h
 
 all: $(LIB) $(ORACLE)

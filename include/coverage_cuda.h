@@ -37,7 +37,7 @@ extern "C" {
 #define COV_ABI_VERSION 3 /* 2: COV_OPT_PROGRESSIVE_INDEX, COV_KERNEL_ORDERED, cov_get_class_weights, cov_eval_batch_best;
                              3: cov_eval_batch_packed (COV_PACK_*); later, with no existing symbol changed:
                                 cov_mads_solve_batch; cov_set_region, cov_eval_region_batch,
-                                cov_mads_solve_batch_region (the grid-free static objective) */
+                                cov_mads_solve_batch_region (the grid-free static objective); cov_run_horizon */
 
 #if defined(__GNUC__)
 #define COV_API __attribute__((visibility("default")))
@@ -283,6 +283,39 @@ COV_API int cov_mads_solve(cov_handle *h, const double *x0, int64_t n_iter, doub
  * launch; cov_last_launch and the kernel timers are left unchanged. */
 COV_API int cov_mads_solve_batch(cov_handle *h, const double *X0, int64_t S, int64_t n_iter, double granularity,
                                  uint64_t seed, double *X_out, double *obj_out, int64_t *stats);
+
+/* The receding-horizon simulation on the device (FullSimulation.run_simulation, src/FullSimulation.jl:42-107, static
+ * environment): T timesteps of rmvCoveredPOI and multi-start MADS, all enqueued before ONE synchronise at the end.
+ * Needs a cell store with area_exact == 1 and cov_set_params with prev_xyR (cons3 on); the penalty, cons3's d_lim,
+ * cons7 and cons8 are the ones set there.  Let cur = x_start (3N).  For t = 1 .. T:
+ *  1. rmvCoveredPOI(cur), as cov_remove_covered;
+ *  2. for t >= 2 and n_boxes > 0 the r_max rule of FullSimulation.py:80-87 in its FP64 operations: for each UAV i with
+ *     fabs(h_focus - R_i / tan_half_fov) < 1 and m = h_max * tan_half_fov, r_max[i] = h_focus * tan_half_fov if some
+ *     box k has x_i < xu_k + m && x_i > xl_k - m && y_i < yu_k + m && y_i > yl_k - m, else m.  boxes: n_boxes x 4
+ *     doubles x_LB, x_UB, y_LB, y_UB; tan_half_fov: cov_set_params's;
+ *  3. cons3's previous swarm := cur (prev_z = R / tan_half_fov, as cov_set_params forms it);
+ *  4. S starts: start 0 is cur; start k >= 1 moves x_i and y_i (never R) to v = cur + spread * z, snapped to
+ *     nearbyint(v / g) * g when granularity g > 0.  z = s * 2^-32 - 6.0 with s the sum of the 12 words of the
+ *     Philox4x32-10 blocks keyed by (low, high 32 bits of seed) with counter (t, k, j, 3 + q), q = 0, 1, 2 (t and k
+ *     taken mod 2^32; j = i for x_i, N + i for y_i).  The direction stream of cov_mads_solve_batch only uses 0 .. 2 in
+ *     that word.  The initial mesh of every start is cov_mads_solve_batch's, with floor(log10(target)) taken as the
+ *     largest b >= 0 whose host-libm 10^b is <= target: the same b except for targets a few ulps below a power of
+ *     ten, which mesh points are not (checked for every point |x| <= 10^4 of granularity 1, 0.5 and 0.25);
+ *  5. the S solves of cov_mads_solve_batch (n_iter, granularity), solve k keyed by seed + (t - 1) S + k (mod 2^64);
+ *  6. cur := X of the solve with the smallest barrier value (NaN counts as +Inf, ties to the smallest k; k = 0, whose
+ *     X is cur itself, when none is finite); X_out row t-1 = cur;
+ *  7. obj_out[t-1] (nullable) = AreaMaxObjective(cur) without the barrier, on step t's store and r_max.
+ * stats (nullable): T x 4 [winner k, evaluations summed over the S solves, solves that found a feasible point,
+ * entries removed in step 1]; step_ms (nullable): T device times between CUDA events recorded between the steps.
+ * Afterwards the store holds every removal and the parameters are step T's (r_max, previous swarm), exactly as the
+ * same sequence of existing calls leaves them.  T == 0 does nothing.  COV_ERR_STATE: no grid or parameters, cons3 off,
+ * or area_exact == 0; COV_ERR_LIMIT: cov_mads_solve_batch's limits; COV_ERR_INVALID: T < 0, S < 1, n_iter < 0, NULL
+ * x_start or X_out when T > 0, spread not finite or < 0, granularity < 0 or NaN, n_boxes < 0 or n_boxes > 0 with
+ * NULL boxes.  A refused call changes nothing.  cov_last_launch and the kernel timers are left unchanged. */
+COV_API int cov_run_horizon(cov_handle *h, const double *x_start, int64_t T, int64_t S, double spread,
+                            int64_t n_iter, double granularity, uint64_t seed,
+                            const double *boxes, int64_t n_boxes, double h_focus, double h_max,
+                            double *X_out, double *obj_out, int64_t *stats, double *step_ms);
 
 /* Covered-cell mask of ONE candidate: nx*ny bytes, 1 where the cell is inside some disc (whether
  * or not it holds entries). Lets the host replay an ordered Float64 sum over a weighted list. */

@@ -46,11 +46,37 @@ class SimulationParameters:
         self.Nt_sim = int(self.tf / self.dt_sim)
 
 
+H_FOCUS = 15.0  # the altitude the r_max rule looks for (src/FullSimulation.jl:66)
+
+
+def _boxes(p: SimulationParameters) -> np.ndarray:
+    """The high-interest rectangles as K x 4 rows x_LB, x_UB, y_LB, y_UB."""
+    return np.stack([np.asarray(v, dtype=np.float64).ravel() for v in (p.x_LB, p.x_UB, p.y_LB, p.y_UB)], axis=1)
+
+
+def apply_r_max_rule(drone_locs, r_max, N: int, p: SimulationParameters, t_half: float):
+    """src/FullSimulation.jl:65-76, in place on r_max: a UAV flying at H_FOCUS keeps the focus radius near a
+    high-interest rectangle (within h_max * tan(FOV/2) of it) and gets the h_max radius elsewhere."""
+    xl, xu, yl, yu = _boxes(p).T
+    for i in range(N):
+        if abs(H_FOCUS - drone_locs[i + 2 * N] / t_half) < 1:
+            m = p.h_max * t_half
+            check = ((drone_locs[i] < xu + m) & (drone_locs[i] > xl - m) &
+                     (drone_locs[i + N] < yu + m) & (drone_locs[i + N] > yl - m))
+            r_max[i] = H_FOCUS * t_half if check.any() else p.h_max * t_half
+
+
 def run_simulation(cells, starting_circles, cons_ext, cons_prog, N, r_max, params: SimulationParameters,
-                   Nt_sim: int | None = None, objective: str = "grid", covered_pb: list | None = None):
+                   Nt_sim: int | None = None, objective: str = "grid", covered_pb: list | None = None,
+                   starts: int | None = None, spread: float = 3.0):
     """Returns (single_input_pb, single_output_pb, runtime_data_MADS, objective_pb).  objective: "grid" (the
     reference's) or "region"; with "region", covered_pb (if given) receives the covered set (M x 3 rows x, y, R) each
-    timestep's objective was built on."""
+    timestep's objective was built on.
+
+    starts=S runs the whole horizon on the device in one call (CoverageEngine.run_horizon): per timestep S MADS
+    solves, from the swarm and from S - 1 copies of it moved by N(0, spread^2) metres in x and y, and the best result
+    becomes the next swarm.  Static environment and the grid objective only, with constraints that all fuse;
+    runtime_data_MADS then holds the device time of each timestep."""
     p = params
     if objective not in ("grid", "region"):
         raise ValueError("objective must be 'grid' or 'region'")
@@ -63,6 +89,10 @@ def run_simulation(cells, starting_circles, cons_ext, cons_prog, N, r_max, param
     r_max = np.ascontiguousarray(r_max, dtype=np.float64)
     d_lim = p.d_lim * np.ones(N)
     steps = p.Nt_sim if Nt_sim is None else Nt_sim
+    if starts is not None:
+        if p.environment_type != "static" or objective != "grid":
+            raise ValueError("starts= runs the static environment with the grid objective only")
+        return _run_horizon(cells, pre, cons_ext, N, r_max, p, steps, int(starts), spread, t_half, d_lim)
     engine, covered = None, np.zeros((0, 3))
     if objective == "region":
         from .engine import CoverageEngine
@@ -78,13 +108,7 @@ def run_simulation(cells, starting_circles, cons_ext, cons_prog, N, r_max, param
         else:
             cells = CellFunctions.rmvCoveredPOI(cells, drone_locs)
         if t != 1:  # :65-76
-            xl, xu, yl, yu = (np.asarray(v, dtype=np.float64) for v in (p.x_LB, p.x_UB, p.y_LB, p.y_UB))
-            for i in range(N):
-                if abs(15 - drone_locs[i + 2 * N] / t_half) < 1:
-                    m = p.h_max * t_half
-                    check = ((drone_locs[i] < xu + m) & (drone_locs[i] > xl - m) &
-                             (drone_locs[i + N] < yu + m) & (drone_locs[i + N] > yl - m))
-                    r_max[i] = 15 * t_half if check.any() else p.h_max * t_half
+            apply_r_max_rule(drone_locs, r_max, N, p, t_half)
         cons3 = create_cons3(pre, p.FOV, d_lim)
         if t < 3:
             single_input = drone_locs
@@ -108,3 +132,24 @@ def run_simulation(cells, starting_circles, cons_ext, cons_prog, N, r_max, param
     if engine is not None:
         engine.close()
     return single_input_pb, single_output_pb, runtime_data_MADS, objective_pb
+
+
+def _run_horizon(cells, pre, cons_ext, N, r_max, p, steps, S, spread, t_half, d_lim):
+    """run_simulation(starts=S): the loop above with S solves per timestep, in one cov_run_horizon call."""
+    from .mads import _flatten_constraints
+    boxes = _boxes(p)
+    if not len(boxes):
+        raise ValueError("starts= needs at least one high-interest rectangle")
+    obj = TDM_STATIC_opt.createObjective(cells, N, r_max)
+    if obj.native_batch_solver(_flatten_constraints([cons_ext, create_cons3(pre, p.FOV, d_lim)])) is None:
+        raise ValueError("starts= needs constraints that all fuse into the objective's launch")
+    res, eng = obj._engine()  # the store synced, the parameters of timestep 1's solves (cons3 from pre) set
+    X, objs, _, step_ms = eng.run_horizon(pre, steps, S, spread, p.N_iter, 1.0, 0 if p.seed is None else p.seed,
+                                          boxes, H_FOCUS, p.h_max)
+    # the host list after every rmvCoveredPOI: the entries whose cell still holds some
+    res.points.keep(eng.grid_cells()[res.cell_index()] > 0)
+    res.mark_synced()
+    for t in range(2, steps + 1):  # the caller's r_max as the host loop leaves it
+        apply_r_max_rule(X[t - 2], r_max, N, p, t_half)
+    inputs = [pre.copy()] + [X[t].copy() for t in range(steps - 1)]
+    return inputs, [x.copy() for x in X], [float(ms) / 1e3 for ms in step_ms], [float(v) for v in objs]

@@ -1956,6 +1956,22 @@ extern "C" int cov_mads_solve(cov_handle *h, const double *x0, int64_t n_iter, d
     return COV_OK;
 }
 
+// The solver's launch plan: N <= kMadsMaxUavs and, with the cell store's objective (grid), one warp's framebuffer.
+static int check_mads_limits(cov_handle *h, const char *who, bool grid)
+{
+    const int N = h->o.N;
+    int warps = 0, smem = 0, planes_smem = 0;
+    if (N > kMadsMaxUavs)
+        return fail(h, COV_ERR_LIMIT, std::string(who) + ": N = " + std::to_string(N) + " exceeds the " +
+                                          std::to_string(kMadsMaxUavs) + " UAVs of the solver's launch plan");
+    if (grid && !mads_plan(h->g, N, h->cfg, &warps, &smem, &planes_smem))
+        return fail(h, COV_ERR_LIMIT, std::string(who) + ": one warp's framebuffer of the " +
+                                          std::to_string(h->g.nx) + " x " + std::to_string(h->g.ny) +
+                                          " grid does not fit the " + std::to_string(h->cfg.max_smem_optin) +
+                                          " bytes of shared memory per CTA");
+    return COV_OK;
+}
+
 // S solves of the same loop on the device, one launch for all of them (cov_mads.cu).  The host contributes what
 // must carry its libm's bits: the initial mesh of every start and the table of powers of ten.  region: the objective
 // of cov_eval_region_batch instead of the cell store's.
@@ -1967,18 +1983,8 @@ static int mads_solve_batch(cov_handle *h, bool region, const double *X0, int64_
         return fail(h, COV_ERR_INVALID, std::string(who) + ": bad arguments");
     if (S == 0) return COV_OK;
     const int N = h->o.N, n = 3 * N;
-    int warps = 0, smem = 0, planes_smem = 0;
-    if (N > kMadsMaxUavs)
-        return fail(h, COV_ERR_LIMIT, std::string(who) + ": N = " + std::to_string(N) + " exceeds the " +
-                                          std::to_string(kMadsMaxUavs) + " UAVs of the solver's launch plan");
-    if (!region) {
-        if (!mads_plan(h->g, N, h->cfg, &warps, &smem, &planes_smem))
-            return fail(h, COV_ERR_LIMIT, std::string(who) + ": one warp's framebuffer of the " +
-                                              std::to_string(h->g.nx) + " x " + std::to_string(h->g.ny) +
-                                              " grid does not fit the " + std::to_string(h->cfg.max_smem_optin) +
-                                              " bytes of shared memory per CTA");
-        if (!h->area_exact) OK(entries_on_device(h)); // non-dyadic weights: the list-order sum
-    }
+    OK(check_mads_limits(h, who, !region));
+    if (!region && !h->area_exact) OK(entries_on_device(h)); // non-dyadic weights: the list-order sum
     // in: [pow10: 801 doubles | X0: S n doubles | a0: S n doubles | b0: S n ints]; out: [X_out | obj | stats]
     constexpr int kPow = 1 - 2 * kMadsPow10Min;
     const size_t sn = (size_t)S * n;
@@ -2033,6 +2039,161 @@ extern "C" int cov_mads_solve_batch(cov_handle *h, const double *X0, int64_t S, 
     DeviceGuard dg(h->device);
     OK(check_ready(h, "cov_mads_solve_batch"));
     return mads_solve_batch(h, false, X0, S, n_iter, granularity, seed, X_out, obj_out, stats);
+}
+
+// T timesteps of FullSimulation.py's MADS loop (lines 72-107) with S starts per timestep, all enqueued before the one
+// synchronise at the end.  Per timestep: rmvCoveredPOI of cur into the stats row, the bit planes repacked (the plane
+// set stays fixed: removals only clear multiplicities), the r_max rule / cons3's previous swarm / the starts
+// (horizon_start_kernel), S solves (launch_mads), the winner to cur (horizon_commit_kernel), AreaMaxObjective(cur).
+extern "C" int cov_run_horizon(cov_handle *h, const double *x_start, int64_t T, int64_t S, double spread,
+                               int64_t n_iter, double granularity, uint64_t seed, const double *boxes, int64_t n_boxes,
+                               double h_focus, double h_max, double *X_out, double *obj_out, int64_t *stats,
+                               double *step_ms)
+{
+    const char *who = "cov_run_horizon";
+    if (!h) return fail(nullptr, COV_ERR_INVALID, "NULL handle");
+    DeviceGuard dg(h->device);
+    OK(check_ready(h, who));
+    if (!h->o.use_cons3)
+        return fail(h, COV_ERR_STATE, "cov_run_horizon: the parameters have no previous swarm (cons3 is off)");
+    if (!h->area_exact)
+        return fail(h, COV_ERR_STATE, "cov_run_horizon: the store's area depends on the list order (area_exact == 0)");
+    if (T < 0 || S < 1 || n_iter < 0 || (T > 0 && (!x_start || !X_out)) || !std::isfinite(spread) || spread < 0 ||
+        !(granularity >= 0) || n_boxes < 0 || (n_boxes > 0 && !boxes))
+        return fail(h, COV_ERR_INVALID, "cov_run_horizon: bad arguments");
+    if (T == 0) return COV_OK;
+    OK(check_mads_limits(h, who, true));
+    const int N = h->o.N, n = 3 * N;
+    // in: [pow10: 801 doubles | x_start: n | boxes: 4 n_boxes | X0: S n | a0: S n | b0: S n ints]
+    // out: [solves' X: S n | obj: S | stats: S x 4 | X_out: T n | obj_out: T | stats: T x 4]
+    constexpr int kPow = 1 - 2 * kMadsPow10Min;
+    const size_t sn = (size_t)S * n, tn = (size_t)T * n;
+    const size_t o_x = (size_t)kPow * 8, o_box = o_x + (size_t)n * 8, o_X0 = o_box + (size_t)n_boxes * 32;
+    const size_t o_a = o_X0 + sn * 8, o_b = o_a + sn * 8, in_bytes = o_b + sn * 4;
+    const size_t o_obj = sn * 8, o_mst = o_obj + (size_t)S * 8, o_Xo = o_mst + (size_t)S * 32;
+    const size_t res_bytes = tn * 8 + (size_t)T * 8 + (size_t)T * 32, out_bytes = o_Xo + res_bytes;
+    std::vector<unsigned char> hin(o_X0);
+    double *p10 = (double *)hin.data();
+    for (int b = kMadsPow10Min; b <= -kMadsPow10Min; ++b) p10[b - kMadsPow10Min] = std::pow(10.0, b);
+    memcpy(hin.data() + o_x, x_start, (size_t)n * 8);
+    if (n_boxes) memcpy(hin.data() + o_box, boxes, (size_t)n_boxes * 32);
+    OK(ensure(h, h->mads_in, in_bytes));
+    OK(ensure(h, h->mads_out, out_bytes));
+    OK(ensure(h, h->xyT, (size_t)n * 8));
+    OK(ensure_pinned(h, &h->h_out, &h->h_out_cap, res_bytes));
+    unsigned char *din = (unsigned char *)h->mads_in.p, *dout = (unsigned char *)h->mads_out.p;
+    const double *d_x0 = (const double *)(din + o_x);
+    double *d_Xo = (double *)(dout + o_Xo), *d_oo = d_Xo + tn, *xyT = (double *)h->xyT.p;
+    long long *d_st = (long long *)(d_oo + T);
+    MadsArgs a{};
+    a.pow10 = (const double *)din;
+    a.X0 = (const double *)(din + o_X0);
+    a.a0 = (const double *)(din + o_a);
+    a.b0 = (const int *)(din + o_b);
+    a.X_out = (double *)dout;
+    a.obj_out = (double *)(dout + o_obj);
+    a.stats = (long long *)(dout + o_mst);
+    a.S = S;
+    a.n_iter = n_iter;
+    a.granularity = granularity;
+    a.force_exact = h->cfg.force_exact;
+    a.ordered = 0;
+    HorizonStep hs{};
+    hs.N = N;
+    hs.n_boxes = (int)n_boxes;
+    hs.S = S;
+    hs.spread = spread;
+    hs.granularity = granularity;
+    hs.seed = seed;
+    hs.pow10 = a.pow10;
+    hs.boxes = (const double *)(din + o_box);
+    hs.h_focus = h_focus;
+    hs.h_max = h_max;
+    hs.tan_half_fov = h->o.tan_half_fov;
+    LaunchCfg cfg = h->cfg; // a dyadic store: every kernel gives the list-order sum, the stale device list is not needed
+    cfg.ordered = 0;
+    if (cfg.kernel == COV_KERNEL_ORDERED) cfg.kernel = COV_KERNEL_AUTO;
+    unsigned char *mult = (unsigned char *)h->mult.p, *cls = (unsigned char *)h->cls.p;
+    std::vector<cudaEvent_t> ev;
+    if (step_ms)
+        for (int64_t t = 0; t <= T; ++t) ev.push_back(get_event(h));
+
+    cudaError_t e = cudaMemcpyAsync(din, hin.data(), o_X0, cudaMemcpyHostToDevice, h->stream);
+    const char *what = "upload";
+    if (e == cudaSuccess) e = launch_thresholds(d_x0, N, xyT, h->stream), what = "launch_thresholds";
+    h->launches += 1;
+    int rc = COV_OK;
+    for (int64_t t = 1; t <= T && e == cudaSuccess && rc == COV_OK; ++t) {
+        const double *cur = t == 1 ? d_x0 : d_Xo + (size_t)(t - 2) * n;
+        double *next = d_Xo + (size_t)(t - 1) * n;
+        long long *row = d_st + 4 * (t - 1);
+        if (step_ms && (e = cudaEventRecord(ev[(size_t)t - 1], h->stream)) != cudaSuccess) break;
+        what = "rmvCoveredPOI";
+        if ((e = launch_remove_covered(mult, cls, h->g, xyT, N, (unsigned long long *)(row + 3), h->stream)) != cudaSuccess) break;
+        what = "repack";
+        if ((e = launch_pack_planes(mult, cls, h->g, (uint32_t *)h->planes.p, h->stream)) != cudaSuccess) break;
+        if (h->g.planes_q && (e = launch_requad_plane(h->g, (uint32_t *)h->planes_q.p, h->stream)) != cudaSuccess) break;
+        hs.t = t;
+        what = "horizon_start";
+        if ((e = launch_horizon_start(hs, cur, (double *)h->params.p, (double *)(din + o_X0), (double *)(din + o_a),
+                                      (int *)(din + o_b), h->stream)) != cudaSuccess)
+            break;
+        a.seed = seed + (uint64_t)(t - 1) * (uint64_t)S;
+        unsigned long long *counter = nullptr;
+        if ((rc = take_counter(h, &counter)) != COV_OK) break;
+        what = "MADS kernel";
+        if ((e = launch_mads(h->g, h->o, cfg, a, counter, h->stream)) != cudaSuccess) break;
+        what = "horizon_commit";
+        if ((e = launch_horizon_commit(S, N, a.X_out, a.obj_out, a.stats, next, row, xyT, h->stream)) != cudaSuccess) break;
+        if ((rc = take_counter(h, &counter)) != COV_OK) break;
+        EvalOut out{};
+        out.obj = d_oo + (t - 1);
+        LaunchInfo li{};
+        what = "coverage kernel";
+        if ((e = launch_eval(h->g, h->o, cfg, next, 1, out, counter, h->stream, &li)) != cudaSuccess) break;
+        h->launches += h->g.planes_q ? 7 : 6;
+    }
+    if (e == cudaSuccess && rc == COV_OK && step_ms) e = cudaEventRecord(ev[(size_t)T], h->stream), what = "event";
+    if (e == cudaSuccess && rc == COV_OK)
+        e = cudaMemcpyAsync(h->h_out, d_Xo, res_bytes, cudaMemcpyDeviceToHost, h->stream), what = "download";
+    if (e != cudaSuccess || rc != COV_OK) { // the removals enqueued so far stand: refresh what the host knows of them
+        if (rc == COV_OK) rc = fail_cuda(h, e, (std::string(who) + ": " + what).c_str());
+        const std::string msg = h->err;
+        h->ent_removed_pending = h->ent_known;
+        h->ent_dev_valid = false;
+        double cw[kMaxClasses];
+        for (int k = 0; k < kMaxClasses; ++k) cw[k] = h->g.class_weight[k];
+        if (rebuild_planes(h, h->g.n_classes, cw) != COV_OK) h->have_grid = false;
+        for (cudaEvent_t x : ev) h->ev_pool.push_back(x);
+        h->err = msg;
+        return rc;
+    }
+    double cw[kMaxClasses];
+    for (int k = 0; k < kMaxClasses; ++k) cw[k] = h->g.class_weight[k];
+    rc = rebuild_planes(h, h->g.n_classes, cw); // the one synchronise
+    const double *hX = (const double *)h->h_out, *hobj = hX + tn;
+    const int64_t *hst = (const int64_t *)(hobj + T);
+    if (rc == COV_OK) {
+        bool removed = false;
+        for (int64_t t = 0; t < T; ++t) removed |= hst[4 * t + 3] != 0;
+        if (removed) {
+            h->ent_removed_pending = h->ent_known;
+            h->ent_dev_valid = false;
+        }
+        memcpy(X_out, hX, tn * 8);
+        if (obj_out) memcpy(obj_out, hobj, (size_t)T * 8);
+        if (stats) memcpy(stats, hst, (size_t)T * 32);
+        for (int64_t t = 0; step_ms && t < T; ++t) {
+            float ms = 0;
+            if ((e = cudaEventElapsedTime(&ms, ev[(size_t)t], ev[(size_t)t + 1])) != cudaSuccess) {
+                rc = fail_cuda(h, e, "cov_run_horizon: cudaEventElapsedTime");
+                break;
+            }
+            step_ms[t] = ms;
+        }
+    }
+    for (cudaEvent_t x : ev) h->ev_pool.push_back(x);
+    return rc;
 }
 
 extern "C" int cov_argmin(cov_handle *h, const double *X, int64_t B, int32_t barrier, double *best_obj,

@@ -70,6 +70,24 @@ bool mads_plan(const GridDesc &g, int N, const LaunchCfg &cfg, int *warps, int *
 cudaError_t launch_mads(const GridDesc &g, const ObjParams &o, const LaunchCfg &cfg, const MadsArgs &a,
                         unsigned long long *counter, cudaStream_t stream);
 
+// ---- cov_run_horizon (cov_horizon.cu): the kernels between the launchers above, per timestep t (1-based) ----
+struct HorizonStep {
+    int N, n_boxes;
+    long long t, S;
+    double spread, granularity;
+    unsigned long long seed;  // Philox key of the starts' perturbations
+    const double *pow10;      // the solver's table (MadsArgs::pow10)
+    const double *boxes;      // n_boxes x 4: x_LB, x_UB, y_LB, y_UB (device)
+    double h_focus, h_max, tan_half_fov;
+};
+// The r_max rule (t >= 2, n_boxes > 0) and cons3's previous swarm := cur into params (cov_handle's 5N doubles:
+// r_max, prev_x, prev_y, prev_z, cons3_G), and S starts with their initial meshes (start 0 = cur).
+cudaError_t launch_horizon_start(const HorizonStep &s, const double *cur, double *params, double *X0, double *a0,
+                                 int *b0, cudaStream_t stream);
+// One CTA: the winner of S solves (Xs S x 3N, objs S, mstats S x 4) to cur, stats_row[0..2], and xyT of cur.
+cudaError_t launch_horizon_commit(long long S, int N, const double *Xs, const double *objs, const long long *mstats,
+                                  double *cur, long long *stats_row, double *xyT, cudaStream_t stream);
+
 // ---- the grid-free static objective (cov_region.cu, cov_mads.cu; geometry and limits in cov_region.cuh) ----
 // The arcs of the covered set's boundary inside the domain (r.arcs / r.K unused): at most cap of them to out, the
 // count of all of them to *count (device).

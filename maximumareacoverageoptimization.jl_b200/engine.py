@@ -343,6 +343,32 @@ class CoverageEngine:
         names = ("iterations", "evaluations", "successes", "converged")
         return X, obj, {name: st[:, q].copy() for q, name in enumerate(names)}
 
+    def run_horizon(self, x_start, T: int, S: int = 1, spread: float = 3.0, n_iter: int = 100,
+                    granularity: float = 1.0, seed: int = 0, boxes=None, h_focus: float = 15.0,
+                    h_max: float = 30.0):
+        """T timesteps of FullSimulation's MADS loop on the device in one call (cov_run_horizon): per timestep
+        rmvCoveredPOI of the current swarm, the r_max rule near the boxes (K x 4 rows x_LB, x_UB, y_LB, y_UB; None:
+        off), cons3 from the current swarm, S solves from the swarm and S - 1 perturbations of it, the best one as
+        the next swarm.  Needs set_params with prev_xyR.  Returns (X (T, 3N), obj (T,), stats, step_ms (T,)) with
+        stats a dict of int64 arrays: winner, evaluations, feasible, removed.  The r_max and previous swarm of the
+        last timestep stay set on the engine."""
+        x_start = _f64(x_start).ravel()
+        if self.N is None or x_start.size != 3 * self.N:
+            raise ValueError("x_start must have 3N entries")
+        B = np.zeros((0, 4)) if boxes is None else _f64(boxes).reshape(-1, 4)
+        T = int(T)
+        X = np.empty((max(T, 0), 3 * self.N))
+        obj = np.empty(max(T, 0))
+        st = np.empty((max(T, 0), 4), dtype=np.int64)
+        ms = np.empty(max(T, 0))
+        self.param_owner = None  # r_max and the previous swarm change on the device
+        self._check(lib.cov_run_horizon(self._h, _ptr(x_start), T, int(S), float(spread), int(n_iter),
+                                        float(granularity), int(seed) & (2**64 - 1), _ptr(B) if len(B) else None,
+                                        len(B), float(h_focus), float(h_max), _ptr(X), _ptr(obj), _ptr(st),
+                                        _ptr(ms)))
+        names = ("winner", "evaluations", "feasible", "removed")
+        return X, obj, {name: st[:, q].copy() for q, name in enumerate(names)}, ms
+
     # ---- grid-free static objective ----
     def set_region(self, x_lo: float, y_lo: float, x_hi: float, y_hi: float, covered=None):
         """The domain rectangle and the discs already covered (cov_set_region): covered is M x 3 rows (x, y, R), or

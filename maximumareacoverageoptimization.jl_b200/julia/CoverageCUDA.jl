@@ -286,6 +286,28 @@ function mads_solve_batch(h::Handle, X0::Matrix{Float64}; N_iter = 100, granular
 end
 
 """
+    run_horizon(h, x_start; T, S = 1, spread = 3.0, N_iter = 100, granularity = 1.0, seed = 0,
+                boxes = zeros(Float64, 4, 0), h_focus = 15.0, h_max = 30.0)
+
+T timesteps of FullSimulation's MADS loop on the device in one call (`cov_run_horizon`): per timestep
+rmvCoveredPOI of the current swarm, the r_max rule near the boxes (columns [x_LB; x_UB; y_LB; y_UB]), cons3 from the
+current swarm, S solves (from the swarm and S - 1 perturbations of it) and the best as the next swarm. Needs
+`set_params!` with a previous swarm. Returns `(X, objectives, stats, step_ms)`: `X` 3N x T, `stats` 4 x T with rows
+winner, evaluations, feasible solves, entries removed; `step_ms` the device time of every timestep.
+"""
+function run_horizon(h::Handle, x_start::Vector{Float64}; T, S = 1, spread = 3.0, N_iter = 100, granularity = 1.0,
+                     seed = 0, boxes::Matrix{Float64} = zeros(Float64, 4, 0), h_focus = 15.0, h_max = 30.0)
+    n = length(x_start); K = size(boxes, 2)
+    X = zeros(Float64, n, T); obj = zeros(Float64, T); stats = zeros(Int64, 4, T); ms = zeros(Float64, T)
+    GC.@preserve x_start boxes X obj stats ms check(h, ccall((:cov_run_horizon, LIB), Cint,
+        (Ptr{Cvoid}, Ptr{Float64}, Int64, Int64, Float64, Int64, Float64, UInt64, Ptr{Float64}, Int64, Float64,
+         Float64, Ptr{Float64}, Ptr{Float64}, Ptr{Int64}, Ptr{Float64}),
+        h.ptr, x_start, T, S, spread, N_iter, granularity, seed, K == 0 ? C_NULL : pointer(boxes), K, h_focus, h_max,
+        X, obj, stats, ms))
+    return X, obj, stats, ms
+end
+
+"""
     set_region!(h, x_lo, y_lo, x_hi, y_hi, covered)
 
 The grid-free static objective's region: the domain rectangle and the discs already covered, `covered` a 3 x M
