@@ -134,6 +134,19 @@ struct DevBuf {
     size_t cap = 0;
 };
 
+// Pinned host scratch for the few words a call brings back or sends (one field per use, allocated once per handle).
+struct HostScratch {
+    unsigned long long stats[2 + kMaxClasses]; // rebuild_planes: entries, cells, per-class OR of the multiplicities
+    int overflow;                              // upload_points, cov_fire_step
+    unsigned long long removed;                // cov_remove_covered, cov_fire_step: entries removed / pushed
+    double fire_p[9];                          // cov_fire_step: direction probabilities
+    double win_obj;                            // the poll winner of one device window (enqueue_winner)
+    long long win_idx;
+    int region_arcs;                           // cov_set_region
+};
+// h_poll, the pinned scratch of the small-batch path: candidates at 0 (<= 256 KiB), results from kPollOut on
+constexpr size_t kPollBytes = 2u << 20, kPollOut = 512u << 10;
+
 struct cov_handle {
     int device = 0;
     cudaStream_t own_stream = nullptr, stream = nullptr; // stream = own_stream or an adopted one
@@ -184,8 +197,9 @@ struct cov_handle {
     size_t h_in_cap = 0;
     void *h_out = nullptr;
     size_t h_out_cap = 0;
-    void *h_small = nullptr; // pinned scratch: 4 KiB of scalars, then one candidate
-    void *h_poll = nullptr;  // pinned scratch of the small-batch path
+    HostScratch *h_small = nullptr;
+    void *h_poll = nullptr; // pinned scratch of the small-batch path (kPollBytes)
+    size_t h_poll_cap = 0;
 
     std::vector<cudaEvent_t> ev_pool; // recycled
     // (start, stop) events around every coverage-kernel launch since the last drain
@@ -403,7 +417,7 @@ extern "C" int cov_create(int device, cov_handle **out)
     nh->cfg.plane_mode = -1;
     nh->cfg.num_sms = prop.multiProcessorCount;
     nh->cfg.max_smem_optin = (int)prop.sharedMemPerBlockOptin;
-    if ((e = cudaMallocHost(&nh->h_small, 4096 + 3 * kMaxUavs * 8)) != cudaSuccess) return bail(e, "cudaMallocHost");
+    if ((e = cudaMallocHost(&nh->h_small, sizeof(HostScratch))) != cudaSuccess) return bail(e, "cudaMallocHost");
     int rc = ensure(nh, nh->counter, kCounterSlots * sizeof(unsigned long long));
     if (rc == COV_OK && cudaMemset(nh->counter.p, 0, kCounterSlots * sizeof(unsigned long long)) != cudaSuccess)
         rc = fail_cuda(nh, cudaGetLastError(), "cudaMemset");
@@ -585,7 +599,8 @@ static void odd_decompose(double v, uint64_t &m, int &e)
     }
 }
 
-// Derive the bit planes from the device-resident mult/cls bytes and refresh the statistics.
+// Derive the bit planes from the device-resident mult/cls bytes and refresh the statistics.  class_weight may be
+// g.class_weight itself: each weight is read only by its own assignment below.
 static int rebuild_planes(cov_handle *h, int n_classes, const double *class_weight)
 {
     GridDesc &g = h->g;
@@ -594,7 +609,7 @@ static int rebuild_planes(cov_handle *h, int n_classes, const double *class_weig
     CK(launch_grid_stats((const unsigned char *)h->mult.p, (const unsigned char *)h->cls.p, ncell, d_stats,
                          h->stream));
     h->launches += 1;
-    unsigned long long *hs = (unsigned long long *)h->h_small;
+    unsigned long long *hs = h->h_small->stats;
     CK(cudaMemcpyAsync(hs, d_stats, (2 + kMaxClasses) * sizeof(unsigned long long), cudaMemcpyDeviceToHost,
                        h->stream));
     CK(cudaStreamSynchronize(h->stream));
@@ -674,14 +689,6 @@ static int rebuild_planes(cov_handle *h, int n_classes, const double *class_weig
     return COV_OK;
 }
 
-static int alloc_cells(cov_handle *h)
-{
-    const size_t ncell = (size_t)h->g.nx * h->g.ny;
-    OK(ensure(h, h->mult, ncell + 4)); // add_points works on aligned 4-byte words
-    OK(ensure(h, h->cls, ncell + 4));
-    return COV_OK;
-}
-
 // ---- the ordered point list ------------------------------------------------------------------------------
 static void entries_forget(cov_handle *h) // the store was re-created without a list: order = createPOI's, on demand
 {
@@ -693,6 +700,22 @@ static void entries_forget(cov_handle *h) // the store was re-created without a 
     h->g.ent_cell = nullptr;
     h->g.ent_cls = nullptr;
     h->g.n_ent = 0;
+}
+// A setter re-creates the store (arguments checked): the automaton's state and the point list go with the old one.
+static int reset_store(cov_handle *h, int64_t nx, int64_t ny, double dx, double dy)
+{
+    h->have_grid = false;
+    h->have_fire = false;
+    entries_forget(h);
+    describe_lattice(h, nx, ny, dx, dy);
+    OK(ensure(h, h->mult, (size_t)nx * ny + 4)); // add_points works on aligned 4-byte words
+    return ensure(h, h->cls, (size_t)nx * ny + 4);
+}
+// Covered cells lost their entries: a known list drops them lazily (entries_apply_removals), the device list is stale.
+static void entries_note_removals(cov_handle *h)
+{
+    h->ent_removed_pending = h->ent_known;
+    h->ent_dev_valid = false;
 }
 // rmvCoveredPOI deletes every entry of a covered cell and keeps the order of the rest
 // (src/CellFunctions.jl:81-108): drop the mirror's entries whose cell is now empty.
@@ -798,11 +821,7 @@ extern "C" int cov_set_grid_bits(cov_handle *h, int64_t nx, int64_t ny, double d
     DeviceGuard dg(h->device);
     if (!bits) return fail(h, COV_ERR_INVALID, "cov_set_grid_bits: bits is NULL");
     OK(check_lattice(h, nx, ny, dx, dy));
-    h->have_grid = false;
-    h->have_fire = false; // the automaton's state belongs to the lattice it was initialised on
-    entries_forget(h);
-    describe_lattice(h, nx, ny, dx, dy);
-    OK(alloc_cells(h));
+    OK(reset_store(h, nx, ny, dx, dy));
     const size_t words = (size_t)ny * ((nx + 31) / 32);
     DevBuf tmp;
     OK(ensure(h, tmp, words * 4));
@@ -831,11 +850,7 @@ extern "C" int cov_set_grid_cells(cov_handle *h, int64_t nx, int64_t ny, double 
     if (cls)
         for (size_t t = 0; t < ncell; ++t)
             if (cls[t] >= n_classes) return fail(h, COV_ERR_INVALID, "cov_set_grid_cells: class index out of range");
-    h->have_grid = false;
-    h->have_fire = false; // the automaton's state belongs to the lattice it was initialised on
-    entries_forget(h);
-    describe_lattice(h, nx, ny, dx, dy);
-    OK(alloc_cells(h));
+    OK(reset_store(h, nx, ny, dx, dy));
     CK(cudaMemcpyAsync(h->mult.p, mult, ncell, cudaMemcpyHostToDevice, h->stream));
     if (cls) CK(cudaMemcpyAsync(h->cls.p, cls, ncell, cudaMemcpyHostToDevice, h->stream));
     else CK(cudaMemsetAsync(h->cls.p, 0, ncell, h->stream));
@@ -850,11 +865,7 @@ extern "C" int cov_set_grid_full(cov_handle *h, int64_t nx, int64_t ny, double d
     if (!h) return fail(nullptr, COV_ERR_INVALID, "NULL handle");
     DeviceGuard dg(h->device);
     OK(check_lattice(h, nx, ny, dx, dy));
-    h->have_grid = false;
-    h->have_fire = false; // the automaton's state belongs to the lattice it was initialised on
-    entries_forget(h);
-    describe_lattice(h, nx, ny, dx, dy);
-    OK(alloc_cells(h));
+    OK(reset_store(h, nx, ny, dx, dy));
     CK(launch_fill_full((unsigned char *)h->mult.p, (unsigned char *)h->cls.p, (long long)nx * ny, h->stream));
     h->launches += 1;
     const double w = dx * dy; // createPOI: area = weight = dx*dy
@@ -910,7 +921,7 @@ static int upload_points(cov_handle *h, const std::vector<int> &cell, const std:
     int rc = ensure(h, dcell, P * sizeof(int));
     if (rc == COV_OK) rc = ensure(h, dcls, P);
     cudaError_t e = cudaSuccess;
-    int *hov = (int *)h->h_small;
+    int *hov = &h->h_small->overflow;
     if (rc == COV_OK) {
         e = cudaMemcpyAsync(dcell.p, cell.data(), P * sizeof(int), cudaMemcpyHostToDevice, h->stream);
         if (e == cudaSuccess) e = cudaMemcpyAsync(dcls.p, pcls.data(), P, cudaMemcpyHostToDevice, h->stream);
@@ -939,10 +950,7 @@ extern "C" int cov_set_points(cov_handle *h, const double *pts5, int64_t P, int6
     DeviceGuard dg(h->device);
     if (P < 0 || (P > 0 && !pts5)) return fail(h, COV_ERR_INVALID, "cov_set_points: bad list");
     OK(check_lattice(h, nx, ny, dx, dy));
-    h->have_grid = false;
-    h->have_fire = false; // the automaton's state belongs to the lattice it was initialised on
-    entries_forget(h);
-    describe_lattice(h, nx, ny, dx, dy);
+    OK(reset_store(h, nx, ny, dx, dy));
     std::vector<int> cell;
     std::vector<unsigned char> pcls;
     int n_classes = 0;
@@ -952,7 +960,6 @@ extern "C" int cov_set_points(cov_handle *h, const double *pts5, int64_t P, int6
         n_classes = 1;
         cw[0] = dx * dy;
     }
-    OK(alloc_cells(h));
     const size_t ncell = (size_t)nx * ny;
     CK(cudaMemsetAsync(h->mult.p, 0, ncell + 4, h->stream));
     CK(cudaMemsetAsync(h->cls.p, 0xff, ncell + 4, h->stream));
@@ -1074,17 +1081,12 @@ extern "C" int cov_remove_covered(cov_handle *h, const double *xyR, int64_t N, i
     CK(launch_remove_covered((unsigned char *)h->mult.p, (unsigned char *)h->cls.p, h->g, (const double *)h->xyT.p, (int)N,
                              (unsigned long long *)h->removed.p, h->stream));
     h->launches += 1;
-    unsigned long long *hr = (unsigned long long *)h->h_small + 16;
+    unsigned long long *hr = &h->h_small->removed;
     CK(cudaMemcpyAsync(hr, h->removed.p, sizeof(unsigned long long), cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
     if (removed) *removed = (int64_t)*hr;
-    if (*hr) {
-        h->ent_removed_pending = h->ent_known;
-        h->ent_dev_valid = false;
-    }
-    double cw[kMaxClasses];
-    for (int k = 0; k < kMaxClasses; ++k) cw[k] = h->g.class_weight[k];
-    return rebuild_planes(h, h->g.n_classes, cw);
+    if (*hr) entries_note_removals(h);
+    return rebuild_planes(h, h->g.n_classes, h->g.class_weight);
 }
 
 extern "C" int cov_covered_mask(cov_handle *h, const double *x, uint8_t *mask)
@@ -1120,11 +1122,7 @@ extern "C" int cov_fire_init(cov_handle *h, int64_t nx, int64_t ny, double dx, d
     const size_t ncell = (size_t)nx * ny;
     for (size_t t = 0; t < ncell; ++t)
         if (state[t] > 2) return fail(h, COV_ERR_INVALID, "cov_fire_init: cell states must be 0 (empty), 1 (tree), 2 (fire)");
-    h->have_grid = false;
-    h->have_fire = false;
-    entries_forget(h);
-    describe_lattice(h, nx, ny, dx, dy);
-    OK(alloc_cells(h));
+    OK(reset_store(h, nx, ny, dx, dy));
     OK(ensure(h, h->fire[0], ncell));
     OK(ensure(h, h->fire[1], ncell));
     OK(ensure(h, h->fire_p, 9 * sizeof(double)));
@@ -1153,7 +1151,7 @@ extern "C" int cov_fire_step(cov_handle *h, double wind_speed, double wind_direc
                                       "automaton pushes");
     // the probability of ignition from the neighbour at window index (a, b), a, b = 1..3, exactly as the
     // reference forms it: wind_speed * cos(wind_direction - atan(2-b, 2-a)) * prob_spread
-    double *hp = (double *)h->h_small + 64;
+    double *hp = h->h_small->fire_p;
     for (int b = 1; b <= 3; ++b)
         for (int a = 1; a <= 3; ++a) {
             volatile double ang = atan2((double)(2 - b), (double)(2 - a));
@@ -1171,8 +1169,8 @@ extern "C" int cov_fire_step(cov_handle *h, double wind_speed, double wind_direc
                         (unsigned int)step, (const double *)h->fire_p.p, append, (unsigned long long *)h->removed.p,
                         (int *)h->overflow.p, h->stream));
     h->launches += 1;
-    unsigned long long *hr = (unsigned long long *)h->h_small + 16;
-    int *hov = (int *)h->h_small;
+    unsigned long long *hr = &h->h_small->removed;
+    int *hov = &h->h_small->overflow;
     CK(cudaMemcpyAsync(hr, h->removed.p, sizeof(unsigned long long), cudaMemcpyDeviceToHost, h->stream));
     CK(cudaMemcpyAsync(hov, h->overflow.p, sizeof(int), cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
@@ -1187,9 +1185,7 @@ extern "C" int cov_fire_step(cov_handle *h, double wind_speed, double wind_direc
     // The automaton pushes in cell order; from here on the list order is createPOI's.  The store has one weight
     // class, so every covered entry adds the same weight and the list-order sum is the same in any order.
     entries_forget(h);
-    double cw[kMaxClasses];
-    for (int k = 0; k < kMaxClasses; ++k) cw[k] = h->g.class_weight[k];
-    return rebuild_planes(h, 1, cw);
+    return rebuild_planes(h, 1, h->g.class_weight);
 }
 
 extern "C" int cov_fire_get_state(cov_handle *h, uint8_t *state)
@@ -1265,29 +1261,29 @@ static int take_counter(cov_handle *h, unsigned long long **counter)
     return COV_OK;
 }
 
-static int launch_on_main(cov_handle *h, const double *dX, int64_t B, const EvalOut &out, bool timed)
+// One kernel launch on the main stream; timed: inside a (start, stop) event pair for cov_last_kernel_ms, with the
+// counter slot (when asked for) taken inside it.  cudaErrorInvalidConfiguration is COV_ERR_LIMIT with limit_msg.
+template <class Launch>
+static int timed_launch(cov_handle *h, bool timed, unsigned long long **counter, const char *what, const char *limit_msg,
+                        Launch &&launch)
 {
-    h->cfg.ordered = h->area_exact ? 0 : 1; // non-dyadic weights: the sum is replayed in list order
-    if (h->cfg.ordered || h->cfg.kernel == COV_KERNEL_ORDERED) OK(entries_on_device(h));
     cudaEvent_t e0 = nullptr, e1 = nullptr;
     if (timed) {
         e0 = get_event(h);
         e1 = get_event(h);
         CK(cudaEventRecord(e0, h->stream));
     }
-    unsigned long long *counter = nullptr;
-    OK(take_counter(h, &counter));
-    cudaError_t e = launch_eval(h->g, h->o, h->cfg, dX, (long long)B, out, counter, h->stream, &h->last_info);
-    if (e != cudaSuccess) {
+    const int rc = counter ? take_counter(h, counter) : COV_OK;
+    const cudaError_t e = rc == COV_OK ? launch() : cudaSuccess;
+    if (rc != COV_OK || e != cudaSuccess) {
         if (timed) {
             h->ev_pool.push_back(e0);
             h->ev_pool.push_back(e1);
         }
-        if (e == cudaErrorInvalidConfiguration) {
-            (void)cudaGetLastError();
-            return fail(h, COV_ERR_LIMIT, "grid row / N too large for the shared-memory plan of this kernel");
-        }
-        return fail_cuda(h, e, "coverage kernel launch");
+        if (rc != COV_OK) return rc;
+        if (e != cudaErrorInvalidConfiguration) return fail_cuda(h, e, what);
+        (void)cudaGetLastError();
+        return fail(h, COV_ERR_LIMIT, limit_msg);
     }
     h->launches += 1;
     if (timed) {
@@ -1297,10 +1293,52 @@ static int launch_on_main(cov_handle *h, const double *dX, int64_t B, const Eval
     return COV_OK;
 }
 
+static int launch_on_main(cov_handle *h, const double *dX, int64_t B, const EvalOut &out, bool timed)
+{
+    h->cfg.ordered = h->area_exact ? 0 : 1; // non-dyadic weights: the sum is replayed in list order
+    if (h->cfg.ordered || h->cfg.kernel == COV_KERNEL_ORDERED) OK(entries_on_device(h));
+    unsigned long long *counter = nullptr;
+    return timed_launch(h, timed, &counter, "coverage kernel launch",
+                        "grid row / N too large for the shared-memory plan of this kernel", [&] {
+                            return launch_eval(h->g, h->o, h->cfg, dX, (long long)B, out, counter, h->stream, &h->last_info);
+                        });
+}
+
 static int check_ready(cov_handle *h, const char *who)
 {
     if (!h->have_grid) return fail(h, COV_ERR_STATE, std::string(who) + ": no grid set");
     if (!h->have_params) return fail(h, COV_ERR_STATE, std::string(who) + ": no parameters set");
+    return COV_OK;
+}
+
+// Candidates per device window: as many as fit cap_bytes, at least one.
+static int64_t window_rows(int64_t B, size_t row_bytes, size_t cap_bytes)
+{
+    return std::max<int64_t>(1, std::min<int64_t>(std::max<int64_t>(B, 1), (int64_t)(cap_bytes / row_bytes)));
+}
+
+// The poll winner: the lowest objective, a tie to the earlier index; no winner is (INFINITY, -1).  offer: candidate i
+// (< 0: none) of a window or shard that starts at candidate base.
+struct Winner {
+    double obj = INFINITY;
+    int64_t idx = -1;
+    void offer(double o, int64_t i, int64_t base = 0)
+    {
+        if (i >= 0 && (idx < 0 || o < obj)) {
+            obj = o;
+            idx = base + i;
+        }
+    }
+};
+// Enqueue the winner of one device window (objectives, feasibility flags, wn candidates) and its 16 bytes' way home;
+// once the main stream is synchronised, offer h_small->win_obj / win_idx.
+static int enqueue_winner(cov_handle *h, const double *d_obj, const unsigned char *d_feas, int64_t wn, int barrier)
+{
+    CK(launch_argmin(d_obj, d_feas, wn, barrier, (double *)h->argmin_obj.p, (long long *)h->argmin_idx.p, 1024,
+                     h->stream));
+    h->launches += 2;
+    CK(cudaMemcpyAsync(&h->h_small->win_obj, h->argmin_obj.p, 8, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaMemcpyAsync(&h->h_small->win_idx, h->argmin_idx.p, 8, cudaMemcpyDeviceToHost, h->stream));
     return COV_OK;
 }
 
@@ -1342,6 +1380,53 @@ static void host_copy(cov_handle *h, void *dst, const void *src, size_t bytes)
     }
 }
 
+// The per-candidate results of a host-path call, in the order of every packed layout: the 8-byte columns before the
+// 1-byte feasibility flags, which keeps each column of a packed block 8-byte aligned.
+enum { COL_OBJ, COL_COUNT, COL_CLS, COL_PROG, COL_FEAS, kCols };
+struct Col {
+    char *host;           // the caller's buffer; null: not requested
+    size_t row;           // bytes per candidate
+    DevBuf *dev;          // the column of the device window
+    bool pinned = false;  // host is null or pinned: written in place, not staged
+    size_t at = 0;        // offset in a packed layout (the small path's scratch, the staging block)
+};
+using Cols = Col[kCols];
+
+// Lays the requested columns that are not pinned one after the other, n candidates each; returns the bytes.
+static size_t pack_cols(Cols &c, size_t n)
+{
+    size_t bytes = 0;
+    for (Col &col : c)
+        if (col.host && !col.pinned) {
+            col.at = bytes;
+            bytes += n * col.row;
+        }
+    return bytes;
+}
+static EvalOut eval_out(char *const at[kCols])
+{
+    EvalOut out{};
+    out.obj = (double *)at[COL_OBJ];
+    out.count = (long long *)at[COL_COUNT];
+    out.class_count = (long long *)at[COL_CLS];
+    out.progressive = (double *)at[COL_PROG];
+    out.feasible = (unsigned char *)at[COL_FEAS];
+    return out;
+}
+// Device views of the host homes (pinned buffer, or staging block so) of the requested columns of the slice from
+// candidate g0 (c0 in its window); false when the device cannot address one.
+static bool view_cols(const Cols &c, char *so, int64_t g0, int64_t c0, char *at[kCols])
+{
+    for (int k = 0; k < kCols; ++k) {
+        at[k] = nullptr;
+        if (!c[k].host) continue;
+        char *v = (char *)device_view(c[k].pinned ? c[k].host : so + c[k].at);
+        if (!v) return false;
+        at[k] = v + (size_t)(c[k].pinned ? g0 : c0) * c[k].row;
+    }
+    return true;
+}
+
 // Small batches (a MADS poll set): one stream, pinned scratch, one synchronisation.
 #ifndef COV_ZC_IN_LIMIT
 #define COV_ZC_IN_LIMIT (256u << 10) // the whole small-batch path; measured against 32 KiB: 512 candidates 53 -> 42 us, 2184 candidates 74 -> 62 us
@@ -1352,79 +1437,34 @@ static void host_copy(cov_handle *h, void *dst, const void *src, size_t bytes)
 // ~49 GB/s over PCIe, the DMA engine 55 GB/s), behind it at 1 M
 #define COV_ZC_MID_LIMIT (48u << 20)
 #endif
-static int eval_host_small(cov_handle *h, const double *X, int64_t B, double *obj, int64_t *count, uint8_t *feasible,
-                           int64_t *class_count, double *progressive)
+static int eval_host_small(cov_handle *h, const double *X, int64_t B, Cols &c, bool timed = true)
 {
-    const int N = h->o.N;
-    const int ncls = h->g.n_classes;
-    const size_t in_bytes = (size_t)B * 3 * N * 8;
-    const size_t o_obj = 0, o_cnt = o_obj + (size_t)B * 8, o_cls = o_cnt + (count ? (size_t)B * 8 : 0),
-                 o_prg = o_cls + (class_count ? (size_t)B * 8 * ncls : 0), o_fea = o_prg + (progressive ? (size_t)B * 8 : 0),
-                 out_bytes = o_fea + (feasible ? (size_t)B : 0);
-    if (!h->h_poll) { // 2 MiB of pinned scratch: candidates at 0 (<= 256 KiB), results from 512 KiB on
-        cudaError_t e = cudaMallocHost(&h->h_poll, 2u << 20);
-        if (e != cudaSuccess) {
-            (void)cudaGetLastError();
-            h->h_poll = nullptr;
-            return fail(h, COV_ERR_NOMEM, std::string("cudaMallocHost: ") + cudaGetErrorString(e));
-        }
-    }
-    char *hin = (char *)h->h_poll, *hout = (char *)h->h_poll + (512u << 10);
+    const size_t in_bytes = (size_t)B * 3 * h->o.N * 8;
+    const size_t out_bytes = pack_cols(c, (size_t)B);
+    OK(ensure_pinned(h, &h->h_poll, &h->h_poll_cap, kPollBytes));
+    char *hin = (char *)h->h_poll, *hout = (char *)h->h_poll + kPollOut;
     memcpy(hin, X, in_bytes);
     // poll-sized calls (a MADS poll set, the scalar closure): no copy engines at all -- the kernel reads the
     // candidates from the pinned scratch and writes the results into it over PCIe; the stream synchronise is
     // the only wait.  Saves two DMA set-ups per call, which is most of what a poll costs.
-    char *vin = nullptr, *vout = nullptr;
-    if (h->zero_copy_out && in_bytes <= (COV_ZC_IN_LIMIT)) {
-        vin = (char *)device_view(hin);
-        vout = (char *)device_view(hout);
+    char *vin = h->zero_copy_out && in_bytes <= (COV_ZC_IN_LIMIT) ? (char *)device_view(hin) : nullptr;
+    char *vout = vin ? (char *)device_view(hout) : nullptr;
+    const bool zc = vin && vout;
+    if (!zc) {
+        OK(ensure(h, h->dX, std::max<size_t>(in_bytes, 1 << 20)));
+        OK(ensure(h, h->d_obj, std::max<size_t>(out_bytes, 1 << 20))); // one device block for every output
+        CK(cudaMemcpyAsync(h->dX.p, hin, in_bytes, cudaMemcpyHostToDevice, h->stream));
     }
-    if (vin && vout) {
-        EvalOut out{};
-        out.obj = (double *)(vout + o_obj);
-        out.count = count ? (long long *)(vout + o_cnt) : nullptr;
-        out.class_count = class_count ? (long long *)(vout + o_cls) : nullptr;
-        out.progressive = progressive ? (double *)(vout + o_prg) : nullptr;
-        out.feasible = feasible ? (unsigned char *)(vout + o_fea) : nullptr;
-        OK(launch_on_main(h, (const double *)vin, B, out, true));
-        CK(cudaStreamSynchronize(h->stream));
-        const char *so = hout;
-        memcpy(obj, so + o_obj, (size_t)B * 8);
-        if (count) memcpy(count, so + o_cnt, (size_t)B * 8);
-        if (class_count) memcpy(class_count, so + o_cls, (size_t)B * 8 * ncls);
-        if (progressive) memcpy(progressive, so + o_prg, (size_t)B * 8);
-        if (feasible) memcpy(feasible, so + o_fea, (size_t)B);
-        return COV_OK;
-    }
-    OK(ensure(h, h->dX, std::max<size_t>(in_bytes, 1 << 20)));
-    OK(ensure(h, h->d_obj, std::max<size_t>(out_bytes, 1 << 20))); // one device block for every output
-    CK(cudaMemcpyAsync(h->dX.p, hin, in_bytes, cudaMemcpyHostToDevice, h->stream));
-    char *dbase = (char *)h->d_obj.p;
-    EvalOut out{};
-    out.obj = (double *)(dbase + o_obj);
-    out.count = count ? (long long *)(dbase + o_cnt) : nullptr;
-    out.class_count = class_count ? (long long *)(dbase + o_cls) : nullptr;
-    out.progressive = progressive ? (double *)(dbase + o_prg) : nullptr;
-    out.feasible = feasible ? (unsigned char *)(dbase + o_fea) : nullptr;
-    OK(launch_on_main(h, (const double *)h->dX.p, B, out, true));
-    CK(cudaMemcpyAsync(hout, dbase, out_bytes, cudaMemcpyDeviceToHost, h->stream)); // ONE copy back
+    char *base = zc ? vout : (char *)h->d_obj.p;
+    char *at[kCols];
+    for (int k = 0; k < kCols; ++k) at[k] = c[k].host ? base + c[k].at : nullptr;
+    OK(launch_on_main(h, zc ? (const double *)vin : (const double *)h->dX.p, B, eval_out(at), timed));
+    if (!zc) CK(cudaMemcpyAsync(hout, base, out_bytes, cudaMemcpyDeviceToHost, h->stream)); // ONE copy back
     CK(cudaStreamSynchronize(h->stream));
-    const char *so = hout;
-    memcpy(obj, so + o_obj, (size_t)B * 8);
-    if (count) memcpy(count, so + o_cnt, (size_t)B * 8);
-    if (class_count) memcpy(class_count, so + o_cls, (size_t)B * 8 * ncls);
-    if (progressive) memcpy(progressive, so + o_prg, (size_t)B * 8);
-    if (feasible) memcpy(feasible, so + o_fea, (size_t)B);
+    for (const Col &col : c)
+        if (col.host) memcpy(col.host, hout + col.at, (size_t)B * col.row);
     return COV_OK;
 }
-
-// The poll winner of a host-path call (cov_argmin, cov_eval_batch_best): reduced on the device from the
-// device-resident copy of the objectives and flags, 16 bytes come back per window.
-struct BestReq {
-    int barrier;
-    double best = INFINITY;
-    int64_t idx = -1;
-};
 
 // Packed candidates (cov_eval_batch_packed): `elem`-byte values that the device widens to doubles, value * g.
 struct PackedIn {
@@ -1448,8 +1488,11 @@ static void unpack_host(const PackedIn &pk, size_t n, double *out) // the same a
     }
 }
 
+// best: the poll winner too (cov_argmin, cov_eval_batch_best), reduced on the device from the device-resident copy of
+// the objectives and flags; 16 bytes come back per window.
 static int eval_host(cov_handle *h, const double *X, int64_t B, double *obj, int64_t *count, uint8_t *feasible,
-                     int64_t *class_count, double *progressive, BestReq *best = nullptr, const PackedIn *pk = nullptr)
+                     int64_t *class_count, double *progressive, Winner *best = nullptr, int barrier = 0,
+                     const PackedIn *pk = nullptr)
 {
     OK(check_ready(h, "cov_eval_batch"));
     if (B < 0 || (B > 0 && ((pk ? !pk->Q : !X) || (!obj && !best))))
@@ -1462,35 +1505,34 @@ static int eval_host(cov_handle *h, const double *X, int64_t B, double *obj, int
     const int N = h->o.N;
     const int ncls = h->g.n_classes;
     const size_t row_bytes = (size_t)3 * N * 8;
+    Cols c = {{(char *)obj, 8, &h->d_obj},
+              {(char *)count, 8, &h->d_count},
+              {(char *)class_count, (size_t)8 * ncls, &h->d_clscnt},
+              {(char *)progressive, 8, &h->d_prog},
+              {(char *)feasible, 1, &h->d_feas}};
     if (!best && (size_t)B * row_bytes <= (256u << 10) && (size_t)B * (25 + 8 * (size_t)ncls) <= (1536u << 10) && h->chunk == 0) {
-        if (!pk) return eval_host_small(h, X, B, obj, count, feasible, class_count, progressive);
+        if (!pk) return eval_host_small(h, X, B, c);
         std::vector<double> wide((size_t)B * 3 * N); // a poll set: widened on the host, then the poll path as it is
         unpack_host(*pk, wide.size(), wide.data());
-        return eval_host_small(h, wide.data(), B, obj, count, feasible, class_count, progressive);
+        return eval_host_small(h, wide.data(), B, c);
     }
+    for (Col &col : c) col.pinned = !col.host || is_pinned_host(col.host);
 #if COV_ZC_MID_LIMIT > 0
     // mid-size batches in pinned buffers: one launch that reads the candidates straight over PCIe (the
     // kernel's own unit prefetch overlaps transfer and compute) and writes the results back the same way
     if (!pk && !best && h->zero_copy_out && h->chunk == 0 && N <= 8 && (size_t)B * row_bytes <= (size_t)(COV_ZC_MID_LIMIT) && is_pinned_host(X) &&
-        is_pinned_host(obj) && (!count || is_pinned_host(count)) && (!feasible || is_pinned_host(feasible)) &&
-        (!class_count || is_pinned_host(class_count)) && (!progressive || is_pinned_host(progressive))) {
+        std::all_of(c, c + kCols, [](const Col &col) { return col.pinned; })) {
         const double *vx = (const double *)device_view((void *)X);
-        EvalOut out{};
-        out.obj = (double *)device_view(obj);
-        out.count = count ? (long long *)device_view(count) : nullptr;
-        out.feasible = feasible ? (unsigned char *)device_view(feasible) : nullptr;
-        out.class_count = class_count ? (long long *)device_view(class_count) : nullptr;
-        out.progressive = progressive ? (double *)device_view(progressive) : nullptr;
-        if (vx && out.obj && (!count || out.count) && (!feasible || out.feasible) && (!class_count || out.class_count) &&
-            (!progressive || out.progressive)) {
-            OK(launch_on_main(h, vx, B, out, true));
+        char *at[kCols];
+        if (vx && view_cols(c, nullptr, 0, 0, at)) {
+            OK(launch_on_main(h, vx, B, eval_out(at), true));
             CK(cudaStreamSynchronize(h->stream));
             return COV_OK;
         }
     }
 #endif
     // device window: at most ~1 GiB of candidates at a time
-    const int64_t window = std::max<int64_t>(1, std::min<int64_t>(B, (int64_t)((1ull << 30) / row_bytes)));
+    const int64_t window = window_rows(B, row_bytes, 1ull << 30);
     // slice size: ~16 MiB of candidates, a multiple of 32 candidates (keeps device slices 16-byte aligned).
     // Packed input is compute-bound, not PCIe-bound (5 UAVs, int16: 0.54 ms of copies beside 0.7 ms of kernels per
     // 1 M candidates), so fewer, larger slices win: ~32 MiB of widened candidates (measured on B200, 1 M x 5 UAVs:
@@ -1501,12 +1543,11 @@ static int eval_host(cov_handle *h, const double *X, int64_t B, double *obj, int
     // (two experiments lost here, DESIGN.md 5: a quarter- and a half-size first slice so that the kernels start sooner,
     // 1.107 -> 1.125 ms; and no copy engine at all, the widening kernel reading the pinned buffer over PCIe beside the
     // previous slice's objective kernel, 1.107 -> 1.21 ms)
+    // the device columns: every requested one, obj always (the winner's input, or its mirror), feasible with best
+    auto on_device = [&](int k) { return c[k].host || k == COL_OBJ || (k == COL_FEAS && best); };
     OK(ensure(h, h->dX, (size_t)window * row_bytes));
-    OK(ensure(h, h->d_obj, (size_t)window * 8));
-    if (count) OK(ensure(h, h->d_count, (size_t)window * 8));
-    if (feasible || best) OK(ensure(h, h->d_feas, (size_t)window));
-    if (class_count) OK(ensure(h, h->d_clscnt, (size_t)window * 8 * ncls));
-    if (progressive) OK(ensure(h, h->d_prog, (size_t)window * 8));
+    for (int k = 0; k < kCols; ++k)
+        if (on_device(k)) OK(ensure(h, *c[k].dev, (size_t)window * c[k].row));
     // what crosses PCIe per candidate: the doubles themselves, or the packed values (widened on the device)
     const size_t in_row_bytes = pk ? (size_t)3 * N * pk->elem : row_bytes;
     const char *in_base = pk ? (const char *)pk->Q : (const char *)X;
@@ -1520,16 +1561,7 @@ static int eval_host(cov_handle *h, const double *X, int64_t B, double *obj, int
     if (pk)
         for (int k = 0; k < 2; ++k) OK(ensure(h, h->d_raw[k], (size_t)chunk * in_row_bytes));
     // outputs that are not pinned are staged per window and copied out at the window's end
-    const bool obj_p = !obj || is_pinned_host(obj), cnt_p = !count || is_pinned_host(count),
-               fea_p = !feasible || is_pinned_host(feasible), cls_p = !class_count || is_pinned_host(class_count),
-               prg_p = !progressive || is_pinned_host(progressive);
-    size_t stage_out = 0;
-    size_t off_obj = 0, off_cnt = 0, off_fea = 0, off_cls = 0, off_prg = 0;
-    if (!obj_p) { off_obj = stage_out; stage_out += (size_t)window * 8; }
-    if (!cnt_p) { off_cnt = stage_out; stage_out += (size_t)window * 8; }
-    if (!cls_p) { off_cls = stage_out; stage_out += (size_t)window * 8 * ncls; }
-    if (!prg_p) { off_prg = stage_out; stage_out += (size_t)window * 8; }
-    if (!fea_p) { off_fea = stage_out; stage_out += (size_t)window; }
+    const size_t stage_out = pack_cols(c, (size_t)window);
     if (stage_out) OK(ensure_pinned(h, &h->h_out, &h->h_out_cap, stage_out));
     char *so = (char *)h->h_out;
 
@@ -1538,12 +1570,7 @@ static int eval_host(cov_handle *h, const double *X, int64_t B, double *obj, int
     bool free_armed[2] = {false, false}, raw_armed[2] = {false, false};
     int rc = COV_OK;
     auto done = [&](int code) {
-        h->ev_pool.push_back(ev_in);
-        h->ev_pool.push_back(ev_k);
-        h->ev_pool.push_back(ev_free[0]);
-        h->ev_pool.push_back(ev_free[1]);
-        h->ev_pool.push_back(ev_raw[0]);
-        h->ev_pool.push_back(ev_raw[1]);
+        for (cudaEvent_t e : {ev_in, ev_k, ev_free[0], ev_free[1], ev_raw[0], ev_raw[1]}) h->ev_pool.push_back(e);
         return code;
     };
 #define CKD(call)                                                         \
@@ -1596,37 +1623,19 @@ static int eval_host(cov_handle *h, const double *X, int64_t B, double *obj, int
                 CKD(cudaEventRecord(ev_raw[slot], h->stream));
                 raw_armed[slot] = true;
             }
-            EvalOut out{};
             const int64_t g0 = w0 + c0;
-            bool zc = h->zero_copy_out != 0 && (obj != nullptr || !best); // (cov_argmin has no per-candidate outputs)
-            if (zc) {
-                // results go straight to pinned host memory (the caller's buffer, or the staging block): posted
-                // PCIe writes of 17 B per candidate instead of three D2H copies per slice beside the H2D stream
-                char *v_obj = (char *)device_view(obj_p ? (void *)obj : (void *)(so + off_obj));
-                char *v_cnt = !count ? nullptr : (char *)device_view(cnt_p ? (void *)count : (void *)(so + off_cnt));
-                char *v_fea = !feasible ? nullptr : (char *)device_view(fea_p ? (void *)feasible : (void *)(so + off_fea));
-                char *v_cls = !class_count ? nullptr : (char *)device_view(cls_p ? (void *)class_count : (void *)(so + off_cls));
-                char *v_prg = !progressive ? nullptr : (char *)device_view(prg_p ? (void *)progressive : (void *)(so + off_prg));
-                if (!v_obj || (count && !v_cnt) || (feasible && !v_fea) || (class_count && !v_cls) || (progressive && !v_prg)) {
-                    zc = false; // a buffer the device cannot address: copy back instead
-                } else {
-                    out.obj = (double *)v_obj + (obj_p ? g0 : c0);
-                    out.count = !count ? nullptr : (long long *)v_cnt + (cnt_p ? g0 : c0);
-                    out.feasible = !feasible ? nullptr : (unsigned char *)v_fea + (fea_p ? g0 : c0);
-                    out.class_count = !class_count ? nullptr : (long long *)v_cls + (size_t)(cls_p ? g0 : c0) * ncls;
-                    out.progressive = !progressive ? nullptr : (double *)v_prg + (prg_p ? g0 : c0);
-                    if (best) { // results straight to the host as usual; the winner is reduced from device mirrors
-                        out.obj_mirror = (double *)h->d_obj.p + c0;
-                        out.feasible_mirror = (unsigned char *)h->d_feas.p + c0;
-                    }
-                }
-            }
-            if (!zc) {
-                out.obj = (double *)h->d_obj.p + c0;
-                out.count = count ? (long long *)h->d_count.p + c0 : nullptr;
-                out.feasible = (feasible || best) ? (unsigned char *)h->d_feas.p + c0 : nullptr;
-                out.class_count = class_count ? (long long *)h->d_clscnt.p + (size_t)c0 * ncls : nullptr;
-                out.progressive = progressive ? (double *)h->d_prog.p + c0 : nullptr;
+            // results straight to pinned host memory (the caller's buffer, or the staging block): posted PCIe writes
+            // of 17 B per candidate instead of three D2H copies per slice beside the H2D stream.  Not when a buffer is
+            // one the device cannot address, nor for cov_argmin, which has no per-candidate outputs.
+            char *at[kCols];
+            const bool zc = h->zero_copy_out != 0 && (obj != nullptr || !best) && view_cols(c, so, g0, c0, at);
+            if (!zc)
+                for (int k = 0; k < kCols; ++k)
+                    at[k] = on_device(k) ? (char *)c[k].dev->p + (size_t)c0 * c[k].row : nullptr;
+            EvalOut out = eval_out(at);
+            if (zc && best) { // results straight to the host as usual; the winner is reduced from device mirrors
+                out.obj_mirror = (double *)h->d_obj.p + c0;
+                out.feasible_mirror = (unsigned char *)h->d_feas.p + c0;
             }
             rc = launch_on_main(h, dst, cn, out, true);
             if (rc != COV_OK) return done(rc);
@@ -1634,47 +1643,23 @@ static int eval_host(cov_handle *h, const double *X, int64_t B, double *obj, int
             tr(h->stream);
             if (!zc) {
                 CKD(cudaStreamWaitEvent(h->s_out, ev_k, 0));
-                if (obj)
-                    CKD(cudaMemcpyAsync(obj_p ? (void *)(obj + g0) : (void *)(so + off_obj + (size_t)c0 * 8), out.obj,
-                                        (size_t)cn * 8, cudaMemcpyDeviceToHost, h->s_out));
-                if (count)
-                    CKD(cudaMemcpyAsync(cnt_p ? (void *)(count + g0) : (void *)(so + off_cnt + (size_t)c0 * 8),
-                                        out.count, (size_t)cn * 8, cudaMemcpyDeviceToHost, h->s_out));
-                if (feasible)
-                    CKD(cudaMemcpyAsync(fea_p ? (void *)(feasible + g0) : (void *)(so + off_fea + (size_t)c0),
-                                        out.feasible, (size_t)cn, cudaMemcpyDeviceToHost, h->s_out));
-                if (class_count)
-                    CKD(cudaMemcpyAsync(cls_p ? (void *)(class_count + (size_t)g0 * ncls)
-                                              : (void *)(so + off_cls + (size_t)c0 * 8 * ncls),
-                                        out.class_count, (size_t)cn * 8 * ncls, cudaMemcpyDeviceToHost, h->s_out));
-                if (progressive)
-                    CKD(cudaMemcpyAsync(prg_p ? (void *)(progressive + g0) : (void *)(so + off_prg + (size_t)c0 * 8),
-                                        out.progressive, (size_t)cn * 8, cudaMemcpyDeviceToHost, h->s_out));
+                for (int k : {COL_OBJ, COL_COUNT, COL_FEAS, COL_CLS, COL_PROG}) {
+                    const Col &col = c[k];
+                    if (col.host)
+                        CKD(cudaMemcpyAsync(col.pinned ? col.host + (size_t)g0 * col.row : so + col.at + (size_t)c0 * col.row,
+                                            at[k], (size_t)cn * col.row, cudaMemcpyDeviceToHost, h->s_out));
+                }
             }
             tr(zc ? h->stream : h->s_out);
         }
         // end of window: results home, device window reusable
-        if (best) {
-            CKD(launch_argmin((const double *)h->d_obj.p, (const unsigned char *)h->d_feas.p, wn, best->barrier,
-                              (double *)h->argmin_obj.p, (long long *)h->argmin_idx.p, 1024, h->stream));
-            h->launches += 2;
-            double *ho = (double *)h->h_small + 40;
-            long long *hi = (long long *)h->h_small + 41;
-            CKD(cudaMemcpyAsync(ho, h->argmin_obj.p, 8, cudaMemcpyDeviceToHost, h->stream));
-            CKD(cudaMemcpyAsync(hi, h->argmin_idx.p, 8, cudaMemcpyDeviceToHost, h->stream));
-            CKD(cudaStreamSynchronize(h->stream));
-            if (*hi >= 0 && (best->idx < 0 || *ho < best->best)) { // ties keep the earlier window's index
-                best->best = *ho;
-                best->idx = w0 + *hi;
-            }
-        }
+        if (best && (rc = enqueue_winner(h, (const double *)h->d_obj.p, (const unsigned char *)h->d_feas.p, wn, barrier)) != COV_OK)
+            return done(rc);
         CKD(cudaStreamSynchronize(h->stream));
         CKD(cudaStreamSynchronize(h->s_out));
-        if (!obj_p) host_copy(h, obj + w0, so + off_obj, (size_t)wn * 8);
-        if (!cnt_p) host_copy(h, count + w0, so + off_cnt, (size_t)wn * 8);
-        if (!fea_p) host_copy(h, feasible + w0, so + off_fea, (size_t)wn);
-        if (!cls_p) memcpy(class_count + (size_t)w0 * ncls, so + off_cls, (size_t)wn * 8 * ncls);
-        if (!prg_p) memcpy(progressive + w0, so + off_prg, (size_t)wn * 8);
+        if (best) best->offer(h->h_small->win_obj, h->h_small->win_idx, w0);
+        for (const Col &col : c)
+            if (!col.pinned) host_copy(h, col.host + (size_t)w0 * col.row, so + col.at, (size_t)wn * col.row);
     }
 #undef CKD
     if (h->trace && h->trace_ev.size() > 1) {
@@ -1687,14 +1672,6 @@ static int eval_host(cov_handle *h, const double *X, int64_t B, double *obj, int
     return done(COV_OK);
 }
 
-extern "C" int cov_eval_batch(cov_handle *h, const double *X, int64_t B, double *obj, int64_t *count,
-                              uint8_t *feasible)
-{
-    if (!h) return fail(nullptr, COV_ERR_INVALID, "NULL handle");
-    DeviceGuard dg(h->device);
-    return eval_host(h, X, B, obj, count, feasible, nullptr, nullptr);
-}
-
 extern "C" int cov_eval_batch_ex(cov_handle *h, const double *X, int64_t B, double *obj, int64_t *count,
                                  uint8_t *feasible, int64_t *class_count, double *progressive)
 {
@@ -1703,16 +1680,22 @@ extern "C" int cov_eval_batch_ex(cov_handle *h, const double *X, int64_t B, doub
     return eval_host(h, X, B, obj, count, feasible, class_count, progressive);
 }
 
+extern "C" int cov_eval_batch(cov_handle *h, const double *X, int64_t B, double *obj, int64_t *count,
+                              uint8_t *feasible)
+{
+    return cov_eval_batch_ex(h, X, B, obj, count, feasible, nullptr, nullptr);
+}
+
 extern "C" int cov_eval_batch_best(cov_handle *h, const double *X, int64_t B, double *obj, int64_t *count,
                                    uint8_t *feasible, int32_t barrier, double *best_obj, int64_t *best_idx)
 {
     if (!h) return fail(nullptr, COV_ERR_INVALID, "NULL handle");
     DeviceGuard dg(h->device);
     if (!best_obj || !best_idx) return fail(h, COV_ERR_INVALID, "cov_eval_batch_best: NULL winner outputs");
-    BestReq br{barrier};
-    OK(eval_host(h, X, B, obj, count, feasible, nullptr, nullptr, &br));
-    *best_obj = br.idx >= 0 ? br.best : INFINITY;
-    *best_idx = br.idx;
+    Winner w;
+    OK(eval_host(h, X, B, obj, count, feasible, nullptr, nullptr, &w, barrier));
+    *best_obj = w.obj;
+    *best_idx = w.idx;
     return COV_OK;
 }
 
@@ -1729,15 +1712,15 @@ extern "C" int cov_eval_batch_packed(cov_handle *h, const void *Q, int32_t pack,
     if ((best_obj == nullptr) != (best_idx == nullptr))
         return fail(h, COV_ERR_INVALID, "cov_eval_batch_packed: best_obj and best_idx go together");
     PackedIn pk{Q, pack, granularity, elem};
-    if (!best_obj) return eval_host(h, nullptr, B, obj, count, feasible, nullptr, nullptr, nullptr, &pk);
-    BestReq br{barrier};
-    OK(eval_host(h, nullptr, B, obj, count, feasible, nullptr, nullptr, &br, &pk));
-    *best_obj = br.idx >= 0 ? br.best : INFINITY;
-    *best_idx = br.idx;
+    if (!best_obj) return eval_host(h, nullptr, B, obj, count, feasible, nullptr, nullptr, nullptr, 0, &pk);
+    Winner w;
+    OK(eval_host(h, nullptr, B, obj, count, feasible, nullptr, nullptr, &w, barrier, &pk));
+    *best_obj = w.obj;
+    *best_idx = w.idx;
     return COV_OK;
 }
 
-// One candidate through pinned scratch: copy in, one launch, copy out, one synchronisation.
+// One candidate through the small path, its launch untimed: copy in, one launch, copy out, one synchronisation.
 extern "C" int cov_eval_one(cov_handle *h, const double *x, double *obj)
 {
     if (!h) return fail(nullptr, COV_ERR_INVALID, "NULL handle");
@@ -1745,35 +1728,8 @@ extern "C" int cov_eval_one(cov_handle *h, const double *x, double *obj)
     OK(check_ready(h, "cov_eval_one"));
     if (!x || !obj) return fail(h, COV_ERR_INVALID, "cov_eval_one: NULL argument");
     recycle_spans(h);
-    const int N = h->o.N;
-    const size_t bytes = (size_t)3 * N * 8;
-    char *hx = (char *)h->h_small + 4096; // pinned scratch for one candidate (3 * kMaxUavs doubles)
-    memcpy(hx, x, bytes);
-    if (h->zero_copy_out) {
-        // no copy engines: the kernel reads the candidate from, and writes the objective to, pinned host memory
-        double *hres = (double *)h->h_small + 32;
-        const double *vx = (const double *)device_view(hx);
-        double *vres = (double *)device_view(hres);
-        if (vx && vres) {
-            EvalOut out{};
-            out.obj = vres;
-            OK(launch_on_main(h, vx, 1, out, false));
-            CK(cudaStreamSynchronize(h->stream));
-            *obj = *hres;
-            return COV_OK;
-        }
-    }
-    OK(ensure(h, h->dX, bytes));
-    OK(ensure(h, h->d_obj, 8));
-    CK(cudaMemcpyAsync(h->dX.p, hx, bytes, cudaMemcpyHostToDevice, h->stream));
-    EvalOut out{};
-    out.obj = (double *)h->d_obj.p;
-    OK(launch_on_main(h, (const double *)h->dX.p, 1, out, false));
-    double *hres = (double *)h->h_small + 32;
-    CK(cudaMemcpyAsync(hres, h->d_obj.p, 8, cudaMemcpyDeviceToHost, h->stream));
-    CK(cudaStreamSynchronize(h->stream));
-    *obj = *hres;
-    return COV_OK;
+    Cols c = {{(char *)obj, 8, &h->d_obj}}; // the objective alone
+    return eval_host_small(h, x, 1, c, false);
 }
 
 
@@ -1972,6 +1928,30 @@ static int check_mads_limits(cov_handle *h, const char *who, bool grid)
     return COV_OK;
 }
 
+constexpr size_t kPow10Bytes = (1 - 2 * kMadsPow10Min) * 8;
+// The device buffers of S solves of n variables, allocated and pointed at by a: mads_in = [prefix, which opens with the
+// powers of ten from the host's libm | X0: S n doubles | a0: S n doubles | b0: S n ints], mads_out = [X_out: S n doubles |
+// obj: S | stats: S x 4 | extra_out bytes].  Fills pow10 into hin, the host copy of mads_in (at least prefix bytes).
+static int mads_buffers(cov_handle *h, size_t prefix, int64_t S, int n, size_t extra_out, std::vector<unsigned char> &hin,
+                        MadsArgs &a)
+{
+    const size_t sn = (size_t)S * n;
+    OK(ensure(h, h->mads_in, prefix + sn * 20));
+    OK(ensure(h, h->mads_out, sn * 8 + (size_t)S * 40 + extra_out));
+    for (int b = kMadsPow10Min; b <= -kMadsPow10Min; ++b) ((double *)hin.data())[b - kMadsPow10Min] = std::pow(10.0, b);
+    a = MadsArgs{};
+    a.pow10 = (const double *)h->mads_in.p;
+    a.X0 = (const double *)((const char *)h->mads_in.p + prefix);
+    a.a0 = a.X0 + sn;
+    a.b0 = (const int *)(a.a0 + sn);
+    a.X_out = (double *)h->mads_out.p;
+    a.obj_out = a.X_out + sn;
+    a.stats = (long long *)(a.obj_out + S);
+    a.S = S;
+    a.force_exact = h->cfg.force_exact;
+    return COV_OK;
+}
+
 // S solves of the same loop on the device, one launch for all of them (cov_mads.cu).  The host contributes what
 // must carry its libm's bits: the initial mesh of every start and the table of powers of ten.  region: the objective
 // of cov_eval_region_batch instead of the cell store's.
@@ -1985,38 +1965,23 @@ static int mads_solve_batch(cov_handle *h, bool region, const double *X0, int64_
     const int N = h->o.N, n = 3 * N;
     OK(check_mads_limits(h, who, !region));
     if (!region && !h->area_exact) OK(entries_on_device(h)); // non-dyadic weights: the list-order sum
-    // in: [pow10: 801 doubles | X0: S n doubles | a0: S n doubles | b0: S n ints]; out: [X_out | obj | stats]
-    constexpr int kPow = 1 - 2 * kMadsPow10Min;
-    const size_t sn = (size_t)S * n;
-    const size_t o_x = (size_t)kPow * 8, o_a = o_x + sn * 8, o_b = o_a + sn * 8, in_bytes = o_b + sn * 4;
-    const size_t o_obj = sn * 8, o_st = o_obj + (size_t)S * 8, out_bytes = o_st + (size_t)S * 4 * 8;
+    const size_t sn = (size_t)S * n, in_bytes = kPow10Bytes + sn * 20, out_bytes = sn * 8 + (size_t)S * 40;
     std::vector<unsigned char> hin(in_bytes), hout(out_bytes);
-    double *p10 = (double *)hin.data(), *ha = (double *)(hin.data() + o_a);
-    int *hb = (int *)(hin.data() + o_b);
-    for (int b = kMadsPow10Min; b <= -kMadsPow10Min; ++b) p10[b - kMadsPow10Min] = std::pow(10.0, b);
-    memcpy(hin.data() + o_x, X0, sn * 8);
+    MadsArgs a;
+    OK(mads_buffers(h, kPow10Bytes, S, n, 0, hin, a)); // the prefix: pow10
+    double *hx = (double *)(hin.data() + kPow10Bytes), *ha = hx + sn;
+    int *hb = (int *)(ha + sn);
+    memcpy(hx, X0, sn * 8);
     for (size_t q = 0; q < sn; ++q) {
         const MeshVar m = initial_mesh(X0[q], granularity);
         ha[q] = m.a;
         hb[q] = m.b;
     }
-    OK(ensure(h, h->mads_in, in_bytes));
-    OK(ensure(h, h->mads_out, out_bytes));
     unsigned char *din = (unsigned char *)h->mads_in.p, *dout = (unsigned char *)h->mads_out.p;
     CK(cudaMemcpyAsync(din, hin.data(), in_bytes, cudaMemcpyHostToDevice, h->stream));
-    MadsArgs a{};
-    a.pow10 = (const double *)din;
-    a.X0 = (const double *)(din + o_x);
-    a.a0 = (const double *)(din + o_a);
-    a.b0 = (const int *)(din + o_b);
-    a.X_out = (double *)dout;
-    a.obj_out = (double *)(dout + o_obj);
-    a.stats = (long long *)(dout + o_st);
-    a.S = S;
     a.n_iter = n_iter;
     a.granularity = granularity;
     a.seed = seed;
-    a.force_exact = h->cfg.force_exact;
     a.ordered = h->area_exact ? 0 : 1;
     unsigned long long *counter = nullptr;
     OK(take_counter(h, &counter));
@@ -2027,8 +1992,8 @@ static int mads_solve_batch(cov_handle *h, bool region, const double *X0, int64_
     CK(cudaMemcpyAsync(hout.data(), dout, out_bytes, cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
     memcpy(X_out, hout.data(), sn * 8);
-    if (obj_out) memcpy(obj_out, hout.data() + o_obj, (size_t)S * 8);
-    if (stats) memcpy(stats, hout.data() + o_st, (size_t)S * 4 * 8);
+    if (obj_out) memcpy(obj_out, hout.data() + sn * 8, (size_t)S * 8);
+    if (stats) memcpy(stats, hout.data() + sn * 8 + (size_t)S * 8, (size_t)S * 4 * 8);
     return COV_OK;
 }
 
@@ -2064,39 +2029,24 @@ extern "C" int cov_run_horizon(cov_handle *h, const double *x_start, int64_t T, 
     if (T == 0) return COV_OK;
     OK(check_mads_limits(h, who, true));
     const int N = h->o.N, n = 3 * N;
-    // in: [pow10: 801 doubles | x_start: n | boxes: 4 n_boxes | X0: S n | a0: S n | b0: S n ints]
-    // out: [solves' X: S n | obj: S | stats: S x 4 | X_out: T n | obj_out: T | stats: T x 4]
-    constexpr int kPow = 1 - 2 * kMadsPow10Min;
-    const size_t sn = (size_t)S * n, tn = (size_t)T * n;
-    const size_t o_x = (size_t)kPow * 8, o_box = o_x + (size_t)n * 8, o_X0 = o_box + (size_t)n_boxes * 32;
-    const size_t o_a = o_X0 + sn * 8, o_b = o_a + sn * 8, in_bytes = o_b + sn * 4;
-    const size_t o_obj = sn * 8, o_mst = o_obj + (size_t)S * 8, o_Xo = o_mst + (size_t)S * 32;
-    const size_t res_bytes = tn * 8 + (size_t)T * 8 + (size_t)T * 32, out_bytes = o_Xo + res_bytes;
+    // in: [pow10 | x_start: n | boxes: 4 n_boxes | the solves' inputs]
+    // out: [the solves' outputs | X_out: T n | obj_out: T | stats: T x 4]
+    const size_t tn = (size_t)T * n;
+    const size_t o_x = kPow10Bytes, o_box = o_x + (size_t)n * 8, o_X0 = o_box + (size_t)n_boxes * 32;
+    const size_t res_bytes = tn * 8 + (size_t)T * 8 + (size_t)T * 32;
     std::vector<unsigned char> hin(o_X0);
-    double *p10 = (double *)hin.data();
-    for (int b = kMadsPow10Min; b <= -kMadsPow10Min; ++b) p10[b - kMadsPow10Min] = std::pow(10.0, b);
+    MadsArgs a;
+    OK(mads_buffers(h, o_X0, S, n, res_bytes, hin, a));
     memcpy(hin.data() + o_x, x_start, (size_t)n * 8);
     if (n_boxes) memcpy(hin.data() + o_box, boxes, (size_t)n_boxes * 32);
-    OK(ensure(h, h->mads_in, in_bytes));
-    OK(ensure(h, h->mads_out, out_bytes));
     OK(ensure(h, h->xyT, (size_t)n * 8));
     OK(ensure_pinned(h, &h->h_out, &h->h_out_cap, res_bytes));
-    unsigned char *din = (unsigned char *)h->mads_in.p, *dout = (unsigned char *)h->mads_out.p;
+    unsigned char *din = (unsigned char *)h->mads_in.p;
     const double *d_x0 = (const double *)(din + o_x);
-    double *d_Xo = (double *)(dout + o_Xo), *d_oo = d_Xo + tn, *xyT = (double *)h->xyT.p;
+    double *d_Xo = (double *)(a.stats + 4 * S), *d_oo = d_Xo + tn, *xyT = (double *)h->xyT.p;
     long long *d_st = (long long *)(d_oo + T);
-    MadsArgs a{};
-    a.pow10 = (const double *)din;
-    a.X0 = (const double *)(din + o_X0);
-    a.a0 = (const double *)(din + o_a);
-    a.b0 = (const int *)(din + o_b);
-    a.X_out = (double *)dout;
-    a.obj_out = (double *)(dout + o_obj);
-    a.stats = (long long *)(dout + o_mst);
-    a.S = S;
     a.n_iter = n_iter;
     a.granularity = granularity;
-    a.force_exact = h->cfg.force_exact;
     a.ordered = 0;
     HorizonStep hs{};
     hs.N = N;
@@ -2135,8 +2085,8 @@ extern "C" int cov_run_horizon(cov_handle *h, const double *x_start, int64_t T, 
         if (h->g.planes_q && (e = launch_requad_plane(h->g, (uint32_t *)h->planes_q.p, h->stream)) != cudaSuccess) break;
         hs.t = t;
         what = "horizon_start";
-        if ((e = launch_horizon_start(hs, cur, (double *)h->params.p, (double *)(din + o_X0), (double *)(din + o_a),
-                                      (int *)(din + o_b), h->stream)) != cudaSuccess)
+        if ((e = launch_horizon_start(hs, cur, (double *)h->params.p, (double *)a.X0, (double *)a.a0, (int *)a.b0,
+                                      h->stream)) != cudaSuccess)
             break;
         a.seed = seed + (uint64_t)(t - 1) * (uint64_t)S;
         unsigned long long *counter = nullptr;
@@ -2159,27 +2109,19 @@ extern "C" int cov_run_horizon(cov_handle *h, const double *x_start, int64_t T, 
     if (e != cudaSuccess || rc != COV_OK) { // the removals enqueued so far stand: refresh what the host knows of them
         if (rc == COV_OK) rc = fail_cuda(h, e, (std::string(who) + ": " + what).c_str());
         const std::string msg = h->err;
-        h->ent_removed_pending = h->ent_known;
-        h->ent_dev_valid = false;
-        double cw[kMaxClasses];
-        for (int k = 0; k < kMaxClasses; ++k) cw[k] = h->g.class_weight[k];
-        if (rebuild_planes(h, h->g.n_classes, cw) != COV_OK) h->have_grid = false;
+        entries_note_removals(h);
+        if (rebuild_planes(h, h->g.n_classes, h->g.class_weight) != COV_OK) h->have_grid = false;
         for (cudaEvent_t x : ev) h->ev_pool.push_back(x);
         h->err = msg;
         return rc;
     }
-    double cw[kMaxClasses];
-    for (int k = 0; k < kMaxClasses; ++k) cw[k] = h->g.class_weight[k];
-    rc = rebuild_planes(h, h->g.n_classes, cw); // the one synchronise
+    rc = rebuild_planes(h, h->g.n_classes, h->g.class_weight); // the one synchronise
     const double *hX = (const double *)h->h_out, *hobj = hX + tn;
     const int64_t *hst = (const int64_t *)(hobj + T);
     if (rc == COV_OK) {
         bool removed = false;
         for (int64_t t = 0; t < T; ++t) removed |= hst[4 * t + 3] != 0;
-        if (removed) {
-            h->ent_removed_pending = h->ent_known;
-            h->ent_dev_valid = false;
-        }
+        if (removed) entries_note_removals(h);
         memcpy(X_out, hX, tn * 8);
         if (obj_out) memcpy(obj_out, hobj, (size_t)T * 8);
         if (stats) memcpy(stats, hst, (size_t)T * 32);
@@ -2203,44 +2145,31 @@ extern "C" int cov_argmin(cov_handle *h, const double *X, int64_t B, int32_t bar
     DeviceGuard dg(h->device);
     OK(check_ready(h, "cov_argmin"));
     if (B < 0 || (B > 0 && !X) || !best_obj || !best_idx) return fail(h, COV_ERR_INVALID, "cov_argmin: bad arguments");
-    double best = INFINITY;
-    int64_t bidx = -1;
+    Winner w;
     const int N = h->o.N;
     const size_t row_bytes = (size_t)3 * N * 8;
     if ((size_t)B * row_bytes > (4u << 20)) { // big sets: the sliced pipeline (H2D of slice k+1 beside the kernel of slice k)
-        BestReq br{barrier};
-        OK(eval_host(h, X, B, nullptr, nullptr, nullptr, nullptr, nullptr, &br));
-        *best_obj = br.idx >= 0 ? br.best : INFINITY;
-        *best_idx = br.idx;
-        return COV_OK;
-    }
-    recycle_spans(h);
-    const int64_t window = std::max<int64_t>(1, std::min<int64_t>(std::max<int64_t>(B, 1), (int64_t)((1ull << 30) / row_bytes)));
-    OK(ensure(h, h->dX, (size_t)window * row_bytes));
-    OK(ensure(h, h->d_obj, (size_t)window * 8));
-    OK(ensure(h, h->d_feas, (size_t)window));
-    for (int64_t w0 = 0; w0 < B; w0 += window) {
-        const int64_t wn = std::min(window, B - w0);
-        CK(cudaMemcpyAsync(h->dX.p, X + (size_t)w0 * 3 * N, (size_t)wn * row_bytes, cudaMemcpyHostToDevice, h->stream));
-        EvalOut out{};
-        out.obj = (double *)h->d_obj.p;
-        out.feasible = (unsigned char *)h->d_feas.p;
-        OK(launch_on_main(h, (const double *)h->dX.p, wn, out, true));
-        CK(launch_argmin(out.obj, out.feasible, wn, barrier, (double *)h->argmin_obj.p, (long long *)h->argmin_idx.p,
-                         1024, h->stream));
-        h->launches += 2;
-        double *ho = (double *)h->h_small + 40;
-        long long *hi = (long long *)h->h_small + 41;
-        CK(cudaMemcpyAsync(ho, h->argmin_obj.p, 8, cudaMemcpyDeviceToHost, h->stream));
-        CK(cudaMemcpyAsync(hi, h->argmin_idx.p, 8, cudaMemcpyDeviceToHost, h->stream));
-        CK(cudaStreamSynchronize(h->stream));
-        if (*hi >= 0 && (bidx < 0 || *ho < best)) { // ties keep the earlier window's index
-            best = *ho;
-            bidx = w0 + *hi;
+        OK(eval_host(h, X, B, nullptr, nullptr, nullptr, nullptr, nullptr, &w, barrier));
+    } else {
+        recycle_spans(h);
+        const int64_t window = window_rows(B, row_bytes, 1ull << 30);
+        OK(ensure(h, h->dX, (size_t)window * row_bytes));
+        OK(ensure(h, h->d_obj, (size_t)window * 8));
+        OK(ensure(h, h->d_feas, (size_t)window));
+        for (int64_t w0 = 0; w0 < B; w0 += window) {
+            const int64_t wn = std::min(window, B - w0);
+            CK(cudaMemcpyAsync(h->dX.p, X + (size_t)w0 * 3 * N, (size_t)wn * row_bytes, cudaMemcpyHostToDevice, h->stream));
+            EvalOut out{};
+            out.obj = (double *)h->d_obj.p;
+            out.feasible = (unsigned char *)h->d_feas.p;
+            OK(launch_on_main(h, (const double *)h->dX.p, wn, out, true));
+            OK(enqueue_winner(h, out.obj, out.feasible, wn, barrier));
+            CK(cudaStreamSynchronize(h->stream));
+            w.offer(h->h_small->win_obj, h->h_small->win_idx, w0);
         }
     }
-    *best_obj = bidx >= 0 ? best : INFINITY;
-    *best_idx = bidx;
+    *best_obj = w.obj;
+    *best_idx = w.idx;
     return COV_OK;
 }
 
@@ -2255,7 +2184,7 @@ extern "C" int cov_union_area_batch(cov_handle *h, const double *X, int64_t B, i
     if (N < 1 || N > kMaxUavs) return fail(h, COV_ERR_LIMIT, "cov_union_area_batch: N must be 1..1024");
     if (B < 0 || (B > 0 && (!X || !area))) return fail(h, COV_ERR_INVALID, "cov_union_area_batch: bad arguments");
     const size_t row_bytes = (size_t)3 * N * 8;
-    const int64_t window = std::max<int64_t>(1, std::min<int64_t>(std::max<int64_t>(B, 1), (int64_t)((256ull << 20) / row_bytes)));
+    const int64_t window = window_rows(B, row_bytes, 256ull << 20);
     OK(ensure(h, h->dX, (size_t)window * row_bytes));
     OK(ensure(h, h->d_obj, (size_t)window * 8));
     for (int64_t w0 = 0; w0 < B; w0 += window) {
@@ -2319,14 +2248,14 @@ extern "C" int cov_set_region(cov_handle *h, double x_lo, double y_lo, double x_
     if (e == cudaSuccess && Mk > 0) e = launch_region_arcs(rd, (RegionArc *)da.p, kRegionMaxArcs, (int *)h->region_count.p, h->stream);
     if (e == cudaSuccess && Mk > 0) {
         h->launches += 1;
-        e = cudaMemcpyAsync((int *)h->h_small + 96, h->region_count.p, sizeof(int), cudaMemcpyDeviceToHost, h->stream);
+        e = cudaMemcpyAsync(&h->h_small->region_arcs, h->region_count.p, sizeof(int), cudaMemcpyDeviceToHost, h->stream);
     }
     if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
     if (e != cudaSuccess) {
         release();
         return fail_cuda(h, e, "cov_set_region");
     }
-    if (Mk > 0) K = *((int *)h->h_small + 96);
+    if (Mk > 0) K = h->h_small->region_arcs;
     if (K > kRegionMaxArcs) {
         release();
         return fail(h, COV_ERR_LIMIT, "cov_set_region: the covered discs' boundary has " + std::to_string(K) +
@@ -2363,56 +2292,33 @@ extern "C" int cov_eval_region_batch(cov_handle *h, const double *X, int64_t B, 
     const bool want_best = best_obj != nullptr;
     const int N = h->o.N;
     const size_t row_bytes = (size_t)3 * N * 8;
-    const int64_t window = std::max<int64_t>(1, std::min<int64_t>(std::max<int64_t>(B, 1), (int64_t)((1ull << 30) / row_bytes)));
+    const int64_t window = window_rows(B, row_bytes, 1ull << 30);
     OK(ensure(h, h->dX, (size_t)window * row_bytes));
     OK(ensure(h, h->d_obj, (size_t)window * 8));
     OK(ensure(h, h->d_area, (size_t)window * 8));
     OK(ensure(h, h->d_feas, (size_t)window));
-    double best = INFINITY;
-    int64_t bidx = -1;
+    Winner w;
     recycle_spans(h);
     for (int64_t w0 = 0; w0 < B; w0 += window) {
         const int64_t wn = std::min(window, B - w0);
         CK(cudaMemcpyAsync(h->dX.p, X + (size_t)w0 * 3 * N, (size_t)wn * row_bytes, cudaMemcpyHostToDevice, h->stream));
         double *d_obj = (double *)h->d_obj.p, *d_area = (double *)h->d_area.p;
         unsigned char *d_feas = (unsigned char *)h->d_feas.p;
-        cudaEvent_t e0 = get_event(h), e1 = get_event(h); // the kernel's device time, for cov_last_kernel_ms
-        CK(cudaEventRecord(e0, h->stream));
-        cudaError_t e = launch_region_eval(h->region, h->o, h->cfg, (const double *)h->dX.p, wn, d_obj, area ? d_area : nullptr,
-                                           d_feas, h->stream);
-        if (e != cudaSuccess) {
-            h->ev_pool.push_back(e0);
-            h->ev_pool.push_back(e1);
-            if (e != cudaErrorInvalidConfiguration) return fail_cuda(h, e, "cov_eval_region_batch: kernel launch");
-            (void)cudaGetLastError();
-            return fail(h, COV_ERR_LIMIT, "cov_eval_region_batch: the region does not fit the shared-memory plan");
-        }
-        CK(cudaEventRecord(e1, h->stream));
-        h->kernel_spans.emplace_back(e0, e1);
-        h->launches += 1;
-        if (want_best) {
-            CK(launch_argmin(d_obj, d_feas, wn, barrier, (double *)h->argmin_obj.p, (long long *)h->argmin_idx.p, 1024,
-                             h->stream));
-            h->launches += 2;
-            CK(cudaMemcpyAsync((double *)h->h_small + 40, h->argmin_obj.p, 8, cudaMemcpyDeviceToHost, h->stream));
-            CK(cudaMemcpyAsync((long long *)h->h_small + 41, h->argmin_idx.p, 8, cudaMemcpyDeviceToHost, h->stream));
-        }
+        OK(timed_launch(h, true, nullptr, "cov_eval_region_batch: kernel launch",
+                        "cov_eval_region_batch: the region does not fit the shared-memory plan", [&] {
+                            return launch_region_eval(h->region, h->o, h->cfg, (const double *)h->dX.p, wn, d_obj,
+                                                      area ? d_area : nullptr, d_feas, h->stream);
+                        }));
+        if (want_best) OK(enqueue_winner(h, d_obj, d_feas, wn, barrier));
         if (obj) CK(cudaMemcpyAsync(obj + w0, d_obj, (size_t)wn * 8, cudaMemcpyDeviceToHost, h->stream));
         if (area) CK(cudaMemcpyAsync(area + w0, d_area, (size_t)wn * 8, cudaMemcpyDeviceToHost, h->stream));
         if (feasible) CK(cudaMemcpyAsync(feasible + w0, d_feas, (size_t)wn, cudaMemcpyDeviceToHost, h->stream));
         CK(cudaStreamSynchronize(h->stream));
-        if (want_best) {
-            const double ho = *((double *)h->h_small + 40);
-            const long long hi = *((long long *)h->h_small + 41);
-            if (hi >= 0 && (bidx < 0 || ho < best)) { // ties keep the earlier window's index
-                best = ho;
-                bidx = w0 + hi;
-            }
-        }
+        if (want_best) w.offer(h->h_small->win_obj, h->h_small->win_idx, w0);
     }
     if (want_best) {
-        *best_obj = bidx >= 0 ? best : INFINITY;
-        *best_idx = bidx;
+        *best_obj = w.obj;
+        *best_idx = w.idx;
     }
     return COV_OK;
 }
@@ -2613,14 +2519,11 @@ static void shard(int64_t B, int G, int k, int64_t &b0, int64_t &bn)
     bn = std::min<int64_t>(B, b0 + per) - b0;
 }
 
-extern "C" int cov_multi_eval_batch(cov_multi *m, const double *X, int64_t B, double *obj, int64_t *count,
-                                    uint8_t *feasible)
+// run(k, handle, candidates, b0, bn) on every non-empty shard k of X, one host thread per device; the first shard that
+// failed is the call's error.
+template <class Run>
+static int run_shards(cov_multi *m, const double *X, int64_t B, Run &&run)
 {
-    if (!m) return fail(nullptr, COV_ERR_INVALID, "NULL multi handle");
-    if (B < 0 || (B > 0 && (!X || !obj))) {
-        m->err = "cov_multi_eval_batch: bad arguments";
-        return COV_ERR_INVALID;
-    }
     const int G = (int)m->hs.size();
     std::vector<int> rcs((size_t)G, COV_OK);
     std::vector<std::thread> th;
@@ -2628,11 +2531,8 @@ extern "C" int cov_multi_eval_batch(cov_multi *m, const double *X, int64_t B, do
         th.emplace_back([&, k]() {
             int64_t b0, bn;
             shard(B, G, k, b0, bn);
-            if (bn <= 0) return;
             cov_handle *h = m->hs[k];
-            const int N = h->have_params ? h->o.N : 0;
-            rcs[k] = cov_eval_batch(h, X + (size_t)b0 * 3 * N, bn, obj + b0, count ? count + b0 : nullptr,
-                                    feasible ? feasible + b0 : nullptr);
+            if (bn > 0) rcs[k] = run(k, h, X + (size_t)b0 * 3 * (h->have_params ? h->o.N : 0), b0, bn);
         });
     for (auto &t : th) t.join();
     for (int k = 0; k < G; ++k)
@@ -2641,6 +2541,19 @@ extern "C" int cov_multi_eval_batch(cov_multi *m, const double *X, int64_t B, do
             return rcs[k];
         }
     return COV_OK;
+}
+
+extern "C" int cov_multi_eval_batch(cov_multi *m, const double *X, int64_t B, double *obj, int64_t *count,
+                                    uint8_t *feasible)
+{
+    if (!m) return fail(nullptr, COV_ERR_INVALID, "NULL multi handle");
+    if (B < 0 || (B > 0 && (!X || !obj))) {
+        m->err = "cov_multi_eval_batch: bad arguments";
+        return COV_ERR_INVALID;
+    }
+    return run_shards(m, X, B, [&](int, cov_handle *h, const double *Xk, int64_t b0, int64_t bn) {
+        return cov_eval_batch(h, Xk, bn, obj + b0, count ? count + b0 : nullptr, feasible ? feasible + b0 : nullptr);
+    });
 }
 
 extern "C" int cov_multi_argmin(cov_multi *m, const double *X, int64_t B, int32_t barrier, double *best_obj,
@@ -2652,34 +2565,16 @@ extern "C" int cov_multi_argmin(cov_multi *m, const double *X, int64_t B, int32_
         return COV_ERR_INVALID;
     }
     const int G = (int)m->hs.size();
-    std::vector<int> rcs((size_t)G, COV_OK);
     std::vector<double> bo((size_t)G, INFINITY);
     std::vector<int64_t> bi((size_t)G, -1);
-    std::vector<std::thread> th;
-    for (int k = 0; k < G; ++k)
-        th.emplace_back([&, k]() {
-            int64_t b0, bn;
-            shard(B, G, k, b0, bn);
-            if (bn <= 0) return;
-            cov_handle *h = m->hs[k];
-            const int N = h->have_params ? h->o.N : 0;
-            rcs[k] = cov_argmin(h, X + (size_t)b0 * 3 * N, bn, barrier, &bo[k], &bi[k]);
-            if (rcs[k] == COV_OK && bi[k] >= 0) bi[k] += b0;
-        });
-    for (auto &t : th) t.join();
-    double best = INFINITY;
-    int64_t idx = -1;
-    for (int k = 0; k < G; ++k) {
-        if (rcs[k] != COV_OK) {
-            m->err = "device shard " + std::to_string(k) + ": " + m->hs[k]->err;
-            return rcs[k];
-        }
-        if (bi[k] >= 0 && (idx < 0 || bo[k] < best)) { // 16-byte (min, index) pair per GPU, host gather
-            best = bo[k];
-            idx = bi[k];
-        }
-    }
-    *best_obj = best;
-    *best_idx = idx;
+    OK(run_shards(m, X, B, [&](int k, cov_handle *h, const double *Xk, int64_t b0, int64_t bn) {
+        const int rc = cov_argmin(h, Xk, bn, barrier, &bo[k], &bi[k]);
+        if (rc == COV_OK && bi[k] >= 0) bi[k] += b0;
+        return rc;
+    }));
+    Winner w; // 16-byte (min, index) pair per GPU, host gather
+    for (int k = 0; k < G; ++k) w.offer(bo[k], bi[k]);
+    *best_obj = w.obj;
+    *best_idx = w.idx;
     return COV_OK;
 }
