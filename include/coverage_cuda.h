@@ -37,7 +37,8 @@ extern "C" {
 #define COV_ABI_VERSION 3 /* 2: COV_OPT_PROGRESSIVE_INDEX, COV_KERNEL_ORDERED, cov_get_class_weights, cov_eval_batch_best;
                              3: cov_eval_batch_packed (COV_PACK_*); later, with no existing symbol changed:
                                 cov_mads_solve_batch; cov_set_region, cov_eval_region_batch,
-                                cov_mads_solve_batch_region (the grid-free static objective); cov_run_horizon */
+                                cov_mads_solve_batch_region (the grid-free static objective); cov_run_horizon;
+                                cov_run_horizon_points, cov_run_horizon_fire (the dynamic horizon) */
 
 #if defined(__GNUC__)
 #define COV_API __attribute__((visibility("default")))
@@ -316,6 +317,64 @@ COV_API int cov_run_horizon(cov_handle *h, const double *x_start, int64_t T, int
                             int64_t n_iter, double granularity, uint64_t seed,
                             const double *boxes, int64_t n_boxes, double h_focus, double h_max,
                             double *X_out, double *obj_out, int64_t *stats, double *step_ms);
+
+/* The dynamic receding horizon (FullSimulation.run_simulation with environment_type = "dynamic"): cov_run_horizon
+ * with an append step that opens every timestep, before step 1 (update_POI before rmvCoveredPOI, as the reference
+ * orders them).  Arguments, outputs and errors are cov_run_horizon's, except that stats is T x 5: [winner k,
+ * evaluations, solves with a feasible point, entries removed, entries appended].
+ *
+ * The store's envelope.  The plane set stays fixed inside the loop, so before anything is enqueued the call reads the
+ * cell store (one download) and bounds every cell's multiplicity over the whole call, ignoring removals:
+ *  - classes: the store's, then the new weights in order of first appearance in the schedule (cov_add_points'
+ *    numbering; a store without entries starts afresh, as there).  More than 4: COV_ERR_LIMIT;
+ *  - planes: for class k, bits 0 .. floor(log2(the largest bound of its cells)).  More than 8, or a bound over 255:
+ *    COV_ERR_LIMIT;
+ *  - area_exact of the store with n_entries replaced by n_entries plus every entry the call can add: 0 gives
+ *    COV_ERR_STATE (list-order stores are out of scope, as for cov_run_horizon);
+ *  - cov_mads_solve_batch's limits on that plane set: COV_ERR_LIMIT.
+ * An empty plane adds nothing to any count, so every objective, iterate and winner is the one the sequence of single
+ * calls computes on its smaller plane sets; one rebuild at the end leaves the minimal plane set and the statistics.
+ * Because removals are ignored, the checks are conservative: a call can be refused that the sequence of single calls
+ * would accept (e.g. a cell whose bound passes 255 although a removal would have emptied it first).
+ *
+ * Afterwards the handle is exactly as the sequence of single calls leaves it (per timestep: the appends, then
+ * cov_remove_covered, cov_set_params, cov_mads_solve_batch on the documented starts, the argmin and the evaluation):
+ * cell store, cov_get_grid_info, cov_get_class_weights, the parameters of step T, the automaton's state and the
+ * ordered point list.  The one exception: when the store empties completely inside the loop, cov_add_points would
+ * restart its class numbering and this call does not (counts and objectives are the same).  A refused call changes
+ * nothing: every check runs before the first enqueue.  A CUDA failure inside the loop leaves what was enqueued, the
+ * store rebuilt, and the list order forgotten (createPOI's from then on).  T == 0 does nothing.
+ *
+ * cov_run_horizon_points: the reference's fire list (update_POI's push!).  Timestep t appends rows offsets[t-1] ..
+ * offsets[t] - 1 of pts5 (reference 5-tuples, P = offsets[T] rows).  COV_ERR_INVALID: offsets NULL, offsets[0] != 0,
+ * decreasing, or T > 2^31 - 1; pts5 NULL with P > 0; a NaN weight; entries of different weights on one cell, checked
+ * against the cell's class at the call and across the whole schedule (conservatively).  COV_ERR_OFF_LATTICE: a point
+ * that is not a cell centre.  stats[t][4] = offsets[t+1] - offsets[t].  last_removed (nullable, nx*ny ints indexed
+ * (i-1) + nx*(j-1)): the last timestep of this call in which rmvCoveredPOI removed entries from the cell, 0 if none.
+ * The ordered list afterwards is the single calls': an entry appended at timestep ta (ta = 1 for the entries listed
+ * before the call) survives iff last_removed[cell] < ta; a store without a known list first fixes createPOI's order,
+ * as cov_add_points does. */
+COV_API int cov_run_horizon_points(cov_handle *h, const double *x_start, int64_t T, int64_t S, double spread,
+                                   int64_t n_iter, double granularity, uint64_t seed,
+                                   const double *boxes, int64_t n_boxes, double h_focus, double h_max,
+                                   const double *pts5, const int64_t *offsets,
+                                   double *X_out, double *obj_out, int64_t *stats, double *step_ms,
+                                   int *last_removed);
+
+/* cov_run_horizon_fire: the device automaton (cov_fire_step with append = 1).  Timestep t runs fire_steps[t-1] >= 0
+ * steps, numbered consecutively from first_step (the last is first_step + sum(fire_steps) - 1 <= 2^32 - 1), with the
+ * direction probabilities cov_fire_step forms from wind_speed, wind_direction and prob_spread, keyed by fire_seed.
+ * The envelope bounds a cell by its multiplicity plus 8 for every interior TREE cell (one ignition, at most one entry
+ * per burning Moore neighbour).  stats[t][4]: the entries the timestep's steps pushed.  If any entry is pushed, the
+ * list order is createPOI's afterwards, as after cov_fire_step.  COV_ERR_STATE: cov_fire_step's preconditions
+ * (cov_fire_init called, one weight class of weight dx*dy); COV_ERR_INVALID: fire_steps NULL with T > 0 or negative,
+ * first_step < 0 or the step range past 2^32 - 1. */
+COV_API int cov_run_horizon_fire(cov_handle *h, const double *x_start, int64_t T, int64_t S, double spread,
+                                 int64_t n_iter, double granularity, uint64_t seed,
+                                 const double *boxes, int64_t n_boxes, double h_focus, double h_max,
+                                 const int64_t *fire_steps, double wind_speed, double wind_direction,
+                                 double prob_spread, uint64_t fire_seed, int64_t first_step,
+                                 double *X_out, double *obj_out, int64_t *stats, double *step_ms);
 
 /* Covered-cell mask of ONE candidate: nx*ny bytes, 1 where the cell is inside some disc (whether
  * or not it holds entries). Lets the host replay an ordered Float64 sum over a weighted list. */

@@ -92,6 +92,22 @@ def update_POI(self: Cells, t: int) -> Cells:
     return self
 
 
+def update_POI_schedule(self: Cells, T: int) -> list:
+    """What update_POI appends at timesteps 1 .. T, as T arrays (n_t x 5): nothing at t = 1, then row
+    t + initial_rows of the table (reweighted) while rows remain.  The appends of CoverageEngine.run_horizon_points."""
+    if self.fire_rows is None:
+        raise ValueError("the dynamic schedule needs fire_rows (see initialise_POI)")
+    first = getattr(self, "_initial_rows", 10)
+    out = []
+    for t in range(1, T + 1):
+        k = t + first  # 1-based row number
+        if t != 1 and k <= len(self.fire_rows):
+            out.append(self._reweight(np.asarray(self.fire_rows[k - 1], dtype=np.float64).reshape(-1, 5)))
+        else:
+            out.append(np.zeros((0, 5)))
+    return out
+
+
 def rmvCoveredPOI(self: Cells, circles) -> Cells:
     """src/CellFunctions.jl:81-108 -- delete every entry covered by the current discs."""
     ACC.rmvCoveredPOI(circles, self.resident())

@@ -43,6 +43,16 @@ class ForestFire:
         return self.engine.fire_step(self.wind_speed, self.wind_direction, self.prob_spread, self.seed, self.t,
                                      append=append)
 
+    def run_horizon(self, x_start, fire_steps, **kw):
+        """CoverageEngine.run_horizon_fire on this fire: timestep t runs fire_steps[t-1] of this fire's steps before
+        its rmvCoveredPOI, continuing the step numbers of step(), so that later step() calls continue the same stream.
+        kw: run_horizon's S, spread, n_iter, granularity, seed, boxes, h_focus, h_max."""
+        fire_steps = np.ascontiguousarray(fire_steps, dtype=np.int64).ravel()
+        out = self.engine.run_horizon_fire(x_start, fire_steps, self.wind_speed, self.wind_direction,
+                                           self.prob_spread, self.seed, self.t + 1, **kw)
+        self.t += int(fire_steps.sum())
+        return out
+
     def grid(self) -> np.ndarray:
         """Current state as grid[i-1, j-1]."""
         return self.engine.fire_state().reshape(self.ny, self.nx).T

@@ -75,8 +75,9 @@ def run_simulation(cells, starting_circles, cons_ext, cons_prog, N, r_max, param
 
     starts=S runs the whole horizon on the device in one call (CoverageEngine.run_horizon): per timestep S MADS
     solves, from the swarm and from S - 1 copies of it moved by N(0, spread^2) metres in x and y, and the best result
-    becomes the next swarm.  Static environment and the grid objective only, with constraints that all fuse;
-    runtime_data_MADS then holds the device time of each timestep."""
+    becomes the next swarm.  The grid objective only, with constraints that all fuse; runtime_data_MADS then holds the
+    device time of each timestep.  The dynamic environment appends update_POI's rows inside the same call
+    (CoverageEngine.run_horizon_points) and leaves cells as the host loop does."""
     p = params
     if objective not in ("grid", "region"):
         raise ValueError("objective must be 'grid' or 'region'")
@@ -90,8 +91,10 @@ def run_simulation(cells, starting_circles, cons_ext, cons_prog, N, r_max, param
     d_lim = p.d_lim * np.ones(N)
     steps = p.Nt_sim if Nt_sim is None else Nt_sim
     if starts is not None:
-        if p.environment_type != "static" or objective != "grid":
-            raise ValueError("starts= runs the static environment with the grid objective only")
+        if objective != "grid":
+            raise ValueError("starts= runs the grid objective only")
+        if p.environment_type == "dynamic" and getattr(cells, "fire_rows", None) is None:
+            raise ValueError("starts= with the dynamic environment needs cells with fire_rows (initialise_POI)")
         return _run_horizon(cells, pre, cons_ext, N, r_max, p, steps, int(starts), spread, t_half, d_lim)
     engine, covered = None, np.zeros((0, 3))
     if objective == "region":
@@ -144,10 +147,24 @@ def _run_horizon(cells, pre, cons_ext, N, r_max, p, steps, S, spread, t_half, d_
     if obj.native_batch_solver(_flatten_constraints([cons_ext, create_cons3(pre, p.FOV, d_lim)])) is None:
         raise ValueError("starts= needs constraints that all fuse into the objective's launch")
     res, eng = obj._engine()  # the store synced, the parameters of timestep 1's solves (cons3 from pre) set
-    X, objs, _, step_ms = eng.run_horizon(pre, steps, S, spread, p.N_iter, 1.0, 0 if p.seed is None else p.seed,
-                                          boxes, H_FOCUS, p.h_max)
-    # the host list after every rmvCoveredPOI: the entries whose cell still holds some
-    res.points.keep(eng.grid_cells()[res.cell_index()] > 0)
+    kw = dict(S=S, spread=spread, n_iter=p.N_iter, granularity=1.0, seed=0 if p.seed is None else p.seed,
+              boxes=boxes, h_focus=H_FOCUS, h_max=p.h_max)
+    if p.environment_type == "dynamic":
+        appends = CellFunctions.update_POI_schedule(cells, steps)
+        X, objs, _, step_ms, last = eng.run_horizon_points(pre, appends, **kw)
+        # the host list as update_POI and rmvCoveredPOI leave it: an entry appended at timestep ta (1 for the
+        # initial list) is gone iff its cell lost entries at ta or later
+        ta = np.concatenate([np.ones(len(res.points), dtype=np.int64)] +
+                            [np.full(len(a), t, dtype=np.int64) for t, a in enumerate(appends, start=1)])
+        for a in appends:
+            if len(a):
+                res.points.append(a)
+                cells.fire_point_xy_ccordinates.extend(q[:2].copy() for q in a)
+        res.points.keep(last[res.points.cell_index()] < ta)
+    else:
+        X, objs, _, step_ms = eng.run_horizon(pre, steps, **kw)
+        # the host list after every rmvCoveredPOI: the entries whose cell still holds some
+        res.points.keep(eng.grid_cells()[res.cell_index()] > 0)
     res.mark_synced()
     for t in range(2, steps + 1):  # the caller's r_max as the host loop leaves it
         apply_r_max_rule(X[t - 2], r_max, N, p, t_half)

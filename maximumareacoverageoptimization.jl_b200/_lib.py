@@ -79,6 +79,10 @@ SIGNATURES = {
     "cov_mads_solve": (_i, [_vp, _vp, _i64, _d, C.c_uint64, _vp, _pd, _pi64]),
     "cov_mads_solve_batch": (_i, [_vp, _vp, _i64, _i64, _d, C.c_uint64, _vp, _vp, _vp]),
     "cov_run_horizon": (_i, [_vp, _vp, _i64, _i64, _d, _i64, _d, C.c_uint64, _vp, _i64, _d, _d, _vp, _vp, _vp, _vp]),
+    "cov_run_horizon_points": (_i, [_vp, _vp, _i64, _i64, _d, _i64, _d, C.c_uint64, _vp, _i64, _d, _d, _vp, _vp,
+                                    _vp, _vp, _vp, _vp, _vp]),
+    "cov_run_horizon_fire": (_i, [_vp, _vp, _i64, _i64, _d, _i64, _d, C.c_uint64, _vp, _i64, _d, _d, _vp, _d, _d, _d,
+                                  C.c_uint64, _i64, _vp, _vp, _vp, _vp]),
     "cov_covered_mask": (_i, [_vp, _vp, _vp]),
     "cov_set_region": (_i, [_vp, _d, _d, _d, _d, _vp, _i64]),
     "cov_eval_region_batch": (_i, [_vp, _vp, _i64, _vp, _vp, _vp, C.c_int32, _pd, _pi64]),

@@ -599,6 +599,33 @@ static void odd_decompose(double v, uint64_t &m, int &e)
     }
 }
 
+// area_exact: every partial sum of the reference's list-order Float64 accumulation over n_entries entries of the
+// classes of g is an integer multiple of a common power of two and stays below 2^53 of them, hence exact in any
+// order, and so is sum_k fl(w_k * count_k).
+static bool sums_exact(const GridDesc &g, int64_t n_entries)
+{
+    int qmin = 0;
+    bool first = true;
+    uint64_t ms[kMaxClasses];
+    int es[kMaxClasses];
+    for (int k = 0; k < g.n_classes; ++k) {
+        const double w = g.class_weight[k];
+        if (w == 0.0) {
+            ms[k] = 0;
+            es[k] = 0;
+            continue;
+        }
+        if (!(w > 0) || std::isinf(w)) return false;
+        odd_decompose(w, ms[k], es[k]);
+        if (first || es[k] < qmin) qmin = es[k];
+        first = false;
+    }
+    long double total = 0;
+    for (int k = 0; k < g.n_classes; ++k)
+        if (ms[k]) total += std::ldexp((long double)ms[k], es[k] - qmin) * (long double)n_entries;
+    return total < 9007199254740992.0L;
+}
+
 // Derive the bit planes from the device-resident mult/cls bytes and refresh the statistics.  class_weight may be
 // g.class_weight itself: each weight is read only by its own assignment below.
 static int rebuild_planes(cov_handle *h, int n_classes, const double *class_weight)
@@ -653,38 +680,7 @@ static int rebuild_planes(cov_handle *h, int n_classes, const double *class_weig
         h->launches += 1;
         g.planes_q = (const uint32_t *)h->planes_q.p;
     }
-    // area_exact: every partial sum of the reference's list-order Float64 accumulation is an
-    // integer multiple of a common power of two and stays below 2^53 of them, hence exact in any
-    // order, and so is sum_k fl(w_k * count_k).
-    h->area_exact = 1;
-    {
-        int qmin = 0;
-        bool first = true, ok = true;
-        uint64_t ms[kMaxClasses];
-        int es[kMaxClasses];
-        for (int k = 0; k < g.n_classes; ++k) {
-            const double w = g.class_weight[k];
-            if (w == 0.0) {
-                ms[k] = 0;
-                es[k] = 0;
-                continue;
-            }
-            if (!(w > 0) || std::isinf(w)) {
-                ok = false;
-                break;
-            }
-            odd_decompose(w, ms[k], es[k]);
-            if (first || es[k] < qmin) qmin = es[k];
-            first = false;
-        }
-        if (ok) {
-            long double total = 0;
-            for (int k = 0; k < g.n_classes; ++k)
-                if (ms[k]) total += std::ldexp((long double)ms[k], es[k] - qmin) * (long double)h->n_entries;
-            ok = total < 9007199254740992.0L;
-        }
-        h->area_exact = ok ? 1 : 0;
-    }
+    h->area_exact = sums_exact(g, h->n_entries) ? 1 : 0;
     h->have_grid = true;
     return COV_OK;
 }
@@ -719,13 +715,10 @@ static void entries_note_removals(cov_handle *h)
 }
 // rmvCoveredPOI deletes every entry of a covered cell and keeps the order of the rest
 // (src/CellFunctions.jl:81-108): drop the mirror's entries whose cell is now empty.
-static int entries_apply_removals(cov_handle *h)
+// m: the multiplicity bytes as they are now (host copy).
+static void entries_apply_removals(cov_handle *h, const unsigned char *m)
 {
-    if (!h->ent_known || !h->ent_removed_pending) return COV_OK;
-    const size_t ncell = (size_t)h->g.nx * h->g.ny;
-    std::vector<unsigned char> m(ncell);
-    CK(cudaMemcpyAsync(m.data(), h->mult.p, ncell, cudaMemcpyDeviceToHost, h->stream));
-    CK(cudaStreamSynchronize(h->stream));
+    if (!h->ent_known || !h->ent_removed_pending) return;
     size_t keep = 0;
     for (size_t p = 0; p < h->ent_cell_h.size(); ++p)
         if (m[(size_t)h->ent_cell_h[p]]) {
@@ -737,18 +730,22 @@ static int entries_apply_removals(cov_handle *h)
     h->ent_cls_h.resize(keep);
     h->ent_removed_pending = false;
     h->ent_dev_valid = false;
+}
+static int entries_apply_removals(cov_handle *h)
+{
+    if (!h->ent_known || !h->ent_removed_pending) return COV_OK;
+    const size_t ncell = (size_t)h->g.nx * h->g.ny;
+    std::vector<unsigned char> m(ncell);
+    CK(cudaMemcpyAsync(m.data(), h->mult.p, ncell, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    entries_apply_removals(h, m.data());
     return COV_OK;
 }
 // The host list of a store that no list was ever given for (bit grid, cell bytes, createPOI, automaton), built from
 // the cell store as it is now: createPOI's order, i outer and j inner (src/AreaCoverageCalculation.jl:14-15), the
 // entries of a cell together.
-static int entries_from_cells(cov_handle *h)
+static void entries_from_cells(cov_handle *h, const unsigned char *m, const unsigned char *k)
 {
-    const size_t ncell = (size_t)h->g.nx * h->g.ny;
-    std::vector<unsigned char> m(ncell), k(ncell);
-    CK(cudaMemcpyAsync(m.data(), h->mult.p, ncell, cudaMemcpyDeviceToHost, h->stream));
-    CK(cudaMemcpyAsync(k.data(), h->cls.p, ncell, cudaMemcpyDeviceToHost, h->stream));
-    CK(cudaStreamSynchronize(h->stream));
     h->ent_cell_h.clear();
     h->ent_cls_h.clear();
     for (int i = 0; i < h->g.nx; ++i)
@@ -759,6 +756,15 @@ static int entries_from_cells(cov_handle *h)
                 h->ent_cls_h.push_back((unsigned char)(k[cell] & (kMaxClasses - 1)));
             }
         }
+}
+static int entries_from_cells(cov_handle *h)
+{
+    const size_t ncell = (size_t)h->g.nx * h->g.ny;
+    std::vector<unsigned char> m(ncell), k(ncell);
+    CK(cudaMemcpyAsync(m.data(), h->mult.p, ncell, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaMemcpyAsync(k.data(), h->cls.p, ncell, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    entries_from_cells(h, m.data(), k.data());
     return COV_OK;
 }
 // Make g.ent_cell / g.ent_cls / g.n_ent describe the current list on the device.
@@ -1137,21 +1143,10 @@ extern "C" int cov_fire_init(cov_handle *h, int64_t nx, int64_t ny, double dx, d
     return rebuild_planes(h, 1, &w);
 }
 
-extern "C" int cov_fire_step(cov_handle *h, double wind_speed, double wind_direction, double prob_spread,
-                             uint64_t seed, int64_t step, int32_t append, int64_t *n_pushed)
+// The probability of ignition from the neighbour at window index (a, b), a, b = 1..3, exactly as the reference forms
+// it: wind_speed * cos(wind_direction - atan(2-b, 2-a)) * prob_spread, to hp[(a-1) + 3(b-1)].
+static void fire_probs(double wind_speed, double wind_direction, double prob_spread, double *hp)
 {
-    if (!h) return fail(nullptr, COV_ERR_INVALID, "NULL handle");
-    DeviceGuard dg(h->device);
-    if (!h->have_fire) return fail(h, COV_ERR_STATE, "cov_fire_step: cov_fire_init has not been called");
-    if (step < 0 || step > 0xffffffffll) return fail(h, COV_ERR_INVALID, "cov_fire_step: step out of range");
-    if (h->g.n_classes != 1)
-        return fail(h, COV_ERR_STATE, "cov_fire_step: the cell store holds several weight classes");
-    if (h->g.class_weight[0] != h->g.dx * h->g.dy) // DynamicArea.jl:65: every pushed entry weighs dx*dy
-        return fail(h, COV_ERR_STATE, "cov_fire_step: the cell store's weight class is not dx*dy, the weight the "
-                                      "automaton pushes");
-    // the probability of ignition from the neighbour at window index (a, b), a, b = 1..3, exactly as the
-    // reference forms it: wind_speed * cos(wind_direction - atan(2-b, 2-a)) * prob_spread
-    double *hp = h->h_small->fire_p;
     for (int b = 1; b <= 3; ++b)
         for (int a = 1; a <= 3; ++a) {
             volatile double ang = atan2((double)(2 - b), (double)(2 - a));
@@ -1159,6 +1154,30 @@ extern "C" int cov_fire_step(cov_handle *h, double wind_speed, double wind_direc
             volatile double p = wind_speed * c;
             hp[(a - 1) + 3 * (b - 1)] = p * prob_spread;
         }
+}
+
+// cov_fire_step's preconditions on the store (cov_run_horizon_fire shares them).
+static int check_fire_store(cov_handle *h, const char *who)
+{
+    if (!h->have_fire) return fail(h, COV_ERR_STATE, std::string(who) + ": cov_fire_init has not been called");
+    if (h->g.n_classes != 1)
+        return fail(h, COV_ERR_STATE, std::string(who) + ": the cell store holds several weight classes");
+    if (h->g.class_weight[0] != h->g.dx * h->g.dy) // DynamicArea.jl:65: every pushed entry weighs dx*dy
+        return fail(h, COV_ERR_STATE, std::string(who) + ": the cell store's weight class is not dx*dy, the weight "
+                                                          "the automaton pushes");
+    return COV_OK;
+}
+
+extern "C" int cov_fire_step(cov_handle *h, double wind_speed, double wind_direction, double prob_spread,
+                             uint64_t seed, int64_t step, int32_t append, int64_t *n_pushed)
+{
+    if (!h) return fail(nullptr, COV_ERR_INVALID, "NULL handle");
+    DeviceGuard dg(h->device);
+    if (!h->have_fire) return fail(h, COV_ERR_STATE, "cov_fire_step: cov_fire_init has not been called");
+    if (step < 0 || step > 0xffffffffll) return fail(h, COV_ERR_INVALID, "cov_fire_step: step out of range");
+    OK(check_fire_store(h, "cov_fire_step"));
+    double *hp = h->h_small->fire_p;
+    fire_probs(wind_speed, wind_direction, prob_spread, hp);
     CK(cudaMemcpyAsync(h->fire_p.p, hp, 9 * sizeof(double), cudaMemcpyHostToDevice, h->stream));
     CK(cudaMemsetAsync(h->removed.p, 0, sizeof(unsigned long long), h->stream));
     CK(cudaMemsetAsync(h->overflow.p, 0, sizeof(int), h->stream));
@@ -1912,15 +1931,16 @@ extern "C" int cov_mads_solve(cov_handle *h, const double *x0, int64_t n_iter, d
     return COV_OK;
 }
 
-// The solver's launch plan: N <= kMadsMaxUavs and, with the cell store's objective (grid), one warp's framebuffer.
-static int check_mads_limits(cov_handle *h, const char *who, bool grid)
+// The solver's launch plan: N <= kMadsMaxUavs and, with the cell store's objective (grid: its description, NULL for
+// the region objective), one warp's framebuffer.
+static int check_mads_limits(cov_handle *h, const char *who, const GridDesc *grid)
 {
     const int N = h->o.N;
     int warps = 0, smem = 0, planes_smem = 0;
     if (N > kMadsMaxUavs)
         return fail(h, COV_ERR_LIMIT, std::string(who) + ": N = " + std::to_string(N) + " exceeds the " +
                                           std::to_string(kMadsMaxUavs) + " UAVs of the solver's launch plan");
-    if (grid && !mads_plan(h->g, N, h->cfg, &warps, &smem, &planes_smem))
+    if (grid && !mads_plan(*grid, N, h->cfg, &warps, &smem, &planes_smem))
         return fail(h, COV_ERR_LIMIT, std::string(who) + ": one warp's framebuffer of the " +
                                           std::to_string(h->g.nx) + " x " + std::to_string(h->g.ny) +
                                           " grid does not fit the " + std::to_string(h->cfg.max_smem_optin) +
@@ -1963,7 +1983,7 @@ static int mads_solve_batch(cov_handle *h, bool region, const double *X0, int64_
         return fail(h, COV_ERR_INVALID, std::string(who) + ": bad arguments");
     if (S == 0) return COV_OK;
     const int N = h->o.N, n = 3 * N;
-    OK(check_mads_limits(h, who, !region));
+    OK(check_mads_limits(h, who, region ? nullptr : &h->g));
     if (!region && !h->area_exact) OK(entries_on_device(h)); // non-dyadic weights: the list-order sum
     const size_t sn = (size_t)S * n, in_bytes = kPow10Bytes + sn * 20, out_bytes = sn * 8 + (size_t)S * 40;
     std::vector<unsigned char> hin(in_bytes), hout(out_bytes);
@@ -2006,45 +2026,154 @@ extern "C" int cov_mads_solve_batch(cov_handle *h, const double *X0, int64_t S, 
     return mads_solve_batch(h, false, X0, S, n_iter, granularity, seed, X_out, obj_out, stats);
 }
 
-// T timesteps of FullSimulation.py's MADS loop (lines 72-107) with S starts per timestep, all enqueued before the one
-// synchronise at the end.  Per timestep: rmvCoveredPOI of cur into the stats row, the bit planes repacked (the plane
-// set stays fixed: removals only clear multiplicities), the r_max rule / cons3's previous swarm / the starts
-// (horizon_start_kernel), S solves (launch_mads), the winner to cur (horizon_commit_kernel), AreaMaxObjective(cur).
-extern "C" int cov_run_horizon(cov_handle *h, const double *x_start, int64_t T, int64_t S, double spread,
-                               int64_t n_iter, double granularity, uint64_t seed, const double *boxes, int64_t n_boxes,
-                               double h_focus, double h_max, double *X_out, double *obj_out, int64_t *stats,
-                               double *step_ms)
+// The append step that opens every timestep of a dynamic horizon (run_horizon; NULL: the static loop).  g is the
+// store's envelope: a plane set that holds every multiplicity the loop can reach, fixed for the whole loop.  An empty
+// plane adds nothing to any count, so every objective value is the one of the smaller plane set the host path has.
+struct HorizonAppend {
+    GridDesc g{};
+    int n_classes = 0; // the classes after the call: the store's, then the new weights in order of first appearance
+    double cw[kMaxClasses] = {0, 0, 0, 0};
+    // the fire list (cov_run_horizon_points): timestep t appends entries offsets[t-1] .. offsets[t]-1 of (cell, pcls)
+    const int64_t *offsets = nullptr;
+    std::vector<int> cell;
+    std::vector<unsigned char> pcls;
+    bool stamps = false; // record the last timestep that removed entries from each cell
+    // the automaton (cov_run_horizon_fire): fire_steps[t-1] steps with append at timestep t, numbered from first_step
+    const int64_t *fire_steps = nullptr;
+    uint64_t fire_seed = 0;
+    int64_t first_step = 0;
+};
+
+// The arguments and store every horizon call needs (cov_run_horizon's checks, in its order).
+static int check_horizon(cov_handle *h, const char *who, const double *x_start, int64_t T, int64_t S, double spread,
+                         int64_t n_iter, double granularity, const double *boxes, int64_t n_boxes, const double *X_out)
 {
-    const char *who = "cov_run_horizon";
-    if (!h) return fail(nullptr, COV_ERR_INVALID, "NULL handle");
-    DeviceGuard dg(h->device);
     OK(check_ready(h, who));
     if (!h->o.use_cons3)
-        return fail(h, COV_ERR_STATE, "cov_run_horizon: the parameters have no previous swarm (cons3 is off)");
+        return fail(h, COV_ERR_STATE, std::string(who) + ": the parameters have no previous swarm (cons3 is off)");
     if (!h->area_exact)
-        return fail(h, COV_ERR_STATE, "cov_run_horizon: the store's area depends on the list order (area_exact == 0)");
+        return fail(h, COV_ERR_STATE, std::string(who) + ": the store's area depends on the list order (area_exact == 0)");
     if (T < 0 || S < 1 || n_iter < 0 || (T > 0 && (!x_start || !X_out)) || !std::isfinite(spread) || spread < 0 ||
         !(granularity >= 0) || n_boxes < 0 || (n_boxes > 0 && !boxes))
-        return fail(h, COV_ERR_INVALID, "cov_run_horizon: bad arguments");
-    if (T == 0) return COV_OK;
-    OK(check_mads_limits(h, who, true));
-    const int N = h->o.N, n = 3 * N;
-    // in: [pow10 | x_start: n | boxes: 4 n_boxes | the solves' inputs]
-    // out: [the solves' outputs | X_out: T n | obj_out: T | stats: T x 4]
+        return fail(h, COV_ERR_INVALID, std::string(who) + ": bad arguments");
+    return COV_OK;
+}
+
+// The envelope's plane set: for class k, planes for bits 0 .. floor(log2(max_mult[k])), where max_mult[k] bounds the
+// multiplicity of every cell of class k over the whole loop; n_entries bounds the entries.  Removals are ignored, so
+// the refusals are conservative.
+static int horizon_envelope(cov_handle *h, const char *who, HorizonAppend &app, const unsigned *max_mult,
+                            int64_t n_entries)
+{
+    GridDesc &g = app.g;
+    g = h->g;
+    g.n_classes = app.n_classes;
+    for (int k = 0; k < kMaxClasses; ++k) g.class_weight[k] = k < app.n_classes ? app.cw[k] : 0.0;
+    int np = 0;
+    for (int k = 0; k < g.n_classes; ++k)
+        for (int b = 0; b < 8 && (max_mult[k] >> b); ++b) {
+            if (np >= kMaxPlanes)
+                return fail(h, COV_ERR_LIMIT, std::string(who) + ": the store can reach more than 8 bit planes "
+                                                                 "(weight classes x multiplicity bits, removals ignored)");
+            g.plane_class[np] = k;
+            g.plane_mult[np] = 1 << b;
+            ++np;
+        }
+    if (np == 0) { // an empty store: one all-zero plane, as rebuild_planes keeps it
+        g.plane_class[0] = 0;
+        g.plane_mult[0] = 1;
+        np = 1;
+    }
+    for (int l = np; l < kMaxPlanes; ++l) {
+        g.plane_class[l] = 0;
+        g.plane_mult[l] = 0;
+    }
+    g.n_planes = np;
+    g.planes = nullptr; // run_horizon points them at the handle's buffers
+    g.planes_q = nullptr;
+    if (!sums_exact(g, n_entries))
+        return fail(h, COV_ERR_STATE, std::string(who) + ": with every entry the call can add, the store's area "
+                                                         "would depend on the list order (area_exact == 0)");
+    return check_mads_limits(h, who, &g);
+}
+
+// The list mirror after a fire-list horizon (the pending removals of the call's start already applied): an entry
+// appended at timestep ta (ta = 1 for those in the list before the call) survives iff no timestep >= ta removed
+// entries from its cell, i.e. iff stamp[cell] < ta.
+static void entries_replay(cov_handle *h, const HorizonAppend &app, int64_t T, const int *stamp)
+{
+    size_t keep = 0;
+    for (size_t p = 0; p < h->ent_cell_h.size(); ++p)
+        if (stamp[h->ent_cell_h[p]] < 1) {
+            h->ent_cell_h[keep] = h->ent_cell_h[p];
+            h->ent_cls_h[keep] = h->ent_cls_h[p];
+            ++keep;
+        }
+    h->ent_cell_h.resize(keep);
+    h->ent_cls_h.resize(keep);
+    for (int64_t t = 1; t <= T; ++t)
+        for (int64_t q = app.offsets[t - 1]; q < app.offsets[t]; ++q)
+            if (stamp[app.cell[(size_t)q]] < t) {
+                h->ent_cell_h.push_back(app.cell[(size_t)q]);
+                h->ent_cls_h.push_back(app.pcls[(size_t)q]);
+            }
+    h->ent_removed_pending = false;
+    h->ent_dev_valid = false;
+}
+
+// T >= 1 timesteps of FullSimulation.py's MADS loop (lines 72-107) with S starts per timestep, all enqueued before the
+// one synchronise at the end (arguments and solver limits checked by the caller).  Per timestep: the append step of
+// app (update_POI's push! or the automaton), rmvCoveredPOI of cur into the stats row, the bit planes repacked (the
+// plane set stays fixed: removals only clear multiplicities, and app's envelope holds every append), the r_max rule /
+// cons3's previous swarm / the starts (horizon_start_kernel), S solves (launch_mads), the winner to cur
+// (horizon_commit_kernel), AreaMaxObjective(cur).  stamps_out (nullable, nx*ny): app's removal stamps.
+static int run_horizon(cov_handle *h, const char *who, const double *x_start, int64_t T, int64_t S, double spread,
+                       int64_t n_iter, double granularity, uint64_t seed, const double *boxes, int64_t n_boxes,
+                       double h_focus, double h_max, double *X_out, double *obj_out, int64_t *stats, double *step_ms,
+                       HorizonAppend *app, int *stamps_out)
+{
+    GridDesc lg = app ? app->g : h->g;
+    const int N = h->o.N, n = 3 * N, cols = app ? 5 : 4;
+    const size_t ncell = (size_t)h->g.nx * h->g.ny, P = app ? app->cell.size() : 0;
+    const bool stamps = app && app->stamps;
+    // in: [pow10 | x_start: n | boxes: 4 n_boxes | appended cells: P ints | their classes: P bytes | the solves' inputs]
+    // out: [the solves' outputs | X_out: T n | obj_out: T | stats: T x cols | removal stamps: nx*ny ints]
     const size_t tn = (size_t)T * n;
-    const size_t o_x = kPow10Bytes, o_box = o_x + (size_t)n * 8, o_X0 = o_box + (size_t)n_boxes * 32;
-    const size_t res_bytes = tn * 8 + (size_t)T * 8 + (size_t)T * 32;
+    const size_t o_x = kPow10Bytes, o_box = o_x + (size_t)n * 8, o_cell = o_box + (size_t)n_boxes * 32;
+    const size_t o_cls = o_cell + P * 4, o_X0 = (o_cls + P + 7) / 8 * 8;
+    const size_t o_stamp = tn * 8 + (size_t)T * 8 + (size_t)T * cols * 8;
+    const size_t res_bytes = o_stamp + (stamps ? ncell * 4 : 0);
     std::vector<unsigned char> hin(o_X0);
     MadsArgs a;
     OK(mads_buffers(h, o_X0, S, n, res_bytes, hin, a));
     memcpy(hin.data() + o_x, x_start, (size_t)n * 8);
     if (n_boxes) memcpy(hin.data() + o_box, boxes, (size_t)n_boxes * 32);
+    if (P) {
+        memcpy(hin.data() + o_cell, app->cell.data(), P * 4);
+        memcpy(hin.data() + o_cls, app->pcls.data(), P);
+    }
     OK(ensure(h, h->xyT, (size_t)n * 8));
     OK(ensure_pinned(h, &h->h_out, &h->h_out_cap, res_bytes));
+    const size_t q_bytes = ((size_t)h->g.ny * h->g.qstride + 8) * 4;
+    if (app) { // the envelope's planes; rebuild_planes sizes them for the store again at the end
+        int rc = ensure(h, h->planes, (size_t)lg.n_planes * lg.plane_words * 4);
+        if (rc == COV_OK && lg.n_planes == 1) rc = ensure(h, h->planes_q, q_bytes);
+        if (rc != COV_OK) { // a buffer may have moved: describe the unchanged store again
+            const std::string msg = h->err;
+            if (rebuild_planes(h, h->g.n_classes, h->g.class_weight) != COV_OK) h->have_grid = false;
+            h->err = msg;
+            return rc;
+        }
+        lg.planes = (const uint32_t *)h->planes.p;
+        lg.planes_q = lg.n_planes == 1 ? (const uint32_t *)h->planes_q.p : nullptr;
+    }
     unsigned char *din = (unsigned char *)h->mads_in.p;
     const double *d_x0 = (const double *)(din + o_x);
+    const int *d_cell = (const int *)(din + o_cell);
+    const unsigned char *d_cls = din + o_cls;
     double *d_Xo = (double *)(a.stats + 4 * S), *d_oo = d_Xo + tn, *xyT = (double *)h->xyT.p;
     long long *d_st = (long long *)(d_oo + T);
+    int *d_stamp = stamps ? (int *)((unsigned char *)d_Xo + o_stamp) : nullptr;
     a.n_iter = n_iter;
     a.granularity = granularity;
     a.ordered = 0;
@@ -2064,6 +2193,9 @@ extern "C" int cov_run_horizon(cov_handle *h, const double *x_start, int64_t T, 
     cfg.ordered = 0;
     if (cfg.kernel == COV_KERNEL_ORDERED) cfg.kernel = COV_KERNEL_AUTO;
     unsigned char *mult = (unsigned char *)h->mult.p, *cls = (unsigned char *)h->cls.p;
+    int *overflow = (int *)h->overflow.p;
+    int fire_cur = h->fire_cur;
+    int64_t step = app ? app->first_step : 0;
     std::vector<cudaEvent_t> ev;
     if (step_ms)
         for (int64_t t = 0; t <= T; ++t) ev.push_back(get_event(h));
@@ -2072,17 +2204,47 @@ extern "C" int cov_run_horizon(cov_handle *h, const double *x_start, int64_t T, 
     const char *what = "upload";
     if (e == cudaSuccess) e = launch_thresholds(d_x0, N, xyT, h->stream), what = "launch_thresholds";
     h->launches += 1;
+    if (app && e == cudaSuccess) {
+        what = "append setup";
+        e = cudaMemsetAsync(overflow, 0, sizeof(int), h->stream);
+        if (e == cudaSuccess && d_stamp) e = cudaMemsetAsync(d_stamp, 0, ncell * 4, h->stream);
+        if (e == cudaSuccess && lg.planes_q) e = cudaMemsetAsync((void *)lg.planes_q, 0, q_bytes, h->stream);
+        if (e == cudaSuccess && app->fire_steps)
+            e = cudaMemcpyAsync(h->fire_p.p, h->h_small->fire_p, 9 * sizeof(double), cudaMemcpyHostToDevice, h->stream);
+    }
     int rc = COV_OK;
     for (int64_t t = 1; t <= T && e == cudaSuccess && rc == COV_OK; ++t) {
         const double *cur = t == 1 ? d_x0 : d_Xo + (size_t)(t - 2) * n;
         double *next = d_Xo + (size_t)(t - 1) * n;
-        long long *row = d_st + 4 * (t - 1);
+        long long *row = d_st + cols * (t - 1);
         if (step_ms && (e = cudaEventRecord(ev[(size_t)t - 1], h->stream)) != cudaSuccess) break;
+        if (app && app->offsets) { // update_POI: this timestep's rows of the fire list
+            const int64_t q0 = app->offsets[t - 1], q1 = app->offsets[t];
+            what = "append";
+            if (q1 > q0) {
+                if ((e = launch_add_points(mult, cls, d_cell + q0, d_cls + q0, q1 - q0, overflow, h->stream)) != cudaSuccess) break;
+                h->launches += 1;
+            }
+        } else if (app) { // the automaton, its pushes counted into the stats row
+            what = "fire step";
+            if ((e = cudaMemsetAsync(row + 4, 0, sizeof(long long), h->stream)) != cudaSuccess) break;
+            for (int64_t k = 0; k < app->fire_steps[t - 1] && e == cudaSuccess; ++k, ++step) {
+                e = launch_fire_step((const unsigned char *)h->fire[fire_cur].p, (unsigned char *)h->fire[fire_cur ^ 1].p,
+                                     mult, cls, h->g.nx, h->g.ny, app->fire_seed, (unsigned int)step,
+                                     (const double *)h->fire_p.p, 1, (unsigned long long *)(row + 4), overflow,
+                                     h->stream);
+                if (e == cudaSuccess) fire_cur ^= 1;
+                h->launches += 1;
+            }
+            if (e != cudaSuccess) break;
+        }
         what = "rmvCoveredPOI";
-        if ((e = launch_remove_covered(mult, cls, h->g, xyT, N, (unsigned long long *)(row + 3), h->stream)) != cudaSuccess) break;
+        if ((e = launch_remove_covered(mult, cls, lg, xyT, N, (unsigned long long *)(row + 3), h->stream, d_stamp,
+                                       (int)t)) != cudaSuccess)
+            break;
         what = "repack";
-        if ((e = launch_pack_planes(mult, cls, h->g, (uint32_t *)h->planes.p, h->stream)) != cudaSuccess) break;
-        if (h->g.planes_q && (e = launch_requad_plane(h->g, (uint32_t *)h->planes_q.p, h->stream)) != cudaSuccess) break;
+        if ((e = launch_pack_planes(mult, cls, lg, (uint32_t *)lg.planes, h->stream)) != cudaSuccess) break;
+        if (lg.planes_q && (e = launch_requad_plane(lg, (uint32_t *)lg.planes_q, h->stream)) != cudaSuccess) break;
         hs.t = t;
         what = "horizon_start";
         if ((e = launch_horizon_start(hs, cur, (double *)h->params.p, (double *)a.X0, (double *)a.a0, (int *)a.b0,
@@ -2092,7 +2254,7 @@ extern "C" int cov_run_horizon(cov_handle *h, const double *x_start, int64_t T, 
         unsigned long long *counter = nullptr;
         if ((rc = take_counter(h, &counter)) != COV_OK) break;
         what = "MADS kernel";
-        if ((e = launch_mads(h->g, h->o, cfg, a, counter, h->stream)) != cudaSuccess) break;
+        if ((e = launch_mads(lg, h->o, cfg, a, counter, h->stream)) != cudaSuccess) break;
         what = "horizon_commit";
         if ((e = launch_horizon_commit(S, N, a.X_out, a.obj_out, a.stats, next, row, xyT, h->stream)) != cudaSuccess) break;
         if ((rc = take_counter(h, &counter)) != COV_OK) break;
@@ -2100,35 +2262,51 @@ extern "C" int cov_run_horizon(cov_handle *h, const double *x_start, int64_t T, 
         out.obj = d_oo + (t - 1);
         LaunchInfo li{};
         what = "coverage kernel";
-        if ((e = launch_eval(h->g, h->o, cfg, next, 1, out, counter, h->stream, &li)) != cudaSuccess) break;
-        h->launches += h->g.planes_q ? 7 : 6;
+        if ((e = launch_eval(lg, h->o, cfg, next, 1, out, counter, h->stream, &li)) != cudaSuccess) break;
+        h->launches += lg.planes_q ? 7 : 6;
     }
+    h->fire_cur = fire_cur; // the automaton steps enqueued stand
     if (e == cudaSuccess && rc == COV_OK && step_ms) e = cudaEventRecord(ev[(size_t)T], h->stream), what = "event";
     if (e == cudaSuccess && rc == COV_OK)
         e = cudaMemcpyAsync(h->h_out, d_Xo, res_bytes, cudaMemcpyDeviceToHost, h->stream), what = "download";
-    if (e != cudaSuccess || rc != COV_OK) { // the removals enqueued so far stand: refresh what the host knows of them
+    if (app && e == cudaSuccess && rc == COV_OK)
+        e = cudaMemcpyAsync(&h->h_small->overflow, overflow, sizeof(int), cudaMemcpyDeviceToHost, h->stream);
+    const int n_classes = app ? app->n_classes : h->g.n_classes;
+    const double *cw = app ? app->cw : h->g.class_weight;
+    if (e != cudaSuccess || rc != COV_OK) { // the steps enqueued so far stand: refresh what the host knows of them
         if (rc == COV_OK) rc = fail_cuda(h, e, (std::string(who) + ": " + what).c_str());
         const std::string msg = h->err;
-        entries_note_removals(h);
-        if (rebuild_planes(h, h->g.n_classes, h->g.class_weight) != COV_OK) h->have_grid = false;
+        if (app) entries_forget(h); // the list's per-timestep history is incomplete
+        else entries_note_removals(h);
+        if (rebuild_planes(h, n_classes, cw) != COV_OK) h->have_grid = false;
         for (cudaEvent_t x : ev) h->ev_pool.push_back(x);
         h->err = msg;
         return rc;
     }
-    rc = rebuild_planes(h, h->g.n_classes, h->g.class_weight); // the one synchronise
+    rc = rebuild_planes(h, n_classes, cw); // the one synchronise
+    if (rc == COV_OK && app && h->h_small->overflow)
+        rc = fail(h, COV_ERR_STATE, std::string(who) + ": internal: an append went past the store's envelope");
     const double *hX = (const double *)h->h_out, *hobj = hX + tn;
-    const int64_t *hst = (const int64_t *)(hobj + T);
+    int64_t *hst = (int64_t *)(hobj + T);
+    const int *hstamp = (const int *)((const unsigned char *)h->h_out + o_stamp);
     if (rc == COV_OK) {
-        bool removed = false;
-        for (int64_t t = 0; t < T; ++t) removed |= hst[4 * t + 3] != 0;
-        if (removed) entries_note_removals(h);
+        bool removed = false, pushed = false;
+        for (int64_t t = 0; t < T; ++t) {
+            removed |= hst[cols * t + 3] != 0;
+            if (app && app->offsets) hst[cols * t + 4] = app->offsets[t + 1] - app->offsets[t];
+            if (app) pushed |= hst[cols * t + 4] != 0;
+        }
+        if (app && app->fire_steps && pushed) entries_forget(h); // cov_fire_step: the automaton's order is createPOI's
+        else if (app && app->offsets && h->ent_known) entries_replay(h, *app, T, hstamp);
+        else if (removed) entries_note_removals(h);
         memcpy(X_out, hX, tn * 8);
         if (obj_out) memcpy(obj_out, hobj, (size_t)T * 8);
-        if (stats) memcpy(stats, hst, (size_t)T * 32);
+        if (stats) memcpy(stats, hst, (size_t)T * cols * 8);
+        if (stamps && stamps_out) memcpy(stamps_out, hstamp, ncell * 4);
         for (int64_t t = 0; step_ms && t < T; ++t) {
             float ms = 0;
             if ((e = cudaEventElapsedTime(&ms, ev[(size_t)t], ev[(size_t)t + 1])) != cudaSuccess) {
-                rc = fail_cuda(h, e, "cov_run_horizon: cudaEventElapsedTime");
+                rc = fail_cuda(h, e, (std::string(who) + ": cudaEventElapsedTime").c_str());
                 break;
             }
             step_ms[t] = ms;
@@ -2136,6 +2314,151 @@ extern "C" int cov_run_horizon(cov_handle *h, const double *x_start, int64_t T, 
     }
     for (cudaEvent_t x : ev) h->ev_pool.push_back(x);
     return rc;
+}
+
+extern "C" int cov_run_horizon(cov_handle *h, const double *x_start, int64_t T, int64_t S, double spread,
+                               int64_t n_iter, double granularity, uint64_t seed, const double *boxes, int64_t n_boxes,
+                               double h_focus, double h_max, double *X_out, double *obj_out, int64_t *stats,
+                               double *step_ms)
+{
+    const char *who = "cov_run_horizon";
+    if (!h) return fail(nullptr, COV_ERR_INVALID, "NULL handle");
+    DeviceGuard dg(h->device);
+    OK(check_horizon(h, who, x_start, T, S, spread, n_iter, granularity, boxes, n_boxes, X_out));
+    if (T == 0) return COV_OK;
+    OK(check_mads_limits(h, who, &h->g));
+    return run_horizon(h, who, x_start, T, S, spread, n_iter, granularity, seed, boxes, n_boxes, h_focus, h_max, X_out,
+                       obj_out, stats, step_ms, nullptr, nullptr);
+}
+
+// The cell store's bytes as they are (one download, one synchronise).
+static int download_cells(cov_handle *h, std::vector<unsigned char> &m, std::vector<unsigned char> &k,
+                          std::vector<unsigned char> *fire_state)
+{
+    const size_t ncell = (size_t)h->g.nx * h->g.ny;
+    m.resize(ncell);
+    k.resize(ncell);
+    CK(cudaMemcpyAsync(m.data(), h->mult.p, ncell, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaMemcpyAsync(k.data(), h->cls.p, ncell, cudaMemcpyDeviceToHost, h->stream));
+    if (fire_state) {
+        fire_state->resize(ncell);
+        CK(cudaMemcpyAsync(fire_state->data(), h->fire[h->fire_cur].p, ncell, cudaMemcpyDeviceToHost, h->stream));
+    }
+    CK(cudaStreamSynchronize(h->stream));
+    return COV_OK;
+}
+
+extern "C" int cov_run_horizon_points(cov_handle *h, const double *x_start, int64_t T, int64_t S, double spread,
+                                      int64_t n_iter, double granularity, uint64_t seed, const double *boxes,
+                                      int64_t n_boxes, double h_focus, double h_max, const double *pts5,
+                                      const int64_t *offsets, double *X_out, double *obj_out, int64_t *stats,
+                                      double *step_ms, int *last_removed)
+{
+    const char *who = "cov_run_horizon_points";
+    if (!h) return fail(nullptr, COV_ERR_INVALID, "NULL handle");
+    DeviceGuard dg(h->device);
+    OK(check_horizon(h, who, x_start, T, S, spread, n_iter, granularity, boxes, n_boxes, X_out));
+    if (!offsets || offsets[0] != 0 || T > 0x7fffffffll)
+        return fail(h, COV_ERR_INVALID, "cov_run_horizon_points: offsets must hold T + 1 non-decreasing values from 0");
+    for (int64_t t = 1; t <= T; ++t)
+        if (offsets[t] < offsets[t - 1])
+            return fail(h, COV_ERR_INVALID, "cov_run_horizon_points: offsets must hold T + 1 non-decreasing values from 0");
+    const int64_t P = offsets[T];
+    if (P > 0 && !pts5) return fail(h, COV_ERR_INVALID, "cov_run_horizon_points: pts5 is NULL");
+    if (T == 0) return COV_OK;
+    HorizonAppend app;
+    app.offsets = offsets;
+    app.n_classes = (h->n_entries == 0 && P > 0) ? 0 : h->g.n_classes; // cov_add_points: an empty store has no weight yet
+    for (int k = 0; k < kMaxClasses; ++k) app.cw[k] = h->g.class_weight[k];
+    OK(map_points(h, pts5, P, app.cell, app.pcls, app.n_classes, app.cw));
+    std::vector<unsigned char> m, k;
+    OK(download_cells(h, m, k, nullptr));
+    // every cell's multiplicity bound and class: the store's entries plus all the schedule puts there
+    const size_t ncell = m.size();
+    std::vector<int> bound(m.begin(), m.end());
+    std::vector<unsigned char> bc(ncell, 0xff);
+    for (size_t c = 0; c < ncell; ++c)
+        if (m[c]) bc[c] = k[c] & (kMaxClasses - 1);
+    for (int64_t q = 0; q < P; ++q) {
+        const int c = app.cell[(size_t)q];
+        if (bc[c] == 0xff) bc[c] = app.pcls[(size_t)q];
+        else if (bc[c] != app.pcls[(size_t)q])
+            return fail(h, COV_ERR_INVALID, "cov_run_horizon_points: entries on one cell carry different weights (the "
+                                            "store's and the schedule's, removals ignored)");
+        ++bound[c];
+    }
+    unsigned max_mult[kMaxClasses] = {0, 0, 0, 0};
+    for (size_t c = 0; c < ncell; ++c) {
+        if (bound[c] > 255)
+            return fail(h, COV_ERR_LIMIT, "cov_run_horizon_points: more than 255 list entries on one cell (removals "
+                                          "ignored)");
+        if (bound[c]) max_mult[bc[c]] = std::max(max_mult[bc[c]], (unsigned)bound[c]);
+    }
+    OK(horizon_envelope(h, who, app, max_mult, h->n_entries + P));
+    // the ordered list: removals pending from earlier calls first, and push! appends after the entries already in
+    // the list, whatever setter built it (cov_add_points)
+    entries_apply_removals(h, m.data());
+    if (!h->ent_known && P > 0) {
+        entries_from_cells(h, m.data(), k.data());
+        h->ent_known = true;
+        h->ent_dev_valid = false;
+    }
+    app.stamps = h->ent_known || last_removed;
+    return run_horizon(h, who, x_start, T, S, spread, n_iter, granularity, seed, boxes, n_boxes, h_focus, h_max, X_out,
+                       obj_out, stats, step_ms, &app, last_removed);
+}
+
+extern "C" int cov_run_horizon_fire(cov_handle *h, const double *x_start, int64_t T, int64_t S, double spread,
+                                    int64_t n_iter, double granularity, uint64_t seed, const double *boxes,
+                                    int64_t n_boxes, double h_focus, double h_max, const int64_t *fire_steps,
+                                    double wind_speed, double wind_direction, double prob_spread, uint64_t fire_seed,
+                                    int64_t first_step, double *X_out, double *obj_out, int64_t *stats,
+                                    double *step_ms)
+{
+    const char *who = "cov_run_horizon_fire";
+    if (!h) return fail(nullptr, COV_ERR_INVALID, "NULL handle");
+    DeviceGuard dg(h->device);
+    OK(check_horizon(h, who, x_start, T, S, spread, n_iter, granularity, boxes, n_boxes, X_out));
+    OK(check_fire_store(h, who));
+    if (T > 0 && !fire_steps) return fail(h, COV_ERR_INVALID, "cov_run_horizon_fire: fire_steps is NULL");
+    constexpr int64_t kSteps = 0x100000000ll; // step numbers are 32-bit (cov_fire_step)
+    int64_t total = 0;
+    for (int64_t t = 0; t < T; ++t) {
+        if (fire_steps[t] < 0 || fire_steps[t] > kSteps - total)
+            return fail(h, COV_ERR_INVALID, "cov_run_horizon_fire: fire_steps must be >= 0 with step numbers below 2^32");
+        total += fire_steps[t];
+    }
+    if (first_step < 0 || first_step > kSteps - total)
+        return fail(h, COV_ERR_INVALID, "cov_run_horizon_fire: the steps first_step .. first_step + sum(fire_steps) - 1 "
+                                        "must lie in 0 .. 2^32 - 1");
+    if (T == 0) return COV_OK;
+    std::vector<unsigned char> m, k, st;
+    OK(download_cells(h, m, k, &st));
+    // a TREE cell ignites at most once and pushes at most one entry per burning Moore neighbour (fire_step_kernel)
+    const int nx = h->g.nx, ny = h->g.ny;
+    unsigned max_mult[kMaxClasses] = {0, 0, 0, 0};
+    int64_t trees = 0;
+    for (int j = 1; j <= ny; ++j)
+        for (int i = 1; i <= nx; ++i) {
+            const size_t c = (size_t)(i - 1) + (size_t)nx * (j - 1);
+            const bool tree = total > 0 && st[c] == 1 && i >= 2 && i <= nx - 1 && j >= 2 && j <= ny - 1;
+            const unsigned b = m[c] + (tree ? 8u : 0u);
+            trees += tree ? 1 : 0;
+            if (b > 255)
+                return fail(h, COV_ERR_LIMIT, "cov_run_horizon_fire: more than 255 list entries on one cell (removals "
+                                              "ignored)");
+            max_mult[0] = std::max(max_mult[0], b);
+        }
+    HorizonAppend app;
+    app.n_classes = 1;
+    app.cw[0] = h->g.class_weight[0];
+    OK(horizon_envelope(h, who, app, max_mult, h->n_entries + 8 * trees));
+    app.fire_steps = fire_steps;
+    app.fire_seed = fire_seed;
+    app.first_step = first_step;
+    fire_probs(wind_speed, wind_direction, prob_spread, h->h_small->fire_p);
+    return run_horizon(h, who, x_start, T, S, spread, n_iter, granularity, seed, boxes, n_boxes, h_focus, h_max, X_out,
+                       obj_out, stats, step_ms, &app, nullptr);
 }
 
 extern "C" int cov_argmin(cov_handle *h, const double *X, int64_t B, int32_t barrier, double *best_obj,

@@ -176,8 +176,10 @@ __device__ __forceinline__ bool cell_covered(const GridDesc &g, int i1, int j1, 
     return false;
 }
 
+// stamp (nullable): stamp[cell] = t for every cell that loses entries (cov_run_horizon_points' last_removed)
 __global__ void remove_covered_kernel(unsigned char *mult, unsigned char *cls, const __grid_constant__ GridDesc g,
-                                      const double *__restrict__ xyT, int N, unsigned long long *removed)
+                                      const double *__restrict__ xyT, int N, unsigned long long *removed, int *stamp,
+                                      int t_stamp)
 {
     const long long ncell = (long long)g.nx * g.ny;
     unsigned long long mine = 0;
@@ -190,6 +192,7 @@ __global__ void remove_covered_kernel(unsigned char *mult, unsigned char *cls, c
                 mine += m;
                 mult[t] = 0;
                 cls[t] = 0xffu;
+                if (stamp) stamp[t] = t_stamp;
             }
         }
     }
@@ -197,14 +200,14 @@ __global__ void remove_covered_kernel(unsigned char *mult, unsigned char *cls, c
     if ((threadIdx.x & 31) == 0 && mine) atomicAdd(removed, mine);
 }
 cudaError_t launch_remove_covered(unsigned char *mult, unsigned char *cls, const GridDesc &g, const double *xyT, int N,
-                                  unsigned long long *removed, cudaStream_t s)
+                                  unsigned long long *removed, cudaStream_t s, int *stamp, int t_stamp)
 {
     cudaError_t e = cudaMemsetAsync(removed, 0, sizeof(unsigned long long), s);
     if (e != cudaSuccess) return e;
     const long long ncell = (long long)g.nx * g.ny;
     const int block = 256;
     const int grid = (int)std::min<long long>((ncell + block - 1) / block, 148 * 8);
-    remove_covered_kernel<<<max(grid, 1), block, 0, s>>>(mult, cls, g, xyT, N, removed);
+    remove_covered_kernel<<<max(grid, 1), block, 0, s>>>(mult, cls, g, xyT, N, removed, stamp, t_stamp);
     return cudaGetLastError();
 }
 

@@ -111,9 +111,10 @@ cudaError_t launch_requad_plane(const GridDesc &g, uint32_t *planes_q, cudaStrea
 cudaError_t launch_fill_full(unsigned char *mult, unsigned char *cls, long long ncell, cudaStream_t s);
 cudaError_t launch_bits_to_cells(const uint32_t *bits, int nx, int ny, unsigned char *mult,
                                  unsigned char *cls, cudaStream_t s);
-// xyT: 3N doubles on the device: cx[N], cy[N], T[N]. removed: one unsigned long long.
+// xyT: 3N doubles on the device: cx[N], cy[N], T[N]. removed: one unsigned long long.  stamp (nullable, nx*ny ints):
+// stamp[cell] = t_stamp for every cell whose entries are removed.
 cudaError_t launch_remove_covered(unsigned char *mult, unsigned char *cls, const GridDesc &g, const double *xyT, int N,
-                                  unsigned long long *removed, cudaStream_t s);
+                                  unsigned long long *removed, cudaStream_t s, int *stamp = nullptr, int t_stamp = 0);
 cudaError_t launch_normalize_cls(const unsigned char *mult, unsigned char *cls, long long ncell, cudaStream_t s);
 cudaError_t launch_covered_mask(unsigned char *mask, const GridDesc &g, const double *xyT, int N,
                                 cudaStream_t s);

@@ -352,6 +352,40 @@ class CoverageEngine:
         the next swarm.  Needs set_params with prev_xyR.  Returns (X (T, 3N), obj (T,), stats, step_ms (T,)) with
         stats a dict of int64 arrays: winner, evaluations, feasible, removed.  The r_max and previous swarm of the
         last timestep stay set on the engine."""
+        return self._horizon(lib.cov_run_horizon, x_start, T, 4, S, spread, n_iter, granularity, seed, boxes, h_focus,
+                             h_max, ())
+
+    def run_horizon_points(self, x_start, appends, S: int = 1, spread: float = 3.0, n_iter: int = 100,
+                           granularity: float = 1.0, seed: int = 0, boxes=None, h_focus: float = 15.0,
+                           h_max: float = 30.0):
+        """run_horizon with the reference's fire list (cov_run_horizon_points): appends is a list of T arrays
+        (n_t x 5 reference 5-tuples), timestep t appending appends[t-1] before its rmvCoveredPOI (update_POI's push!).
+        Returns (X, obj, stats, step_ms, last_removed): stats gains "appended"; last_removed (nx*ny int32, indexed
+        (i-1) + nx*(j-1)) holds the last timestep that removed entries from each cell, 0 if none."""
+        rows = [_f64(a).reshape(-1, 5) for a in appends]
+        offsets = np.zeros(len(rows) + 1, dtype=np.int64)
+        offsets[1:] = np.cumsum([r.shape[0] for r in rows], dtype=np.int64)
+        pts = np.concatenate(rows) if offsets[-1] else None
+        gi = self.grid_info()
+        last = np.zeros(gi["nx"] * gi["ny"], dtype=np.int32)
+        out = self._horizon(lib.cov_run_horizon_points, x_start, len(rows), 5, S, spread, n_iter, granularity, seed,
+                            boxes, h_focus, h_max, (_ptr(pts), _ptr(offsets)), (_ptr(last),))
+        return out + (last,)
+
+    def run_horizon_fire(self, x_start, fire_steps, wind_speed: float, wind_direction: float, prob_spread: float,
+                         fire_seed: int, first_step: int, S: int = 1, spread: float = 3.0, n_iter: int = 100,
+                         granularity: float = 1.0, seed: int = 0, boxes=None, h_focus: float = 15.0,
+                         h_max: float = 30.0):
+        """run_horizon with the device automaton (cov_run_horizon_fire): timestep t first runs fire_steps[t-1] steps
+        of fire_step(append=True), numbered from first_step.  Returns (X, obj, stats, step_ms) with stats["appended"]
+        the entries each timestep's steps pushed."""
+        fs = np.ascontiguousarray(fire_steps, dtype=np.int64).ravel()
+        return self._horizon(lib.cov_run_horizon_fire, x_start, fs.size, 5, S, spread, n_iter, granularity, seed,
+                             boxes, h_focus, h_max, (_ptr(fs), float(wind_speed), float(wind_direction),
+                                                     float(prob_spread), int(fire_seed) & (2**64 - 1), int(first_step)))
+
+    def _horizon(self, fn, x_start, T, cols, S, spread, n_iter, granularity, seed, boxes, h_focus, h_max, source,
+                 tail=()):
         x_start = _f64(x_start).ravel()
         if self.N is None or x_start.size != 3 * self.N:
             raise ValueError("x_start must have 3N entries")
@@ -359,14 +393,13 @@ class CoverageEngine:
         T = int(T)
         X = np.empty((max(T, 0), 3 * self.N))
         obj = np.empty(max(T, 0))
-        st = np.empty((max(T, 0), 4), dtype=np.int64)
+        st = np.empty((max(T, 0), cols), dtype=np.int64)
         ms = np.empty(max(T, 0))
         self.param_owner = None  # r_max and the previous swarm change on the device
-        self._check(lib.cov_run_horizon(self._h, _ptr(x_start), T, int(S), float(spread), int(n_iter),
-                                        float(granularity), int(seed) & (2**64 - 1), _ptr(B) if len(B) else None,
-                                        len(B), float(h_focus), float(h_max), _ptr(X), _ptr(obj), _ptr(st),
-                                        _ptr(ms)))
-        names = ("winner", "evaluations", "feasible", "removed")
+        self._check(fn(self._h, _ptr(x_start), T, int(S), float(spread), int(n_iter), float(granularity),
+                       int(seed) & (2**64 - 1), _ptr(B) if len(B) else None, len(B), float(h_focus), float(h_max),
+                       *source, _ptr(X), _ptr(obj), _ptr(st), _ptr(ms), *tail))
+        names = ("winner", "evaluations", "feasible", "removed", "appended")[:cols]
         return X, obj, {name: st[:, q].copy() for q, name in enumerate(names)}, ms
 
     # ---- grid-free static objective ----

@@ -308,6 +308,60 @@ function run_horizon(h::Handle, x_start::Vector{Float64}; T, S = 1, spread = 3.0
 end
 
 """
+    run_horizon_points(h, x_start, appends; S = 1, spread = 3.0, N_iter = 100, granularity = 1.0, seed = 0,
+                       boxes = zeros(Float64, 4, 0), h_focus = 15.0, h_max = 30.0, nx = 100, ny = 100)
+
+`run_horizon` with the reference's fire list (`cov_run_horizon_points`): `appends` holds T matrices of reference
+points (5 x n_t, columns [x; y; area; weight; covered]), timestep t appending `appends[t]` before its rmvCoveredPOI
+(update_POI's push!). Returns `(X, objectives, stats, step_ms, last_removed)`: `stats` 5 x T with the entries appended
+as row 5, `last_removed` (nx*ny of the store's lattice, index (i-1) + nx*(j-1)) the last timestep that removed entries
+from each cell (0: none).
+"""
+function run_horizon_points(h::Handle, x_start::Vector{Float64}, appends::Vector{Matrix{Float64}}; S = 1,
+                            spread = 3.0, N_iter = 100, granularity = 1.0, seed = 0,
+                            boxes::Matrix{Float64} = zeros(Float64, 4, 0), h_focus = 15.0, h_max = 30.0, nx = 100,
+                            ny = 100)
+    T = length(appends); n = length(x_start); K = size(boxes, 2)
+    offsets = zeros(Int64, T + 1)
+    for t in 1:T
+        offsets[t + 1] = offsets[t] + size(appends[t], 2)
+    end
+    pts = T == 0 ? zeros(Float64, 5, 0) : reduce(hcat, appends)  # column p = the 5-tuple of entry p
+    last = zeros(Cint, nx * ny)
+    X = zeros(Float64, n, T); obj = zeros(Float64, T); stats = zeros(Int64, 5, T); ms = zeros(Float64, T)
+    GC.@preserve x_start boxes pts offsets X obj stats ms last check(h, ccall((:cov_run_horizon_points, LIB), Cint,
+        (Ptr{Cvoid}, Ptr{Float64}, Int64, Int64, Float64, Int64, Float64, UInt64, Ptr{Float64}, Int64, Float64,
+         Float64, Ptr{Float64}, Ptr{Int64}, Ptr{Float64}, Ptr{Float64}, Ptr{Int64}, Ptr{Float64}, Ptr{Cint}),
+        h.ptr, x_start, T, S, spread, N_iter, granularity, seed, K == 0 ? C_NULL : pointer(boxes), K, h_focus, h_max,
+        offsets[end] == 0 ? C_NULL : pointer(pts), offsets, X, obj, stats, ms, last))
+    return X, obj, stats, ms, last
+end
+
+"""
+    run_horizon_fire(h, x_start, fire_steps; wind_speed = 4.0, wind_direction = deg2rad(270.0), prob_spread = 0.5,
+                     fire_seed = 0, first_step = 1, S = 1, spread = 3.0, N_iter = 100, granularity = 1.0, seed = 0,
+                     boxes = zeros(Float64, 4, 0), h_focus = 15.0, h_max = 30.0)
+
+`run_horizon` with the device forest-fire automaton (`cov_run_horizon_fire`, after `fire_init!`): timestep t first
+runs `fire_steps[t]` automaton steps with append, numbered from `first_step`. Returns `(X, objectives, stats,
+step_ms)` with `stats` 5 x T, row 5 the entries each timestep's steps pushed.
+"""
+function run_horizon_fire(h::Handle, x_start::Vector{Float64}, fire_steps::Vector{Int64}; wind_speed = 4.0,
+                          wind_direction = deg2rad(270.0), prob_spread = 0.5, fire_seed = 0, first_step = 1, S = 1,
+                          spread = 3.0, N_iter = 100, granularity = 1.0, seed = 0,
+                          boxes::Matrix{Float64} = zeros(Float64, 4, 0), h_focus = 15.0, h_max = 30.0)
+    T = length(fire_steps); n = length(x_start); K = size(boxes, 2)
+    X = zeros(Float64, n, T); obj = zeros(Float64, T); stats = zeros(Int64, 5, T); ms = zeros(Float64, T)
+    GC.@preserve x_start boxes fire_steps X obj stats ms check(h, ccall((:cov_run_horizon_fire, LIB), Cint,
+        (Ptr{Cvoid}, Ptr{Float64}, Int64, Int64, Float64, Int64, Float64, UInt64, Ptr{Float64}, Int64, Float64,
+         Float64, Ptr{Int64}, Float64, Float64, Float64, UInt64, Int64, Ptr{Float64}, Ptr{Float64}, Ptr{Int64},
+         Ptr{Float64}),
+        h.ptr, x_start, T, S, spread, N_iter, granularity, seed, K == 0 ? C_NULL : pointer(boxes), K, h_focus, h_max,
+        fire_steps, wind_speed, wind_direction, prob_spread, fire_seed, first_step, X, obj, stats, ms))
+    return X, obj, stats, ms
+end
+
+"""
     set_region!(h, x_lo, y_lo, x_hi, y_hi, covered)
 
 The grid-free static objective's region: the domain rectangle and the discs already covered, `covered` a 3 x M
