@@ -38,7 +38,8 @@ extern "C" {
                              3: cov_eval_batch_packed (COV_PACK_*); later, with no existing symbol changed:
                                 cov_mads_solve_batch; cov_set_region, cov_eval_region_batch,
                                 cov_mads_solve_batch_region (the grid-free static objective); cov_run_horizon;
-                                cov_run_horizon_points, cov_run_horizon_fire (the dynamic horizon) */
+                                cov_run_horizon_points, cov_run_horizon_fire (the dynamic horizon);
+                                cov_run_horizon_ensemble, cov_multi_run_horizon_ensemble */
 
 #if defined(__GNUC__)
 #define COV_API __attribute__((visibility("default")))
@@ -376,6 +377,30 @@ COV_API int cov_run_horizon_fire(cov_handle *h, const double *x_start, int64_t T
                                  double prob_spread, uint64_t fire_seed, int64_t first_step,
                                  double *X_out, double *obj_out, int64_t *stats, double *step_ms);
 
+/* E independent static receding horizons in one call, on the device side by side: scenario e (0 <= e < E) is exactly
+ * cov_run_horizon(x_starts + e * 3N, T, S, spread, n_iter, granularity, seed + e * T * S (mod 2^64), boxes, ...) run on
+ * a private copy of the handle's current cell store and parameters.  Solve k of timestep t of scenario e is keyed by
+ * seed + e * T * S + (t - 1) * S + k, so the scenarios' keys are disjoint and a scenario's results do not depend on E
+ * or on the other scenarios.  Static environment only (no append step).  Every step of a timestep is one launch for
+ * the whole ensemble.
+ *
+ * x_starts: E x 3N.  X_out: E x T x 3N; obj_out (nullable): E x T; stats (nullable): E x T x 4 with cov_run_horizon's
+ * columns [winner k, evaluations, feasible solves, entries removed]; step_ms (nullable): T device times of the whole
+ * ensemble per timestep; cells_out (nullable): E x nx*ny bytes, row e the multiplicities scenario e leaves (what
+ * cov_get_grid_cells returns after the equivalent cov_run_horizon).
+ *
+ * The handle is not changed: unlike cov_run_horizon, which consumes the store, the cell store, cov_get_grid_info, the
+ * class weights, the parameters (r_max and the previous swarm), the ordered point list and the automaton's state are
+ * as before the call.  cov_launch_count counts the launches; cov_last_launch and the kernel timers are left unchanged.
+ * Errors: cov_run_horizon's, in its order; COV_ERR_INVALID also for E < 1, E * S > 2^31 - 1 or E * T * S > 2^63 - 1;
+ * a failed device allocation as the other calls report it.  T == 0 does nothing, and a refused or failed call changes
+ * nothing on the handle. */
+COV_API int cov_run_horizon_ensemble(cov_handle *h, const double *x_starts, int64_t E, int64_t T, int64_t S,
+                                     double spread, int64_t n_iter, double granularity, uint64_t seed,
+                                     const double *boxes, int64_t n_boxes, double h_focus, double h_max,
+                                     double *X_out, double *obj_out, int64_t *stats, double *step_ms,
+                                     uint8_t *cells_out);
+
 /* Covered-cell mask of ONE candidate: nx*ny bytes, 1 where the cell is inside some disc (whether
  * or not it holds entries). Lets the host replay an ordered Float64 sum over a weighted list. */
 COV_API int cov_covered_mask(cov_handle *h, const double *x, uint8_t *mask);
@@ -475,6 +500,13 @@ COV_API int cov_multi_size(const cov_multi *m);
 COV_API cov_handle *cov_multi_handle(cov_multi *m, int k); /* borrow shard k's handle (set grid/params on each) */
 COV_API int cov_multi_eval_batch(cov_multi *m, const double *X, int64_t B, double *obj, int64_t *count,
                          uint8_t *feasible);
+/* cov_run_horizon_ensemble over the devices (without step_ms): contiguous shards of scenarios (ceil(E / G) each),
+ * shard k from scenario b0 on with seed + b0 * T * S, so its results equal the single-device call's bit for bit.  Set
+ * the same store and parameters on every shard's handle (cov_multi_handle). */
+COV_API int cov_multi_run_horizon_ensemble(cov_multi *m, const double *x_starts, int64_t E, int64_t T, int64_t S,
+                                           double spread, int64_t n_iter, double granularity, uint64_t seed,
+                                           const double *boxes, int64_t n_boxes, double h_focus, double h_max,
+                                           double *X_out, double *obj_out, int64_t *stats, uint8_t *cells_out);
 COV_API int cov_multi_argmin(cov_multi *m, const double *X, int64_t B, int32_t barrier, double *best_obj,
                      int64_t *best_idx);
 

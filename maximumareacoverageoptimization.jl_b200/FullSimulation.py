@@ -170,3 +170,37 @@ def _run_horizon(cells, pre, cons_ext, N, r_max, p, steps, S, spread, t_half, d_
         apply_r_max_rule(X[t - 2], r_max, N, p, t_half)
     inputs = [pre.copy()] + [X[t].copy() for t in range(steps - 1)]
     return inputs, [x.copy() for x in X], [float(ms) / 1e3 for ms in step_ms], [float(v) for v in objs]
+
+
+def run_simulation_ensemble(cells, starting_swarms, cons_ext, N, r_max, params: SimulationParameters,
+                            Nt_sim: int | None = None, starts: int = 1, spread: float = 3.0):
+    """run_simulation(starts=S) from E starting swarms at once, in one cov_run_horizon_ensemble call: scenario e is
+    run_simulation(starts=S) from starting_swarms[e] with params.seed + e * Nt_sim * S (base seed 0 when params.seed is
+    None).  Static environment only.  Returns a list of E tuples (single_input_pb, single_output_pb,
+    runtime_data_MADS, objective_pb), each what run_simulation(starts=S) returns for that scenario, except that
+    runtime_data_MADS holds the device time of each timestep of the whole ensemble.  Unlike run_simulation, cells (its
+    point list and the store on the device) and the caller's r_max are left untouched."""
+    from .mads import _flatten_constraints
+    p = params
+    if p.environment_type != "static":
+        raise ValueError("run_simulation_ensemble runs the static environment only")
+    pres = [np.ascontiguousarray(s if not hasattr(s[0], "x") else ACC.make_MADS(s), dtype=np.float64)
+            for s in starting_swarms]
+    if not pres:
+        raise ValueError("starting_swarms must hold at least one swarm")
+    d_lim = p.d_lim * np.ones(N)
+    steps = p.Nt_sim if Nt_sim is None else Nt_sim
+    S = int(starts)
+    if not len(_boxes(p)):
+        raise ValueError("starts= needs at least one high-interest rectangle")
+    obj = TDM_STATIC_opt.createObjective(cells, N, np.array(r_max, dtype=np.float64))
+    for pre in pres:  # the last one's cons3 stays set; every timestep replaces the previous swarm on the device
+        if obj.native_batch_solver(_flatten_constraints([cons_ext, create_cons3(pre, p.FOV, d_lim)])) is None:
+            raise ValueError("starts= needs constraints that all fuse into the objective's launch")
+    _, eng = obj._engine()
+    X, objs, _, step_ms = eng.run_horizon_ensemble(np.stack(pres), steps, S=S, spread=spread, n_iter=p.N_iter,
+                                                   granularity=1.0, seed=0 if p.seed is None else p.seed,
+                                                   boxes=_boxes(p), h_focus=H_FOCUS, h_max=p.h_max)
+    runtime = [float(ms) / 1e3 for ms in step_ms]
+    return [([pre.copy()] + [Xe[t].copy() for t in range(steps - 1)], [x.copy() for x in Xe], list(runtime),
+             [float(v) for v in oe]) for pre, Xe, oe in zip(pres, X, objs)]

@@ -193,6 +193,8 @@ struct cov_handle {
     DevBuf dX, d_obj, d_count, d_feas, d_clscnt, d_prog;
     DevBuf d_raw[2]; // packed slices as they arrive (cov_eval_batch_packed), widened into dX
     DevBuf mads_in, mads_out; // cov_mads_solve_batch: starts, initial meshes, powers of ten / results
+    DevBuf ens;               // cov_run_horizon_ensemble: the scenarios' stores, plane sets, parameters and thresholds
+                              // (E times the store: freed when the call ends, never kept between calls)
     void *h_in[2] = {nullptr, nullptr};
     size_t h_in_cap = 0;
     void *h_out = nullptr;
@@ -446,7 +448,7 @@ extern "C" void cov_destroy(cov_handle *h)
                       &h->small_in, &h->argmin_obj, &h->argmin_idx, &h->removed, &h->overflow, &h->dX,
                       &h->d_obj, &h->d_count, &h->d_feas, &h->d_clscnt, &h->d_prog, &h->fire[0], &h->fire[1], &h->fire_p,
                       &h->backup, &h->ent_cell, &h->ent_cls, &h->d_raw[0], &h->d_raw[1], &h->mads_in, &h->mads_out,
-                      &h->region_discs, &h->region_arcs, &h->region_count, &h->d_area};
+                      &h->ens, &h->region_discs, &h->region_arcs, &h->region_count, &h->d_area};
     for (DevBuf *b : bufs)
         if (b->p) cudaFree(b->p);
     for (int k = 0; k < 2; ++k)
@@ -2121,40 +2123,69 @@ static void entries_replay(cov_handle *h, const HorizonAppend &app, int64_t T, c
     h->ent_dev_valid = false;
 }
 
+// The scenarios of cov_run_horizon_ensemble (run_horizon; NULL: one scenario on the handle's own store): E copies of
+// the handle's store and parameters, made on the device when the call starts and dropped when it ends.
+struct HorizonEnsemble {
+    int64_t E = 1;
+    uint8_t *cells_out = nullptr; // E x nx*ny (nullable): the multiplicities each scenario leaves
+};
+
+// E copies of `bytes` bytes at src side by side at dst (device memory), in 1 + ceil(log2(E)) copies.
+static cudaError_t replicate(void *dst, const void *src, size_t bytes, int64_t E, cudaStream_t s)
+{
+    cudaError_t e = cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToDevice, s);
+    for (int64_t have = 1; have < E && e == cudaSuccess; have *= 2)
+        e = cudaMemcpyAsync((char *)dst + (size_t)have * bytes, dst, (size_t)std::min(have, E - have) * bytes,
+                            cudaMemcpyDeviceToDevice, s);
+    return e;
+}
+
 // T >= 1 timesteps of FullSimulation.py's MADS loop (lines 72-107) with S starts per timestep, all enqueued before the
 // one synchronise at the end (arguments and solver limits checked by the caller).  Per timestep: the append step of
 // app (update_POI's push! or the automaton), rmvCoveredPOI of cur into the stats row, the bit planes repacked (the
 // plane set stays fixed: removals only clear multiplicities, and app's envelope holds every append), the r_max rule /
 // cons3's previous swarm / the starts (horizon_start_kernel), S solves (launch_mads), the winner to cur
 // (horizon_commit_kernel), AreaMaxObjective(cur).  stamps_out (nullable, nx*ny): app's removal stamps.
+// ens: the same loop over ens->E scenarios side by side (one launch per step for all of them) on copies of the store
+// and parameters; x_start and the outputs then hold E scenarios, each of them as the single call lays it out.
 static int run_horizon(cov_handle *h, const char *who, const double *x_start, int64_t T, int64_t S, double spread,
                        int64_t n_iter, double granularity, uint64_t seed, const double *boxes, int64_t n_boxes,
                        double h_focus, double h_max, double *X_out, double *obj_out, int64_t *stats, double *step_ms,
-                       HorizonAppend *app, int *stamps_out)
+                       HorizonAppend *app, int *stamps_out, const HorizonEnsemble *ens = nullptr)
 {
     GridDesc lg = app ? app->g : h->g;
+    const int64_t E = ens ? ens->E : 1;
     const int N = h->o.N, n = 3 * N, cols = app ? 5 : 4;
     const size_t ncell = (size_t)h->g.nx * h->g.ny, P = app ? app->cell.size() : 0;
     const bool stamps = app && app->stamps;
-    // in: [pow10 | x_start: n | boxes: 4 n_boxes | appended cells: P ints | their classes: P bytes | the solves' inputs]
-    // out: [the solves' outputs | X_out: T n | obj_out: T | stats: T x cols | removal stamps: nx*ny ints]
-    const size_t tn = (size_t)T * n;
-    const size_t o_x = kPow10Bytes, o_box = o_x + (size_t)n * 8, o_cell = o_box + (size_t)n_boxes * 32;
+    // in: [pow10 | x_start: E n | boxes: 4 n_boxes | appended cells: P ints | their classes: P bytes | the solves'
+    // inputs]; out: [the solves' outputs | X_out: T E n | obj_out: T E | stats: T E cols | removal stamps: nx*ny ints],
+    // timestep-major (a timestep's rows side by side); pinned: [the out rows after the solves' | the cells: E nx*ny]
+    const size_t tn = (size_t)T * E * n;
+    const size_t o_x = kPow10Bytes, o_box = o_x + (size_t)E * n * 8, o_cell = o_box + (size_t)n_boxes * 32;
     const size_t o_cls = o_cell + P * 4, o_X0 = (o_cls + P + 7) / 8 * 8;
-    const size_t o_stamp = tn * 8 + (size_t)T * 8 + (size_t)T * cols * 8;
+    const size_t o_stamp = tn * 8 + (size_t)T * E * 8 + (size_t)T * E * cols * 8;
     const size_t res_bytes = o_stamp + (stamps ? ncell * 4 : 0);
+    const size_t cells_bytes = ens && ens->cells_out ? (size_t)E * ncell : 0;
     std::vector<unsigned char> hin(o_X0);
     MadsArgs a;
-    OK(mads_buffers(h, o_X0, S, n, res_bytes, hin, a));
-    memcpy(hin.data() + o_x, x_start, (size_t)n * 8);
+    OK(mads_buffers(h, o_X0, E * S, n, res_bytes, hin, a));
+    memcpy(hin.data() + o_x, x_start, (size_t)E * n * 8);
     if (n_boxes) memcpy(hin.data() + o_box, boxes, (size_t)n_boxes * 32);
     if (P) {
         memcpy(hin.data() + o_cell, app->cell.data(), P * 4);
         memcpy(hin.data() + o_cls, app->pcls.data(), P);
     }
-    OK(ensure(h, h->xyT, (size_t)n * 8));
-    OK(ensure_pinned(h, &h->h_out, &h->h_out_cap, res_bytes));
-    const size_t q_bytes = ((size_t)h->g.ny * h->g.qstride + 8) * 4;
+    // the scenarios' device state: [mult: E nx*ny | cls: E nx*ny | plane sets: E | the single-plane swizzled copy, for
+    // E = 1 (launch_eval's CTA kernel may read it; the E > 1 kernels read the packed planes) | parameters: E 5N |
+    // thresholds: E 3N]
+    const size_t pw = (size_t)lg.n_planes * lg.plane_words * 4, q_bytes = ((size_t)h->g.ny * h->g.qstride + 8) * 4;
+    const bool quad = lg.planes_q && E == 1;
+    const size_t o_epl = ((size_t)2 * E * ncell + 15) / 16 * 16, o_eq = o_epl + (size_t)E * pw;
+    const size_t o_epar = o_eq + (quad ? q_bytes : 0), o_exyT = o_epar + (size_t)E * 5 * N * 8;
+    if (ens) OK(ensure(h, h->ens, o_exyT + (size_t)E * n * 8));
+    else OK(ensure(h, h->xyT, (size_t)n * 8));
+    OK(ensure_pinned(h, &h->h_out, &h->h_out_cap, res_bytes + cells_bytes));
     if (app) { // the envelope's planes; rebuild_planes sizes them for the store again at the end
         int rc = ensure(h, h->planes, (size_t)lg.n_planes * lg.plane_words * 4);
         if (rc == COV_OK && lg.n_planes == 1) rc = ensure(h, h->planes_q, q_bytes);
@@ -2171,8 +2202,25 @@ static int run_horizon(cov_handle *h, const char *who, const double *x_start, in
     const double *d_x0 = (const double *)(din + o_x);
     const int *d_cell = (const int *)(din + o_cell);
     const unsigned char *d_cls = din + o_cls;
-    double *d_Xo = (double *)(a.stats + 4 * S), *d_oo = d_Xo + tn, *xyT = (double *)h->xyT.p;
-    long long *d_st = (long long *)(d_oo + T);
+    double *d_Xo = (double *)(a.stats + 4 * E * S), *d_oo = d_Xo + tn, *xyT = (double *)h->xyT.p;
+    long long *d_st = (long long *)(d_oo + T * E);
+    unsigned char *mult = (unsigned char *)h->mult.p, *cls = (unsigned char *)h->cls.p;
+    double *params = (double *)h->params.p;
+    ObjParams o = h->o;
+    if (ens) {
+        unsigned char *eb = (unsigned char *)h->ens.p;
+        mult = eb;
+        cls = eb + (size_t)E * ncell;
+        lg.planes = (const uint32_t *)(eb + o_epl);
+        lg.planes_q = quad ? (const uint32_t *)(eb + o_eq) : nullptr;
+        params = (double *)(eb + o_epar);
+        xyT = (double *)(eb + o_exyT);
+        o.r_max = params; // scenario e's block at e * 5N (the kernels shift these by it)
+        o.prev_x = params + N;
+        o.prev_y = params + 2 * N;
+        o.prev_z = params + 3 * N;
+        o.cons3_G = params + 4 * N;
+    }
     int *d_stamp = stamps ? (int *)((unsigned char *)d_Xo + o_stamp) : nullptr;
     a.n_iter = n_iter;
     a.granularity = granularity;
@@ -2181,9 +2229,11 @@ static int run_horizon(cov_handle *h, const char *who, const double *x_start, in
     hs.N = N;
     hs.n_boxes = (int)n_boxes;
     hs.S = S;
+    hs.E = E;
     hs.spread = spread;
     hs.granularity = granularity;
     hs.seed = seed;
+    hs.seed_stride = (uint64_t)T * (uint64_t)S;
     hs.pow10 = a.pow10;
     hs.boxes = (const double *)(din + o_box);
     hs.h_focus = h_focus;
@@ -2192,7 +2242,6 @@ static int run_horizon(cov_handle *h, const char *who, const double *x_start, in
     LaunchCfg cfg = h->cfg; // a dyadic store: every kernel gives the list-order sum, the stale device list is not needed
     cfg.ordered = 0;
     if (cfg.kernel == COV_KERNEL_ORDERED) cfg.kernel = COV_KERNEL_AUTO;
-    unsigned char *mult = (unsigned char *)h->mult.p, *cls = (unsigned char *)h->cls.p;
     int *overflow = (int *)h->overflow.p;
     int fire_cur = h->fire_cur;
     int64_t step = app ? app->first_step : 0;
@@ -2202,7 +2251,14 @@ static int run_horizon(cov_handle *h, const char *who, const double *x_start, in
 
     cudaError_t e = cudaMemcpyAsync(din, hin.data(), o_X0, cudaMemcpyHostToDevice, h->stream);
     const char *what = "upload";
-    if (e == cudaSuccess) e = launch_thresholds(d_x0, N, xyT, h->stream), what = "launch_thresholds";
+    if (ens && e == cudaSuccess) { // the scenarios start from the handle's store and parameters
+        what = "scenario copies";
+        e = replicate(mult, h->mult.p, ncell, E, h->stream);
+        if (e == cudaSuccess) e = replicate(cls, h->cls.p, ncell, E, h->stream);
+        if (e == cudaSuccess) e = replicate(params, h->params.p, (size_t)5 * N * 8, E, h->stream);
+        if (e == cudaSuccess && quad) e = cudaMemsetAsync((void *)lg.planes_q, 0, q_bytes, h->stream);
+    }
+    if (e == cudaSuccess) e = launch_thresholds(d_x0, N, xyT, h->stream, E), what = "launch_thresholds";
     h->launches += 1;
     if (app && e == cudaSuccess) {
         what = "append setup";
@@ -2214,9 +2270,9 @@ static int run_horizon(cov_handle *h, const char *who, const double *x_start, in
     }
     int rc = COV_OK;
     for (int64_t t = 1; t <= T && e == cudaSuccess && rc == COV_OK; ++t) {
-        const double *cur = t == 1 ? d_x0 : d_Xo + (size_t)(t - 2) * n;
-        double *next = d_Xo + (size_t)(t - 1) * n;
-        long long *row = d_st + cols * (t - 1);
+        const double *cur = t == 1 ? d_x0 : d_Xo + (size_t)(t - 2) * E * n;
+        double *next = d_Xo + (size_t)(t - 1) * E * n;
+        long long *row = d_st + cols * E * (t - 1);
         if (step_ms && (e = cudaEventRecord(ev[(size_t)t - 1], h->stream)) != cudaSuccess) break;
         if (app && app->offsets) { // update_POI: this timestep's rows of the fire list
             const int64_t q0 = app->offsets[t - 1], q1 = app->offsets[t];
@@ -2240,41 +2296,57 @@ static int run_horizon(cov_handle *h, const char *who, const double *x_start, in
         }
         what = "rmvCoveredPOI";
         if ((e = launch_remove_covered(mult, cls, lg, xyT, N, (unsigned long long *)(row + 3), h->stream, d_stamp,
-                                       (int)t)) != cudaSuccess)
+                                       (int)t, E, cols)) != cudaSuccess)
             break;
         what = "repack";
-        if ((e = launch_pack_planes(mult, cls, lg, (uint32_t *)lg.planes, h->stream)) != cudaSuccess) break;
+        if ((e = launch_pack_planes(mult, cls, lg, (uint32_t *)lg.planes, h->stream, E)) != cudaSuccess) break;
         if (lg.planes_q && (e = launch_requad_plane(lg, (uint32_t *)lg.planes_q, h->stream)) != cudaSuccess) break;
         hs.t = t;
         what = "horizon_start";
-        if ((e = launch_horizon_start(hs, cur, (double *)h->params.p, (double *)a.X0, (double *)a.a0, (int *)a.b0,
-                                      h->stream)) != cudaSuccess)
+        if ((e = launch_horizon_start(hs, cur, params, (double *)a.X0, (double *)a.a0, (int *)a.b0, h->stream)) !=
+            cudaSuccess)
             break;
         a.seed = seed + (uint64_t)(t - 1) * (uint64_t)S;
         unsigned long long *counter = nullptr;
         if ((rc = take_counter(h, &counter)) != COV_OK) break;
         what = "MADS kernel";
-        if ((e = launch_mads(lg, h->o, cfg, a, counter, h->stream)) != cudaSuccess) break;
+        // one scenario: mads_kernel, its planes staged in shared memory once per CTA
+        e = E == 1 ? launch_mads(lg, o, cfg, a, counter, h->stream)
+                   : launch_scenario_mads(lg, o, cfg, a, S, hs.seed_stride, counter, h->stream);
+        if (e != cudaSuccess) break;
         what = "horizon_commit";
-        if ((e = launch_horizon_commit(S, N, a.X_out, a.obj_out, a.stats, next, row, xyT, h->stream)) != cudaSuccess) break;
-        if ((rc = take_counter(h, &counter)) != COV_OK) break;
-        EvalOut out{};
-        out.obj = d_oo + (t - 1);
-        LaunchInfo li{};
+        if ((e = launch_horizon_commit(S, N, a.X_out, a.obj_out, a.stats, next, row, xyT, h->stream, E, cols)) !=
+            cudaSuccess)
+            break;
         what = "coverage kernel";
-        if ((e = launch_eval(lg, h->o, cfg, next, 1, out, counter, h->stream, &li)) != cudaSuccess) break;
+        if (E == 1) {
+            if ((rc = take_counter(h, &counter)) != COV_OK) break;
+            EvalOut out{};
+            out.obj = d_oo + (t - 1);
+            LaunchInfo li{};
+            if ((e = launch_eval(lg, o, cfg, next, 1, out, counter, h->stream, &li)) != cudaSuccess) break;
+        } else if ((e = launch_scenario_eval(lg, o, cfg, next, E, d_oo + (t - 1) * E, h->stream)) != cudaSuccess) {
+            break;
+        }
         h->launches += lg.planes_q ? 7 : 6;
     }
     h->fire_cur = fire_cur; // the automaton steps enqueued stand
     if (e == cudaSuccess && rc == COV_OK && step_ms) e = cudaEventRecord(ev[(size_t)T], h->stream), what = "event";
     if (e == cudaSuccess && rc == COV_OK)
         e = cudaMemcpyAsync(h->h_out, d_Xo, res_bytes, cudaMemcpyDeviceToHost, h->stream), what = "download";
+    if (cells_bytes && e == cudaSuccess && rc == COV_OK)
+        e = cudaMemcpyAsync((unsigned char *)h->h_out + res_bytes, mult, cells_bytes, cudaMemcpyDeviceToHost, h->stream);
     if (app && e == cudaSuccess && rc == COV_OK)
         e = cudaMemcpyAsync(&h->h_small->overflow, overflow, sizeof(int), cudaMemcpyDeviceToHost, h->stream);
     const int n_classes = app ? app->n_classes : h->g.n_classes;
     const double *cw = app ? app->cw : h->g.class_weight;
+    if (ens && e == cudaSuccess && rc == COV_OK) e = cudaStreamSynchronize(h->stream), what = "synchronise";
     if (e != cudaSuccess || rc != COV_OK) { // the steps enqueued so far stand: refresh what the host knows of them
         if (rc == COV_OK) rc = fail_cuda(h, e, (std::string(who) + ": " + what).c_str());
+        if (ens) { // they only touched the scenarios' copies
+            for (cudaEvent_t x : ev) h->ev_pool.push_back(x);
+            return rc;
+        }
         const std::string msg = h->err;
         if (app) entries_forget(h); // the list's per-timestep history is incomplete
         else entries_note_removals(h);
@@ -2283,25 +2355,30 @@ static int run_horizon(cov_handle *h, const char *who, const double *x_start, in
         h->err = msg;
         return rc;
     }
-    rc = rebuild_planes(h, n_classes, cw); // the one synchronise
+    if (!ens) rc = rebuild_planes(h, n_classes, cw); // the one synchronise
     if (rc == COV_OK && app && h->h_small->overflow)
         rc = fail(h, COV_ERR_STATE, std::string(who) + ": internal: an append went past the store's envelope");
     const double *hX = (const double *)h->h_out, *hobj = hX + tn;
-    int64_t *hst = (int64_t *)(hobj + T);
+    int64_t *hst = (int64_t *)(hobj + T * E);
     const int *hstamp = (const int *)((const unsigned char *)h->h_out + o_stamp);
     if (rc == COV_OK) {
         bool removed = false, pushed = false;
-        for (int64_t t = 0; t < T; ++t) {
+        for (int64_t t = 0; t < T * E; ++t) {
             removed |= hst[cols * t + 3] != 0;
             if (app && app->offsets) hst[cols * t + 4] = app->offsets[t + 1] - app->offsets[t];
             if (app) pushed |= hst[cols * t + 4] != 0;
         }
         if (app && app->fire_steps && pushed) entries_forget(h); // cov_fire_step: the automaton's order is createPOI's
         else if (app && app->offsets && h->ent_known) entries_replay(h, *app, T, hstamp);
-        else if (removed) entries_note_removals(h);
-        memcpy(X_out, hX, tn * 8);
-        if (obj_out) memcpy(obj_out, hobj, (size_t)T * 8);
-        if (stats) memcpy(stats, hst, (size_t)T * cols * 8);
+        else if (removed && !ens) entries_note_removals(h);
+        for (int64_t q = 0; q < E; ++q) // timestep-major rows to the scenario-major outputs
+            for (int64_t t = 0; t < T; ++t) {
+                const size_t src = (size_t)(t * E + q), dst = (size_t)(q * T + t);
+                memcpy(X_out + dst * n, hX + src * n, (size_t)n * 8);
+                if (obj_out) obj_out[dst] = hobj[src];
+                if (stats) memcpy(stats + dst * cols, hst + src * cols, (size_t)cols * 8);
+            }
+        if (cells_bytes) memcpy(ens->cells_out, (const unsigned char *)h->h_out + res_bytes, cells_bytes);
         if (stamps && stamps_out) memcpy(stamps_out, hstamp, ncell * 4);
         for (int64_t t = 0; step_ms && t < T; ++t) {
             float ms = 0;
@@ -2329,6 +2406,34 @@ extern "C" int cov_run_horizon(cov_handle *h, const double *x_start, int64_t T, 
     OK(check_mads_limits(h, who, &h->g));
     return run_horizon(h, who, x_start, T, S, spread, n_iter, granularity, seed, boxes, n_boxes, h_focus, h_max, X_out,
                        obj_out, stats, step_ms, nullptr, nullptr);
+}
+
+extern "C" int cov_run_horizon_ensemble(cov_handle *h, const double *x_starts, int64_t E, int64_t T, int64_t S,
+                                        double spread, int64_t n_iter, double granularity, uint64_t seed,
+                                        const double *boxes, int64_t n_boxes, double h_focus, double h_max,
+                                        double *X_out, double *obj_out, int64_t *stats, double *step_ms,
+                                        uint8_t *cells_out)
+{
+    const char *who = "cov_run_horizon_ensemble";
+    if (!h) return fail(nullptr, COV_ERR_INVALID, "NULL handle");
+    DeviceGuard dg(h->device);
+    OK(check_horizon(h, who, x_starts, T, S, spread, n_iter, granularity, boxes, n_boxes, X_out));
+    // E * S solves per launch (counted in int by the grid and the dispenser), E * T * S keys without wrapping
+    if (E < 1 || E > INT32_MAX / S || (T > 0 && E * S > INT64_MAX / T))
+        return fail(h, COV_ERR_INVALID, std::string(who) + ": E must be >= 1 with E * S <= 2^31 - 1 and E * T * S <= "
+                                                           "2^63 - 1");
+    if (T == 0) return COV_OK;
+    OK(check_mads_limits(h, who, &h->g));
+    const HorizonEnsemble ens{E, cells_out};
+    const int rc = run_horizon(h, who, x_starts, T, S, spread, n_iter, granularity, seed, boxes, n_boxes, h_focus, h_max,
+                               X_out, obj_out, stats, step_ms, nullptr, nullptr, &ens);
+    if (h->ens.p) { // a large ensemble would otherwise pin E copies of the store for the handle's lifetime
+        (void)cudaStreamSynchronize(h->stream); // a failed call may still have copies in flight
+        (void)cudaFree(h->ens.p);
+        (void)cudaGetLastError();
+        h->ens = DevBuf{};
+    }
+    return rc;
 }
 
 // The cell store's bytes as they are (one download, one synchronise).
@@ -2876,6 +2981,27 @@ extern "C" int cov_multi_eval_batch(cov_multi *m, const double *X, int64_t B, do
     }
     return run_shards(m, X, B, [&](int, cov_handle *h, const double *Xk, int64_t b0, int64_t bn) {
         return cov_eval_batch(h, Xk, bn, obj + b0, count ? count + b0 : nullptr, feasible ? feasible + b0 : nullptr);
+    });
+}
+
+// Scenarios b0 .. b0 + bn - 1 on shard k with the keys they have in the single-device call.
+extern "C" int cov_multi_run_horizon_ensemble(cov_multi *m, const double *x_starts, int64_t E, int64_t T, int64_t S,
+                                              double spread, int64_t n_iter, double granularity, uint64_t seed,
+                                              const double *boxes, int64_t n_boxes, double h_focus, double h_max,
+                                              double *X_out, double *obj_out, int64_t *stats, uint8_t *cells_out)
+{
+    if (!m) return fail(nullptr, COV_ERR_INVALID, "NULL multi handle");
+    if (E < 1 || T < 0 || (T > 0 && (!x_starts || !X_out))) {
+        m->err = "cov_multi_run_horizon_ensemble: bad arguments";
+        return COV_ERR_INVALID;
+    }
+    return run_shards(m, x_starts, E, [&](int, cov_handle *h, const double *Xk, int64_t b0, int64_t bn) {
+        const size_t n = h->have_params ? 3 * (size_t)h->o.N : 0, ncell = (size_t)h->g.nx * h->g.ny;
+        const size_t r0 = (size_t)b0 * (size_t)T;
+        return cov_run_horizon_ensemble(h, Xk, bn, T, S, spread, n_iter, granularity,
+                                        seed + (uint64_t)b0 * (uint64_t)T * (uint64_t)S, boxes, n_boxes, h_focus, h_max,
+                                        X_out + r0 * n, obj_out ? obj_out + r0 : nullptr, stats ? stats + r0 * 4 : nullptr,
+                                        nullptr, cells_out ? cells_out + (size_t)b0 * ncell : nullptr);
     });
 }
 

@@ -31,10 +31,11 @@ struct CandScalars {
 // Per-candidate prologue, executed by one warp.
 //   stage : the candidate's 3N doubles in shared memory (already visible to the warp)
 //   dp    : N DiscParam records to fill
+//   poff  : offset of the parameter block read through o's five arrays (cov_run_horizon_ensemble's scenarios)
 template <bool WANT_DP>
 __device__ __forceinline__ CandScalars candidate_prologue(const GridDesc &g, const ObjParams &o,
                                                           const double *stage, DiscParam *dp,
-                                                          bool want_progressive)
+                                                          bool want_progressive, long long poff = 0)
 {
     const int N = o.N;
     const uint32_t lane = lane_id();
@@ -97,12 +98,12 @@ __device__ __forceinline__ CandScalars candidate_prologue(const GridDesc &g, con
     double viol = 0.0, prog = 0.0;
     if (lane == 0) {
         for (int i = 0; i < N; ++i) {
-            const double diff = __dsub_rn(stage[2 * N + i], o.r_max[i]);
+            const double diff = __dsub_rn(stage[2 * N + i], o.r_max[poff + i]);
             viol = __dadd_rn(viol, fabs(diff));
         }
         if (want_progressive)
             for (int i = 0; i < N; ++i) {
-                const double diff = __dsub_rn(stage[2 * N + i], o.r_max[i]);
+                const double diff = __dsub_rn(stage[2 * N + i], o.r_max[poff + i]);
                 if (prog_takes(o, i)) prog = __dadd_rn(prog, julia_max0(diff));
             }
     }
@@ -112,13 +113,13 @@ __device__ __forceinline__ CandScalars candidate_prologue(const GridDesc &g, con
     bool bad = false;
     if (o.use_cons3) {
         for (int i = lane; i < N; i += 32) {
-            const double ax = __dsub_rn(o.prev_x[i], stage[i]);
-            const double ay = __dsub_rn(o.prev_y[i], stage[N + i]);
+            const double ax = __dsub_rn(o.prev_x[poff + i], stage[i]);
+            const double ay = __dsub_rn(o.prev_y[poff + i], stage[N + i]);
             const double z2 = __ddiv_rn(stage[2 * N + i], o.tan_half_fov);
-            const double az = __dsub_rn(o.prev_z[i], z2);
+            const double az = __dsub_rn(o.prev_z[poff + i], z2);
             const double s =
                 __dadd_rn(__dadd_rn(__dmul_rn(ax, ax), __dmul_rn(ay, ay)), __dmul_rn(az, az));
-            bad |= (s >= o.cons3_G[i]);
+            bad |= (s >= o.cons3_G[poff + i]);
         }
     }
     if (o.use_cons7) {

@@ -56,40 +56,51 @@ cudaError_t launch_grid_stats(const unsigned char *mult, const unsigned char *cl
     return cudaGetLastError();
 }
 
+// The grid of a launch over E stores side by side: blockIdx.y strides over the stores, and the blocks of one store
+// shrink so that the whole launch stays near `cap` blocks (E = 1: the single-store grid).
+static dim3 store_grid(long long work, int block, int cap, long long E)
+{
+    const int gy = (int)std::min<long long>(E, 65535);
+    const long long gx = std::min<long long>((work + block - 1) / block, std::max(cap / gy, 1));
+    return dim3((unsigned)std::max<long long>(gx, 1), (unsigned)gy);
+}
+
 // one warp per (row, word): lane b reads cell i = 32w + b + 1 and the ballot is the plane word
 __global__ void pack_planes_kernel(const unsigned char *__restrict__ mult, const unsigned char *__restrict__ cls,
-                                   const __grid_constant__ GridDesc g, uint32_t *__restrict__ planes)
+                                   const __grid_constant__ GridDesc g, uint32_t *__restrict__ planes, long long E)
 {
     const long long warp_global = (blockIdx.x * (long long)blockDim.x + threadIdx.x) >> 5;
     const int lane = threadIdx.x & 31;
-    const long long n_words = (long long)g.ny * g.stride;
+    const long long n_words = (long long)g.ny * g.stride, ncell = (long long)g.nx * g.ny;
     const long long n_warps = ((long long)gridDim.x * blockDim.x) >> 5;
-    for (long long t = warp_global; t < n_words; t += n_warps) {
-        const int row = (int)(t / g.stride), w = (int)(t % g.stride);
-        const int i = 32 * w + lane; // 0-based column
-        unsigned m = 0, k = 0;
-        if (w < g.wpr && i < g.nx) {
-            const long long cell = (long long)i + (long long)g.nx * row;
-            m = mult[cell];
-            k = cls[cell];
-        }
-        for (int l = 0; l < g.n_planes; ++l) {
-            const bool bit = (m & (unsigned)g.plane_mult[l]) && ((int)k == g.plane_class[l]);
-            const uint32_t word = __ballot_sync(0xffffffffu, bit);
-            if (lane == 0) planes[(size_t)l * g.plane_words + t] = word;
+    for (long long e = blockIdx.y; e < E; e += gridDim.y) {
+        const unsigned char *me = mult + e * ncell, *ce = cls + e * ncell;
+        uint32_t *pe = planes + e * g.n_planes * (long long)g.plane_words;
+        for (long long t = warp_global; t < n_words; t += n_warps) {
+            const int row = (int)(t / g.stride), w = (int)(t % g.stride);
+            const int i = 32 * w + lane; // 0-based column
+            unsigned m = 0, k = 0;
+            if (w < g.wpr && i < g.nx) {
+                const long long cell = (long long)i + (long long)g.nx * row;
+                m = me[cell];
+                k = ce[cell];
+            }
+            for (int l = 0; l < g.n_planes; ++l) {
+                const bool bit = (m & (unsigned)g.plane_mult[l]) && ((int)k == g.plane_class[l]);
+                const uint32_t word = __ballot_sync(0xffffffffu, bit);
+                if (lane == 0) pe[(size_t)l * g.plane_words + t] = word;
+            }
         }
     }
 }
 
 cudaError_t launch_pack_planes(const unsigned char *mult, const unsigned char *cls, const GridDesc &g,
-                               uint32_t *planes, cudaStream_t s)
+                               uint32_t *planes, cudaStream_t s, long long E)
 {
-    cudaError_t e = cudaMemsetAsync(planes, 0, (size_t)g.n_planes * g.plane_words * 4, s);
+    cudaError_t e = cudaMemsetAsync(planes, 0, (size_t)E * g.n_planes * g.plane_words * 4, s);
     if (e != cudaSuccess) return e;
     const long long n_words = (long long)g.ny * g.stride;
-    const int block = 256;
-    const int grid = (int)std::min<long long>((n_words * 32 + block - 1) / block, 148 * 16);
-    pack_planes_kernel<<<max(grid, 1), block, 0, s>>>(mult, cls, g, planes);
+    pack_planes_kernel<<<store_grid(n_words * 32, 256, 148 * 16, E), 256, 0, s>>>(mult, cls, g, planes, E);
     return cudaGetLastError();
 }
 
@@ -151,18 +162,20 @@ cudaError_t launch_bits_to_cells(const uint32_t *bits, int nx, int ny, unsigned 
     return cudaGetLastError();
 }
 
-__global__ void thresholds_kernel(const double *xyR, int N, double *xyT)
+__global__ void thresholds_kernel(const double *xyR, int N, double *xyT, long long E)
 {
     const int c = blockIdx.x * blockDim.x + threadIdx.x;
-    if (c < N) {
-        xyT[c] = xyR[c];
-        xyT[N + c] = xyR[N + c];
-        xyT[2 * N + c] = threshold(xyR[2 * N + c]);
+    for (long long e = blockIdx.y; e < E && c < N; e += gridDim.y) {
+        const double *in = xyR + e * 3 * N;
+        double *out = xyT + e * 3 * N;
+        out[c] = in[c];
+        out[N + c] = in[N + c];
+        out[2 * N + c] = threshold(in[2 * N + c]);
     }
 }
-cudaError_t launch_thresholds(const double *xyR, int N, double *xyT, cudaStream_t s)
+cudaError_t launch_thresholds(const double *xyR, int N, double *xyT, cudaStream_t s, long long E)
 {
-    thresholds_kernel<<<(N + 127) / 128, 128, 0, s>>>(xyR, N, xyT);
+    thresholds_kernel<<<dim3((N + 127) / 128, (unsigned)std::min<long long>(E, 65535)), 128, 0, s>>>(xyR, N, xyT, E);
     return cudaGetLastError();
 }
 
@@ -179,35 +192,40 @@ __device__ __forceinline__ bool cell_covered(const GridDesc &g, int i1, int j1, 
 // stamp (nullable): stamp[cell] = t for every cell that loses entries (cov_run_horizon_points' last_removed)
 __global__ void remove_covered_kernel(unsigned char *mult, unsigned char *cls, const __grid_constant__ GridDesc g,
                                       const double *__restrict__ xyT, int N, unsigned long long *removed, int *stamp,
-                                      int t_stamp)
+                                      int t_stamp, long long E, long long removed_stride)
 {
     const long long ncell = (long long)g.nx * g.ny;
-    unsigned long long mine = 0;
-    for (long long t = blockIdx.x * (long long)blockDim.x + threadIdx.x; t < ncell;
-         t += (long long)gridDim.x * blockDim.x) {
-        const unsigned m = mult[t];
-        if (m) {
-            const int i1 = (int)(t % g.nx) + 1, j1 = (int)(t / g.nx) + 1;
-            if (cell_covered(g, i1, j1, xyT, N)) {
-                mine += m;
-                mult[t] = 0;
-                cls[t] = 0xffu;
-                if (stamp) stamp[t] = t_stamp;
+    for (long long e = blockIdx.y; e < E; e += gridDim.y) {
+        unsigned char *me = mult + e * ncell, *ce = cls + e * ncell;
+        const double *xe = xyT + e * 3 * N;
+        unsigned long long mine = 0;
+        for (long long t = blockIdx.x * (long long)blockDim.x + threadIdx.x; t < ncell;
+             t += (long long)gridDim.x * blockDim.x) {
+            const unsigned m = me[t];
+            if (m) {
+                const int i1 = (int)(t % g.nx) + 1, j1 = (int)(t / g.nx) + 1;
+                if (cell_covered(g, i1, j1, xe, N)) {
+                    mine += m;
+                    me[t] = 0;
+                    ce[t] = 0xffu;
+                    if (stamp) stamp[t] = t_stamp;
+                }
             }
         }
+        for (int off = 16; off; off >>= 1) mine += __shfl_xor_sync(0xffffffffu, mine, off);
+        if ((threadIdx.x & 31) == 0 && mine) atomicAdd(removed + e * removed_stride, mine);
     }
-    for (int off = 16; off; off >>= 1) mine += __shfl_xor_sync(0xffffffffu, mine, off);
-    if ((threadIdx.x & 31) == 0 && mine) atomicAdd(removed, mine);
 }
 cudaError_t launch_remove_covered(unsigned char *mult, unsigned char *cls, const GridDesc &g, const double *xyT, int N,
-                                  unsigned long long *removed, cudaStream_t s, int *stamp, int t_stamp)
+                                  unsigned long long *removed, cudaStream_t s, int *stamp, int t_stamp, long long E,
+                                  long long removed_stride)
 {
-    cudaError_t e = cudaMemsetAsync(removed, 0, sizeof(unsigned long long), s);
+    // the counters of the E stores and whatever lies between them (the callers' rows are rewritten afterwards)
+    cudaError_t e = cudaMemsetAsync(removed, 0, (size_t)((E - 1) * removed_stride + 1) * sizeof(unsigned long long), s);
     if (e != cudaSuccess) return e;
     const long long ncell = (long long)g.nx * g.ny;
-    const int block = 256;
-    const int grid = (int)std::min<long long>((ncell + block - 1) / block, 148 * 8);
-    remove_covered_kernel<<<max(grid, 1), block, 0, s>>>(mult, cls, g, xyT, N, removed, stamp, t_stamp);
+    remove_covered_kernel<<<store_grid(ncell, 256, 148 * 8, E), 256, 0, s>>>(mult, cls, g, xyT, N, removed, stamp,
+                                                                             t_stamp, E, removed_stride);
     return cudaGetLastError();
 }
 

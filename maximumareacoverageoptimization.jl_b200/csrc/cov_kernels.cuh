@@ -69,13 +69,26 @@ struct MadsArgs {
 bool mads_plan(const GridDesc &g, int N, const LaunchCfg &cfg, int *warps, int *smem, int *planes_smem);
 cudaError_t launch_mads(const GridDesc &g, const ObjParams &o, const LaunchCfg &cfg, const MadsArgs &a,
                         unsigned long long *counter, cudaStream_t stream);
+// The solves of E scenarios in one launch (cov_run_horizon_ensemble): a.S = E * S solves, solve j of scenario j / S.
+// Scenario e reads plane set e (g.planes + e * n_planes * plane_words, read through L2) and parameter block e (o's
+// five arrays shifted by e * 5N); solve k of scenario e is keyed by a.seed + e * key_stride + k.
+cudaError_t launch_scenario_mads(const GridDesc &g, const ObjParams &o, const LaunchCfg &cfg, const MadsArgs &a,
+                                 long long S, unsigned long long key_stride, unsigned long long *counter,
+                                 cudaStream_t stream);
+// AreaMaxObjective without the barrier of E swarms (X: E x 3N, device), swarm e on plane set e and parameter block e
+// as above, one warp per swarm: obj[e].
+cudaError_t launch_scenario_eval(const GridDesc &g, const ObjParams &o, const LaunchCfg &cfg, const double *X,
+                                 long long E, double *obj, cudaStream_t stream);
 
 // ---- cov_run_horizon (cov_horizon.cu): the kernels between the launchers above, per timestep t (1-based) ----
+// A launch covers E scenarios side by side (cov_run_horizon_ensemble; E = 1: cov_run_horizon): scenario e's cur,
+// parameter block and starts at e * 3N, e * 5N and e * S * 3N doubles.
 struct HorizonStep {
     int N, n_boxes;
-    long long t, S;
+    long long t, S, E;
     double spread, granularity;
-    unsigned long long seed;  // Philox key of the starts' perturbations
+    unsigned long long seed;        // Philox key of scenario 0's perturbations
+    unsigned long long seed_stride; // scenario e's key: seed + e * seed_stride
     const double *pow10;      // the solver's table (MadsArgs::pow10)
     const double *boxes;      // n_boxes x 4: x_LB, x_UB, y_LB, y_UB (device)
     double h_focus, h_max, tan_half_fov;
@@ -84,9 +97,11 @@ struct HorizonStep {
 // r_max, prev_x, prev_y, prev_z, cons3_G), and S starts with their initial meshes (start 0 = cur).
 cudaError_t launch_horizon_start(const HorizonStep &s, const double *cur, double *params, double *X0, double *a0,
                                  int *b0, cudaStream_t stream);
-// One CTA: the winner of S solves (Xs S x 3N, objs S, mstats S x 4) to cur, stats_row[0..2], and xyT of cur.
+// One CTA per scenario: the winner of S solves (Xs S x 3N, objs S, mstats S x 4) to cur, stats_row[0..2], and xyT of
+// cur.  Scenario e's arrays are at e times their size, its stats row at e * row_stride.
 cudaError_t launch_horizon_commit(long long S, int N, const double *Xs, const double *objs, const long long *mstats,
-                                  double *cur, long long *stats_row, double *xyT, cudaStream_t stream);
+                                  double *cur, long long *stats_row, double *xyT, cudaStream_t stream, long long E = 1,
+                                  long long row_stride = 0);
 
 // ---- the grid-free static objective (cov_region.cu, cov_mads.cu; geometry and limits in cov_region.cuh) ----
 // The arcs of the covered set's boundary inside the domain (r.arcs / r.K unused): at most cap of them to out, the
@@ -104,21 +119,25 @@ cudaError_t launch_mads_region(const RegionDesc &r, const ObjParams &o, const La
 // stats[0] = entries, stats[1] = cells, stats[2 + k] = OR of the multiplicities of class k
 cudaError_t launch_grid_stats(const unsigned char *mult, const unsigned char *cls, long long ncell,
                               unsigned long long *stats, cudaStream_t s);
+// The launchers below that take E work on E stores side by side (cov_run_horizon_ensemble): store e's mult / cls at
+// e * nx*ny bytes, its plane set at e * n_planes * plane_words words, its xyT at e * 3N doubles.
 cudaError_t launch_pack_planes(const unsigned char *mult, const unsigned char *cls, const GridDesc &g,
-                               uint32_t *planes, cudaStream_t s);
+                               uint32_t *planes, cudaStream_t s, long long E = 1);
 // plane 0 in the pair-aligned, swizzled layout of the CTA kernel's sweep mode (GridDesc::planes_q)
 cudaError_t launch_requad_plane(const GridDesc &g, uint32_t *planes_q, cudaStream_t s);
 cudaError_t launch_fill_full(unsigned char *mult, unsigned char *cls, long long ncell, cudaStream_t s);
 cudaError_t launch_bits_to_cells(const uint32_t *bits, int nx, int ny, unsigned char *mult,
                                  unsigned char *cls, cudaStream_t s);
-// xyT: 3N doubles on the device: cx[N], cy[N], T[N]. removed: one unsigned long long.  stamp (nullable, nx*ny ints):
-// stamp[cell] = t_stamp for every cell whose entries are removed.
+// xyT: 3N doubles on the device: cx[N], cy[N], T[N]. removed: one unsigned long long (store e's at e *
+// removed_stride).  stamp (nullable, nx*ny ints, E = 1 only): stamp[cell] = t_stamp for every cell whose entries are
+// removed.
 cudaError_t launch_remove_covered(unsigned char *mult, unsigned char *cls, const GridDesc &g, const double *xyT, int N,
-                                  unsigned long long *removed, cudaStream_t s, int *stamp = nullptr, int t_stamp = 0);
+                                  unsigned long long *removed, cudaStream_t s, int *stamp = nullptr, int t_stamp = 0,
+                                  long long E = 1, long long removed_stride = 0);
 cudaError_t launch_normalize_cls(const unsigned char *mult, unsigned char *cls, long long ncell, cudaStream_t s);
 cudaError_t launch_covered_mask(unsigned char *mask, const GridDesc &g, const double *xyT, int N,
                                 cudaStream_t s);
-cudaError_t launch_thresholds(const double *xyR, int N, double *xyT, cudaStream_t s);
+cudaError_t launch_thresholds(const double *xyR, int N, double *xyT, cudaStream_t s, long long E = 1); // E swarms
 cudaError_t launch_add_points(unsigned char *mult, unsigned char *cls, const int *cell_idx,
                               const unsigned char *cell_cls, long long P, int *overflow, cudaStream_t s);
 cudaError_t launch_argmin(const double *obj, const unsigned char *feasible, long long B, int barrier,

@@ -106,15 +106,17 @@ __device__ __forceinline__ bool poll_point(int kk, int n, const double *x, const
 
 // The objective with the extreme barrier for the candidate in `stage`, by one warp: +Inf where a fused constraint
 // fails (its coverage is never counted) or the objective is NaN.  fb: the warp's framebuffer, all-zero on entry and
-// on return (the list-order path keeps the thresholds there instead and never paints it).
+// on return (the list-order path keeps the thresholds there instead and never paints it).  poff: the parameter
+// block's offset (candidate_prologue); barrier = false: AreaMaxObjective itself, as the objective kernels give it.
 template <bool MULTI, bool PLANES_SMEM>
 __device__ double mads_eval(const GridDesc &g, const ObjParams &o, const double *stage, SDisc *sd, int *pre,
-                            uint32_t *fb, const uint32_t *planes, int force_exact, int ordered)
+                            uint32_t *fb, const uint32_t *planes, int force_exact, int ordered, long long poff = 0,
+                            bool barrier = true)
 {
     const int N = o.N;
     const uint32_t lane = lane_id();
-    const CandScalars cs = candidate_prologue<false>(g, o, stage, nullptr, false);
-    if (!cs.feasible) return __longlong_as_double(0x7ff0000000000000ll);
+    const CandScalars cs = candidate_prologue<false>(g, o, stage, nullptr, false, poff);
+    if (barrier && !cs.feasible) return __longlong_as_double(0x7ff0000000000000ll);
     double obj;
     long long cls[kMaxClasses];
     if (ordered) {
@@ -180,16 +182,17 @@ __device__ double mads_eval(const GridDesc &g, const ObjParams &o, const double 
             cls[k] = k < (MULTI ? kMaxClasses : 1) ? (long long)__reduce_add_sync(0xffffffffu, cnt[MULTI ? k : 0]) : 0;
         obj = assemble_objective(g, o, cls, cs.violation);
     }
-    return (obj == obj) ? obj : __longlong_as_double(0x7ff0000000000000ll);
+    return (obj == obj || !barrier) ? obj : __longlong_as_double(0x7ff0000000000000ll);
 }
 
 // The solves of cov_mads_solve_batch from the dispenser `counter` until none is left, by the whole CTA: the loop
-// shared by mads_kernel (the grid objective) and region_solve_kernel (the region objective).  state: mads_state_bytes(n)
-// bytes of shared memory; stage: the calling warp's 3N doubles; eval(p): the barrier value of the point p (shared
-// memory) by the calling warp.
-template <class Eval>
+// shared by mads_kernel (the grid objective), scenario_solve_kernel (the grid objective of several stores) and
+// region_solve_kernel (the region objective).  state: mads_state_bytes(n) bytes of shared memory; stage: the calling
+// warp's 3N doubles; key_of(k): the Philox key of solve k, called by every thread before the solve's first evaluation;
+// eval(p): the barrier value of the point p (shared memory) by the calling warp.
+template <class Key, class Eval>
 __device__ __forceinline__ void mads_solves(const MadsArgs &a, int n, unsigned char *state, double *stage,
-                                            unsigned long long *counter, const Eval &eval)
+                                            unsigned long long *counter, const Key &key_of, const Eval &eval)
 {
     const int W = blockDim.x >> 5;
     const int warp = threadIdx.x >> 5;
@@ -206,6 +209,7 @@ __device__ __forceinline__ void mads_solves(const MadsArgs &a, int n, unsigned c
         __syncthreads();
         const unsigned long long k = sh->solve;
         if ((long long)k >= a.S) break;
+        const unsigned long long key = key_of(k);
         const double *x0 = a.X0 + (long long)k * n;
         for (int i = tid; i < n; i += nthr) {
             x[i] = x0[i];
@@ -222,7 +226,6 @@ __device__ __forceinline__ void mads_solves(const MadsArgs &a, int n, unsigned c
         }
         long long iterations = 0, evaluations = 1, successes = 0; // kept by thread 0
         int converged = 0;
-        const unsigned long long key = a.seed + k;
         for (long long it = 0; it < a.n_iter; ++it) {
             ++iterations;
             for (int i = tid; i < n; i += nthr) {
@@ -343,9 +346,68 @@ mads_kernel(const __grid_constant__ GridDesc g, const __grid_constant__ ObjParam
     const uint32_t *planes = PLANES_SMEM ? planes_s : g.planes;
     for (int t = lane; t < mads_fb_bytes(g, N) / 16; t += 32) reinterpret_cast<uint4 *>(fb)[t] = make_uint4(0, 0, 0, 0);
     __syncwarp();
-    mads_solves(a, n, sbase, stage, counter, [&](const double *p) {
+    mads_solves(a, n, sbase, stage, counter, [&](unsigned long long k) { return a.seed + k; }, [&](const double *p) {
         return mads_eval<MULTI, PLANES_SMEM>(g, o, p, sd, pre, fb, planes, a.force_exact, a.ordered);
     });
+}
+
+// The solves of E scenarios (launch_scenario_mads): mads_kernel's shared-memory layout without the staged planes.
+// Solve k belongs to scenario k / S, whose plane set is read through L2 (E stores rarely fit one SM's shared memory,
+// and consecutive solves of a persistent CTA belong to different scenarios).
+template <bool MULTI>
+__global__ void __launch_bounds__(kMadsThreads, kMadsCtas)
+scenario_solve_kernel(const __grid_constant__ GridDesc g, const __grid_constant__ ObjParams o,
+                      const __grid_constant__ MadsArgs a, long long S, unsigned long long key_stride,
+                      unsigned long long *counter)
+{
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    const int warp = threadIdx.x >> 5;
+    const uint32_t lane = lane_id();
+    const int N = o.N, n = 3 * N;
+    const int warp_bytes = mads_warp_bytes(g, N);
+    unsigned char *wbase = smem_raw + mads_state_bytes(n) + (size_t)warp * warp_bytes;
+    double *stage = reinterpret_cast<double *>(wbase);
+    SDisc *sd = reinterpret_cast<SDisc *>(wbase + round_up(3 * N * 8, 16));
+    int *pre = reinterpret_cast<int *>(wbase + round_up(3 * N * 8, 16) + N * 32);
+    uint32_t *fb = reinterpret_cast<uint32_t *>(wbase + round_up(3 * N * 8, 16) + N * 32 + round_up(N * 4, 16));
+    for (int t = lane; t < mads_fb_bytes(g, N) / 16; t += 32) reinterpret_cast<uint4 *>(fb)[t] = make_uint4(0, 0, 0, 0);
+    __syncwarp();
+    const long long pstride = (long long)g.n_planes * g.plane_words;
+    long long e = 0; // the scenario of the current solve
+    mads_solves(
+        a, n, smem_raw, stage, counter,
+        [&](unsigned long long k) {
+            e = (long long)(k / (unsigned long long)S);
+            return a.seed + (unsigned long long)e * key_stride + (k - (unsigned long long)e * S);
+        },
+        [&](const double *p) {
+            return mads_eval<MULTI, false>(g, o, p, sd, pre, fb, g.planes + e * pstride, a.force_exact, 0, e * 5 * N);
+        });
+}
+
+// AreaMaxObjective of E swarms, one warp per swarm (launch_scenario_eval).  Shared memory: W x mads_warp_bytes.
+template <bool MULTI>
+__global__ void __launch_bounds__(kMadsThreads)
+scenario_eval_kernel(const __grid_constant__ GridDesc g, const __grid_constant__ ObjParams o,
+                     const double *__restrict__ X, long long E, int force_exact, double *__restrict__ obj)
+{
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    const int W = blockDim.x >> 5, warp = threadIdx.x >> 5;
+    const uint32_t lane = lane_id();
+    const int N = o.N, n = 3 * N;
+    const long long e = (long long)blockIdx.x * W + warp;
+    if (e >= E) return;
+    unsigned char *wbase = smem_raw + (size_t)warp * mads_warp_bytes(g, N);
+    double *stage = reinterpret_cast<double *>(wbase);
+    SDisc *sd = reinterpret_cast<SDisc *>(wbase + round_up(3 * N * 8, 16));
+    int *pre = reinterpret_cast<int *>(wbase + round_up(3 * N * 8, 16) + N * 32);
+    uint32_t *fb = reinterpret_cast<uint32_t *>(wbase + round_up(3 * N * 8, 16) + N * 32 + round_up(N * 4, 16));
+    for (int t = lane; t < mads_fb_bytes(g, N) / 16; t += 32) reinterpret_cast<uint4 *>(fb)[t] = make_uint4(0, 0, 0, 0);
+    for (int i = lane; i < n; i += 32) stage[i] = X[e * n + i];
+    __syncwarp();
+    const double f = mads_eval<MULTI, false>(g, o, stage, sd, pre, fb, g.planes + e * g.n_planes * (long long)g.plane_words,
+                                             force_exact, 0, e * 5 * N, false);
+    if (lane == 0) obj[e] = f;
 }
 
 bool mads_plan(const GridDesc &g, int N, const LaunchCfg &cfg, int *warps, int *smem, int *planes_smem)
@@ -378,17 +440,61 @@ static cudaError_t launch_mads_variant(const GridDesc &g, const ObjParams &o, co
     return cudaGetLastError();
 }
 
+static bool plane_multi(const GridDesc &g) { return !(g.n_planes == 1 && g.n_classes == 1 && g.plane_mult[0] == 1); }
+
 cudaError_t launch_mads(const GridDesc &g, const ObjParams &o, const LaunchCfg &cfg, const MadsArgs &a,
                         unsigned long long *counter, cudaStream_t stream)
 {
     if (a.S <= 0) return cudaSuccess;
     int warps = 0, smem = 0, ps = 0;
     if (!mads_plan(g, o.N, cfg, &warps, &smem, &ps)) return cudaErrorInvalidConfiguration;
-    const bool multi = !(g.n_planes == 1 && g.n_classes == 1 && g.plane_mult[0] == 1);
-    if (multi) return ps ? launch_mads_variant<true, true>(g, o, cfg, a, counter, stream, warps, smem)
-                         : launch_mads_variant<true, false>(g, o, cfg, a, counter, stream, warps, smem);
+    if (plane_multi(g)) return ps ? launch_mads_variant<true, true>(g, o, cfg, a, counter, stream, warps, smem)
+                                  : launch_mads_variant<true, false>(g, o, cfg, a, counter, stream, warps, smem);
     return ps ? launch_mads_variant<false, true>(g, o, cfg, a, counter, stream, warps, smem)
               : launch_mads_variant<false, false>(g, o, cfg, a, counter, stream, warps, smem);
+}
+
+// Persistent CTAs of kern with smem bytes, at most `work` of them.
+template <class K>
+static cudaError_t persistent_grid(K kern, int threads, int smem, long long work, const LaunchCfg &cfg, int *grid)
+{
+    cudaError_t err = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+    if (err != cudaSuccess) return err;
+    int per_sm = 0;
+    err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, threads, smem);
+    if (err != cudaSuccess) return err;
+    *grid = (int)std::min<long long>(work, (long long)cfg.num_sms * std::max(per_sm, 1));
+    return cudaSuccess;
+}
+
+cudaError_t launch_scenario_mads(const GridDesc &g, const ObjParams &o, const LaunchCfg &cfg, const MadsArgs &a,
+                                 long long S, unsigned long long key_stride, unsigned long long *counter,
+                                 cudaStream_t stream)
+{
+    if (a.S <= 0) return cudaSuccess;
+    int warps = 0, smem = 0, ps = 0;
+    if (!mads_plan(g, o.N, cfg, &warps, &smem, &ps)) return cudaErrorInvalidConfiguration;
+    if (ps) smem -= g.n_planes * g.plane_words * 4; // the planes stay in global memory
+    auto kern = plane_multi(g) ? scenario_solve_kernel<true> : scenario_solve_kernel<false>;
+    int grid = 0;
+    cudaError_t err = persistent_grid(kern, warps * 32, smem, a.S, cfg, &grid);
+    if (err != cudaSuccess) return err;
+    kern<<<grid, warps * 32, smem, stream>>>(g, o, a, S, key_stride, counter);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_scenario_eval(const GridDesc &g, const ObjParams &o, const LaunchCfg &cfg, const double *X,
+                                 long long E, double *obj, cudaStream_t stream)
+{
+    if (E <= 0) return cudaSuccess;
+    int warps = 0, smem = 0, ps = 0;
+    if (!mads_plan(g, o.N, cfg, &warps, &smem, &ps)) return cudaErrorInvalidConfiguration;
+    smem = warps * mads_warp_bytes(g, o.N);
+    auto kern = plane_multi(g) ? scenario_eval_kernel<true> : scenario_eval_kernel<false>;
+    cudaError_t err = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+    if (err != cudaSuccess) return err;
+    kern<<<(unsigned)((E + warps - 1) / warps), warps * 32, smem, stream>>>(g, o, X, E, cfg.force_exact, obj);
+    return cudaGetLastError();
 }
 
 // The solves of cov_mads_solve_batch with the region objective.  Shared memory: [solve state] [region] [W x (stage,
@@ -406,7 +512,8 @@ region_solve_kernel(const __grid_constant__ RegionDesc r, const __grid_constant_
     double *stage = reinterpret_cast<double *>(wbase);
     double *ia = reinterpret_cast<double *>(wbase + round_up(3 * N * 8, 16)), *ib = ia + region_list_cap(N, r.M);
     __syncthreads();
-    mads_solves(a, n, smem_raw, stage, counter, [&](const double *p) { // region_objective with the extreme barrier
+    mads_solves(a, n, smem_raw, stage, counter, [&](unsigned long long k) { return a.seed + k; },
+                [&](const double *p) { // region_objective with the extreme barrier
         const CandScalars cs = candidate_prologue<false>(GridDesc{}, o, p, nullptr, false);
         if (!cs.feasible) return __longlong_as_double(0x7ff0000000000000ll);
         const double obj = objective_from_area(region_area(v, p, N, ia, ib), cs.violation, o);

@@ -384,6 +384,37 @@ class CoverageEngine:
                              boxes, h_focus, h_max, (_ptr(fs), float(wind_speed), float(wind_direction),
                                                      float(prob_spread), int(fire_seed) & (2**64 - 1), int(first_step)))
 
+    def run_horizon_ensemble(self, x_starts, T: int, S: int = 1, spread: float = 3.0, n_iter: int = 100,
+                             granularity: float = 1.0, seed: int = 0, boxes=None, h_focus: float = 15.0,
+                             h_max: float = 30.0, want_cells: bool = False):
+        """E independent run_horizon scenarios in one call (cov_run_horizon_ensemble), each on a private copy of the
+        engine's current store and parameters: scenario e starts from x_starts[e] ((E, 3N)) and equals run_horizon
+        with seed + e * T * S.  The engine is left unchanged.  Returns (X (E, T, 3N), obj (E, T), stats, step_ms (T,))
+        with stats a dict of (E, T) int64 arrays (run_horizon's), and with want_cells=True also cells (E, nx*ny), the
+        multiplicities each scenario leaves (grid_cells after the equivalent run_horizon)."""
+        X0 = _f64(x_starts)
+        if X0.ndim == 1:
+            X0 = X0.reshape(1, -1)
+        if self.N is None or X0.ndim != 2 or X0.shape[1] != 3 * self.N:
+            raise ValueError("x_starts must be (E, 3N) with the N given to set_params")
+        E, T, n = X0.shape[0], max(int(T), 0), 3 * self.N
+        B = np.zeros((0, 4)) if boxes is None else _f64(boxes).reshape(-1, 4)
+        X = np.empty((E, T, n))
+        obj = np.empty((E, T))
+        st = np.empty((E, T, 4), dtype=np.int64)
+        ms = np.empty(T)
+        cells = None
+        if want_cells:
+            gi = self.grid_info()
+            cells = np.empty((E, gi["nx"] * gi["ny"]), dtype=np.uint8)
+        self._check(lib.cov_run_horizon_ensemble(self._h, _ptr(X0), E, int(T), int(S), float(spread), int(n_iter),
+                                                 float(granularity), int(seed) & (2**64 - 1),
+                                                 _ptr(B) if len(B) else None, len(B), float(h_focus), float(h_max),
+                                                 _ptr(X), _ptr(obj), _ptr(st), _ptr(ms), _ptr(cells)))
+        names = ("winner", "evaluations", "feasible", "removed")
+        out = (X, obj, {name: st[:, :, q].copy() for q, name in enumerate(names)}, ms)
+        return out + (cells,) if want_cells else out
+
     def _horizon(self, fn, x_start, T, cols, S, spread, n_iter, granularity, seed, boxes, h_focus, h_max, source,
                  tail=()):
         x_start = _f64(x_start).ravel()

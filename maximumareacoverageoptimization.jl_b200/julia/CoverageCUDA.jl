@@ -20,14 +20,16 @@ end
 mutable struct Handle
     ptr::Ptr{Cvoid}
     N::Int
+    ncells::Int # nx * ny of the lattice last set through this binding (0: none yet)
     function Handle(device::Integer = 0)
         out = Ref{Ptr{Cvoid}}(C_NULL)
         rc = ccall((:cov_create, LIB), Cint, (Cint, Ref{Ptr{Cvoid}}), device, out)
         rc == 0 || throw(CovError(rc, unsafe_string(ccall((:cov_last_error, LIB), Cstring, (Ptr{Cvoid},), C_NULL))))
-        h = new(out[], 0)
+        h = new(out[], 0, 0)
         finalizer(h -> (h.ptr == C_NULL || ccall((:cov_destroy, LIB), Cvoid, (Ptr{Cvoid},), h.ptr); h.ptr = C_NULL), h)
         return h
     end
+    Handle(ptr::Ptr{Cvoid}, N::Int) = new(ptr, N, 0) # borrowed (a MultiHandle's shard): never destroyed here
 end
 
 check(h::Handle, rc::Cint) =
@@ -42,11 +44,14 @@ function set_points!(h::Handle, points::Vector{Vector{Float64}}; nx = 100, ny = 
     GC.@preserve flat check(h, ccall((:cov_set_points, LIB), Cint,
         (Ptr{Cvoid}, Ptr{Float64}, Int64, Int64, Int64, Float64, Float64),
         h.ptr, flat, length(points), nx, ny, dx, dy))
+    h.ncells = nx * ny
 end
 
 "createPOI(dx, dy, nx, ny) built on the device (src/AreaCoverageCalculation.jl:11-21)."
-set_grid_full!(h::Handle, nx, ny, dx, dy) =
+function set_grid_full!(h::Handle, nx, ny, dx, dy)
     check(h, ccall((:cov_set_grid_full, LIB), Cint, (Ptr{Cvoid}, Int64, Int64, Float64, Float64), h.ptr, nx, ny, dx, dy))
+    h.ncells = nx * ny
+end
 
 "rmvCoveredPOI on the device-resident store (src/CellFunctions.jl:81-108); returns entries removed."
 function remove_covered!(h::Handle, xyR::Vector{Float64})
@@ -78,6 +83,7 @@ function fire_init!(h::Handle, state::Matrix{UInt8}; dx = 5.0, dy = 5.0, push_in
     nx, ny = size(state)
     GC.@preserve state check(h, ccall((:cov_fire_init, LIB), Cint,
         (Ptr{Cvoid}, Int64, Int64, Float64, Float64, Ptr{UInt8}, Int32), h.ptr, nx, ny, dx, dy, state, push_initial ? 1 : 0))
+    h.ncells = nx * ny
 end
 function fire_step!(h::Handle, wind_speed, wind_direction, prob_spread; seed = 0, step = 0, append = true)
     pushed = Ref{Int64}(0)
@@ -359,6 +365,96 @@ function run_horizon_fire(h::Handle, x_start::Vector{Float64}, fire_steps::Vecto
         h.ptr, x_start, T, S, spread, N_iter, granularity, seed, K == 0 ? C_NULL : pointer(boxes), K, h_focus, h_max,
         fire_steps, wind_speed, wind_direction, prob_spread, fire_seed, first_step, X, obj, stats, ms))
     return X, obj, stats, ms
+end
+
+"""
+    run_horizon_ensemble(h, x_starts; T, S = 1, spread = 3.0, N_iter = 100, granularity = 1.0, seed = 0,
+                         boxes = zeros(Float64, 4, 0), h_focus = 15.0, h_max = 30.0, want_cells = false)
+
+E independent `run_horizon` scenarios in one call (`cov_run_horizon_ensemble`), each on a private copy of the
+handle's current store and parameters: column e of `x_starts` (3N x E) starts scenario e, which equals `run_horizon`
+with `seed + (e - 1) * T * S`. The handle is left unchanged. Returns `(X, objectives, stats, step_ms, cells)`: `X`
+3N x T x E, `objectives` T x E, `stats` 4 x T x E (`run_horizon`'s rows), `step_ms` the device time of every timestep
+of the whole ensemble, `cells` (nx*ny x E, with `want_cells`; else `nothing`) the multiplicities each scenario leaves. `want_cells` needs the
+lattice set through this binding (`set_points!`, `set_grid_full!` or `fire_init!`), which sizes `cells`.
+"""
+function run_horizon_ensemble(h::Handle, x_starts::Matrix{Float64}; T, S = 1, spread = 3.0, N_iter = 100,
+                              granularity = 1.0, seed = 0, boxes::Matrix{Float64} = zeros(Float64, 4, 0),
+                              h_focus = 15.0, h_max = 30.0, want_cells = false)
+    n, E = size(x_starts); K = size(boxes, 2)
+    X = zeros(Float64, n, T, E); obj = zeros(Float64, T, E); stats = zeros(Int64, 4, T, E); ms = zeros(Float64, T)
+    cells = want_cells ? zeros(UInt8, lattice_cells(h), E) : nothing
+    GC.@preserve x_starts boxes X obj stats ms cells check(h, ccall((:cov_run_horizon_ensemble, LIB), Cint,
+        (Ptr{Cvoid}, Ptr{Float64}, Int64, Int64, Int64, Float64, Int64, Float64, UInt64, Ptr{Float64}, Int64, Float64,
+         Float64, Ptr{Float64}, Ptr{Float64}, Ptr{Int64}, Ptr{Float64}, Ptr{UInt8}),
+        h.ptr, x_starts, E, T, S, spread, N_iter, granularity, seed, K == 0 ? C_NULL : pointer(boxes), K, h_focus,
+        h_max, X, obj, stats, ms, want_cells ? pointer(cells) : C_NULL))
+    return X, obj, stats, ms, cells
+end
+
+"The cells of the lattice set through the binding on h (`cells_out` rows of the ensemble calls)."
+function lattice_cells(h::Handle)
+    h.ncells > 0 || throw(CovError(-2, "want_cells needs the lattice set through set_points!, set_grid_full! or fire_init!"))
+    return h.ncells
+end
+
+"Several devices of one box (`cov_multi_create`): one handle per device, borrowed with `shard_handle`."
+mutable struct MultiHandle
+    ptr::Ptr{Cvoid}
+    shards::Vector{Handle} # borrowed views of the shards' handles, one per device
+    function MultiHandle(devices::Vector{Cint})
+        out = Ref{Ptr{Cvoid}}(C_NULL)
+        rc = ccall((:cov_multi_create, LIB), Cint, (Ptr{Cint}, Cint, Ref{Ptr{Cvoid}}), devices, length(devices), out)
+        rc == 0 || throw(CovError(rc, unsafe_string(ccall((:cov_last_error, LIB), Cstring, (Ptr{Cvoid},), C_NULL))))
+        m = new(out[], Handle[])
+        for k in 0:length(devices) - 1
+            push!(m.shards, Handle(ccall((:cov_multi_handle, LIB), Ptr{Cvoid}, (Ptr{Cvoid}, Cint), m.ptr, k), 0))
+        end
+        finalizer(m -> (m.ptr == C_NULL || ccall((:cov_multi_destroy, LIB), Cvoid, (Ptr{Cvoid},), m.ptr);
+                        m.ptr = C_NULL), m)
+        return m
+    end
+end
+
+check(m::MultiHandle, rc::Cint) =
+    rc == 0 || throw(CovError(rc, unsafe_string(ccall((:cov_multi_last_error, LIB), Cstring, (Ptr{Cvoid},), m.ptr))))
+
+"""
+    shard_handle(m, k)
+
+Shard k's handle (0-based), owned by `m`: set the same store and parameters on every shard through it. Keep `m`
+alive while it is used.
+"""
+function shard_handle(m::MultiHandle, k::Integer)
+    0 <= k < length(m.shards) || throw(CovError(-1, "no shard $k"))
+    return m.shards[k + 1]
+end
+
+"""
+    multi_run_horizon_ensemble(m, x_starts; T, S = 1, spread = 3.0, N_iter = 100, granularity = 1.0, seed = 0,
+                               boxes = zeros(Float64, 4, 0), h_focus = 15.0, h_max = 30.0, want_cells = false)
+
+`run_horizon_ensemble` over the devices of `m` (`cov_multi_run_horizon_ensemble`): contiguous shards of scenarios,
+each with the keys it has in the single-device call, so the results are the same bits. Returns `(X, objectives,
+stats, cells)`.
+"""
+function multi_run_horizon_ensemble(m::MultiHandle, x_starts::Matrix{Float64}; T, S = 1, spread = 3.0, N_iter = 100,
+                                    granularity = 1.0, seed = 0, boxes::Matrix{Float64} = zeros(Float64, 4, 0),
+                                    h_focus = 15.0, h_max = 30.0, want_cells = false)
+    n, E = size(x_starts); K = size(boxes, 2)
+    X = zeros(Float64, n, T, E); obj = zeros(Float64, T, E); stats = zeros(Int64, 4, T, E)
+    cells = nothing
+    if want_cells # every shard's lattice, as set through the binding, must be the same
+        nc = lattice_cells(m.shards[1])
+        all(s -> lattice_cells(s) == nc, m.shards) || throw(CovError(-2, "the shards hold different lattices"))
+        cells = zeros(UInt8, nc, E)
+    end
+    GC.@preserve x_starts boxes X obj stats cells check(m, ccall((:cov_multi_run_horizon_ensemble, LIB), Cint,
+        (Ptr{Cvoid}, Ptr{Float64}, Int64, Int64, Int64, Float64, Int64, Float64, UInt64, Ptr{Float64}, Int64, Float64,
+         Float64, Ptr{Float64}, Ptr{Float64}, Ptr{Int64}, Ptr{UInt8}),
+        m.ptr, x_starts, E, T, S, spread, N_iter, granularity, seed, K == 0 ? C_NULL : pointer(boxes), K, h_focus,
+        h_max, X, obj, stats, want_cells ? pointer(cells) : C_NULL))
+    return X, obj, stats, cells
 end
 
 """
