@@ -39,7 +39,8 @@ extern "C" {
                                 cov_mads_solve_batch; cov_set_region, cov_eval_region_batch,
                                 cov_mads_solve_batch_region (the grid-free static objective); cov_run_horizon;
                                 cov_run_horizon_points, cov_run_horizon_fire (the dynamic horizon);
-                                cov_run_horizon_ensemble, cov_multi_run_horizon_ensemble */
+                                cov_run_horizon_ensemble, cov_multi_run_horizon_ensemble;
+                                cov_run_horizon_fire_ensemble, cov_multi_run_horizon_fire_ensemble */
 
 #if defined(__GNUC__)
 #define COV_API __attribute__((visibility("default")))
@@ -401,6 +402,35 @@ COV_API int cov_run_horizon_ensemble(cov_handle *h, const double *x_starts, int6
                                      double *X_out, double *obj_out, int64_t *stats, double *step_ms,
                                      uint8_t *cells_out);
 
+/* E independent dynamic receding horizons with the device automaton in one call, on the device side by side: scenario
+ * e (0 <= e < E) is exactly cov_run_horizon_fire(x_starts + e * 3N, T, S, spread, n_iter, granularity, seed + e * T * S,
+ * boxes, ..., fire_steps, winds[3e], winds[3e + 1], winds[3e + 2], fire_seed + e * fire_seed_stride, first_step, ...)
+ * (arithmetic mod 2^64) run on a private copy of the handle's current cell store, parameters and automaton state.  Each
+ * scenario has its own fire realisation (its fire seed), its own wind and its own starting swarm; fire_seed_stride = 1
+ * gives independent realisations (Monte Carlo), 0 gives every scenario the same fire.  fire_steps (T values) and
+ * first_step are shared by every scenario.  Every step of a timestep, each automaton step included, is one launch for
+ * the whole ensemble.
+ *
+ * x_starts: E x 3N; winds: E x 3 doubles (wind_speed, wind_direction, prob_spread).  X_out: E x T x 3N; obj_out
+ * (nullable): E x T; stats (nullable): E x T x 5 with cov_run_horizon_fire's columns [winner k, evaluations, feasible
+ * solves, entries removed, entries appended]; step_ms (nullable): T device times of the whole ensemble per timestep;
+ * cells_out (nullable): E x nx*ny bytes, the multiplicities each scenario leaves; states_out (nullable): E x nx*ny
+ * bytes, the automaton state each scenario leaves, laid out as cov_fire_get_state returns it.
+ *
+ * Every scenario starts from the same store and state, so one envelope (cov_run_horizon_fire's) serves all of them.
+ * The handle is not changed: the cell store, cov_get_grid_info, the class weights, the parameters, the ordered point
+ * list, the automaton's state and its current buffer are as before the call, so the next cov_fire_step gives what it
+ * would have given without it.  Errors: cov_run_horizon_fire's, in its order, with cov_run_horizon_ensemble's E checks
+ * after cov_run_horizon's; COV_ERR_INVALID also for winds NULL with T > 0.  T == 0 does nothing, and a refused or
+ * failed call changes nothing on the handle. */
+COV_API int cov_run_horizon_fire_ensemble(cov_handle *h, const double *x_starts, int64_t E, int64_t T, int64_t S,
+                                          double spread, int64_t n_iter, double granularity, uint64_t seed,
+                                          const double *boxes, int64_t n_boxes, double h_focus, double h_max,
+                                          const int64_t *fire_steps, const double *winds, uint64_t fire_seed,
+                                          uint64_t fire_seed_stride, int64_t first_step,
+                                          double *X_out, double *obj_out, int64_t *stats, double *step_ms,
+                                          uint8_t *cells_out, uint8_t *states_out);
+
 /* Covered-cell mask of ONE candidate: nx*ny bytes, 1 where the cell is inside some disc (whether
  * or not it holds entries). Lets the host replay an ordered Float64 sum over a weighted list. */
 COV_API int cov_covered_mask(cov_handle *h, const double *x, uint8_t *mask);
@@ -507,6 +537,16 @@ COV_API int cov_multi_run_horizon_ensemble(cov_multi *m, const double *x_starts,
                                            double spread, int64_t n_iter, double granularity, uint64_t seed,
                                            const double *boxes, int64_t n_boxes, double h_focus, double h_max,
                                            double *X_out, double *obj_out, int64_t *stats, uint8_t *cells_out);
+/* cov_run_horizon_fire_ensemble over the devices (without step_ms): contiguous shards of scenarios, shard k from
+ * scenario b0 on with seed + b0 * T * S, fire_seed + b0 * fire_seed_stride and winds + 3 * b0, so its results equal the
+ * single-device call's bit for bit.  Set the same store, parameters and automaton state on every shard's handle. */
+COV_API int cov_multi_run_horizon_fire_ensemble(cov_multi *m, const double *x_starts, int64_t E, int64_t T, int64_t S,
+                                                double spread, int64_t n_iter, double granularity, uint64_t seed,
+                                                const double *boxes, int64_t n_boxes, double h_focus, double h_max,
+                                                const int64_t *fire_steps, const double *winds, uint64_t fire_seed,
+                                                uint64_t fire_seed_stride, int64_t first_step,
+                                                double *X_out, double *obj_out, int64_t *stats, uint8_t *cells_out,
+                                                uint8_t *states_out);
 COV_API int cov_multi_argmin(cov_multi *m, const double *X, int64_t B, int32_t barrier, double *best_obj,
                      int64_t *best_idx);
 

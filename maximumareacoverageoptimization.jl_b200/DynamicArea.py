@@ -53,6 +53,18 @@ class ForestFire:
         self.t += int(fire_steps.sum())
         return out
 
+    def run_horizon_ensemble(self, x_starts, fire_steps, winds=None, fire_seed_stride: int = 1, **kw):
+        """CoverageEngine.run_horizon_fire_ensemble from this fire's current state: E scenarios, each with its own
+        starting swarm (x_starts (E, 3N)), wind (winds (E, 3) or (3,); None: this fire's wind for every scenario) and
+        fire seed self.seed + e * fire_seed_stride, all continuing at step self.t + 1, so that scenario 0 is this fire's
+        own run_horizon.  Unlike run_horizon it leaves self.t as it is: the engine's fire has not moved.
+        kw: run_horizon_fire_ensemble's S, spread, n_iter, granularity, seed, boxes, h_focus, h_max, want_cells,
+        want_states."""
+        if winds is None:
+            winds = (self.wind_speed, self.wind_direction, self.prob_spread)
+        return self.engine.run_horizon_fire_ensemble(x_starts, fire_steps, winds, self.seed, self.t + 1,
+                                                     fire_seed_stride=fire_seed_stride, **kw)
+
     def grid(self) -> np.ndarray:
         """Current state as grid[i-1, j-1]."""
         return self.engine.fire_state().reshape(self.ny, self.nx).T

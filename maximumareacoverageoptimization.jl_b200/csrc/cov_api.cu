@@ -2040,9 +2040,11 @@ struct HorizonAppend {
     std::vector<int> cell;
     std::vector<unsigned char> pcls;
     bool stamps = false; // record the last timestep that removed entries from each cell
-    // the automaton (cov_run_horizon_fire): fire_steps[t-1] steps with append at timestep t, numbered from first_step
+    // the automaton (cov_run_horizon_fire): fire_steps[t-1] steps with append at timestep t, numbered from first_step,
+    // with scenario e's 9 direction probabilities at fire_p + 9e (host) and its key fire_seed + e * fire_seed_stride
     const int64_t *fire_steps = nullptr;
-    uint64_t fire_seed = 0;
+    const double *fire_p = nullptr;
+    uint64_t fire_seed = 0, fire_seed_stride = 0;
     int64_t first_step = 0;
 };
 
@@ -2123,12 +2125,36 @@ static void entries_replay(cov_handle *h, const HorizonAppend &app, int64_t T, c
     h->ent_dev_valid = false;
 }
 
-// The scenarios of cov_run_horizon_ensemble (run_horizon; NULL: one scenario on the handle's own store): E copies of
-// the handle's store and parameters, made on the device when the call starts and dropped when it ends.
+// The scenarios of cov_run_horizon_ensemble / cov_run_horizon_fire_ensemble (run_horizon; NULL: one scenario on the
+// handle's own store): E copies of the handle's store, parameters and automaton state, made on the device when the call
+// starts and dropped when it ends.
 struct HorizonEnsemble {
     int64_t E = 1;
-    uint8_t *cells_out = nullptr; // E x nx*ny (nullable): the multiplicities each scenario leaves
+    uint8_t *cells_out = nullptr;  // E x nx*ny (nullable): the multiplicities each scenario leaves
+    uint8_t *states_out = nullptr; // E x nx*ny (nullable): the automaton state each scenario leaves
 };
+
+// The scenario counts the ensemble calls accept: E * S solves per launch (counted in int by the grid and the
+// dispenser), E * T * S keys without wrapping.
+static int check_ensemble(cov_handle *h, const char *who, int64_t E, int64_t T, int64_t S)
+{
+    if (E < 1 || E > INT32_MAX / S || (T > 0 && E * S > INT64_MAX / T))
+        return fail(h, COV_ERR_INVALID, std::string(who) + ": E must be >= 1 with E * S <= 2^31 - 1 and E * T * S <= "
+                                                           "2^63 - 1");
+    return COV_OK;
+}
+
+// The end of an ensemble call: a large ensemble would otherwise pin E copies of the store for the handle's lifetime.
+static int drop_ensemble(cov_handle *h, int rc)
+{
+    if (h->ens.p) {
+        (void)cudaStreamSynchronize(h->stream); // a failed call may still have copies in flight
+        (void)cudaFree(h->ens.p);
+        (void)cudaGetLastError();
+        h->ens = DevBuf{};
+    }
+    return rc;
+}
 
 // E copies of `bytes` bytes at src side by side at dst (device memory), in 1 + ceil(log2(E)) copies.
 static cudaError_t replicate(void *dst, const void *src, size_t bytes, int64_t E, cudaStream_t s)
@@ -2147,46 +2173,54 @@ static cudaError_t replicate(void *dst, const void *src, size_t bytes, int64_t E
 // cons3's previous swarm / the starts (horizon_start_kernel), S solves (launch_mads), the winner to cur
 // (horizon_commit_kernel), AreaMaxObjective(cur).  stamps_out (nullable, nx*ny): app's removal stamps.
 // ens: the same loop over ens->E scenarios side by side (one launch per step for all of them) on copies of the store
-// and parameters; x_start and the outputs then hold E scenarios, each of them as the single call lays it out.
+// and parameters (and, with the automaton, of its state); x_start and the outputs then hold E scenarios, each of them
+// as the single call lays it out.  The fire list (app->offsets) stays single-scenario.
 static int run_horizon(cov_handle *h, const char *who, const double *x_start, int64_t T, int64_t S, double spread,
                        int64_t n_iter, double granularity, uint64_t seed, const double *boxes, int64_t n_boxes,
                        double h_focus, double h_max, double *X_out, double *obj_out, int64_t *stats, double *step_ms,
                        HorizonAppend *app, int *stamps_out, const HorizonEnsemble *ens = nullptr)
 {
+    if (ens && app && app->offsets)
+        return fail(h, COV_ERR_INVALID, std::string(who) + ": internal: the fire list has no ensemble");
     GridDesc lg = app ? app->g : h->g;
     const int64_t E = ens ? ens->E : 1;
     const int N = h->o.N, n = 3 * N, cols = app ? 5 : 4;
     const size_t ncell = (size_t)h->g.nx * h->g.ny, P = app ? app->cell.size() : 0;
-    const bool stamps = app && app->stamps;
-    // in: [pow10 | x_start: E n | boxes: 4 n_boxes | appended cells: P ints | their classes: P bytes | the solves'
-    // inputs]; out: [the solves' outputs | X_out: T E n | obj_out: T E | stats: T E cols | removal stamps: nx*ny ints],
-    // timestep-major (a timestep's rows side by side); pinned: [the out rows after the solves' | the cells: E nx*ny]
+    const bool stamps = app && app->stamps, automaton = app && app->fire_steps;
+    // in: [pow10 | x_start: E n | boxes: 4 n_boxes | direction probabilities: E 9 | appended cells: P ints | their
+    // classes: P bytes | the solves' inputs]; out: [the solves' outputs | X_out: T E n | obj_out: T E | stats: T E cols |
+    // removal stamps: nx*ny ints], timestep-major (a timestep's rows side by side); pinned: [the out rows after the
+    // solves' | the cells: E nx*ny | the automaton states: E nx*ny]
     const size_t tn = (size_t)T * E * n;
-    const size_t o_x = kPow10Bytes, o_box = o_x + (size_t)E * n * 8, o_cell = o_box + (size_t)n_boxes * 32;
+    const size_t o_x = kPow10Bytes, o_box = o_x + (size_t)E * n * 8, o_fp = o_box + (size_t)n_boxes * 32;
+    const size_t o_cell = o_fp + (automaton ? (size_t)E * 9 * 8 : 0);
     const size_t o_cls = o_cell + P * 4, o_X0 = (o_cls + P + 7) / 8 * 8;
     const size_t o_stamp = tn * 8 + (size_t)T * E * 8 + (size_t)T * E * cols * 8;
     const size_t res_bytes = o_stamp + (stamps ? ncell * 4 : 0);
     const size_t cells_bytes = ens && ens->cells_out ? (size_t)E * ncell : 0;
+    const size_t states_bytes = ens && automaton && ens->states_out ? (size_t)E * ncell : 0;
     std::vector<unsigned char> hin(o_X0);
     MadsArgs a;
     OK(mads_buffers(h, o_X0, E * S, n, res_bytes, hin, a));
     memcpy(hin.data() + o_x, x_start, (size_t)E * n * 8);
     if (n_boxes) memcpy(hin.data() + o_box, boxes, (size_t)n_boxes * 32);
+    if (automaton) memcpy(hin.data() + o_fp, app->fire_p, (size_t)E * 9 * 8);
     if (P) {
         memcpy(hin.data() + o_cell, app->cell.data(), P * 4);
         memcpy(hin.data() + o_cls, app->pcls.data(), P);
     }
-    // the scenarios' device state: [mult: E nx*ny | cls: E nx*ny | plane sets: E | the single-plane swizzled copy, for
-    // E = 1 (launch_eval's CTA kernel may read it; the E > 1 kernels read the packed planes) | parameters: E 5N |
-    // thresholds: E 3N]
+    // the scenarios' device state: [mult: E nx*ny | cls: E nx*ny | automaton states: 2 E nx*ny, the E of either
+    // ping-pong half side by side | plane sets: E | the single-plane swizzled copy, for E = 1 (launch_eval's CTA kernel
+    // may read it; the E > 1 kernels read the packed planes) | parameters: E 5N | thresholds: E 3N]
     const size_t pw = (size_t)lg.n_planes * lg.plane_words * 4, q_bytes = ((size_t)h->g.ny * h->g.qstride + 8) * 4;
-    const bool quad = lg.planes_q && E == 1;
-    const size_t o_epl = ((size_t)2 * E * ncell + 15) / 16 * 16, o_eq = o_epl + (size_t)E * pw;
+    const bool quad = E == 1 && (app ? lg.n_planes == 1 : lg.planes_q != nullptr); // as the single call has it
+    const size_t o_efire = (size_t)2 * E * ncell, o_epl = (o_efire + (automaton ? o_efire : 0) + 15) / 16 * 16;
+    const size_t o_eq = o_epl + (size_t)E * pw;
     const size_t o_epar = o_eq + (quad ? q_bytes : 0), o_exyT = o_epar + (size_t)E * 5 * N * 8;
     if (ens) OK(ensure(h, h->ens, o_exyT + (size_t)E * n * 8));
     else OK(ensure(h, h->xyT, (size_t)n * 8));
-    OK(ensure_pinned(h, &h->h_out, &h->h_out_cap, res_bytes + cells_bytes));
-    if (app) { // the envelope's planes; rebuild_planes sizes them for the store again at the end
+    OK(ensure_pinned(h, &h->h_out, &h->h_out_cap, res_bytes + cells_bytes + states_bytes));
+    if (app && !ens) { // the envelope's planes; rebuild_planes sizes them for the store again at the end
         int rc = ensure(h, h->planes, (size_t)lg.n_planes * lg.plane_words * 4);
         if (rc == COV_OK && lg.n_planes == 1) rc = ensure(h, h->planes_q, q_bytes);
         if (rc != COV_OK) { // a buffer may have moved: describe the unchanged store again
@@ -2202,15 +2236,21 @@ static int run_horizon(cov_handle *h, const char *who, const double *x_start, in
     const double *d_x0 = (const double *)(din + o_x);
     const int *d_cell = (const int *)(din + o_cell);
     const unsigned char *d_cls = din + o_cls;
+    const double *d_fp = (const double *)(din + o_fp);
     double *d_Xo = (double *)(a.stats + 4 * E * S), *d_oo = d_Xo + tn, *xyT = (double *)h->xyT.p;
     long long *d_st = (long long *)(d_oo + T * E);
     unsigned char *mult = (unsigned char *)h->mult.p, *cls = (unsigned char *)h->cls.p;
     double *params = (double *)h->params.p;
+    unsigned char *fire[2] = {(unsigned char *)h->fire[0].p, (unsigned char *)h->fire[1].p};
+    int fire_cur = h->fire_cur;
     ObjParams o = h->o;
     if (ens) {
         unsigned char *eb = (unsigned char *)h->ens.p;
         mult = eb;
         cls = eb + (size_t)E * ncell;
+        fire[0] = eb + o_efire; // the scenarios start in half 0: one parity for all of them (the schedule is shared)
+        fire[1] = fire[0] + (size_t)E * ncell;
+        fire_cur = 0;
         lg.planes = (const uint32_t *)(eb + o_epl);
         lg.planes_q = quad ? (const uint32_t *)(eb + o_eq) : nullptr;
         params = (double *)(eb + o_epar);
@@ -2243,7 +2283,6 @@ static int run_horizon(cov_handle *h, const char *who, const double *x_start, in
     cfg.ordered = 0;
     if (cfg.kernel == COV_KERNEL_ORDERED) cfg.kernel = COV_KERNEL_AUTO;
     int *overflow = (int *)h->overflow.p;
-    int fire_cur = h->fire_cur;
     int64_t step = app ? app->first_step : 0;
     std::vector<cudaEvent_t> ev;
     if (step_ms)
@@ -2256,6 +2295,7 @@ static int run_horizon(cov_handle *h, const char *who, const double *x_start, in
         e = replicate(mult, h->mult.p, ncell, E, h->stream);
         if (e == cudaSuccess) e = replicate(cls, h->cls.p, ncell, E, h->stream);
         if (e == cudaSuccess) e = replicate(params, h->params.p, (size_t)5 * N * 8, E, h->stream);
+        if (e == cudaSuccess && automaton) e = replicate(fire[0], h->fire[h->fire_cur].p, ncell, E, h->stream);
         if (e == cudaSuccess && quad) e = cudaMemsetAsync((void *)lg.planes_q, 0, q_bytes, h->stream);
     }
     if (e == cudaSuccess) e = launch_thresholds(d_x0, N, xyT, h->stream, E), what = "launch_thresholds";
@@ -2264,9 +2304,7 @@ static int run_horizon(cov_handle *h, const char *who, const double *x_start, in
         what = "append setup";
         e = cudaMemsetAsync(overflow, 0, sizeof(int), h->stream);
         if (e == cudaSuccess && d_stamp) e = cudaMemsetAsync(d_stamp, 0, ncell * 4, h->stream);
-        if (e == cudaSuccess && lg.planes_q) e = cudaMemsetAsync((void *)lg.planes_q, 0, q_bytes, h->stream);
-        if (e == cudaSuccess && app->fire_steps)
-            e = cudaMemcpyAsync(h->fire_p.p, h->h_small->fire_p, 9 * sizeof(double), cudaMemcpyHostToDevice, h->stream);
+        if (e == cudaSuccess && lg.planes_q && !ens) e = cudaMemsetAsync((void *)lg.planes_q, 0, q_bytes, h->stream);
     }
     int rc = COV_OK;
     for (int64_t t = 1; t <= T && e == cudaSuccess && rc == COV_OK; ++t) {
@@ -2281,14 +2319,15 @@ static int run_horizon(cov_handle *h, const char *who, const double *x_start, in
                 if ((e = launch_add_points(mult, cls, d_cell + q0, d_cls + q0, q1 - q0, overflow, h->stream)) != cudaSuccess) break;
                 h->launches += 1;
             }
-        } else if (app) { // the automaton, its pushes counted into the stats row
+        } else if (app) { // the automaton, its pushes counted into the stats rows (column 4 of each scenario)
             what = "fire step";
-            if ((e = cudaMemsetAsync(row + 4, 0, sizeof(long long), h->stream)) != cudaSuccess) break;
+            e = E == 1 ? cudaMemsetAsync(row + 4, 0, sizeof(long long), h->stream)
+                       : cudaMemset2DAsync(row + 4, (size_t)cols * 8, 0, sizeof(long long), (size_t)E, h->stream);
+            if (e != cudaSuccess) break;
             for (int64_t k = 0; k < app->fire_steps[t - 1] && e == cudaSuccess; ++k, ++step) {
-                e = launch_fire_step((const unsigned char *)h->fire[fire_cur].p, (unsigned char *)h->fire[fire_cur ^ 1].p,
-                                     mult, cls, h->g.nx, h->g.ny, app->fire_seed, (unsigned int)step,
-                                     (const double *)h->fire_p.p, 1, (unsigned long long *)(row + 4), overflow,
-                                     h->stream);
+                e = launch_fire_step(fire[fire_cur], fire[fire_cur ^ 1], mult, cls, h->g.nx, h->g.ny, app->fire_seed,
+                                     (unsigned int)step, d_fp, 1, (unsigned long long *)(row + 4), overflow, h->stream,
+                                     E, app->fire_seed_stride, cols);
                 if (e == cudaSuccess) fire_cur ^= 1;
                 h->launches += 1;
             }
@@ -2330,12 +2369,15 @@ static int run_horizon(cov_handle *h, const char *who, const double *x_start, in
         }
         h->launches += lg.planes_q ? 7 : 6;
     }
-    h->fire_cur = fire_cur; // the automaton steps enqueued stand
+    if (!ens) h->fire_cur = fire_cur; // the automaton steps enqueued stand
     if (e == cudaSuccess && rc == COV_OK && step_ms) e = cudaEventRecord(ev[(size_t)T], h->stream), what = "event";
     if (e == cudaSuccess && rc == COV_OK)
         e = cudaMemcpyAsync(h->h_out, d_Xo, res_bytes, cudaMemcpyDeviceToHost, h->stream), what = "download";
     if (cells_bytes && e == cudaSuccess && rc == COV_OK)
         e = cudaMemcpyAsync((unsigned char *)h->h_out + res_bytes, mult, cells_bytes, cudaMemcpyDeviceToHost, h->stream);
+    if (states_bytes && e == cudaSuccess && rc == COV_OK)
+        e = cudaMemcpyAsync((unsigned char *)h->h_out + res_bytes + cells_bytes, fire[fire_cur], states_bytes,
+                            cudaMemcpyDeviceToHost, h->stream);
     if (app && e == cudaSuccess && rc == COV_OK)
         e = cudaMemcpyAsync(&h->h_small->overflow, overflow, sizeof(int), cudaMemcpyDeviceToHost, h->stream);
     const int n_classes = app ? app->n_classes : h->g.n_classes;
@@ -2368,9 +2410,14 @@ static int run_horizon(cov_handle *h, const char *who, const double *x_start, in
             if (app && app->offsets) hst[cols * t + 4] = app->offsets[t + 1] - app->offsets[t];
             if (app) pushed |= hst[cols * t + 4] != 0;
         }
-        if (app && app->fire_steps && pushed) entries_forget(h); // cov_fire_step: the automaton's order is createPOI's
-        else if (app && app->offsets && h->ent_known) entries_replay(h, *app, T, hstamp);
-        else if (removed && !ens) entries_note_removals(h);
+        if (ens) { // the handle's list is untouched
+        } else if (automaton && pushed) {
+            entries_forget(h); // cov_fire_step: the automaton's order is createPOI's
+        } else if (app && app->offsets && h->ent_known) {
+            entries_replay(h, *app, T, hstamp);
+        } else if (removed) {
+            entries_note_removals(h);
+        }
         for (int64_t q = 0; q < E; ++q) // timestep-major rows to the scenario-major outputs
             for (int64_t t = 0; t < T; ++t) {
                 const size_t src = (size_t)(t * E + q), dst = (size_t)(q * T + t);
@@ -2379,6 +2426,7 @@ static int run_horizon(cov_handle *h, const char *who, const double *x_start, in
                 if (stats) memcpy(stats + dst * cols, hst + src * cols, (size_t)cols * 8);
             }
         if (cells_bytes) memcpy(ens->cells_out, (const unsigned char *)h->h_out + res_bytes, cells_bytes);
+        if (states_bytes) memcpy(ens->states_out, (const unsigned char *)h->h_out + res_bytes + cells_bytes, states_bytes);
         if (stamps && stamps_out) memcpy(stamps_out, hstamp, ncell * 4);
         for (int64_t t = 0; step_ms && t < T; ++t) {
             float ms = 0;
@@ -2418,22 +2466,12 @@ extern "C" int cov_run_horizon_ensemble(cov_handle *h, const double *x_starts, i
     if (!h) return fail(nullptr, COV_ERR_INVALID, "NULL handle");
     DeviceGuard dg(h->device);
     OK(check_horizon(h, who, x_starts, T, S, spread, n_iter, granularity, boxes, n_boxes, X_out));
-    // E * S solves per launch (counted in int by the grid and the dispenser), E * T * S keys without wrapping
-    if (E < 1 || E > INT32_MAX / S || (T > 0 && E * S > INT64_MAX / T))
-        return fail(h, COV_ERR_INVALID, std::string(who) + ": E must be >= 1 with E * S <= 2^31 - 1 and E * T * S <= "
-                                                           "2^63 - 1");
+    OK(check_ensemble(h, who, E, T, S));
     if (T == 0) return COV_OK;
     OK(check_mads_limits(h, who, &h->g));
-    const HorizonEnsemble ens{E, cells_out};
-    const int rc = run_horizon(h, who, x_starts, T, S, spread, n_iter, granularity, seed, boxes, n_boxes, h_focus, h_max,
-                               X_out, obj_out, stats, step_ms, nullptr, nullptr, &ens);
-    if (h->ens.p) { // a large ensemble would otherwise pin E copies of the store for the handle's lifetime
-        (void)cudaStreamSynchronize(h->stream); // a failed call may still have copies in flight
-        (void)cudaFree(h->ens.p);
-        (void)cudaGetLastError();
-        h->ens = DevBuf{};
-    }
-    return rc;
+    const HorizonEnsemble ens{E, cells_out, nullptr};
+    return drop_ensemble(h, run_horizon(h, who, x_starts, T, S, spread, n_iter, granularity, seed, boxes, n_boxes,
+                                        h_focus, h_max, X_out, obj_out, stats, step_ms, nullptr, nullptr, &ens));
 }
 
 // The cell store's bytes as they are (one download, one synchronise).
@@ -2513,29 +2551,31 @@ extern "C" int cov_run_horizon_points(cov_handle *h, const double *x_start, int6
                        obj_out, stats, step_ms, &app, last_removed);
 }
 
-extern "C" int cov_run_horizon_fire(cov_handle *h, const double *x_start, int64_t T, int64_t S, double spread,
-                                    int64_t n_iter, double granularity, uint64_t seed, const double *boxes,
-                                    int64_t n_boxes, double h_focus, double h_max, const int64_t *fire_steps,
-                                    double wind_speed, double wind_direction, double prob_spread, uint64_t fire_seed,
-                                    int64_t first_step, double *X_out, double *obj_out, int64_t *stats,
-                                    double *step_ms)
+// cov_run_horizon_fire (ens NULL, winds one triple) and cov_run_horizon_fire_ensemble (winds: E triples wind_speed,
+// wind_direction, prob_spread): the checks in cov_run_horizon_fire's order, the envelope, the loop.  Every scenario
+// starts from the handle's store and automaton state, so one envelope serves all of them.
+static int horizon_fire(cov_handle *h, const char *who, const double *x_start, int64_t T, int64_t S, double spread,
+                        int64_t n_iter, double granularity, uint64_t seed, const double *boxes, int64_t n_boxes,
+                        double h_focus, double h_max, const int64_t *fire_steps, const double *winds,
+                        uint64_t fire_seed, uint64_t fire_seed_stride, int64_t first_step, double *X_out,
+                        double *obj_out, int64_t *stats, double *step_ms, const HorizonEnsemble *ens)
 {
-    const char *who = "cov_run_horizon_fire";
-    if (!h) return fail(nullptr, COV_ERR_INVALID, "NULL handle");
-    DeviceGuard dg(h->device);
+    const int64_t E = ens ? ens->E : 1;
     OK(check_horizon(h, who, x_start, T, S, spread, n_iter, granularity, boxes, n_boxes, X_out));
+    if (ens) OK(check_ensemble(h, who, E, T, S));
     OK(check_fire_store(h, who));
-    if (T > 0 && !fire_steps) return fail(h, COV_ERR_INVALID, "cov_run_horizon_fire: fire_steps is NULL");
+    if (T > 0 && !fire_steps) return fail(h, COV_ERR_INVALID, std::string(who) + ": fire_steps is NULL");
+    if (T > 0 && !winds) return fail(h, COV_ERR_INVALID, std::string(who) + ": winds is NULL");
     constexpr int64_t kSteps = 0x100000000ll; // step numbers are 32-bit (cov_fire_step)
     int64_t total = 0;
     for (int64_t t = 0; t < T; ++t) {
         if (fire_steps[t] < 0 || fire_steps[t] > kSteps - total)
-            return fail(h, COV_ERR_INVALID, "cov_run_horizon_fire: fire_steps must be >= 0 with step numbers below 2^32");
+            return fail(h, COV_ERR_INVALID, std::string(who) + ": fire_steps must be >= 0 with step numbers below 2^32");
         total += fire_steps[t];
     }
     if (first_step < 0 || first_step > kSteps - total)
-        return fail(h, COV_ERR_INVALID, "cov_run_horizon_fire: the steps first_step .. first_step + sum(fire_steps) - 1 "
-                                        "must lie in 0 .. 2^32 - 1");
+        return fail(h, COV_ERR_INVALID, std::string(who) + ": the steps first_step .. first_step + sum(fire_steps) - 1 "
+                                                           "must lie in 0 .. 2^32 - 1");
     if (T == 0) return COV_OK;
     std::vector<unsigned char> m, k, st;
     OK(download_cells(h, m, k, &st));
@@ -2550,20 +2590,55 @@ extern "C" int cov_run_horizon_fire(cov_handle *h, const double *x_start, int64_
             const unsigned b = m[c] + (tree ? 8u : 0u);
             trees += tree ? 1 : 0;
             if (b > 255)
-                return fail(h, COV_ERR_LIMIT, "cov_run_horizon_fire: more than 255 list entries on one cell (removals "
-                                              "ignored)");
+                return fail(h, COV_ERR_LIMIT, std::string(who) + ": more than 255 list entries on one cell (removals "
+                                                                 "ignored)");
             max_mult[0] = std::max(max_mult[0], b);
         }
     HorizonAppend app;
     app.n_classes = 1;
     app.cw[0] = h->g.class_weight[0];
     OK(horizon_envelope(h, who, app, max_mult, h->n_entries + 8 * trees));
+    std::vector<double> fp((size_t)E * 9);
+    for (int64_t e = 0; e < E; ++e) fire_probs(winds[3 * e], winds[3 * e + 1], winds[3 * e + 2], fp.data() + 9 * e);
     app.fire_steps = fire_steps;
+    app.fire_p = fp.data();
     app.fire_seed = fire_seed;
+    app.fire_seed_stride = fire_seed_stride;
     app.first_step = first_step;
-    fire_probs(wind_speed, wind_direction, prob_spread, h->h_small->fire_p);
     return run_horizon(h, who, x_start, T, S, spread, n_iter, granularity, seed, boxes, n_boxes, h_focus, h_max, X_out,
-                       obj_out, stats, step_ms, &app, nullptr);
+                       obj_out, stats, step_ms, &app, nullptr, ens);
+}
+
+extern "C" int cov_run_horizon_fire(cov_handle *h, const double *x_start, int64_t T, int64_t S, double spread,
+                                    int64_t n_iter, double granularity, uint64_t seed, const double *boxes,
+                                    int64_t n_boxes, double h_focus, double h_max, const int64_t *fire_steps,
+                                    double wind_speed, double wind_direction, double prob_spread, uint64_t fire_seed,
+                                    int64_t first_step, double *X_out, double *obj_out, int64_t *stats,
+                                    double *step_ms)
+{
+    if (!h) return fail(nullptr, COV_ERR_INVALID, "NULL handle");
+    DeviceGuard dg(h->device);
+    const double wind[3] = {wind_speed, wind_direction, prob_spread};
+    return horizon_fire(h, "cov_run_horizon_fire", x_start, T, S, spread, n_iter, granularity, seed, boxes, n_boxes,
+                        h_focus, h_max, fire_steps, wind, fire_seed, 0, first_step, X_out, obj_out, stats, step_ms,
+                        nullptr);
+}
+
+extern "C" int cov_run_horizon_fire_ensemble(cov_handle *h, const double *x_starts, int64_t E, int64_t T, int64_t S,
+                                             double spread, int64_t n_iter, double granularity, uint64_t seed,
+                                             const double *boxes, int64_t n_boxes, double h_focus, double h_max,
+                                             const int64_t *fire_steps, const double *winds, uint64_t fire_seed,
+                                             uint64_t fire_seed_stride, int64_t first_step, double *X_out,
+                                             double *obj_out, int64_t *stats, double *step_ms, uint8_t *cells_out,
+                                             uint8_t *states_out)
+{
+    if (!h) return fail(nullptr, COV_ERR_INVALID, "NULL handle");
+    DeviceGuard dg(h->device);
+    const HorizonEnsemble ens{E, cells_out, states_out};
+    return drop_ensemble(h, horizon_fire(h, "cov_run_horizon_fire_ensemble", x_starts, T, S, spread, n_iter,
+                                         granularity, seed, boxes, n_boxes, h_focus, h_max, fire_steps, winds,
+                                         fire_seed, fire_seed_stride, first_step, X_out, obj_out, stats, step_ms,
+                                         &ens));
 }
 
 extern "C" int cov_argmin(cov_handle *h, const double *X, int64_t B, int32_t barrier, double *best_obj,
@@ -3002,6 +3077,34 @@ extern "C" int cov_multi_run_horizon_ensemble(cov_multi *m, const double *x_star
                                         seed + (uint64_t)b0 * (uint64_t)T * (uint64_t)S, boxes, n_boxes, h_focus, h_max,
                                         X_out + r0 * n, obj_out ? obj_out + r0 : nullptr, stats ? stats + r0 * 4 : nullptr,
                                         nullptr, cells_out ? cells_out + (size_t)b0 * ncell : nullptr);
+    });
+}
+
+// Scenarios b0 .. b0 + bn - 1 on shard k with the keys, fire seeds and winds they have in the single-device call.
+extern "C" int cov_multi_run_horizon_fire_ensemble(cov_multi *m, const double *x_starts, int64_t E, int64_t T, int64_t S,
+                                                   double spread, int64_t n_iter, double granularity, uint64_t seed,
+                                                   const double *boxes, int64_t n_boxes, double h_focus, double h_max,
+                                                   const int64_t *fire_steps, const double *winds, uint64_t fire_seed,
+                                                   uint64_t fire_seed_stride, int64_t first_step, double *X_out,
+                                                   double *obj_out, int64_t *stats, uint8_t *cells_out,
+                                                   uint8_t *states_out)
+{
+    if (!m) return fail(nullptr, COV_ERR_INVALID, "NULL multi handle");
+    if (E < 1 || T < 0 || (T > 0 && (!x_starts || !X_out || !winds))) {
+        m->err = "cov_multi_run_horizon_fire_ensemble: bad arguments";
+        return COV_ERR_INVALID;
+    }
+    return run_shards(m, x_starts, E, [&](int, cov_handle *h, const double *Xk, int64_t b0, int64_t bn) {
+        const size_t n = h->have_params ? 3 * (size_t)h->o.N : 0, ncell = (size_t)h->g.nx * h->g.ny;
+        const size_t r0 = (size_t)b0 * (size_t)T;
+        return cov_run_horizon_fire_ensemble(h, Xk, bn, T, S, spread, n_iter, granularity,
+                                             seed + (uint64_t)b0 * (uint64_t)T * (uint64_t)S, boxes, n_boxes, h_focus,
+                                             h_max, fire_steps, winds ? winds + 3 * b0 : nullptr,
+                                             fire_seed + (uint64_t)b0 * fire_seed_stride, fire_seed_stride, first_step,
+                                             X_out + r0 * n, obj_out ? obj_out + r0 : nullptr,
+                                             stats ? stats + r0 * 5 : nullptr, nullptr,
+                                             cells_out ? cells_out + (size_t)b0 * ncell : nullptr,
+                                             states_out ? states_out + (size_t)b0 * ncell : nullptr);
     });
 }
 

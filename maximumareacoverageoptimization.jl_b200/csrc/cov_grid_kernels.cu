@@ -220,8 +220,10 @@ cudaError_t launch_remove_covered(unsigned char *mult, unsigned char *cls, const
                                   unsigned long long *removed, cudaStream_t s, int *stamp, int t_stamp, long long E,
                                   long long removed_stride)
 {
-    // the counters of the E stores and whatever lies between them (the callers' rows are rewritten afterwards)
-    cudaError_t e = cudaMemsetAsync(removed, 0, (size_t)((E - 1) * removed_stride + 1) * sizeof(unsigned long long), s);
+    // the counters of the E stores only: what lies between them (a fire step's push counts) stays
+    cudaError_t e = E == 1 ? cudaMemsetAsync(removed, 0, sizeof(unsigned long long), s)
+                           : cudaMemset2DAsync(removed, (size_t)removed_stride * sizeof(unsigned long long), 0,
+                                               sizeof(unsigned long long), (size_t)E, s);
     if (e != cudaSuccess) return e;
     const long long ncell = (long long)g.nx * g.ny;
     remove_covered_kernel<<<store_grid(ncell, 256, 148 * 8, E), 256, 0, s>>>(mult, cls, g, xyT, N, removed, stamp,
@@ -422,42 +424,50 @@ __device__ __forceinline__ double u01_53(uint32_t a, uint32_t b)
 // one list entry (so a cell can be pushed several times in a step: the duplicates of FirePoints.xlsx).
 // rand() is replaced by a counter-based uniform: Philox4x32-10 with counter
 // (cell index, step, neighbour index k = (a-1) + 3(b-1), 0) and key = seed.
+// blockIdx.y strides over E automata side by side (launch_fire_step); E = 1 with zero strides is the single automaton.
 __global__ void fire_step_kernel(const unsigned char *__restrict__ cur, unsigned char *__restrict__ nxt,
                                  unsigned char *mult, unsigned char *cls, int nx, int ny, unsigned long long seed,
                                  unsigned int step, const double *__restrict__ p_dir, int append,
-                                 unsigned long long *pushed, int *overflow)
+                                 unsigned long long *pushed, int *overflow, long long E, unsigned long long seed_stride,
+                                 long long pushed_stride)
 {
     const long long ncell = (long long)nx * ny;
-    unsigned long long mine = 0;
-    for (long long t = blockIdx.x * (long long)blockDim.x + threadIdx.x; t < ncell;
-         t += (long long)gridDim.x * blockDim.x) {
-        const int i = (int)(t % nx) + 1, j = (int)(t / nx) + 1; // 1-based grid[i, j]
-        unsigned char st = cur[t];
-        unsigned pushes = 0;
-        if (st == 1 && i >= 2 && i <= nx - 1 && j >= 2 && j <= ny - 1) {
-            for (int b = 1; b <= 3; ++b)
-                for (int a = 1; a <= 3; ++a) {
-                    const long long nb = (long long)(i - 2 + a - 1) + (long long)nx * (j - 2 + b - 1);
-                    if (cur[nb] != 2) continue;
-                    const int k = (a - 1) + 3 * (b - 1);
-                    uint32_t r[4];
-                    philox4x32_10((uint32_t)t, step, (uint32_t)k, (uint32_t)((unsigned long long)t >> 32),
-                                  (uint32_t)seed, (uint32_t)(seed >> 32), r);
-                    if (p_dir[k] > u01_53(r[0], r[1])) ++pushes;
-                }
-            if (pushes) st = 2;
+    for (long long e = blockIdx.y; e < E; e += gridDim.y) {
+        const unsigned char *ce = cur + e * ncell;
+        unsigned char *ne = nxt + e * ncell, *me = mult + e * ncell, *ke = cls + e * ncell;
+        const double *pe = p_dir + 9 * e;
+        const unsigned long long key = seed + (unsigned long long)e * seed_stride;
+        unsigned long long mine = 0;
+        for (long long t = blockIdx.x * (long long)blockDim.x + threadIdx.x; t < ncell;
+             t += (long long)gridDim.x * blockDim.x) {
+            const int i = (int)(t % nx) + 1, j = (int)(t / nx) + 1; // 1-based grid[i, j]
+            unsigned char st = ce[t];
+            unsigned pushes = 0;
+            if (st == 1 && i >= 2 && i <= nx - 1 && j >= 2 && j <= ny - 1) {
+                for (int b = 1; b <= 3; ++b)
+                    for (int a = 1; a <= 3; ++a) {
+                        const long long nb = (long long)(i - 2 + a - 1) + (long long)nx * (j - 2 + b - 1);
+                        if (ce[nb] != 2) continue;
+                        const int k = (a - 1) + 3 * (b - 1);
+                        uint32_t r[4];
+                        philox4x32_10((uint32_t)t, step, (uint32_t)k, (uint32_t)((unsigned long long)t >> 32),
+                                      (uint32_t)key, (uint32_t)(key >> 32), r);
+                        if (pe[k] > u01_53(r[0], r[1])) ++pushes;
+                    }
+                if (pushes) st = 2;
+            }
+            ne[t] = st;
+            if (pushes && append) {
+                const unsigned m = me[t] + pushes; // one thread per cell: no race
+                if (m > 255u) atomicExch(overflow, 1);
+                me[t] = (unsigned char)(m > 255u ? 255u : m);
+                ke[t] = 0;
+            }
+            mine += pushes;
         }
-        nxt[t] = st;
-        if (pushes && append) {
-            const unsigned m = mult[t] + pushes; // one thread per cell: no race
-            if (m > 255u) atomicExch(overflow, 1);
-            mult[t] = (unsigned char)(m > 255u ? 255u : m);
-            cls[t] = 0;
-        }
-        mine += pushes;
+        for (int off = 16; off; off >>= 1) mine += __shfl_xor_sync(0xffffffffu, mine, off);
+        if ((threadIdx.x & 31) == 0 && mine) atomicAdd(pushed + e * pushed_stride, mine);
     }
-    for (int off = 16; off; off >>= 1) mine += __shfl_xor_sync(0xffffffffu, mine, off);
-    if ((threadIdx.x & 31) == 0 && mine) atomicAdd(pushed, mine);
 }
 
 // initial state -> the list entries of the ignition cells (src/DynamicArea.jl:37-43)
@@ -767,13 +777,13 @@ cudaError_t launch_union_area(const double *dX, long long B, int N, double *d_ar
 
 cudaError_t launch_fire_step(const unsigned char *cur, unsigned char *nxt, unsigned char *mult, unsigned char *cls,
                              int nx, int ny, unsigned long long seed, unsigned int step, const double *p_dir,
-                             int append, unsigned long long *pushed, int *overflow, cudaStream_t s)
+                             int append, unsigned long long *pushed, int *overflow, cudaStream_t s, long long E,
+                             unsigned long long seed_stride, long long pushed_stride)
 {
     const long long ncell = (long long)nx * ny;
-    const int block = 256;
-    const int grid = (int)std::min<long long>((ncell + block - 1) / block, 148 * 8);
-    fire_step_kernel<<<max(grid, 1), block, 0, s>>>(cur, nxt, mult, cls, nx, ny, seed, step, p_dir, append, pushed,
-                                                    overflow);
+    fire_step_kernel<<<store_grid(ncell, 256, 148 * 8, E), 256, 0, s>>>(cur, nxt, mult, cls, nx, ny, seed, step, p_dir,
+                                                                        append, pushed, overflow, E, seed_stride,
+                                                                        pushed_stride);
     return cudaGetLastError();
 }
 cudaError_t launch_fire_seed(const unsigned char *state, unsigned char *mult, unsigned char *cls, long long ncell,

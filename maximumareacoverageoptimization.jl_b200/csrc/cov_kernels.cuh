@@ -143,9 +143,13 @@ cudaError_t launch_add_points(unsigned char *mult, unsigned char *cls, const int
 cudaError_t launch_argmin(const double *obj, const unsigned char *feasible, long long B, int barrier,
                           double *scratch_obj, long long *scratch_idx, int scratch_n, cudaStream_t s);
 cudaError_t launch_union_area(const double *dX, long long B, int N, double *d_area, cudaStream_t s);
+// E automata side by side (cov_run_horizon_fire_ensemble): automaton e's cur / nxt / mult / cls at e * nx*ny bytes, its
+// 9 direction probabilities at p_dir + 9e, its key seed + e * seed_stride (mod 2^64), its push counter at
+// pushed + e * pushed_stride; overflow is shared.
 cudaError_t launch_fire_step(const unsigned char *cur, unsigned char *nxt, unsigned char *mult, unsigned char *cls,
                              int nx, int ny, unsigned long long seed, unsigned int step, const double *p_dir,
-                             int append, unsigned long long *pushed, int *overflow, cudaStream_t s);
+                             int append, unsigned long long *pushed, int *overflow, cudaStream_t s, long long E = 1,
+                             unsigned long long seed_stride = 0, long long pushed_stride = 0);
 cudaError_t launch_fire_seed(const unsigned char *state, unsigned char *mult, unsigned char *cls, long long ncell,
                              int push_initial, cudaStream_t s);
 cudaError_t launch_generate(double *dX, long long B, int N, unsigned long long seed, long long first,

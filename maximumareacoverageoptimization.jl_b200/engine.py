@@ -415,6 +415,49 @@ class CoverageEngine:
         out = (X, obj, {name: st[:, :, q].copy() for q, name in enumerate(names)}, ms)
         return out + (cells,) if want_cells else out
 
+    def run_horizon_fire_ensemble(self, x_starts, fire_steps, winds, fire_seed: int, first_step: int,
+                                  fire_seed_stride: int = 1, S: int = 1, spread: float = 3.0, n_iter: int = 100,
+                                  granularity: float = 1.0, seed: int = 0, boxes=None, h_focus: float = 15.0,
+                                  h_max: float = 30.0, want_cells: bool = False, want_states: bool = False):
+        """E independent run_horizon_fire scenarios in one call (cov_run_horizon_fire_ensemble), each on a private copy
+        of the engine's current store, parameters and automaton state: scenario e starts from x_starts[e] ((E, 3N)),
+        with the wind winds[e] ((E, 3) rows wind_speed, wind_direction, prob_spread, or one (3,) row for every
+        scenario), and equals run_horizon_fire with seed + e * T * S and fire_seed + e * fire_seed_stride (stride 1:
+        independent fires, 0: the same fire).  The engine is left unchanged.  Returns (X (E, T, 3N), obj (E, T), stats,
+        step_ms (T,)) with stats a dict of (E, T) int64 arrays (run_horizon_fire's, "appended" included), then with
+        want_cells=True cells (E, nx*ny), the multiplicities each scenario leaves, and with want_states=True states
+        (E, nx*ny), the automaton state each scenario leaves (fire_state's layout)."""
+        X0 = _f64(x_starts)
+        if X0.ndim == 1:
+            X0 = X0.reshape(1, -1)
+        if self.N is None or X0.ndim != 2 or X0.shape[1] != 3 * self.N:
+            raise ValueError("x_starts must be (E, 3N) with the N given to set_params")
+        E, n = X0.shape[0], 3 * self.N
+        fs = np.ascontiguousarray(fire_steps, dtype=np.int64).ravel()
+        W = _f64(winds)
+        if W.shape == (3,):
+            W = np.repeat(W[None], E, axis=0)
+        if W.shape != (E, 3):
+            raise ValueError("winds must be (E, 3) or (3,): wind_speed, wind_direction, prob_spread")
+        W = np.ascontiguousarray(W)
+        T = fs.size
+        B = np.zeros((0, 4)) if boxes is None else _f64(boxes).reshape(-1, 4)
+        X = np.empty((E, T, n))
+        obj = np.empty((E, T))
+        st = np.empty((E, T, 5), dtype=np.int64)
+        ms = np.empty(T)
+        gi = self.grid_info() if want_cells or want_states else None
+        cells = np.empty((E, gi["nx"] * gi["ny"]), dtype=np.uint8) if want_cells else None
+        states = np.empty((E, gi["nx"] * gi["ny"]), dtype=np.uint8) if want_states else None
+        self._check(lib.cov_run_horizon_fire_ensemble(
+            self._h, _ptr(X0), E, T, int(S), float(spread), int(n_iter), float(granularity), int(seed) & (2**64 - 1),
+            _ptr(B) if len(B) else None, len(B), float(h_focus), float(h_max), _ptr(fs), _ptr(W),
+            int(fire_seed) & (2**64 - 1), int(fire_seed_stride) & (2**64 - 1), int(first_step), _ptr(X), _ptr(obj),
+            _ptr(st), _ptr(ms), _ptr(cells), _ptr(states)))
+        names = ("winner", "evaluations", "feasible", "removed", "appended")
+        out = (X, obj, {name: st[:, :, q].copy() for q, name in enumerate(names)}, ms)
+        return out + tuple(a for a, want in ((cells, want_cells), (states, want_states)) if want)
+
     def _horizon(self, fn, x_start, T, cols, S, spread, n_iter, granularity, seed, boxes, h_focus, h_max, source,
                  tail=()):
         x_start = _f64(x_start).ravel()

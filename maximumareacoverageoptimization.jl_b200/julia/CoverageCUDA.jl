@@ -392,6 +392,50 @@ function run_horizon_ensemble(h::Handle, x_starts::Matrix{Float64}; T, S = 1, sp
     return X, obj, stats, ms, cells
 end
 
+"""
+    run_horizon_fire_ensemble(h, x_starts, fire_steps; winds = [4.0, deg2rad(270.0), 0.5], fire_seed = 0,
+                              fire_seed_stride = 1, first_step = 1, S = 1, spread = 3.0, N_iter = 100,
+                              granularity = 1.0, seed = 0, boxes = zeros(Float64, 4, 0), h_focus = 15.0, h_max = 30.0,
+                              want_cells = false, want_states = false)
+
+E independent `run_horizon_fire` scenarios in one call (`cov_run_horizon_fire_ensemble`, after `fire_init!`), each on
+a private copy of the handle's current store, parameters and automaton state: column e of `x_starts` (3N x E) starts
+scenario e, column e of `winds` (3 x E rows wind_speed, wind_direction, prob_spread; a 3-vector: the same wind for
+every scenario) is its wind, and it equals `run_horizon_fire` with `seed + (e - 1) * T * S` and
+`fire_seed + (e - 1) * fire_seed_stride` (stride 1: independent fires, 0: the same fire). The handle is left
+unchanged. Returns `(X, objectives, stats, step_ms, cells, states)`: `X` 3N x T x E, `objectives` T x E, `stats`
+5 x T x E (`run_horizon_fire`'s rows), `step_ms` the device time of every timestep of the whole ensemble, `cells` and
+`states` (nx*ny x E, with `want_cells` / `want_states`; else `nothing`) the multiplicities and the automaton state
+each scenario leaves.
+"""
+function run_horizon_fire_ensemble(h::Handle, x_starts::Matrix{Float64}, fire_steps::Vector{Int64};
+                                   winds::VecOrMat{Float64} = [4.0, deg2rad(270.0), 0.5], fire_seed = 0,
+                                   fire_seed_stride = 1, first_step = 1, S = 1, spread = 3.0, N_iter = 100,
+                                   granularity = 1.0, seed = 0, boxes::Matrix{Float64} = zeros(Float64, 4, 0),
+                                   h_focus = 15.0, h_max = 30.0, want_cells = false, want_states = false)
+    n, E = size(x_starts); K = size(boxes, 2); T = length(fire_steps)
+    W = fire_winds(winds, E)
+    X = zeros(Float64, n, T, E); obj = zeros(Float64, T, E); stats = zeros(Int64, 5, T, E); ms = zeros(Float64, T)
+    cells = want_cells ? zeros(UInt8, lattice_cells(h), E) : nothing
+    states = want_states ? zeros(UInt8, lattice_cells(h), E) : nothing
+    GC.@preserve x_starts boxes fire_steps W X obj stats ms cells states check(h,
+        ccall((:cov_run_horizon_fire_ensemble, LIB), Cint,
+        (Ptr{Cvoid}, Ptr{Float64}, Int64, Int64, Int64, Float64, Int64, Float64, UInt64, Ptr{Float64}, Int64, Float64,
+         Float64, Ptr{Int64}, Ptr{Float64}, UInt64, UInt64, Int64, Ptr{Float64}, Ptr{Float64}, Ptr{Int64}, Ptr{Float64},
+         Ptr{UInt8}, Ptr{UInt8}),
+        h.ptr, x_starts, E, T, S, spread, N_iter, granularity, seed, K == 0 ? C_NULL : pointer(boxes), K, h_focus,
+        h_max, fire_steps, W, fire_seed, fire_seed_stride, first_step, X, obj, stats, ms,
+        want_cells ? pointer(cells) : C_NULL, want_states ? pointer(states) : C_NULL))
+    return X, obj, stats, ms, cells, states
+end
+
+"The 3 x E winds of the fire ensembles: a 3-vector repeated for every scenario, or 3 x E as given."
+function fire_winds(winds::VecOrMat{Float64}, E::Integer)
+    W = winds isa Vector ? repeat(winds, 1, E) : winds
+    size(W) == (3, E) || throw(CovError(-2, "winds must be 3 x E or a 3-vector"))
+    return W
+end
+
 "The cells of the lattice set through the binding on h (`cells_out` rows of the ensemble calls)."
 function lattice_cells(h::Handle)
     h.ncells > 0 || throw(CovError(-2, "want_cells needs the lattice set through set_points!, set_grid_full! or fire_init!"))
@@ -455,6 +499,43 @@ function multi_run_horizon_ensemble(m::MultiHandle, x_starts::Matrix{Float64}; T
         m.ptr, x_starts, E, T, S, spread, N_iter, granularity, seed, K == 0 ? C_NULL : pointer(boxes), K, h_focus,
         h_max, X, obj, stats, want_cells ? pointer(cells) : C_NULL))
     return X, obj, stats, cells
+end
+
+"""
+    multi_run_horizon_fire_ensemble(m, x_starts, fire_steps; winds = [4.0, deg2rad(270.0), 0.5], fire_seed = 0,
+                                    fire_seed_stride = 1, first_step = 1, S = 1, spread = 3.0, N_iter = 100,
+                                    granularity = 1.0, seed = 0, boxes = zeros(Float64, 4, 0), h_focus = 15.0,
+                                    h_max = 30.0, want_cells = false, want_states = false)
+
+`run_horizon_fire_ensemble` over the devices of `m` (`cov_multi_run_horizon_fire_ensemble`): contiguous shards of
+scenarios, each with the keys, fire seeds and winds it has in the single-device call, so the results are the same
+bits. Call `fire_init!` and set the same parameters on every `shard_handle` first. Returns `(X, objectives, stats,
+cells, states)`.
+"""
+function multi_run_horizon_fire_ensemble(m::MultiHandle, x_starts::Matrix{Float64}, fire_steps::Vector{Int64};
+                                         winds::VecOrMat{Float64} = [4.0, deg2rad(270.0), 0.5], fire_seed = 0,
+                                         fire_seed_stride = 1, first_step = 1, S = 1, spread = 3.0, N_iter = 100,
+                                         granularity = 1.0, seed = 0, boxes::Matrix{Float64} = zeros(Float64, 4, 0),
+                                         h_focus = 15.0, h_max = 30.0, want_cells = false, want_states = false)
+    n, E = size(x_starts); K = size(boxes, 2); T = length(fire_steps)
+    W = fire_winds(winds, E)
+    X = zeros(Float64, n, T, E); obj = zeros(Float64, T, E); stats = zeros(Int64, 5, T, E)
+    cells = states = nothing
+    if want_cells || want_states # every shard's lattice, as set through the binding, must be the same
+        nc = lattice_cells(m.shards[1])
+        all(s -> lattice_cells(s) == nc, m.shards) || throw(CovError(-2, "the shards hold different lattices"))
+        cells = want_cells ? zeros(UInt8, nc, E) : nothing
+        states = want_states ? zeros(UInt8, nc, E) : nothing
+    end
+    GC.@preserve x_starts boxes fire_steps W X obj stats cells states check(m,
+        ccall((:cov_multi_run_horizon_fire_ensemble, LIB), Cint,
+        (Ptr{Cvoid}, Ptr{Float64}, Int64, Int64, Int64, Float64, Int64, Float64, UInt64, Ptr{Float64}, Int64, Float64,
+         Float64, Ptr{Int64}, Ptr{Float64}, UInt64, UInt64, Int64, Ptr{Float64}, Ptr{Float64}, Ptr{Int64}, Ptr{UInt8},
+         Ptr{UInt8}),
+        m.ptr, x_starts, E, T, S, spread, N_iter, granularity, seed, K == 0 ? C_NULL : pointer(boxes), K, h_focus,
+        h_max, fire_steps, W, fire_seed, fire_seed_stride, first_step, X, obj, stats,
+        want_cells ? pointer(cells) : C_NULL, want_states ? pointer(states) : C_NULL))
+    return X, obj, stats, cells, states
 end
 
 """
