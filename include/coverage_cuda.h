@@ -277,7 +277,9 @@ COV_API int cov_mads_solve(cov_handle *h, const double *x0, int64_t n_iter, doub
  *    (0-based), variable i takes the 12 words of the blocks with counter (t low 32, t high 32, i, g), g = 0, 1, 2,
  *    summed as a uint64 s; v_i = s * 2^-32 - 6.0 (an Irwin-Hall(12) normal, mean 0, variance 1, exact in binary64);
  *    v /= sqrt(sum of v_i^2 summed in index order).  Powers of ten and the initial mesh are computed by the host's
- *    libm, so every iterate can be replayed on a host;
+ *    libm, so every iterate can be replayed on a host.  A start component that is +Inf or -Inf gets the poll size
+ *    5 x 10^400 (b clamped to the table's 400), a NaN one 5 x 10^0; n_iter = 0 evaluates the start alone and
+ *    returns it;
  *  - no cache and no duplicate removal: every kept poll point is evaluated (the winner, the first strict minimum in
  *    generation order -- sign + for columns 0..n-1, then sign -, is the same); evaluations counts them and x0.
  * Limits: N <= 64 (384 poll points per iteration) and a grid whose framebuffer (ny x stride words) fits one warp's

@@ -1781,11 +1781,14 @@ struct MeshVar {
     double a;
     int b, b0;
 };
-// initial poll size: about |x0_i| / 10 (at least 1), on the {1, 2, 5} x 10^b ladder
+// initial poll size: about |x0_i| / 10 (at least 1), on the {1, 2, 5} x 10^b ladder.  A non-finite start keeps the
+// conversion defined: +-Inf gets b = -kMadsPow10Min (the device's powers-of-ten table clamps there too), NaN gets b = 0
+// (target >= 1 otherwise, so b >= 0); either way a = 5, as the mantissa is NaN.
 MeshVar initial_mesh(double x0, double g)
 {
     const double target = std::max(std::max(std::fabs(x0) / 10.0, 1.0), g);
-    const int b = (int)std::floor(std::log10(target));
+    const double lb = std::floor(std::log10(target));
+    const int b = lb == lb ? (int)std::min(lb, (double)-kMadsPow10Min) : 0;
     const double mant = target / std::pow(10.0, b);
     return {mant < 2 ? 1.0 : (mant < 5 ? 2.0 : 5.0), b, b};
 }

@@ -79,7 +79,8 @@ class _Model:
         self.a, self.b = np.empty(n), np.empty(n, dtype=np.int64)
         for i in range(n):  # cov_api.cu initial_mesh
             target = max(max(abs(float(x0[i])) / 10.0, 1.0), g)
-            b = int(math.floor(math.log10(target)))
+            lb = math.log10(target)  # +Inf for an infinite start, NaN for a NaN one: b clamped to 400, NaN to 0
+            b = 0 if lb != lb else (400 if lb == math.inf else min(math.floor(lb), 400))
             mant = target / _p10(b)
             self.a[i], self.b[i] = (1.0 if mant < 2 else (2.0 if mant < 5 else 5.0)), b
         self.b0 = self.b.copy()
