@@ -40,7 +40,8 @@ extern "C" {
                                 cov_mads_solve_batch_region (the grid-free static objective); cov_run_horizon;
                                 cov_run_horizon_points, cov_run_horizon_fire (the dynamic horizon);
                                 cov_run_horizon_ensemble, cov_multi_run_horizon_ensemble;
-                                cov_run_horizon_fire_ensemble, cov_multi_run_horizon_fire_ensemble */
+                                cov_run_horizon_fire_ensemble, cov_multi_run_horizon_fire_ensemble;
+                                cov_run_horizon_points_ensemble, cov_multi_run_horizon_points_ensemble */
 
 #if defined(__GNUC__)
 #define COV_API __attribute__((visibility("default")))
@@ -433,6 +434,43 @@ COV_API int cov_run_horizon_fire_ensemble(cov_handle *h, const double *x_starts,
                                           double *X_out, double *obj_out, int64_t *stats, double *step_ms,
                                           uint8_t *cells_out, uint8_t *states_out);
 
+/* E independent dynamic receding horizons over the reference's fire list in one call, on the device side by side, each
+ * scenario with its own starting swarm and one of L fire schedules: scenario e (0 <= e < E) is exactly
+ * cov_run_horizon_points(x_starts + e * 3N, T, S, spread, n_iter, granularity, seed + e * T * S (mod 2^64), boxes, ...,
+ * schedule list_of[e], ...) run on a private copy of the handle's current cell store and parameters.  A schedule is a
+ * forecast of the fire: what it appends to the current store, timestep by timestep.  L = 1 with list_of all zeros is
+ * the Monte Carlo over starting swarms and keys.  Every step of a timestep is one launch for the whole ensemble.
+ *
+ * Schedules: the rows of the L schedules are concatenated in pts5 (reference 5-tuples); offsets holds L * T + 1
+ * non-decreasing values from 0, and schedule l appends rows offsets[l * T + t - 1] .. offsets[l * T + t] - 1 at
+ * timestep t.  list_of: E values in [0, L).
+ *
+ * x_starts: E x 3N.  X_out: E x T x 3N; obj_out (nullable): E x T; stats (nullable): E x T x 5 with
+ * cov_run_horizon_points' columns (column 4 of scenario e counts its own schedule's rows); step_ms (nullable): T device
+ * times of the whole ensemble per timestep; cells_out (nullable): E x nx*ny bytes, the multiplicities each scenario
+ * leaves; last_removed (nullable): E x nx*ny ints, row e what cov_run_horizon_points returns for scenario e, from which
+ * the caller can rebuild each scenario's point list with the rule documented there.
+ *
+ * Every scenario starts from the same store, so one envelope serves all of them: cov_run_horizon_points' with a cell's
+ * bound the store's multiplicity plus the largest count any one schedule puts on it (a scenario holds only its own
+ * schedule); the classes the store's, then the new weights in order of first appearance over the concatenated
+ * schedules; mixed weights on one cell checked across all schedules; the entry count the store's plus the longest
+ * schedule's.  Every schedule counts, whether a scenario uses it or not, so the checks are conservative.  A scenario's
+ * single call may number the classes differently (a weight that schedule 2 brings first); counts and objectives do not
+ * change, since the store is dyadic and classes are not returned.
+ *
+ * The handle is not changed: the cell store, cov_get_grid_info, the class weights, the parameters, the ordered point
+ * list with its pending removals and the automaton's state are as before the call.  Errors: cov_run_horizon_points',
+ * in its order, with cov_run_horizon_ensemble's E checks after cov_run_horizon's; COV_ERR_INVALID also for L < 1, L * T
+ * + 1 past 2^63 - 1, list_of NULL with T > 0 or a value outside [0, L).  T == 0 does nothing, and a refused or failed
+ * call changes nothing on the handle. */
+COV_API int cov_run_horizon_points_ensemble(cov_handle *h, const double *x_starts, int64_t E, int64_t T, int64_t S,
+                                            double spread, int64_t n_iter, double granularity, uint64_t seed,
+                                            const double *boxes, int64_t n_boxes, double h_focus, double h_max,
+                                            const double *pts5, const int64_t *offsets, int64_t L,
+                                            const int64_t *list_of, double *X_out, double *obj_out, int64_t *stats,
+                                            double *step_ms, uint8_t *cells_out, int *last_removed);
+
 /* Covered-cell mask of ONE candidate: nx*ny bytes, 1 where the cell is inside some disc (whether
  * or not it holds entries). Lets the host replay an ordered Float64 sum over a weighted list. */
 COV_API int cov_covered_mask(cov_handle *h, const double *x, uint8_t *mask);
@@ -549,6 +587,15 @@ COV_API int cov_multi_run_horizon_fire_ensemble(cov_multi *m, const double *x_st
                                                 uint64_t fire_seed_stride, int64_t first_step,
                                                 double *X_out, double *obj_out, int64_t *stats, uint8_t *cells_out,
                                                 uint8_t *states_out);
+/* cov_run_horizon_points_ensemble over the devices (without step_ms): contiguous shards of scenarios, shard k from
+ * scenario b0 on with seed + b0 * T * S and list_of + b0 (every shard gets all of pts5 and offsets), so its results
+ * equal the single-device call's bit for bit.  Set the same store and parameters on every shard's handle. */
+COV_API int cov_multi_run_horizon_points_ensemble(cov_multi *m, const double *x_starts, int64_t E, int64_t T, int64_t S,
+                                                  double spread, int64_t n_iter, double granularity, uint64_t seed,
+                                                  const double *boxes, int64_t n_boxes, double h_focus, double h_max,
+                                                  const double *pts5, const int64_t *offsets, int64_t L,
+                                                  const int64_t *list_of, double *X_out, double *obj_out,
+                                                  int64_t *stats, uint8_t *cells_out, int *last_removed);
 COV_API int cov_multi_argmin(cov_multi *m, const double *X, int64_t B, int32_t barrier, double *best_obj,
                      int64_t *best_idx);
 

@@ -174,16 +174,20 @@ def _run_horizon(cells, pre, cons_ext, N, r_max, p, steps, S, spread, t_half, d_
 
 def run_simulation_ensemble(cells, starting_swarms, cons_ext, N, r_max, params: SimulationParameters,
                             Nt_sim: int | None = None, starts: int = 1, spread: float = 3.0):
-    """run_simulation(starts=S) from E starting swarms at once, in one cov_run_horizon_ensemble call: scenario e is
-    run_simulation(starts=S) from starting_swarms[e] with params.seed + e * Nt_sim * S (base seed 0 when params.seed is
-    None).  Static environment only.  Returns a list of E tuples (single_input_pb, single_output_pb,
-    runtime_data_MADS, objective_pb), each what run_simulation(starts=S) returns for that scenario, except that
-    runtime_data_MADS holds the device time of each timestep of the whole ensemble.  Unlike run_simulation, cells (its
-    point list and the store on the device) and the caller's r_max are left untouched."""
+    """run_simulation(starts=S) from E starting swarms at once, in one cov_run_horizon_ensemble call (static
+    environment) or one cov_run_horizon_points_ensemble call (dynamic environment, on cells with fire_rows: every
+    scenario appends update_POI's rows): scenario e is run_simulation(starts=S) from starting_swarms[e] with
+    params.seed + e * Nt_sim * S (base seed 0 when params.seed is None).  Returns a list of E tuples (single_input_pb,
+    single_output_pb, runtime_data_MADS, objective_pb), each what run_simulation(starts=S) returns for that scenario,
+    except that runtime_data_MADS holds the device time of each timestep of the whole ensemble.  Unlike run_simulation,
+    cells (its point list and the store on the device) and the caller's r_max are left untouched."""
     from .mads import _flatten_constraints
     p = params
-    if p.environment_type != "static":
-        raise ValueError("run_simulation_ensemble runs the static environment only")
+    if p.environment_type not in ("static", "dynamic"):
+        raise ValueError("environment_type must be 'static' or 'dynamic'")
+    dynamic = p.environment_type == "dynamic"
+    if dynamic and getattr(cells, "fire_rows", None) is None:
+        raise ValueError("the dynamic environment needs cells with fire_rows (initialise_POI)")
     pres = [np.ascontiguousarray(s if not hasattr(s[0], "x") else ACC.make_MADS(s), dtype=np.float64)
             for s in starting_swarms]
     if not pres:
@@ -198,9 +202,13 @@ def run_simulation_ensemble(cells, starting_swarms, cons_ext, N, r_max, params: 
         if obj.native_batch_solver(_flatten_constraints([cons_ext, create_cons3(pre, p.FOV, d_lim)])) is None:
             raise ValueError("starts= needs constraints that all fuse into the objective's launch")
     _, eng = obj._engine()
-    X, objs, _, step_ms = eng.run_horizon_ensemble(np.stack(pres), steps, S=S, spread=spread, n_iter=p.N_iter,
-                                                   granularity=1.0, seed=0 if p.seed is None else p.seed,
-                                                   boxes=_boxes(p), h_focus=H_FOCUS, h_max=p.h_max)
+    kw = dict(S=S, spread=spread, n_iter=p.N_iter, granularity=1.0, seed=0 if p.seed is None else p.seed,
+              boxes=_boxes(p), h_focus=H_FOCUS, h_max=p.h_max)
+    if dynamic:
+        schedule = CellFunctions.update_POI_schedule(cells, steps)
+        X, objs, _, step_ms = eng.run_horizon_points_ensemble(np.stack(pres), [schedule], **kw)
+    else:
+        X, objs, _, step_ms = eng.run_horizon_ensemble(np.stack(pres), steps, **kw)
     runtime = [float(ms) / 1e3 for ms in step_ms]
     return [([pre.copy()] + [Xe[t].copy() for t in range(steps - 1)], [x.copy() for x in Xe], list(runtime),
              [float(v) for v in oe]) for pre, Xe, oe in zip(pres, X, objs)]

@@ -87,6 +87,8 @@ SIGNATURES = {
                                   C.c_uint64, _i64, _vp, _vp, _vp, _vp]),
     "cov_run_horizon_fire_ensemble": (_i, [_vp, _vp, _i64, _i64, _i64, _d, _i64, _d, C.c_uint64, _vp, _i64, _d, _d,
                                            _vp, _vp, C.c_uint64, C.c_uint64, _i64, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "cov_run_horizon_points_ensemble": (_i, [_vp, _vp, _i64, _i64, _i64, _d, _i64, _d, C.c_uint64, _vp, _i64, _d, _d,
+                                             _vp, _vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "cov_covered_mask": (_i, [_vp, _vp, _vp]),
     "cov_set_region": (_i, [_vp, _d, _d, _d, _d, _vp, _i64]),
     "cov_eval_region_batch": (_i, [_vp, _vp, _i64, _vp, _vp, _vp, C.c_int32, _pd, _pi64]),
@@ -116,6 +118,8 @@ SIGNATURES = {
                                             _vp, _vp, _vp, _vp]),
     "cov_multi_run_horizon_fire_ensemble": (_i, [_vp, _vp, _i64, _i64, _i64, _d, _i64, _d, C.c_uint64, _vp, _i64, _d,
                                                  _d, _vp, _vp, C.c_uint64, C.c_uint64, _i64, _vp, _vp, _vp, _vp, _vp]),
+    "cov_multi_run_horizon_points_ensemble": (_i, [_vp, _vp, _i64, _i64, _i64, _d, _i64, _d, C.c_uint64, _vp, _i64,
+                                                   _d, _d, _vp, _vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp]),
     "cov_multi_argmin": (_i, [_vp, _vp, _i64, C.c_int32, _pd, _pi64]),
     "cov_get_limits": (None, [C.POINTER(Limits)]),
     "cov_threshold": (_d, [_d]),

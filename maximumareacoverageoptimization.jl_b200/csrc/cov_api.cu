@@ -2038,8 +2038,12 @@ struct HorizonAppend {
     GridDesc g{};
     int n_classes = 0; // the classes after the call: the store's, then the new weights in order of first appearance
     double cw[kMaxClasses] = {0, 0, 0, 0};
-    // the fire list (cov_run_horizon_points): timestep t appends entries offsets[t-1] .. offsets[t]-1 of (cell, pcls)
+    // the fire list (cov_run_horizon_points): timestep t appends entries offsets[t-1] .. offsets[t]-1 of (cell, pcls);
+    // with list_of (cov_run_horizon_points_ensemble, E values in [0, L)), scenario e follows schedule l = list_of[e]:
+    // entries offsets[l*T + t-1] .. offsets[l*T + t]-1
     const int64_t *offsets = nullptr;
+    const int64_t *list_of = nullptr;
+    int64_t L = 1;
     std::vector<int> cell;
     std::vector<unsigned char> pcls;
     bool stamps = false; // record the last timestep that removed entries from each cell
@@ -2128,9 +2132,9 @@ static void entries_replay(cov_handle *h, const HorizonAppend &app, int64_t T, c
     h->ent_dev_valid = false;
 }
 
-// The scenarios of cov_run_horizon_ensemble / cov_run_horizon_fire_ensemble (run_horizon; NULL: one scenario on the
-// handle's own store): E copies of the handle's store, parameters and automaton state, made on the device when the call
-// starts and dropped when it ends.
+// The scenarios of cov_run_horizon_ensemble / cov_run_horizon_fire_ensemble / cov_run_horizon_points_ensemble
+// (run_horizon; NULL: one scenario on the handle's own store): E copies of the handle's store, parameters and automaton
+// state, made on the device when the call starts and dropped when it ends.
 struct HorizonEnsemble {
     int64_t E = 1;
     uint8_t *cells_out = nullptr;  // E x nx*ny (nullable): the multiplicities each scenario leaves
@@ -2177,29 +2181,30 @@ static cudaError_t replicate(void *dst, const void *src, size_t bytes, int64_t E
 // (horizon_commit_kernel), AreaMaxObjective(cur).  stamps_out (nullable, nx*ny): app's removal stamps.
 // ens: the same loop over ens->E scenarios side by side (one launch per step for all of them) on copies of the store
 // and parameters (and, with the automaton, of its state); x_start and the outputs then hold E scenarios, each of them
-// as the single call lays it out.  The fire list (app->offsets) stays single-scenario.
+// as the single call lays it out, and with the fire list each scenario appends its own schedule (app->list_of).
 static int run_horizon(cov_handle *h, const char *who, const double *x_start, int64_t T, int64_t S, double spread,
                        int64_t n_iter, double granularity, uint64_t seed, const double *boxes, int64_t n_boxes,
                        double h_focus, double h_max, double *X_out, double *obj_out, int64_t *stats, double *step_ms,
                        HorizonAppend *app, int *stamps_out, const HorizonEnsemble *ens = nullptr)
 {
-    if (ens && app && app->offsets)
-        return fail(h, COV_ERR_INVALID, std::string(who) + ": internal: the fire list has no ensemble");
     GridDesc lg = app ? app->g : h->g;
     const int64_t E = ens ? ens->E : 1;
     const int N = h->o.N, n = 3 * N, cols = app ? 5 : 4;
     const size_t ncell = (size_t)h->g.nx * h->g.ny, P = app ? app->cell.size() : 0;
     const bool stamps = app && app->stamps, automaton = app && app->fire_steps;
-    // in: [pow10 | x_start: E n | boxes: 4 n_boxes | direction probabilities: E 9 | appended cells: P ints | their
-    // classes: P bytes | the solves' inputs]; out: [the solves' outputs | X_out: T E n | obj_out: T E | stats: T E cols |
-    // removal stamps: nx*ny ints], timestep-major (a timestep's rows side by side); pinned: [the out rows after the
-    // solves' | the cells: E nx*ny | the automaton states: E nx*ny]
+    const int64_t *list_of = app ? app->list_of : nullptr;
+    const size_t n_off = list_of ? (size_t)(app->L * T + 1) : 0;
+    // in: [pow10 | x_start: E n | boxes: 4 n_boxes | direction probabilities: E 9 | the schedules' offsets: L T + 1 |
+    // list_of: E | appended cells: P ints | their classes: P bytes | the solves' inputs]; out: [the solves' outputs |
+    // X_out: T E n | obj_out: T E | stats: T E cols | removal stamps: E nx*ny ints], timestep-major (a timestep's rows
+    // side by side); pinned: [the out rows after the solves' | the cells: E nx*ny | the automaton states: E nx*ny]
     const size_t tn = (size_t)T * E * n;
     const size_t o_x = kPow10Bytes, o_box = o_x + (size_t)E * n * 8, o_fp = o_box + (size_t)n_boxes * 32;
-    const size_t o_cell = o_fp + (automaton ? (size_t)E * 9 * 8 : 0);
+    const size_t o_off = o_fp + (automaton ? (size_t)E * 9 * 8 : 0), o_list = o_off + n_off * 8;
+    const size_t o_cell = o_list + (list_of ? (size_t)E * 8 : 0);
     const size_t o_cls = o_cell + P * 4, o_X0 = (o_cls + P + 7) / 8 * 8;
     const size_t o_stamp = tn * 8 + (size_t)T * E * 8 + (size_t)T * E * cols * 8;
-    const size_t res_bytes = o_stamp + (stamps ? ncell * 4 : 0);
+    const size_t res_bytes = o_stamp + (stamps ? (size_t)E * ncell * 4 : 0);
     const size_t cells_bytes = ens && ens->cells_out ? (size_t)E * ncell : 0;
     const size_t states_bytes = ens && automaton && ens->states_out ? (size_t)E * ncell : 0;
     std::vector<unsigned char> hin(o_X0);
@@ -2208,16 +2213,22 @@ static int run_horizon(cov_handle *h, const char *who, const double *x_start, in
     memcpy(hin.data() + o_x, x_start, (size_t)E * n * 8);
     if (n_boxes) memcpy(hin.data() + o_box, boxes, (size_t)n_boxes * 32);
     if (automaton) memcpy(hin.data() + o_fp, app->fire_p, (size_t)E * 9 * 8);
+    if (list_of) {
+        memcpy(hin.data() + o_off, app->offsets, n_off * 8);
+        memcpy(hin.data() + o_list, list_of, (size_t)E * 8);
+    }
     if (P) {
         memcpy(hin.data() + o_cell, app->cell.data(), P * 4);
         memcpy(hin.data() + o_cls, app->pcls.data(), P);
     }
     // the scenarios' device state: [mult: E nx*ny | cls: E nx*ny | automaton states: 2 E nx*ny, the E of either
     // ping-pong half side by side | plane sets: E | the single-plane swizzled copy, for E = 1 (launch_eval's CTA kernel
-    // may read it; the E > 1 kernels read the packed planes) | parameters: E 5N | thresholds: E 3N]
+    // may read it; the E > 1 kernels read the packed planes) | parameters: E 5N | thresholds: E 3N]; cls, the states and
+    // the plane sets from 16-byte boundaries: add_points_kernel's 32-bit atomics need 4-byte aligned bases for mult, cls
     const size_t pw = (size_t)lg.n_planes * lg.plane_words * 4, q_bytes = ((size_t)h->g.ny * h->g.qstride + 8) * 4;
     const bool quad = E == 1 && (app ? lg.n_planes == 1 : lg.planes_q != nullptr); // as the single call has it
-    const size_t o_efire = (size_t)2 * E * ncell, o_epl = (o_efire + (automaton ? o_efire : 0) + 15) / 16 * 16;
+    const size_t store16 = ((size_t)E * ncell + 15) / 16 * 16, o_efire = 2 * store16;
+    const size_t o_epl = (o_efire + (automaton ? 2 * store16 : 0) + 15) / 16 * 16;
     const size_t o_eq = o_epl + (size_t)E * pw;
     const size_t o_epar = o_eq + (quad ? q_bytes : 0), o_exyT = o_epar + (size_t)E * 5 * N * 8;
     if (ens) OK(ensure(h, h->ens, o_exyT + (size_t)E * n * 8));
@@ -2240,6 +2251,7 @@ static int run_horizon(cov_handle *h, const char *who, const double *x_start, in
     const int *d_cell = (const int *)(din + o_cell);
     const unsigned char *d_cls = din + o_cls;
     const double *d_fp = (const double *)(din + o_fp);
+    const long long *d_off = (const long long *)(din + o_off), *d_list = (const long long *)(din + o_list);
     double *d_Xo = (double *)(a.stats + 4 * E * S), *d_oo = d_Xo + tn, *xyT = (double *)h->xyT.p;
     long long *d_st = (long long *)(d_oo + T * E);
     unsigned char *mult = (unsigned char *)h->mult.p, *cls = (unsigned char *)h->cls.p;
@@ -2250,9 +2262,9 @@ static int run_horizon(cov_handle *h, const char *who, const double *x_start, in
     if (ens) {
         unsigned char *eb = (unsigned char *)h->ens.p;
         mult = eb;
-        cls = eb + (size_t)E * ncell;
+        cls = eb + store16;
         fire[0] = eb + o_efire; // the scenarios start in half 0: one parity for all of them (the schedule is shared)
-        fire[1] = fire[0] + (size_t)E * ncell;
+        fire[1] = fire[0] + store16;
         fire_cur = 0;
         lg.planes = (const uint32_t *)(eb + o_epl);
         lg.planes_q = quad ? (const uint32_t *)(eb + o_eq) : nullptr;
@@ -2306,7 +2318,7 @@ static int run_horizon(cov_handle *h, const char *who, const double *x_start, in
     if (app && e == cudaSuccess) {
         what = "append setup";
         e = cudaMemsetAsync(overflow, 0, sizeof(int), h->stream);
-        if (e == cudaSuccess && d_stamp) e = cudaMemsetAsync(d_stamp, 0, ncell * 4, h->stream);
+        if (e == cudaSuccess && d_stamp) e = cudaMemsetAsync(d_stamp, 0, (size_t)E * ncell * 4, h->stream);
         if (e == cudaSuccess && lg.planes_q && !ens) e = cudaMemsetAsync((void *)lg.planes_q, 0, q_bytes, h->stream);
     }
     int rc = COV_OK;
@@ -2315,7 +2327,20 @@ static int run_horizon(cov_handle *h, const char *who, const double *x_start, in
         double *next = d_Xo + (size_t)(t - 1) * E * n;
         long long *row = d_st + cols * E * (t - 1);
         if (step_ms && (e = cudaEventRecord(ev[(size_t)t - 1], h->stream)) != cudaSuccess) break;
-        if (app && app->offsets) { // update_POI: this timestep's rows of the fire list
+        if (app && app->offsets && list_of) { // update_POI, each scenario its schedule's rows of this timestep
+            int64_t longest = 0;
+            for (int64_t q = 0; q < E; ++q) {
+                const int64_t *o = app->offsets + list_of[q] * T + (t - 1);
+                longest = std::max(longest, o[1] - o[0]);
+            }
+            what = "append";
+            if (longest > 0) {
+                if ((e = launch_add_points(mult, cls, d_cell, d_cls, longest, overflow, h->stream, E, d_off + (t - 1),
+                                           T, d_list, (long long)ncell)) != cudaSuccess)
+                    break;
+                h->launches += 1;
+            }
+        } else if (app && app->offsets) { // update_POI: this timestep's rows of the fire list
             const int64_t q0 = app->offsets[t - 1], q1 = app->offsets[t];
             what = "append";
             if (q1 > q0) {
@@ -2408,10 +2433,13 @@ static int run_horizon(cov_handle *h, const char *who, const double *x_start, in
     const int *hstamp = (const int *)((const unsigned char *)h->h_out + o_stamp);
     if (rc == COV_OK) {
         bool removed = false, pushed = false;
-        for (int64_t t = 0; t < T * E; ++t) {
-            removed |= hst[cols * t + 3] != 0;
-            if (app && app->offsets) hst[cols * t + 4] = app->offsets[t + 1] - app->offsets[t];
-            if (app) pushed |= hst[cols * t + 4] != 0;
+        for (int64_t r = 0; r < T * E; ++r) { // row r: timestep r / E of scenario r % E
+            removed |= hst[cols * r + 3] != 0;
+            if (app && app->offsets) {
+                const int64_t *o = app->offsets + (list_of ? list_of[r % E] * T : 0) + r / E;
+                hst[cols * r + 4] = o[1] - o[0];
+            }
+            if (app) pushed |= hst[cols * r + 4] != 0;
         }
         if (ens) { // the handle's list is untouched
         } else if (automaton && pushed) {
@@ -2430,7 +2458,7 @@ static int run_horizon(cov_handle *h, const char *who, const double *x_start, in
             }
         if (cells_bytes) memcpy(ens->cells_out, (const unsigned char *)h->h_out + res_bytes, cells_bytes);
         if (states_bytes) memcpy(ens->states_out, (const unsigned char *)h->h_out + res_bytes + cells_bytes, states_bytes);
-        if (stamps && stamps_out) memcpy(stamps_out, hstamp, ncell * 4);
+        if (stamps && stamps_out) memcpy(stamps_out, hstamp, (size_t)E * ncell * 4);
         for (int64_t t = 0; step_ms && t < T; ++t) {
             float ms = 0;
             if ((e = cudaEventElapsedTime(&ms, ev[(size_t)t], ev[(size_t)t + 1])) != cudaSuccess) {
@@ -2494,53 +2522,85 @@ static int download_cells(cov_handle *h, std::vector<unsigned char> &m, std::vec
     return COV_OK;
 }
 
-extern "C" int cov_run_horizon_points(cov_handle *h, const double *x_start, int64_t T, int64_t S, double spread,
-                                      int64_t n_iter, double granularity, uint64_t seed, const double *boxes,
-                                      int64_t n_boxes, double h_focus, double h_max, const double *pts5,
-                                      const int64_t *offsets, double *X_out, double *obj_out, int64_t *stats,
-                                      double *step_ms, int *last_removed)
+// cov_run_horizon_points (ens NULL, one schedule, list_of NULL) and cov_run_horizon_points_ensemble (L schedules,
+// scenario e on schedule list_of[e]): the checks in cov_run_horizon_points' order, the envelope, the loop.  Every
+// scenario starts from the handle's store, so one envelope serves all of them: a cell's bound is the store's
+// multiplicity plus the largest count one schedule puts there (a scenario holds only its own schedule).
+static int horizon_points(cov_handle *h, const char *who, const double *x_start, int64_t T, int64_t S, double spread,
+                          int64_t n_iter, double granularity, uint64_t seed, const double *boxes, int64_t n_boxes,
+                          double h_focus, double h_max, const double *pts5, const int64_t *offsets, int64_t L,
+                          const int64_t *list_of, double *X_out, double *obj_out, int64_t *stats, double *step_ms,
+                          int *last_removed, const HorizonEnsemble *ens)
 {
-    const char *who = "cov_run_horizon_points";
-    if (!h) return fail(nullptr, COV_ERR_INVALID, "NULL handle");
-    DeviceGuard dg(h->device);
+    const int64_t E = ens ? ens->E : 1;
     OK(check_horizon(h, who, x_start, T, S, spread, n_iter, granularity, boxes, n_boxes, X_out));
-    if (!offsets || offsets[0] != 0 || T > 0x7fffffffll)
-        return fail(h, COV_ERR_INVALID, "cov_run_horizon_points: offsets must hold T + 1 non-decreasing values from 0");
-    for (int64_t t = 1; t <= T; ++t)
-        if (offsets[t] < offsets[t - 1])
-            return fail(h, COV_ERR_INVALID, "cov_run_horizon_points: offsets must hold T + 1 non-decreasing values from 0");
-    const int64_t P = offsets[T];
-    if (P > 0 && !pts5) return fail(h, COV_ERR_INVALID, "cov_run_horizon_points: pts5 is NULL");
+    if (ens) OK(check_ensemble(h, who, E, T, S));
+    if (L < 1 || (T > 0 && L > (INT64_MAX - 1) / T))
+        return fail(h, COV_ERR_INVALID, std::string(who) + ": L must be >= 1 with L * T + 1 <= 2^63 - 1");
+    const int64_t n_off = L * T + 1;
+    const std::string bad_offsets = std::string(who) + ": offsets must hold " + (ens ? "L * T + 1" : "T + 1") +
+                                    " non-decreasing values from 0";
+    if (!offsets || offsets[0] != 0 || T > 0x7fffffffll) return fail(h, COV_ERR_INVALID, bad_offsets);
+    for (int64_t q = 1; q < n_off; ++q)
+        if (offsets[q] < offsets[q - 1]) return fail(h, COV_ERR_INVALID, bad_offsets);
+    const int64_t P = offsets[n_off - 1];
+    if (P > 0 && !pts5) return fail(h, COV_ERR_INVALID, std::string(who) + ": pts5 is NULL");
+    if (ens && T > 0) {
+        if (!list_of) return fail(h, COV_ERR_INVALID, std::string(who) + ": list_of is NULL");
+        for (int64_t e = 0; e < E; ++e)
+            if (list_of[e] < 0 || list_of[e] >= L)
+                return fail(h, COV_ERR_INVALID, std::string(who) + ": list_of must hold E values in [0, L)");
+    }
     if (T == 0) return COV_OK;
     HorizonAppend app;
     app.offsets = offsets;
+    app.list_of = ens ? list_of : nullptr;
+    app.L = L;
     app.n_classes = (h->n_entries == 0 && P > 0) ? 0 : h->g.n_classes; // cov_add_points: an empty store has no weight yet
     for (int k = 0; k < kMaxClasses; ++k) app.cw[k] = h->g.class_weight[k];
     OK(map_points(h, pts5, P, app.cell, app.pcls, app.n_classes, app.cw));
     std::vector<unsigned char> m, k;
     OK(download_cells(h, m, k, nullptr));
-    // every cell's multiplicity bound and class: the store's entries plus all the schedule puts there
+    // every cell's multiplicity bound and class: the store's entries plus the most that one schedule puts there
     const size_t ncell = m.size();
-    std::vector<int> bound(m.begin(), m.end());
+    std::vector<int> extra(ncell, 0), cnt(L > 1 ? ncell : 0, 0);
     std::vector<unsigned char> bc(ncell, 0xff);
     for (size_t c = 0; c < ncell; ++c)
         if (m[c]) bc[c] = k[c] & (kMaxClasses - 1);
-    for (int64_t q = 0; q < P; ++q) {
-        const int c = app.cell[(size_t)q];
-        if (bc[c] == 0xff) bc[c] = app.pcls[(size_t)q];
-        else if (bc[c] != app.pcls[(size_t)q])
-            return fail(h, COV_ERR_INVALID, "cov_run_horizon_points: entries on one cell carry different weights (the "
-                                            "store's and the schedule's, removals ignored)");
-        ++bound[c];
+    int64_t longest = 0;
+    for (int64_t l = 0; l < L; ++l) {
+        const int64_t q0 = offsets[l * T], q1 = offsets[(l + 1) * T];
+        std::vector<int> &mine = L > 1 ? cnt : extra; // one schedule counts straight into the bound
+        for (int64_t q = q0; q < q1; ++q) {
+            const int c = app.cell[(size_t)q];
+            if (bc[c] == 0xff) bc[c] = app.pcls[(size_t)q];
+            else if (bc[c] != app.pcls[(size_t)q])
+                return fail(h, COV_ERR_INVALID, std::string(who) + ": entries on one cell carry different weights (the "
+                                                                   "store's and the schedule's, removals ignored)");
+            ++mine[c];
+        }
+        if (L > 1)
+            for (int64_t q = q0; q < q1; ++q) {
+                const int c = app.cell[(size_t)q];
+                extra[c] = std::max(extra[c], cnt[c]);
+                cnt[c] = 0; // the first row on c resets it; the later ones leave zero
+            }
+        longest = std::max(longest, q1 - q0);
     }
     unsigned max_mult[kMaxClasses] = {0, 0, 0, 0};
     for (size_t c = 0; c < ncell; ++c) {
-        if (bound[c] > 255)
-            return fail(h, COV_ERR_LIMIT, "cov_run_horizon_points: more than 255 list entries on one cell (removals "
-                                          "ignored)");
-        if (bound[c]) max_mult[bc[c]] = std::max(max_mult[bc[c]], (unsigned)bound[c]);
+        const int bound = m[c] + extra[c];
+        if (bound > 255)
+            return fail(h, COV_ERR_LIMIT, std::string(who) + ": more than 255 list entries on one cell (removals "
+                                                             "ignored)");
+        if (bound) max_mult[bc[c]] = std::max(max_mult[bc[c]], (unsigned)bound);
     }
-    OK(horizon_envelope(h, who, app, max_mult, h->n_entries + P));
+    OK(horizon_envelope(h, who, app, max_mult, h->n_entries + longest));
+    if (ens) { // the scenarios' lists are the caller's to rebuild (last_removed); the handle's stays as it is
+        app.stamps = last_removed != nullptr;
+        return run_horizon(h, who, x_start, T, S, spread, n_iter, granularity, seed, boxes, n_boxes, h_focus, h_max,
+                           X_out, obj_out, stats, step_ms, &app, last_removed, ens);
+    }
     // the ordered list: removals pending from earlier calls first, and push! appends after the entries already in
     // the list, whatever setter built it (cov_add_points)
     entries_apply_removals(h, m.data());
@@ -2552,6 +2612,34 @@ extern "C" int cov_run_horizon_points(cov_handle *h, const double *x_start, int6
     app.stamps = h->ent_known || last_removed;
     return run_horizon(h, who, x_start, T, S, spread, n_iter, granularity, seed, boxes, n_boxes, h_focus, h_max, X_out,
                        obj_out, stats, step_ms, &app, last_removed);
+}
+
+extern "C" int cov_run_horizon_points(cov_handle *h, const double *x_start, int64_t T, int64_t S, double spread,
+                                      int64_t n_iter, double granularity, uint64_t seed, const double *boxes,
+                                      int64_t n_boxes, double h_focus, double h_max, const double *pts5,
+                                      const int64_t *offsets, double *X_out, double *obj_out, int64_t *stats,
+                                      double *step_ms, int *last_removed)
+{
+    if (!h) return fail(nullptr, COV_ERR_INVALID, "NULL handle");
+    DeviceGuard dg(h->device);
+    return horizon_points(h, "cov_run_horizon_points", x_start, T, S, spread, n_iter, granularity, seed, boxes,
+                          n_boxes, h_focus, h_max, pts5, offsets, 1, nullptr, X_out, obj_out, stats, step_ms,
+                          last_removed, nullptr);
+}
+
+extern "C" int cov_run_horizon_points_ensemble(cov_handle *h, const double *x_starts, int64_t E, int64_t T, int64_t S,
+                                               double spread, int64_t n_iter, double granularity, uint64_t seed,
+                                               const double *boxes, int64_t n_boxes, double h_focus, double h_max,
+                                               const double *pts5, const int64_t *offsets, int64_t L,
+                                               const int64_t *list_of, double *X_out, double *obj_out, int64_t *stats,
+                                               double *step_ms, uint8_t *cells_out, int *last_removed)
+{
+    if (!h) return fail(nullptr, COV_ERR_INVALID, "NULL handle");
+    DeviceGuard dg(h->device);
+    const HorizonEnsemble ens{E, cells_out, nullptr};
+    return drop_ensemble(h, horizon_points(h, "cov_run_horizon_points_ensemble", x_starts, T, S, spread, n_iter,
+                                           granularity, seed, boxes, n_boxes, h_focus, h_max, pts5, offsets, L,
+                                           list_of, X_out, obj_out, stats, step_ms, last_removed, &ens));
 }
 
 // cov_run_horizon_fire (ens NULL, winds one triple) and cov_run_horizon_fire_ensemble (winds: E triples wind_speed,
@@ -3108,6 +3196,33 @@ extern "C" int cov_multi_run_horizon_fire_ensemble(cov_multi *m, const double *x
                                              stats ? stats + r0 * 5 : nullptr, nullptr,
                                              cells_out ? cells_out + (size_t)b0 * ncell : nullptr,
                                              states_out ? states_out + (size_t)b0 * ncell : nullptr);
+    });
+}
+
+// Scenarios b0 .. b0 + bn - 1 on shard k with the keys and schedules they have in the single-device call.
+extern "C" int cov_multi_run_horizon_points_ensemble(cov_multi *m, const double *x_starts, int64_t E, int64_t T,
+                                                     int64_t S, double spread, int64_t n_iter, double granularity,
+                                                     uint64_t seed, const double *boxes, int64_t n_boxes,
+                                                     double h_focus, double h_max, const double *pts5,
+                                                     const int64_t *offsets, int64_t L, const int64_t *list_of,
+                                                     double *X_out, double *obj_out, int64_t *stats,
+                                                     uint8_t *cells_out, int *last_removed)
+{
+    if (!m) return fail(nullptr, COV_ERR_INVALID, "NULL multi handle");
+    if (E < 1 || T < 0 || (T > 0 && (!x_starts || !X_out || !list_of))) {
+        m->err = "cov_multi_run_horizon_points_ensemble: bad arguments";
+        return COV_ERR_INVALID;
+    }
+    return run_shards(m, x_starts, E, [&](int, cov_handle *h, const double *Xk, int64_t b0, int64_t bn) {
+        const size_t n = h->have_params ? 3 * (size_t)h->o.N : 0, ncell = (size_t)h->g.nx * h->g.ny;
+        const size_t r0 = (size_t)b0 * (size_t)T;
+        return cov_run_horizon_points_ensemble(h, Xk, bn, T, S, spread, n_iter, granularity,
+                                               seed + (uint64_t)b0 * (uint64_t)T * (uint64_t)S, boxes, n_boxes,
+                                               h_focus, h_max, pts5, offsets, L, list_of ? list_of + b0 : nullptr,
+                                               X_out + r0 * n, obj_out ? obj_out + r0 : nullptr,
+                                               stats ? stats + r0 * 5 : nullptr, nullptr,
+                                               cells_out ? cells_out + (size_t)b0 * ncell : nullptr,
+                                               last_removed ? last_removed + (size_t)b0 * ncell : nullptr);
     });
 }
 

@@ -189,7 +189,8 @@ __device__ __forceinline__ bool cell_covered(const GridDesc &g, int i1, int j1, 
     return false;
 }
 
-// stamp (nullable): stamp[cell] = t for every cell that loses entries (cov_run_horizon_points' last_removed)
+// stamp (nullable): stamp[e * ncell + cell] = t for every cell of store e that loses entries (cov_run_horizon_points'
+// last_removed)
 __global__ void remove_covered_kernel(unsigned char *mult, unsigned char *cls, const __grid_constant__ GridDesc g,
                                       const double *__restrict__ xyT, int N, unsigned long long *removed, int *stamp,
                                       int t_stamp, long long E, long long removed_stride)
@@ -197,6 +198,7 @@ __global__ void remove_covered_kernel(unsigned char *mult, unsigned char *cls, c
     const long long ncell = (long long)g.nx * g.ny;
     for (long long e = blockIdx.y; e < E; e += gridDim.y) {
         unsigned char *me = mult + e * ncell, *ce = cls + e * ncell;
+        int *se = stamp ? stamp + e * ncell : nullptr;
         const double *xe = xyT + e * 3 * N;
         unsigned long long mine = 0;
         for (long long t = blockIdx.x * (long long)blockDim.x + threadIdx.x; t < ncell;
@@ -208,7 +210,7 @@ __global__ void remove_covered_kernel(unsigned char *mult, unsigned char *cls, c
                     mine += m;
                     me[t] = 0;
                     ce[t] = 0xffu;
-                    if (stamp) stamp[t] = t_stamp;
+                    if (se) se[t] = t_stamp;
                 }
             }
         }
@@ -268,29 +270,42 @@ __device__ __forceinline__ unsigned byte_cas(unsigned char *base, long long idx,
     } while (old != assumed);
     return expect;
 }
+// blockIdx.y strides over E stores side by side (launch_add_points); list_of NULL: entries 0 .. P-1 into store 0.
+// Store e's bytes start at e * ncell, which need not be a word boundary: the words are formed from the absolute byte
+// index on the 4-byte aligned bases, and two stores sharing a word is safe under the compare-and-swap.
 __global__ void add_points_kernel(unsigned char *mult, unsigned char *cls, const int *__restrict__ cell_idx,
-                                  const unsigned char *__restrict__ cell_cls, long long P, int *overflow)
+                                  const unsigned char *__restrict__ cell_cls, long long P, int *overflow, long long E,
+                                  const long long *__restrict__ offsets, long long offsets_stride,
+                                  const long long *__restrict__ list_of, long long ncell)
 {
-    for (long long t = blockIdx.x * (long long)blockDim.x + threadIdx.x; t < P;
-         t += (long long)gridDim.x * blockDim.x) {
-        const int cell = cell_idx[t];
-        const unsigned k = cell_cls[t];
-        const unsigned seen = byte_cas(cls, cell, kNoClass, k);
-        if (seen != kNoClass && seen != k) {
-            atomicExch(overflow, 2); // entries of different weights on one cell
-            continue;
+    for (long long e = blockIdx.y; e < E; e += gridDim.y) {
+        long long q0 = 0, q1 = P;
+        if (list_of) {
+            const long long *o = offsets + list_of[e] * offsets_stride;
+            q0 = o[0];
+            q1 = o[1];
         }
-        unsigned int *word = reinterpret_cast<unsigned int *>(mult + (cell & ~3));
-        const int sh = (cell & 3) * 8;
-        unsigned int old = *word, assumed;
-        do {
-            assumed = old;
-            if (((assumed >> sh) & 0xffu) >= 255u) {
-                atomicExch(overflow, 1);
-                break;
+        for (long long t = q0 + blockIdx.x * (long long)blockDim.x + threadIdx.x; t < q1;
+             t += (long long)gridDim.x * blockDim.x) {
+            const long long idx = e * ncell + cell_idx[t];
+            const unsigned k = cell_cls[t];
+            const unsigned seen = byte_cas(cls, idx, kNoClass, k);
+            if (seen != kNoClass && seen != k) {
+                atomicExch(overflow, 2); // entries of different weights on one cell
+                continue;
             }
-            old = atomicCAS(word, assumed, assumed + (1u << sh));
-        } while (old != assumed);
+            unsigned int *word = reinterpret_cast<unsigned int *>(mult + (idx & ~3ll));
+            const int sh = (int)(idx & 3) * 8;
+            unsigned int old = *word, assumed;
+            do {
+                assumed = old;
+                if (((assumed >> sh) & 0xffu) >= 255u) {
+                    atomicExch(overflow, 1);
+                    break;
+                }
+                old = atomicCAS(word, assumed, assumed + (1u << sh));
+            } while (old != assumed);
+        }
     }
 }
 // cells without entries carry kNoClass (after uploads and removals)
@@ -308,12 +323,13 @@ cudaError_t launch_normalize_cls(const unsigned char *mult, unsigned char *cls, 
     return cudaGetLastError();
 }
 cudaError_t launch_add_points(unsigned char *mult, unsigned char *cls, const int *cell_idx,
-                              const unsigned char *cell_cls, long long P, int *overflow, cudaStream_t s)
+                              const unsigned char *cell_cls, long long P, int *overflow, cudaStream_t s, long long E,
+                              const long long *offsets, long long offsets_stride, const long long *list_of,
+                              long long ncell)
 {
     if (P <= 0) return cudaSuccess;
-    const int block = 256;
-    const int grid = (int)std::min<long long>((P + block - 1) / block, 148 * 8);
-    add_points_kernel<<<grid, block, 0, s>>>(mult, cls, cell_idx, cell_cls, P, overflow);
+    add_points_kernel<<<store_grid(P, 256, 148 * 8, E), 256, 0, s>>>(mult, cls, cell_idx, cell_cls, P, overflow, E,
+                                                                     offsets, offsets_stride, list_of, ncell);
     return cudaGetLastError();
 }
 

@@ -129,8 +129,8 @@ cudaError_t launch_fill_full(unsigned char *mult, unsigned char *cls, long long 
 cudaError_t launch_bits_to_cells(const uint32_t *bits, int nx, int ny, unsigned char *mult,
                                  unsigned char *cls, cudaStream_t s);
 // xyT: 3N doubles on the device: cx[N], cy[N], T[N]. removed: one unsigned long long (store e's at e *
-// removed_stride).  stamp (nullable, nx*ny ints, E = 1 only): stamp[cell] = t_stamp for every cell whose entries are
-// removed.
+// removed_stride).  stamp (nullable, E x nx*ny ints): stamp[e * nx*ny + cell] = t_stamp for every cell of store e whose
+// entries are removed.
 cudaError_t launch_remove_covered(unsigned char *mult, unsigned char *cls, const GridDesc &g, const double *xyT, int N,
                                   unsigned long long *removed, cudaStream_t s, int *stamp = nullptr, int t_stamp = 0,
                                   long long E = 1, long long removed_stride = 0);
@@ -138,8 +138,13 @@ cudaError_t launch_normalize_cls(const unsigned char *mult, unsigned char *cls, 
 cudaError_t launch_covered_mask(unsigned char *mask, const GridDesc &g, const double *xyT, int N,
                                 cudaStream_t s);
 cudaError_t launch_thresholds(const double *xyR, int N, double *xyT, cudaStream_t s, long long E = 1); // E swarms
+// E stores side by side (cov_run_horizon_points_ensemble): store e's mult / cls at e * ncell bytes from 4-byte aligned
+// bases; it appends entries offsets[list_of[e] * offsets_stride] .. offsets[list_of[e] * offsets_stride + 1] - 1 of
+// (cell_idx, cell_cls), and P bounds the length of every such slice.  list_of NULL (E = 1): entries 0 .. P-1.
 cudaError_t launch_add_points(unsigned char *mult, unsigned char *cls, const int *cell_idx,
-                              const unsigned char *cell_cls, long long P, int *overflow, cudaStream_t s);
+                              const unsigned char *cell_cls, long long P, int *overflow, cudaStream_t s,
+                              long long E = 1, const long long *offsets = nullptr, long long offsets_stride = 0,
+                              const long long *list_of = nullptr, long long ncell = 0);
 cudaError_t launch_argmin(const double *obj, const unsigned char *feasible, long long B, int barrier,
                           double *scratch_obj, long long *scratch_idx, int scratch_n, cudaStream_t s);
 cudaError_t launch_union_area(const double *dX, long long B, int N, double *d_area, cudaStream_t s);

@@ -458,6 +458,53 @@ class CoverageEngine:
         out = (X, obj, {name: st[:, :, q].copy() for q, name in enumerate(names)}, ms)
         return out + tuple(a for a, want in ((cells, want_cells), (states, want_states)) if want)
 
+    def run_horizon_points_ensemble(self, x_starts, schedules, list_of=None, S: int = 1, spread: float = 3.0,
+                                    n_iter: int = 100, granularity: float = 1.0, seed: int = 0, boxes=None,
+                                    h_focus: float = 15.0, h_max: float = 30.0, want_cells: bool = False,
+                                    want_last_removed: bool = False):
+        """E independent run_horizon_points scenarios in one call (cov_run_horizon_points_ensemble), each on a private
+        copy of the engine's current store and parameters: schedules holds L fire schedules (forecasts), each a list of
+        T arrays (n_t x 5 reference 5-tuples) as run_horizon_points takes them, all with the same T; scenario e starts
+        from x_starts[e] ((E, 3N)), appends schedule list_of[e] (default: schedule 0 for every scenario) and equals
+        run_horizon_points with seed + e * T * S.  The engine is left unchanged.  Returns (X (E, T, 3N), obj (E, T),
+        stats, step_ms (T,)) with stats a dict of (E, T) int64 arrays (run_horizon_points'), then with want_cells=True
+        cells (E, nx*ny), the multiplicities each scenario leaves, and with want_last_removed=True last_removed
+        (E, nx*ny int32), row e what run_horizon_points returns as last_removed for scenario e."""
+        X0 = _f64(x_starts)
+        if X0.ndim == 1:
+            X0 = X0.reshape(1, -1)
+        if self.N is None or X0.ndim != 2 or X0.shape[1] != 3 * self.N:
+            raise ValueError("x_starts must be (E, 3N) with the N given to set_params")
+        E, n = X0.shape[0], 3 * self.N
+        if len(schedules) < 1:
+            raise ValueError("schedules must hold at least one schedule")
+        T = len(schedules[0])
+        if any(len(s) != T for s in schedules):
+            raise ValueError("every schedule must have the same number of timesteps")
+        rows = [_f64(a).reshape(-1, 5) for s in schedules for a in s]  # schedule-major: schedule l, timestep t
+        L = len(schedules)
+        offsets = np.zeros(L * T + 1, dtype=np.int64)
+        offsets[1:] = np.cumsum([r.shape[0] for r in rows], dtype=np.int64)
+        pts = np.ascontiguousarray(np.concatenate(rows)) if offsets[-1] else None
+        lo = np.zeros(E, dtype=np.int64) if list_of is None else np.ascontiguousarray(list_of, dtype=np.int64)
+        if lo.shape != (E,) or (E and (lo.min() < 0 or lo.max() >= L)):
+            raise ValueError("list_of must hold E schedule indices in [0, L)")
+        B = np.zeros((0, 4)) if boxes is None else _f64(boxes).reshape(-1, 4)
+        X = np.empty((E, T, n))
+        obj = np.empty((E, T))
+        st = np.empty((E, T, 5), dtype=np.int64)
+        ms = np.empty(T)
+        gi = self.grid_info() if want_cells or want_last_removed else None
+        cells = np.empty((E, gi["nx"] * gi["ny"]), dtype=np.uint8) if want_cells else None
+        last = np.empty((E, gi["nx"] * gi["ny"]), dtype=np.int32) if want_last_removed else None
+        self._check(lib.cov_run_horizon_points_ensemble(
+            self._h, _ptr(X0), E, T, int(S), float(spread), int(n_iter), float(granularity), int(seed) & (2**64 - 1),
+            _ptr(B) if len(B) else None, len(B), float(h_focus), float(h_max), _ptr(pts), _ptr(offsets), L, _ptr(lo),
+            _ptr(X), _ptr(obj), _ptr(st), _ptr(ms), _ptr(cells), _ptr(last)))
+        names = ("winner", "evaluations", "feasible", "removed", "appended")
+        out = (X, obj, {name: st[:, :, q].copy() for q, name in enumerate(names)}, ms)
+        return out + tuple(a for a, want in ((cells, want_cells), (last, want_last_removed)) if want)
+
     def _horizon(self, fn, x_start, T, cols, S, spread, n_iter, granularity, seed, boxes, h_focus, h_max, source,
                  tail=()):
         x_start = _f64(x_start).ravel()

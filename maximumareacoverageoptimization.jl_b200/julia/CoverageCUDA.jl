@@ -429,6 +429,56 @@ function run_horizon_fire_ensemble(h::Handle, x_starts::Matrix{Float64}, fire_st
     return X, obj, stats, ms, cells, states
 end
 
+"""
+    run_horizon_points_ensemble(h, x_starts, schedules; list_of = zeros(Int64, size(x_starts, 2)), S = 1, spread = 3.0,
+                                N_iter = 100, granularity = 1.0, seed = 0, boxes = zeros(Float64, 4, 0),
+                                h_focus = 15.0, h_max = 30.0, want_cells = false, want_last_removed = false)
+
+E independent `run_horizon_points` scenarios in one call (`cov_run_horizon_points_ensemble`), each on a private copy
+of the handle's current store and parameters: `schedules` holds L fire schedules, each T matrices as
+`run_horizon_points` takes them (the same T for all); column e of `x_starts` (3N x E) starts scenario e, which appends
+schedule `list_of[e] + 1` (0-based indices, as the C call takes them) and equals `run_horizon_points` with
+`seed + (e - 1) * T * S`. The handle is left unchanged. Returns `(X, objectives, stats, step_ms, cells, last_removed)`:
+`X` 3N x T x E, `objectives` T x E, `stats` 5 x T x E (`run_horizon_points`' rows), `step_ms` the device time of every
+timestep of the whole ensemble, `cells` and `last_removed` (nx*ny x E, with `want_cells` / `want_last_removed`; else
+`nothing`) the multiplicities each scenario leaves and what `run_horizon_points` returns as `last_removed` for it.
+"""
+function run_horizon_points_ensemble(h::Handle, x_starts::Matrix{Float64}, schedules::Vector{Vector{Matrix{Float64}}};
+                                     list_of::Vector{Int64} = zeros(Int64, size(x_starts, 2)), S = 1, spread = 3.0,
+                                     N_iter = 100, granularity = 1.0, seed = 0,
+                                     boxes::Matrix{Float64} = zeros(Float64, 4, 0), h_focus = 15.0, h_max = 30.0,
+                                     want_cells = false, want_last_removed = false)
+    n, E = size(x_starts); K = size(boxes, 2)
+    T, L, pts, offsets = fire_schedules(schedules)
+    X = zeros(Float64, n, T, E); obj = zeros(Float64, T, E); stats = zeros(Int64, 5, T, E); ms = zeros(Float64, T)
+    cells = want_cells ? zeros(UInt8, lattice_cells(h), E) : nothing
+    last = want_last_removed ? zeros(Cint, lattice_cells(h), E) : nothing
+    GC.@preserve x_starts boxes pts offsets list_of X obj stats ms cells last check(h,
+        ccall((:cov_run_horizon_points_ensemble, LIB), Cint,
+        (Ptr{Cvoid}, Ptr{Float64}, Int64, Int64, Int64, Float64, Int64, Float64, UInt64, Ptr{Float64}, Int64, Float64,
+         Float64, Ptr{Float64}, Ptr{Int64}, Int64, Ptr{Int64}, Ptr{Float64}, Ptr{Float64}, Ptr{Int64}, Ptr{Float64},
+         Ptr{UInt8}, Ptr{Cint}),
+        h.ptr, x_starts, E, T, S, spread, N_iter, granularity, seed, K == 0 ? C_NULL : pointer(boxes), K, h_focus,
+        h_max, offsets[end] == 0 ? C_NULL : pointer(pts), offsets, L, list_of, X, obj, stats, ms,
+        want_cells ? pointer(cells) : C_NULL, want_last_removed ? pointer(last) : C_NULL))
+    return X, obj, stats, ms, cells, last
+end
+
+"The L fire schedules of the fire-list ensembles concatenated: (T, L, 5 x P entries, the L * T + 1 offsets)."
+function fire_schedules(schedules::Vector{Vector{Matrix{Float64}}})
+    L = length(schedules)
+    L >= 1 || throw(CovError(-1, "schedules must hold at least one schedule"))
+    T = length(schedules[1])
+    all(s -> length(s) == T, schedules) || throw(CovError(-1, "every schedule must have the same number of timesteps"))
+    rows = [a for s in schedules for a in s]
+    offsets = zeros(Int64, L * T + 1)
+    for q in 1:L * T
+        offsets[q + 1] = offsets[q] + size(rows[q], 2)
+    end
+    pts = offsets[end] == 0 ? zeros(Float64, 5, 0) : reduce(hcat, rows)
+    return T, L, pts, offsets
+end
+
 "The 3 x E winds of the fire ensembles: a 3-vector repeated for every scenario, or 3 x E as given."
 function fire_winds(winds::VecOrMat{Float64}, E::Integer)
     W = winds isa Vector ? repeat(winds, 1, E) : winds
@@ -536,6 +586,43 @@ function multi_run_horizon_fire_ensemble(m::MultiHandle, x_starts::Matrix{Float6
         h_max, fire_steps, W, fire_seed, fire_seed_stride, first_step, X, obj, stats,
         want_cells ? pointer(cells) : C_NULL, want_states ? pointer(states) : C_NULL))
     return X, obj, stats, cells, states
+end
+
+"""
+    multi_run_horizon_points_ensemble(m, x_starts, schedules; list_of = zeros(Int64, size(x_starts, 2)), S = 1,
+                                      spread = 3.0, N_iter = 100, granularity = 1.0, seed = 0,
+                                      boxes = zeros(Float64, 4, 0), h_focus = 15.0, h_max = 30.0, want_cells = false,
+                                      want_last_removed = false)
+
+`run_horizon_points_ensemble` over the devices of `m` (`cov_multi_run_horizon_points_ensemble`): contiguous shards of
+scenarios, each with the keys and schedules it has in the single-device call, so the results are the same bits. Set
+the same store and parameters on every `shard_handle` first. Returns `(X, objectives, stats, cells, last_removed)`.
+"""
+function multi_run_horizon_points_ensemble(m::MultiHandle, x_starts::Matrix{Float64},
+                                           schedules::Vector{Vector{Matrix{Float64}}};
+                                           list_of::Vector{Int64} = zeros(Int64, size(x_starts, 2)), S = 1,
+                                           spread = 3.0, N_iter = 100, granularity = 1.0, seed = 0,
+                                           boxes::Matrix{Float64} = zeros(Float64, 4, 0), h_focus = 15.0, h_max = 30.0,
+                                           want_cells = false, want_last_removed = false)
+    n, E = size(x_starts); K = size(boxes, 2)
+    T, L, pts, offsets = fire_schedules(schedules)
+    X = zeros(Float64, n, T, E); obj = zeros(Float64, T, E); stats = zeros(Int64, 5, T, E)
+    cells = last = nothing
+    if want_cells || want_last_removed # every shard's lattice, as set through the binding, must be the same
+        nc = lattice_cells(m.shards[1])
+        all(s -> lattice_cells(s) == nc, m.shards) || throw(CovError(-2, "the shards hold different lattices"))
+        cells = want_cells ? zeros(UInt8, nc, E) : nothing
+        last = want_last_removed ? zeros(Cint, nc, E) : nothing
+    end
+    GC.@preserve x_starts boxes pts offsets list_of X obj stats cells last check(m,
+        ccall((:cov_multi_run_horizon_points_ensemble, LIB), Cint,
+        (Ptr{Cvoid}, Ptr{Float64}, Int64, Int64, Int64, Float64, Int64, Float64, UInt64, Ptr{Float64}, Int64, Float64,
+         Float64, Ptr{Float64}, Ptr{Int64}, Int64, Ptr{Int64}, Ptr{Float64}, Ptr{Float64}, Ptr{Int64}, Ptr{UInt8},
+         Ptr{Cint}),
+        m.ptr, x_starts, E, T, S, spread, N_iter, granularity, seed, K == 0 ? C_NULL : pointer(boxes), K, h_focus,
+        h_max, offsets[end] == 0 ? C_NULL : pointer(pts), offsets, L, list_of, X, obj, stats,
+        want_cells ? pointer(cells) : C_NULL, want_last_removed ? pointer(last) : C_NULL))
+    return X, obj, stats, cells, last
 end
 
 """
