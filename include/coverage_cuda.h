@@ -41,7 +41,8 @@ extern "C" {
                                 cov_run_horizon_points, cov_run_horizon_fire (the dynamic horizon);
                                 cov_run_horizon_ensemble, cov_multi_run_horizon_ensemble;
                                 cov_run_horizon_fire_ensemble, cov_multi_run_horizon_fire_ensemble;
-                                cov_run_horizon_points_ensemble, cov_multi_run_horizon_points_ensemble */
+                                cov_run_horizon_points_ensemble, cov_multi_run_horizon_points_ensemble;
+                                COV_OPT_LIST_ORDER_HORIZON */
 
 #if defined(__GNUC__)
 #define COV_API __attribute__((visibility("default")))
@@ -88,11 +89,18 @@ enum {
                                    fourth CTA per SM; what auto picks unless the swarm is tiny for its grid) */
     COV_OPT_ZEROCOPY_OUT = 8,   /* 1 (default): the host path's kernels write their results straight into pinned host
                                    memory; 0: into device buffers, copied back slice by slice */
-    COV_OPT_PROGRESSIVE_INDEX = 10 /* which progressive constraint the `progressive` output of cov_eval_batch_ex is:
+    COV_OPT_PROGRESSIVE_INDEX = 10, /* which progressive constraint the `progressive` output of cov_eval_batch_ex is:
                                    0 (default) cons1_progressive = sum over every UAV of max(R_i - r_max_i, 0.0)
                                    (src/TDM_Constraints.jl:182-195); k >= 1 the single-UAV forms, 1-based index as in
                                    the reference: 2 = cons2_progressive (:197-208), 3 = cons3_progressive (:210-221).
                                    k > N is rejected by the evaluation calls with COV_ERR_INVALID */
+    COV_OPT_LIST_ORDER_HORIZON = 11 /* 0 (default): the horizons refuse a store whose area depends on the list order
+                                   (cov_grid_info.area_exact == 0) with COV_ERR_STATE; 1: cov_run_horizon,
+                                   cov_run_horizon_points and their ensembles (cov_multi_* through their member
+                                   handles) accept it and replay the reference's list-order sum on the device, every
+                                   candidate walking the whole point list (the cost of COV_KERNEL_ORDERED).  Dyadic
+                                   stores run as with 0, and the automaton horizons refuse such stores either way.
+                                   Other values: COV_ERR_INVALID */
 };
 
 typedef struct cov_handle cov_handle;
@@ -292,8 +300,9 @@ COV_API int cov_mads_solve_batch(cov_handle *h, const double *X0, int64_t S, int
 
 /* The receding-horizon simulation on the device (FullSimulation.run_simulation, src/FullSimulation.jl:42-107, static
  * environment): T timesteps of rmvCoveredPOI and multi-start MADS, all enqueued before ONE synchronise at the end.
- * Needs a cell store with area_exact == 1 and cov_set_params with prev_xyR (cons3 on); the penalty, cons3's d_lim,
- * cons7 and cons8 are the ones set there.  Let cur = x_start (3N).  For t = 1 .. T:
+ * Needs a cell store with area_exact == 1 (or COV_OPT_LIST_ORDER_HORIZON at 1, below) and cov_set_params with
+ * prev_xyR (cons3 on); the penalty, cons3's d_lim, cons7 and cons8 are the ones set there.  Let cur = x_start (3N).
+ * For t = 1 .. T:
  *  1. rmvCoveredPOI(cur), as cov_remove_covered;
  *  2. for t >= 2 and n_boxes > 0 the r_max rule of FullSimulation.py:80-87 in its FP64 operations: for each UAV i with
  *     fabs(h_focus - R_i / tan_half_fov) < 1 and m = h_max * tan_half_fov, r_max[i] = h_focus * tan_half_fov if some
@@ -315,9 +324,28 @@ COV_API int cov_mads_solve_batch(cov_handle *h, const double *X0, int64_t S, int
  * entries removed in step 1]; step_ms (nullable): T device times between CUDA events recorded between the steps.
  * Afterwards the store holds every removal and the parameters are step T's (r_max, previous swarm), exactly as the
  * same sequence of existing calls leaves them.  T == 0 does nothing.  COV_ERR_STATE: no grid or parameters, cons3 off,
- * or area_exact == 0; COV_ERR_LIMIT: cov_mads_solve_batch's limits; COV_ERR_INVALID: T < 0, S < 1, n_iter < 0, NULL
- * x_start or X_out when T > 0, spread not finite or < 0, granularity < 0 or NaN, n_boxes < 0 or n_boxes > 0 with
- * NULL boxes.  A refused call changes nothing.  cov_last_launch and the kernel timers are left unchanged. */
+ * or area_exact == 0 unless COV_OPT_LIST_ORDER_HORIZON is 1; COV_ERR_LIMIT: cov_mads_solve_batch's limits;
+ * COV_ERR_INVALID: T < 0, S < 1, n_iter < 0, NULL x_start or X_out when T > 0, spread not finite or < 0,
+ * granularity < 0 or NaN, n_boxes < 0 or n_boxes > 0 with NULL boxes.  A refused call changes nothing.  cov_last_launch and the kernel
+ * timers are left unchanged.
+ *
+ * List-order stores (COV_OPT_LIST_ORDER_HORIZON at 1; cov_run_horizon, cov_run_horizon_points and their ensembles).
+ * A store whose area depends on the order of the list (non-dyadic weights such as update_POI's high-interest weight
+ * (h_max tan(FOV/2))^2 pi) is accepted, and the call still equals its sequence of single calls bit for bit: those
+ * calls already sum in list order, and so does the horizon.  Inside one call the list only loses every entry of a
+ * covered cell (rmvCoveredPOI, order kept) and gains appends at its end (update_POI), so scenario e's list at timestep
+ * t is a filter of one fixed sequence -- the handle's list at the call (its pending removals applied; createPOI's order
+ * when no list is known), then the schedule's entries in timestep order -- in which an entry appended at timestep ta
+ * (ta = 1 for the handle's) is live iff ta <= t and no timestep >= ta removed entries from its cell.  Every candidate
+ * walks that sequence, skipping dead entries, with the warp-wide left fold of the list-order evaluation, so each
+ * objective is the one the single calls compute on their compacted list.  Each scenario keeps its removal stamps on the
+ * device (E x nx*ny ints, allocated for the call whether or not last_removed is asked for), and the bit planes are not
+ * repacked inside the loop (nothing reads them).  Every other check is unchanged, in the same order.  Afterwards the
+ * handle's ordered list is the single calls' (the ensembles leave it unchanged, as always); a CUDA failure inside the
+ * loop of cov_run_horizon_points leaves the store unusable (cov_grid_info's calls fail until a setter rebuilds it),
+ * because its list is not known then.  Dyadic stores run exactly as with the option at 0.  The automaton horizons
+ * (cov_run_horizon_fire and its ensemble) refuse list-order stores whatever the option: after an automaton push the
+ * list order becomes createPOI's, another replay. */
 COV_API int cov_run_horizon(cov_handle *h, const double *x_start, int64_t T, int64_t S, double spread,
                             int64_t n_iter, double granularity, uint64_t seed,
                             const double *boxes, int64_t n_boxes, double h_focus, double h_max,
@@ -335,7 +363,8 @@ COV_API int cov_run_horizon(cov_handle *h, const double *x_start, int64_t T, int
  *  - planes: for class k, bits 0 .. floor(log2(the largest bound of its cells)).  More than 8, or a bound over 255:
  *    COV_ERR_LIMIT;
  *  - area_exact of the store with n_entries replaced by n_entries plus every entry the call can add: 0 gives
- *    COV_ERR_STATE (list-order stores are out of scope, as for cov_run_horizon);
+ *    COV_ERR_STATE unless COV_OPT_LIST_ORDER_HORIZON is 1 (list-order stores, as for cov_run_horizon; never for the
+ *    automaton);
  *  - cov_mads_solve_batch's limits on that plane set: COV_ERR_LIMIT.
  * An empty plane adds nothing to any count, so every objective, iterate and winner is the one the sequence of single
  * calls computes on its smaller plane sets; one rebuild at the end leaves the minimal plane set and the statistics.

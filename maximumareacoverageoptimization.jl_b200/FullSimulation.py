@@ -68,7 +68,7 @@ def apply_r_max_rule(drone_locs, r_max, N: int, p: SimulationParameters, t_half:
 
 def run_simulation(cells, starting_circles, cons_ext, cons_prog, N, r_max, params: SimulationParameters,
                    Nt_sim: int | None = None, objective: str = "grid", covered_pb: list | None = None,
-                   starts: int | None = None, spread: float = 3.0):
+                   starts: int | None = None, spread: float = 3.0, list_order: bool = False):
     """Returns (single_input_pb, single_output_pb, runtime_data_MADS, objective_pb).  objective: "grid" (the
     reference's) or "region"; with "region", covered_pb (if given) receives the covered set (M x 3 rows x, y, R) each
     timestep's objective was built on.
@@ -77,7 +77,9 @@ def run_simulation(cells, starting_circles, cons_ext, cons_prog, N, r_max, param
     solves, from the swarm and from S - 1 copies of it moved by N(0, spread^2) metres in x and y, and the best result
     becomes the next swarm.  The grid objective only, with constraints that all fuse; runtime_data_MADS then holds the
     device time of each timestep.  The dynamic environment appends update_POI's rows inside the same call
-    (CoverageEngine.run_horizon_points) and leaves cells as the host loop does."""
+    (CoverageEngine.run_horizon_points) and leaves cells as the host loop does.  list_order=True lets that call run
+    on a store whose area depends on the list order (a high-interest rectangle where the fire is gives its entries
+    the non-dyadic weight (h_max tan(FOV/2))^2 pi); without it such a store raises COV_ERR_STATE."""
     p = params
     if objective not in ("grid", "region"):
         raise ValueError("objective must be 'grid' or 'region'")
@@ -95,7 +97,7 @@ def run_simulation(cells, starting_circles, cons_ext, cons_prog, N, r_max, param
             raise ValueError("starts= runs the grid objective only")
         if p.environment_type == "dynamic" and getattr(cells, "fire_rows", None) is None:
             raise ValueError("starts= with the dynamic environment needs cells with fire_rows (initialise_POI)")
-        return _run_horizon(cells, pre, cons_ext, N, r_max, p, steps, int(starts), spread, t_half, d_lim)
+        return _run_horizon(cells, pre, cons_ext, N, r_max, p, steps, int(starts), spread, t_half, d_lim, list_order)
     engine, covered = None, np.zeros((0, 3))
     if objective == "region":
         from .engine import CoverageEngine
@@ -137,7 +139,7 @@ def run_simulation(cells, starting_circles, cons_ext, cons_prog, N, r_max, param
     return single_input_pb, single_output_pb, runtime_data_MADS, objective_pb
 
 
-def _run_horizon(cells, pre, cons_ext, N, r_max, p, steps, S, spread, t_half, d_lim):
+def _run_horizon(cells, pre, cons_ext, N, r_max, p, steps, S, spread, t_half, d_lim, list_order=False):
     """run_simulation(starts=S): the loop above with S solves per timestep, in one cov_run_horizon call."""
     from .mads import _flatten_constraints
     boxes = _boxes(p)
@@ -148,7 +150,7 @@ def _run_horizon(cells, pre, cons_ext, N, r_max, p, steps, S, spread, t_half, d_
         raise ValueError("starts= needs constraints that all fuse into the objective's launch")
     res, eng = obj._engine()  # the store synced, the parameters of timestep 1's solves (cons3 from pre) set
     kw = dict(S=S, spread=spread, n_iter=p.N_iter, granularity=1.0, seed=0 if p.seed is None else p.seed,
-              boxes=boxes, h_focus=H_FOCUS, h_max=p.h_max)
+              boxes=boxes, h_focus=H_FOCUS, h_max=p.h_max, list_order=list_order)
     if p.environment_type == "dynamic":
         appends = CellFunctions.update_POI_schedule(cells, steps)
         X, objs, _, step_ms, last = eng.run_horizon_points(pre, appends, **kw)
@@ -173,14 +175,15 @@ def _run_horizon(cells, pre, cons_ext, N, r_max, p, steps, S, spread, t_half, d_
 
 
 def run_simulation_ensemble(cells, starting_swarms, cons_ext, N, r_max, params: SimulationParameters,
-                            Nt_sim: int | None = None, starts: int = 1, spread: float = 3.0):
+                            Nt_sim: int | None = None, starts: int = 1, spread: float = 3.0, list_order: bool = False):
     """run_simulation(starts=S) from E starting swarms at once, in one cov_run_horizon_ensemble call (static
     environment) or one cov_run_horizon_points_ensemble call (dynamic environment, on cells with fire_rows: every
     scenario appends update_POI's rows): scenario e is run_simulation(starts=S) from starting_swarms[e] with
     params.seed + e * Nt_sim * S (base seed 0 when params.seed is None).  Returns a list of E tuples (single_input_pb,
     single_output_pb, runtime_data_MADS, objective_pb), each what run_simulation(starts=S) returns for that scenario,
     except that runtime_data_MADS holds the device time of each timestep of the whole ensemble.  Unlike run_simulation,
-    cells (its point list and the store on the device) and the caller's r_max are left untouched."""
+    cells (its point list and the store on the device) and the caller's r_max are left untouched.  list_order: as for
+    run_simulation."""
     from .mads import _flatten_constraints
     p = params
     if p.environment_type not in ("static", "dynamic"):
@@ -203,7 +206,7 @@ def run_simulation_ensemble(cells, starting_swarms, cons_ext, N, r_max, params: 
             raise ValueError("starts= needs constraints that all fuse into the objective's launch")
     _, eng = obj._engine()
     kw = dict(S=S, spread=spread, n_iter=p.N_iter, granularity=1.0, seed=0 if p.seed is None else p.seed,
-              boxes=_boxes(p), h_focus=H_FOCUS, h_max=p.h_max)
+              boxes=_boxes(p), h_focus=H_FOCUS, h_max=p.h_max, list_order=list_order)
     if dynamic:
         schedule = CellFunctions.update_POI_schedule(cells, steps)
         X, objs, _, step_ms = eng.run_horizon_points_ensemble(np.stack(pres), [schedule], **kw)

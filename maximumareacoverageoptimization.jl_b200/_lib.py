@@ -23,6 +23,7 @@ COV_ERR_NOMEM = -6
 KERNEL_AUTO, KERNEL_SPAN, KERNEL_BRUTE, KERNEL_EXACT, KERNEL_SPAN_GENERAL, KERNEL_ORDERED = 0, 1, 2, 3, 4, 5
 OPT_KERNEL, OPT_WARPS_PER_CTA, OPT_CTAS_PER_SM, OPT_BAND_ROWS, OPT_FORCE_EXACT, OPT_CHUNK, OPT_TRACE, OPT_ZEROCOPY_OUT, OPT_PLANE_MODE = 1, 2, 3, 4, 5, 6, 7, 8, 9
 OPT_PROGRESSIVE_INDEX = 10
+OPT_LIST_ORDER_HORIZON = 11
 PACK_F32, PACK_I32, PACK_I16 = 1, 2, 3
 
 

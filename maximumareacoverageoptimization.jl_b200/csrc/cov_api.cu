@@ -217,6 +217,7 @@ struct cov_handle {
     // COV_OPT_TRACE: per-slice timeline of the last host-path call (ms since its first copy was queued)
     int trace = 0;
     int zero_copy_out = 1; // COV_OPT_ZEROCOPY_OUT: kernels write results straight into pinned host memory
+    int list_order_horizon = 0; // COV_OPT_LIST_ORDER_HORIZON: the horizons accept stores with area_exact == 0
     std::vector<cudaEvent_t> trace_ev; // start, then per slice: h2d done, kernel start, kernel end, d2h done
     std::vector<double> trace_ms;
 };
@@ -510,6 +511,10 @@ extern "C" int cov_set_option(cov_handle *h, int option, int64_t value)
         if (value < 0 || value > kMaxUavs) return fail(h, COV_ERR_INVALID, "progressive index must be 0..1024");
         h->o.prog_which = (int)value;
         return COV_OK;
+    case COV_OPT_LIST_ORDER_HORIZON:
+        if (value != 0 && value != 1) return fail(h, COV_ERR_INVALID, "the list-order horizon option must be 0 or 1");
+        h->list_order_horizon = (int)value;
+        return COV_OK;
     }
     return fail(h, COV_ERR_INVALID, "unknown option");
 }
@@ -528,6 +533,7 @@ extern "C" int cov_get_option(const cov_handle *h, int option, int64_t *value)
     case COV_OPT_ZEROCOPY_OUT: *value = h->zero_copy_out; return COV_OK;
     case COV_OPT_PLANE_MODE: *value = h->cfg.plane_mode; return COV_OK;
     case COV_OPT_PROGRESSIVE_INDEX: *value = h->o.prog_which; return COV_OK;
+    case COV_OPT_LIST_ORDER_HORIZON: *value = h->list_order_horizon; return COV_OK;
     }
     return COV_ERR_INVALID;
 }
@@ -2055,14 +2061,16 @@ struct HorizonAppend {
     int64_t first_step = 0;
 };
 
-// The arguments and store every horizon call needs (cov_run_horizon's checks, in its order).
+// The arguments and store every horizon call needs (cov_run_horizon's checks, in its order).  list_ok: the call can
+// replay the list-order sum (not the automaton), which it does when COV_OPT_LIST_ORDER_HORIZON is 1.
 static int check_horizon(cov_handle *h, const char *who, const double *x_start, int64_t T, int64_t S, double spread,
-                         int64_t n_iter, double granularity, const double *boxes, int64_t n_boxes, const double *X_out)
+                         int64_t n_iter, double granularity, const double *boxes, int64_t n_boxes, const double *X_out,
+                         bool list_ok)
 {
     OK(check_ready(h, who));
     if (!h->o.use_cons3)
         return fail(h, COV_ERR_STATE, std::string(who) + ": the parameters have no previous swarm (cons3 is off)");
-    if (!h->area_exact)
+    if (!h->area_exact && !(list_ok && h->list_order_horizon))
         return fail(h, COV_ERR_STATE, std::string(who) + ": the store's area depends on the list order (area_exact == 0)");
     if (T < 0 || S < 1 || n_iter < 0 || (T > 0 && (!x_start || !X_out)) || !std::isfinite(spread) || spread < 0 ||
         !(granularity >= 0) || n_boxes < 0 || (n_boxes > 0 && !boxes))
@@ -2072,9 +2080,10 @@ static int check_horizon(cov_handle *h, const char *who, const double *x_start, 
 
 // The envelope's plane set: for class k, planes for bits 0 .. floor(log2(max_mult[k])), where max_mult[k] bounds the
 // multiplicity of every cell of class k over the whole loop; n_entries bounds the entries.  Removals are ignored, so
-// the refusals are conservative.
+// the refusals are conservative.  list (NULL: refused, the automaton): whether the loop needs the list-order sum,
+// accepted when COV_OPT_LIST_ORDER_HORIZON is 1.
 static int horizon_envelope(cov_handle *h, const char *who, HorizonAppend &app, const unsigned *max_mult,
-                            int64_t n_entries)
+                            int64_t n_entries, bool *list)
 {
     GridDesc &g = app.g;
     g = h->g;
@@ -2102,9 +2111,11 @@ static int horizon_envelope(cov_handle *h, const char *who, HorizonAppend &app, 
     g.n_planes = np;
     g.planes = nullptr; // run_horizon points them at the handle's buffers
     g.planes_q = nullptr;
-    if (!sums_exact(g, n_entries))
+    const bool exact = sums_exact(g, n_entries);
+    if (!exact && !(list && h->list_order_horizon))
         return fail(h, COV_ERR_STATE, std::string(who) + ": with every entry the call can add, the store's area "
                                                          "would depend on the list order (area_exact == 0)");
+    if (list) *list = !exact;
     return check_mads_limits(h, who, &g);
 }
 
@@ -2182,44 +2193,55 @@ static cudaError_t replicate(void *dst, const void *src, size_t bytes, int64_t E
 // ens: the same loop over ens->E scenarios side by side (one launch per step for all of them) on copies of the store
 // and parameters (and, with the automaton, of its state); x_start and the outputs then hold E scenarios, each of them
 // as the single call lays it out, and with the fire list each scenario appends its own schedule (app->list_of).
+// list: the store's area depends on the list order (COV_OPT_LIST_ORDER_HORIZON): the solves and the objective walk
+// each scenario's point list (ListWalk: the handle's list, then the schedule's entries, live by the removal stamps,
+// which are then always kept), and nothing reads the bit planes, so they are not repacked.
 static int run_horizon(cov_handle *h, const char *who, const double *x_start, int64_t T, int64_t S, double spread,
                        int64_t n_iter, double granularity, uint64_t seed, const double *boxes, int64_t n_boxes,
                        double h_focus, double h_max, double *X_out, double *obj_out, int64_t *stats, double *step_ms,
-                       HorizonAppend *app, int *stamps_out, const HorizonEnsemble *ens = nullptr)
+                       HorizonAppend *app, int *stamps_out, bool list, const HorizonEnsemble *ens = nullptr)
 {
+    if (list) OK(entries_on_device(h)); // the base list: the handle's, its pending removals applied
     GridDesc lg = app ? app->g : h->g;
     const int64_t E = ens ? ens->E : 1;
     const int N = h->o.N, n = 3 * N, cols = app ? 5 : 4;
     const size_t ncell = (size_t)h->g.nx * h->g.ny, P = app ? app->cell.size() : 0;
     const bool stamps = app && app->stamps, automaton = app && app->fire_steps;
     const int64_t *list_of = app ? app->list_of : nullptr;
-    const size_t n_off = list_of ? (size_t)(app->L * T + 1) : 0;
+    const bool walk_sched = list && app && app->offsets; // the list walk reads the schedules' offsets
+    const size_t n_off = list_of || walk_sched ? (size_t)(app->L * T + 1) : 0;
     // in: [pow10 | x_start: E n | boxes: 4 n_boxes | direction probabilities: E 9 | the schedules' offsets: L T + 1 |
-    // list_of: E | appended cells: P ints | their classes: P bytes | the solves' inputs]; out: [the solves' outputs |
-    // X_out: T E n | obj_out: T E | stats: T E cols | removal stamps: E nx*ny ints], timestep-major (a timestep's rows
-    // side by side); pinned: [the out rows after the solves' | the cells: E nx*ny | the automaton states: E nx*ny]
+    // list_of: E | appended cells: P ints | their append timesteps (list): P ints | their classes: P bytes | the
+    // solves' inputs]; out: [the solves' outputs | X_out: T E n | obj_out: T E | stats: T E cols | removal stamps: E nx*ny
+    // ints (on the device, and downloaded with stamps)], timestep-major (a timestep's rows side by side); pinned: [the
+    // out rows after the solves' | the cells: E nx*ny | the automaton states: E nx*ny]
     const size_t tn = (size_t)T * E * n;
     const size_t o_x = kPow10Bytes, o_box = o_x + (size_t)E * n * 8, o_fp = o_box + (size_t)n_boxes * 32;
     const size_t o_off = o_fp + (automaton ? (size_t)E * 9 * 8 : 0), o_list = o_off + n_off * 8;
-    const size_t o_cell = o_list + (list_of ? (size_t)E * 8 : 0);
-    const size_t o_cls = o_cell + P * 4, o_X0 = (o_cls + P + 7) / 8 * 8;
+    const size_t o_cell = o_list + (list_of ? (size_t)E * 8 : 0), o_ta = o_cell + P * 4;
+    const size_t o_cls = o_ta + (list ? P * 4 : 0), o_X0 = (o_cls + P + 7) / 8 * 8;
     const size_t o_stamp = tn * 8 + (size_t)T * E * 8 + (size_t)T * E * cols * 8;
     const size_t res_bytes = o_stamp + (stamps ? (size_t)E * ncell * 4 : 0);
+    const size_t dev_bytes = o_stamp + (stamps || list ? (size_t)E * ncell * 4 : 0);
     const size_t cells_bytes = ens && ens->cells_out ? (size_t)E * ncell : 0;
     const size_t states_bytes = ens && automaton && ens->states_out ? (size_t)E * ncell : 0;
     std::vector<unsigned char> hin(o_X0);
     MadsArgs a;
-    OK(mads_buffers(h, o_X0, E * S, n, res_bytes, hin, a));
+    OK(mads_buffers(h, o_X0, E * S, n, dev_bytes, hin, a));
     memcpy(hin.data() + o_x, x_start, (size_t)E * n * 8);
     if (n_boxes) memcpy(hin.data() + o_box, boxes, (size_t)n_boxes * 32);
     if (automaton) memcpy(hin.data() + o_fp, app->fire_p, (size_t)E * 9 * 8);
-    if (list_of) {
-        memcpy(hin.data() + o_off, app->offsets, n_off * 8);
-        memcpy(hin.data() + o_list, list_of, (size_t)E * 8);
-    }
+    if (n_off) memcpy(hin.data() + o_off, app->offsets, n_off * 8);
+    if (list_of) memcpy(hin.data() + o_list, list_of, (size_t)E * 8);
     if (P) {
         memcpy(hin.data() + o_cell, app->cell.data(), P * 4);
         memcpy(hin.data() + o_cls, app->pcls.data(), P);
+    }
+    if (list && P) { // entry q of schedule l is appended at the t with offsets[l T + t-1] <= q < offsets[l T + t]
+        int *ta = (int *)(hin.data() + o_ta);
+        for (int64_t l = 0; l < app->L; ++l)
+            for (int64_t t = 1; t <= T; ++t)
+                for (int64_t q = app->offsets[l * T + t - 1]; q < app->offsets[l * T + t]; ++q) ta[q] = (int)t;
     }
     // the scenarios' device state: [mult: E nx*ny | cls: E nx*ny | automaton states: 2 E nx*ny, the E of either
     // ping-pong half side by side | plane sets: E | the single-plane swizzled copy, for E = 1 (launch_eval's CTA kernel
@@ -2276,7 +2298,21 @@ static int run_horizon(cov_handle *h, const char *who, const double *x_start, in
         o.prev_z = params + 3 * N;
         o.cons3_G = params + 4 * N;
     }
-    int *d_stamp = stamps ? (int *)((unsigned char *)d_Xo + o_stamp) : nullptr;
+    int *d_stamp = stamps || list ? (int *)((unsigned char *)d_Xo + o_stamp) : nullptr;
+    ListWalk walk{};
+    if (list) {
+        walk.base_cell = h->g.ent_cell;
+        walk.base_cls = h->g.ent_cls;
+        walk.n_base = h->g.n_ent;
+        walk.cell = d_cell;
+        walk.cls = d_cls;
+        walk.ta = (const int *)(din + o_ta);
+        walk.off = walk_sched ? d_off : nullptr;
+        walk.list_of = list_of ? d_list : nullptr;
+        walk.T = T;
+        walk.ncell = (long long)ncell;
+        walk.stamps = d_stamp;
+    }
     a.n_iter = n_iter;
     a.granularity = granularity;
     a.ordered = 0;
@@ -2315,6 +2351,7 @@ static int run_horizon(cov_handle *h, const char *who, const double *x_start, in
     }
     if (e == cudaSuccess) e = launch_thresholds(d_x0, N, xyT, h->stream, E), what = "launch_thresholds";
     h->launches += 1;
+    if (!app && d_stamp && e == cudaSuccess) e = cudaMemsetAsync(d_stamp, 0, (size_t)E * ncell * 4, h->stream);
     if (app && e == cudaSuccess) {
         what = "append setup";
         e = cudaMemsetAsync(overflow, 0, sizeof(int), h->stream);
@@ -2366,8 +2403,10 @@ static int run_horizon(cov_handle *h, const char *who, const double *x_start, in
                                        (int)t, E, cols)) != cudaSuccess)
             break;
         what = "repack";
-        if ((e = launch_pack_planes(mult, cls, lg, (uint32_t *)lg.planes, h->stream, E)) != cudaSuccess) break;
-        if (lg.planes_q && (e = launch_requad_plane(lg, (uint32_t *)lg.planes_q, h->stream)) != cudaSuccess) break;
+        if (!list && (e = launch_pack_planes(mult, cls, lg, (uint32_t *)lg.planes, h->stream, E)) != cudaSuccess) break;
+        if (!list && lg.planes_q && (e = launch_requad_plane(lg, (uint32_t *)lg.planes_q, h->stream)) != cudaSuccess)
+            break;
+        walk.t = t;
         hs.t = t;
         what = "horizon_start";
         if ((e = launch_horizon_start(hs, cur, params, (double *)a.X0, (double *)a.a0, (int *)a.b0, h->stream)) !=
@@ -2378,15 +2417,18 @@ static int run_horizon(cov_handle *h, const char *who, const double *x_start, in
         if ((rc = take_counter(h, &counter)) != COV_OK) break;
         what = "MADS kernel";
         // one scenario: mads_kernel, its planes staged in shared memory once per CTA
-        e = E == 1 ? launch_mads(lg, o, cfg, a, counter, h->stream)
-                   : launch_scenario_mads(lg, o, cfg, a, S, hs.seed_stride, counter, h->stream);
+        e = list     ? launch_list_mads(lg, o, cfg, a, S, hs.seed_stride, walk, counter, h->stream)
+            : E == 1 ? launch_mads(lg, o, cfg, a, counter, h->stream)
+                     : launch_scenario_mads(lg, o, cfg, a, S, hs.seed_stride, counter, h->stream);
         if (e != cudaSuccess) break;
         what = "horizon_commit";
         if ((e = launch_horizon_commit(S, N, a.X_out, a.obj_out, a.stats, next, row, xyT, h->stream, E, cols)) !=
             cudaSuccess)
             break;
         what = "coverage kernel";
-        if (E == 1) {
+        if (list) {
+            if ((e = launch_list_eval(lg, o, walk, next, E, d_oo + (t - 1) * E, h->stream)) != cudaSuccess) break;
+        } else if (E == 1) {
             if ((rc = take_counter(h, &counter)) != COV_OK) break;
             EvalOut out{};
             out.obj = d_oo + (t - 1);
@@ -2395,7 +2437,7 @@ static int run_horizon(cov_handle *h, const char *who, const double *x_start, in
         } else if ((e = launch_scenario_eval(lg, o, cfg, next, E, d_oo + (t - 1) * E, h->stream)) != cudaSuccess) {
             break;
         }
-        h->launches += lg.planes_q ? 7 : 6;
+        h->launches += list ? 5 : (lg.planes_q ? 7 : 6);
     }
     if (!ens) h->fire_cur = fire_cur; // the automaton steps enqueued stand
     if (e == cudaSuccess && rc == COV_OK && step_ms) e = cudaEventRecord(ev[(size_t)T], h->stream), what = "event";
@@ -2420,7 +2462,8 @@ static int run_horizon(cov_handle *h, const char *who, const double *x_start, in
         const std::string msg = h->err;
         if (app) entries_forget(h); // the list's per-timestep history is incomplete
         else entries_note_removals(h);
-        if (rebuild_planes(h, n_classes, cw) != COV_OK) h->have_grid = false;
+        // a list-order store: createPOI's order would give other bits, so the store cannot be vouched for any more
+        if (rebuild_planes(h, n_classes, cw) != COV_OK || (app && list)) h->have_grid = false;
         for (cudaEvent_t x : ev) h->ev_pool.push_back(x);
         h->err = msg;
         return rc;
@@ -2480,11 +2523,11 @@ extern "C" int cov_run_horizon(cov_handle *h, const double *x_start, int64_t T, 
     const char *who = "cov_run_horizon";
     if (!h) return fail(nullptr, COV_ERR_INVALID, "NULL handle");
     DeviceGuard dg(h->device);
-    OK(check_horizon(h, who, x_start, T, S, spread, n_iter, granularity, boxes, n_boxes, X_out));
+    OK(check_horizon(h, who, x_start, T, S, spread, n_iter, granularity, boxes, n_boxes, X_out, true));
     if (T == 0) return COV_OK;
     OK(check_mads_limits(h, who, &h->g));
     return run_horizon(h, who, x_start, T, S, spread, n_iter, granularity, seed, boxes, n_boxes, h_focus, h_max, X_out,
-                       obj_out, stats, step_ms, nullptr, nullptr);
+                       obj_out, stats, step_ms, nullptr, nullptr, !h->area_exact);
 }
 
 extern "C" int cov_run_horizon_ensemble(cov_handle *h, const double *x_starts, int64_t E, int64_t T, int64_t S,
@@ -2496,13 +2539,14 @@ extern "C" int cov_run_horizon_ensemble(cov_handle *h, const double *x_starts, i
     const char *who = "cov_run_horizon_ensemble";
     if (!h) return fail(nullptr, COV_ERR_INVALID, "NULL handle");
     DeviceGuard dg(h->device);
-    OK(check_horizon(h, who, x_starts, T, S, spread, n_iter, granularity, boxes, n_boxes, X_out));
+    OK(check_horizon(h, who, x_starts, T, S, spread, n_iter, granularity, boxes, n_boxes, X_out, true));
     OK(check_ensemble(h, who, E, T, S));
     if (T == 0) return COV_OK;
     OK(check_mads_limits(h, who, &h->g));
     const HorizonEnsemble ens{E, cells_out, nullptr};
     return drop_ensemble(h, run_horizon(h, who, x_starts, T, S, spread, n_iter, granularity, seed, boxes, n_boxes,
-                                        h_focus, h_max, X_out, obj_out, stats, step_ms, nullptr, nullptr, &ens));
+                                        h_focus, h_max, X_out, obj_out, stats, step_ms, nullptr, nullptr,
+                                        !h->area_exact, &ens));
 }
 
 // The cell store's bytes as they are (one download, one synchronise).
@@ -2533,7 +2577,7 @@ static int horizon_points(cov_handle *h, const char *who, const double *x_start,
                           int *last_removed, const HorizonEnsemble *ens)
 {
     const int64_t E = ens ? ens->E : 1;
-    OK(check_horizon(h, who, x_start, T, S, spread, n_iter, granularity, boxes, n_boxes, X_out));
+    OK(check_horizon(h, who, x_start, T, S, spread, n_iter, granularity, boxes, n_boxes, X_out, true));
     if (ens) OK(check_ensemble(h, who, E, T, S));
     if (L < 1 || (T > 0 && L > (INT64_MAX - 1) / T))
         return fail(h, COV_ERR_INVALID, std::string(who) + ": L must be >= 1 with L * T + 1 <= 2^63 - 1");
@@ -2595,11 +2639,12 @@ static int horizon_points(cov_handle *h, const char *who, const double *x_start,
                                                              "ignored)");
         if (bound) max_mult[bc[c]] = std::max(max_mult[bc[c]], (unsigned)bound);
     }
-    OK(horizon_envelope(h, who, app, max_mult, h->n_entries + longest));
+    bool list = false;
+    OK(horizon_envelope(h, who, app, max_mult, h->n_entries + longest, &list));
     if (ens) { // the scenarios' lists are the caller's to rebuild (last_removed); the handle's stays as it is
         app.stamps = last_removed != nullptr;
         return run_horizon(h, who, x_start, T, S, spread, n_iter, granularity, seed, boxes, n_boxes, h_focus, h_max,
-                           X_out, obj_out, stats, step_ms, &app, last_removed, ens);
+                           X_out, obj_out, stats, step_ms, &app, last_removed, list, ens);
     }
     // the ordered list: removals pending from earlier calls first, and push! appends after the entries already in
     // the list, whatever setter built it (cov_add_points)
@@ -2611,7 +2656,7 @@ static int horizon_points(cov_handle *h, const char *who, const double *x_start,
     }
     app.stamps = h->ent_known || last_removed;
     return run_horizon(h, who, x_start, T, S, spread, n_iter, granularity, seed, boxes, n_boxes, h_focus, h_max, X_out,
-                       obj_out, stats, step_ms, &app, last_removed);
+                       obj_out, stats, step_ms, &app, last_removed, list);
 }
 
 extern "C" int cov_run_horizon_points(cov_handle *h, const double *x_start, int64_t T, int64_t S, double spread,
@@ -2652,7 +2697,8 @@ static int horizon_fire(cov_handle *h, const char *who, const double *x_start, i
                         double *obj_out, int64_t *stats, double *step_ms, const HorizonEnsemble *ens)
 {
     const int64_t E = ens ? ens->E : 1;
-    OK(check_horizon(h, who, x_start, T, S, spread, n_iter, granularity, boxes, n_boxes, X_out));
+    // after an automaton push the list order is createPOI's, another replay: list-order stores stay refused
+    OK(check_horizon(h, who, x_start, T, S, spread, n_iter, granularity, boxes, n_boxes, X_out, false));
     if (ens) OK(check_ensemble(h, who, E, T, S));
     OK(check_fire_store(h, who));
     if (T > 0 && !fire_steps) return fail(h, COV_ERR_INVALID, std::string(who) + ": fire_steps is NULL");
@@ -2688,7 +2734,7 @@ static int horizon_fire(cov_handle *h, const char *who, const double *x_start, i
     HorizonAppend app;
     app.n_classes = 1;
     app.cw[0] = h->g.class_weight[0];
-    OK(horizon_envelope(h, who, app, max_mult, h->n_entries + 8 * trees));
+    OK(horizon_envelope(h, who, app, max_mult, h->n_entries + 8 * trees, nullptr));
     std::vector<double> fp((size_t)E * 9);
     for (int64_t e = 0; e < E; ++e) fire_probs(winds[3 * e], winds[3 * e + 1], winds[3 * e + 2], fp.data() + 9 * e);
     app.fire_steps = fire_steps;
@@ -2697,7 +2743,7 @@ static int horizon_fire(cov_handle *h, const char *who, const double *x_start, i
     app.fire_seed_stride = fire_seed_stride;
     app.first_step = first_step;
     return run_horizon(h, who, x_start, T, S, spread, n_iter, granularity, seed, boxes, n_boxes, h_focus, h_max, X_out,
-                       obj_out, stats, step_ms, &app, nullptr, ens);
+                       obj_out, stats, step_ms, &app, nullptr, false, ens);
 }
 
 extern "C" int cov_run_horizon_fire(cov_handle *h, const double *x_start, int64_t T, int64_t S, double spread,

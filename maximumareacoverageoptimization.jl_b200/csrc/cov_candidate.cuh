@@ -143,26 +143,41 @@ __device__ __forceinline__ CandScalars candidate_prologue(const GridDesc &g, con
     return r;
 }
 
+// The store's own point list (g.ent_cell / g.ent_cls / g.n_ent), every entry live.
+struct StoreList {
+    const GridDesc &g;
+    __device__ __forceinline__ long long size() const { return g.n_ent; }
+    __device__ __forceinline__ bool get(long long p, int &cell, int &k) const
+    {
+        cell = g.ent_cell[p];
+        k = g.ent_cls[p] & (kMaxClasses - 1);
+        return true;
+    }
+};
+
 // The reference's own loop (src/AreaCoverageCalculation.jl:63-110) over the point LIST for one candidate, executed
 // by one warp: for each entry in list order, the first covering disc adds the entry's weight to a Float64 running
 // sum.  32 entries are tested at a time and the covered ones added one after the other (every lane forms the same
 // sum).  stage: the candidate's 3N doubles, Ts: the N thresholds T(R_c) (shared memory, visible to the warp).
-// Returns the area; cls_total receives the covered entries per weight class.
+// Returns the area; cls_total receives the covered entries per weight class.  list: the sequence walked, list.size()
+// entries of which list.get(p, cell, k) reads entry p and says whether it is in the list (a dead entry adds nothing,
+// so the sum is the one over the live entries alone, in the same order).
+template <class List>
 __device__ __forceinline__ double ordered_area(const GridDesc &g, int N, const double *stage, const double *Ts,
-                                               long long *cls_total)
+                                               long long *cls_total, const List &list)
 {
     const uint32_t lane = lane_id();
     const double w0 = g.class_weight[0], w1 = g.class_weight[1], w2 = g.class_weight[2], w3 = g.class_weight[3];
 #pragma unroll
     for (int k = 0; k < kMaxClasses; ++k) cls_total[k] = 0;
     double area = 0.0;
-    for (long long p0 = 0; p0 < g.n_ent; p0 += 32) {
+    const long long n_ent = list.size();
+    for (long long p0 = 0; p0 < n_ent; p0 += 32) {
         const long long p = p0 + lane;
         bool cov_entry = false;
         int k = 0;
-        if (p < g.n_ent) {
-            const int cell = g.ent_cell[p];
-            k = g.ent_cls[p] & (kMaxClasses - 1);
+        int cell = 0;
+        if (p < n_ent && list.get(p, cell, k)) {
             const double px = cell_centre(cell % g.nx + 1, g.dx, g.hdx);
             const double py = cell_centre(cell / g.nx + 1, g.dy, g.hdy);
             for (int c = 0; c < N; ++c) {
@@ -184,6 +199,11 @@ __device__ __forceinline__ double ordered_area(const GridDesc &g, int N, const d
         }
     }
     return area;
+}
+__device__ __forceinline__ double ordered_area(const GridDesc &g, int N, const double *stage, const double *Ts,
+                                               long long *cls_total)
+{
+    return ordered_area(g, N, stage, Ts, cls_total, StoreList{g});
 }
 
 } // namespace cov

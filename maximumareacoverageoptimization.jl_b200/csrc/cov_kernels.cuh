@@ -80,6 +80,32 @@ cudaError_t launch_scenario_mads(const GridDesc &g, const ObjParams &o, const La
 cudaError_t launch_scenario_eval(const GridDesc &g, const ObjParams &o, const LaunchCfg &cfg, const double *X,
                                  long long E, double *obj, cudaStream_t stream);
 
+// ---- the horizons on a list-order store (COV_OPT_LIST_ORDER_HORIZON; cov_mads.cu) ----
+// Scenario e's point list after timestep t's removal, as liveness over one fixed sequence: the base list (the handle's
+// at the call's start, append time 1), then the entries of schedule l = list_of[e] (list_of NULL: l = 0) up to
+// off[l * T + t], appended at ta[q].  An entry is live iff stamps[e * ncell + cell] < its append time (stamps: the
+// removal stamps of launch_remove_covered, zero before the call).  off NULL: the base list alone.
+struct ListWalk {
+    const int *base_cell;
+    const unsigned char *base_cls;
+    long long n_base;
+    const int *cell;         // the schedules' entries (device)
+    const unsigned char *cls;
+    const int *ta;           // their append timesteps
+    const long long *off;    // L T + 1 offsets (device, nullable)
+    const long long *list_of; // E schedule numbers (device, nullable)
+    long long T, t, ncell;
+    const int *stamps;       // E x ncell
+};
+// The solves of E scenarios with the list-order sum (launch_scenario_mads' numbering and keys; E = 1: launch_mads'),
+// scenario e on parameter block e and on its list; a.ordered and the plane sets are unused.
+cudaError_t launch_list_mads(const GridDesc &g, const ObjParams &o, const LaunchCfg &cfg, const MadsArgs &a,
+                             long long S, unsigned long long key_stride, const ListWalk &w,
+                             unsigned long long *counter, cudaStream_t stream);
+// AreaMaxObjective without the barrier of E swarms (X: E x 3N) on their lists, one warp per swarm: obj[e].
+cudaError_t launch_list_eval(const GridDesc &g, const ObjParams &o, const ListWalk &w, const double *X, long long E,
+                             double *obj, cudaStream_t stream);
+
 // ---- cov_run_horizon (cov_horizon.cu): the kernels between the launchers above, per timestep t (1-based) ----
 // A launch covers E scenarios side by side (cov_run_horizon_ensemble; E = 1: cov_run_horizon): scenario e's cur,
 // parameter block and starts at e * 3N, e * 5N and e * S * 3N doubles.

@@ -540,4 +540,123 @@ cudaError_t launch_mads_region(const RegionDesc &r, const ObjParams &o, const La
     return cudaGetLastError();
 }
 
+// ---- the horizons on a list-order store (launch_list_mads, launch_list_eval) ----
+// Scenario e's list at timestep w.t (ListWalk): the base list, then its schedule's entries up to the timestep, each
+// live iff no removal since its append reached its cell.  The walk skips dead entries, so the sum is the one over the
+// compacted list the single calls keep, in the same order.
+struct HorizonList {
+    const ListWalk &w;
+    const int *stamp;
+    long long q0, n;
+    __device__ __forceinline__ HorizonList(const ListWalk &w_, long long e)
+        : w(w_), stamp(w_.stamps + e * w_.ncell), q0(0), n(w_.n_base)
+    {
+        if (w.off) {
+            const long long l = w.list_of ? w.list_of[e] : 0;
+            q0 = w.off[l * w.T];
+            n += w.off[l * w.T + w.t] - q0;
+        }
+    }
+    __device__ __forceinline__ long long size() const { return n; }
+    __device__ __forceinline__ bool get(long long p, int &cell, int &k) const
+    {
+        if (p < w.n_base) {
+            cell = w.base_cell[p];
+            k = w.base_cls[p] & (kMaxClasses - 1);
+            return stamp[cell] < 1;
+        }
+        const long long q = q0 + (p - w.n_base);
+        cell = w.cell[q];
+        k = w.cls[q] & (kMaxClasses - 1);
+        return stamp[cell] < w.ta[q];
+    }
+};
+
+__host__ __device__ inline int list_warp_bytes(int N) { return round_up(3 * N * 8, 16) + round_up(N * 8, 16); }
+
+// mads_eval's list-order branch over scenario e's list: the same FP64 operations in the same order.  Ts: the warp's N
+// thresholds; poff: the parameter block's offset.
+__device__ __forceinline__ double list_eval(const GridDesc &g, const ObjParams &o, const double *stage, double *Ts,
+                                            const HorizonList &list, long long poff, bool barrier)
+{
+    const int N = o.N;
+    const uint32_t lane = lane_id();
+    const CandScalars cs = candidate_prologue<false>(g, o, stage, nullptr, false, poff);
+    if (barrier && !cs.feasible) return __longlong_as_double(0x7ff0000000000000ll);
+    for (int c = lane; c < N; c += 32) Ts[c] = threshold(stage[2 * N + c]);
+    __syncwarp();
+    long long cls[kMaxClasses];
+    const double area = ordered_area(g, N, stage, Ts, cls, list);
+    __syncwarp();
+    const double obj = __dadd_rn(-area, __dmul_rn(cs.violation, o.penalty_scale));
+    return (obj == obj || !barrier) ? obj : __longlong_as_double(0x7ff0000000000000ll);
+}
+
+// The solves of E scenarios (launch_list_mads): solve k of scenario k / S, keyed as in scenario_solve_kernel.  Shared
+// memory: [solve state] [W x (stage, thresholds)], no framebuffer and no planes.
+__global__ void __launch_bounds__(kMadsThreads, kMadsCtas)
+list_solve_kernel(const __grid_constant__ GridDesc g, const __grid_constant__ ObjParams o,
+                  const __grid_constant__ MadsArgs a, const __grid_constant__ ListWalk w, long long S,
+                  unsigned long long key_stride, unsigned long long *counter)
+{
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    const int warp = threadIdx.x >> 5;
+    const int N = o.N, n = 3 * N;
+    unsigned char *wbase = smem_raw + mads_state_bytes(n) + (size_t)warp * list_warp_bytes(N);
+    double *stage = reinterpret_cast<double *>(wbase);
+    double *Ts = reinterpret_cast<double *>(wbase + round_up(3 * N * 8, 16));
+    long long e = 0; // the scenario of the current solve
+    mads_solves(
+        a, n, smem_raw, stage, counter,
+        [&](unsigned long long k) {
+            e = (long long)(k / (unsigned long long)S);
+            return a.seed + (unsigned long long)e * key_stride + (k - (unsigned long long)e * S);
+        },
+        [&](const double *p) { return list_eval(g, o, p, Ts, HorizonList(w, e), e * 5 * N, true); });
+}
+
+// AreaMaxObjective of E swarms on their lists, one warp per swarm (launch_list_eval).
+__global__ void __launch_bounds__(kMadsThreads)
+list_eval_kernel(const __grid_constant__ GridDesc g, const __grid_constant__ ObjParams o,
+                 const __grid_constant__ ListWalk w, const double *__restrict__ X, long long E,
+                 double *__restrict__ obj)
+{
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    const int W = blockDim.x >> 5, warp = threadIdx.x >> 5;
+    const uint32_t lane = lane_id();
+    const int N = o.N, n = 3 * N;
+    const long long e = (long long)blockIdx.x * W + warp;
+    if (e >= E) return;
+    unsigned char *wbase = smem_raw + (size_t)warp * list_warp_bytes(N);
+    double *stage = reinterpret_cast<double *>(wbase);
+    double *Ts = reinterpret_cast<double *>(wbase + round_up(3 * N * 8, 16));
+    for (int i = lane; i < n; i += 32) stage[i] = X[e * n + i];
+    __syncwarp();
+    const double f = list_eval(g, o, stage, Ts, HorizonList(w, e), e * 5 * N, false);
+    if (lane == 0) obj[e] = f;
+}
+
+cudaError_t launch_list_mads(const GridDesc &g, const ObjParams &o, const LaunchCfg &cfg, const MadsArgs &a,
+                             long long S, unsigned long long key_stride, const ListWalk &w,
+                             unsigned long long *counter, cudaStream_t stream)
+{
+    if (a.S <= 0) return cudaSuccess;
+    if (o.N < 1 || o.N > kMadsMaxUavs) return cudaErrorInvalidConfiguration;
+    const int warps = kMadsThreads / 32, smem = mads_state_bytes(3 * o.N) + warps * list_warp_bytes(o.N);
+    int grid = 0;
+    cudaError_t err = persistent_grid(list_solve_kernel, kMadsThreads, smem, a.S, cfg, &grid);
+    if (err != cudaSuccess) return err;
+    list_solve_kernel<<<grid, kMadsThreads, smem, stream>>>(g, o, a, w, S, key_stride, counter);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_list_eval(const GridDesc &g, const ObjParams &o, const ListWalk &w, const double *X, long long E,
+                             double *obj, cudaStream_t stream)
+{
+    if (E <= 0) return cudaSuccess;
+    const int warps = kMadsThreads / 32, smem = warps * list_warp_bytes(o.N);
+    list_eval_kernel<<<(unsigned)((E + warps - 1) / warps), kMadsThreads, smem, stream>>>(g, o, w, X, E, obj);
+    return cudaGetLastError();
+}
+
 } // namespace cov

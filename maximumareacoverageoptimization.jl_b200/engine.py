@@ -6,6 +6,7 @@ this class only marshals NumPy buffers.  Citations are relative to /root/referen
 from __future__ import annotations
 
 import ctypes as C
+import functools
 import math
 
 import numpy as np
@@ -25,6 +26,23 @@ def _f64(a, shape=None):
     if shape is not None:
         a = a.reshape(shape)
     return a
+
+
+def _list_order(fn):
+    """A horizon method with the keyword list_order: True runs the call with COV_OPT_LIST_ORDER_HORIZON at 1, so that
+    it accepts a store whose area depends on the list order (cov_grid_info.area_exact == 0), and puts the handle's
+    previous value back afterwards, also when the call raises; False leaves the option as it is."""
+    @functools.wraps(fn)
+    def call(self, *args, list_order: bool = False, **kwargs):
+        if not list_order:
+            return fn(self, *args, **kwargs)
+        prev = self.get_option(_lib.OPT_LIST_ORDER_HORIZON)
+        self.set_option(_lib.OPT_LIST_ORDER_HORIZON, 1)
+        try:
+            return fn(self, *args, **kwargs)
+        finally:
+            self.set_option(_lib.OPT_LIST_ORDER_HORIZON, prev)
+    return call
 
 
 class PinnedArray:
@@ -343,6 +361,7 @@ class CoverageEngine:
         names = ("iterations", "evaluations", "successes", "converged")
         return X, obj, {name: st[:, q].copy() for q, name in enumerate(names)}
 
+    @_list_order
     def run_horizon(self, x_start, T: int, S: int = 1, spread: float = 3.0, n_iter: int = 100,
                     granularity: float = 1.0, seed: int = 0, boxes=None, h_focus: float = 15.0,
                     h_max: float = 30.0):
@@ -351,10 +370,13 @@ class CoverageEngine:
         off), cons3 from the current swarm, S solves from the swarm and S - 1 perturbations of it, the best one as
         the next swarm.  Needs set_params with prev_xyR.  Returns (X (T, 3N), obj (T,), stats, step_ms (T,)) with
         stats a dict of int64 arrays: winner, evaluations, feasible, removed.  The r_max and previous swarm of the
-        last timestep stay set on the engine."""
+        last timestep stay set on the engine.  list_order=True (keyword, on this method and on run_horizon_points and
+        the two ensembles) also accepts a store whose area depends on the list order (non-dyadic weights), replaying
+        the reference's list-order sum on the device (COV_OPT_LIST_ORDER_HORIZON for this call only)."""
         return self._horizon(lib.cov_run_horizon, x_start, T, 4, S, spread, n_iter, granularity, seed, boxes, h_focus,
                              h_max, ())
 
+    @_list_order
     def run_horizon_points(self, x_start, appends, S: int = 1, spread: float = 3.0, n_iter: int = 100,
                            granularity: float = 1.0, seed: int = 0, boxes=None, h_focus: float = 15.0,
                            h_max: float = 30.0):
@@ -384,6 +406,7 @@ class CoverageEngine:
                              boxes, h_focus, h_max, (_ptr(fs), float(wind_speed), float(wind_direction),
                                                      float(prob_spread), int(fire_seed) & (2**64 - 1), int(first_step)))
 
+    @_list_order
     def run_horizon_ensemble(self, x_starts, T: int, S: int = 1, spread: float = 3.0, n_iter: int = 100,
                              granularity: float = 1.0, seed: int = 0, boxes=None, h_focus: float = 15.0,
                              h_max: float = 30.0, want_cells: bool = False):
@@ -458,6 +481,7 @@ class CoverageEngine:
         out = (X, obj, {name: st[:, :, q].copy() for q, name in enumerate(names)}, ms)
         return out + tuple(a for a, want in ((cells, want_cells), (states, want_states)) if want)
 
+    @_list_order
     def run_horizon_points_ensemble(self, x_starts, schedules, list_of=None, S: int = 1, spread: float = 3.0,
                                     n_iter: int = 100, granularity: float = 1.0, seed: int = 0, boxes=None,
                                     h_focus: float = 15.0, h_max: float = 30.0, want_cells: bool = False,

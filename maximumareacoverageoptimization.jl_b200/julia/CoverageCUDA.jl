@@ -292,6 +292,26 @@ function mads_solve_batch(h::Handle, X0::Matrix{Float64}; N_iter = 100, granular
 end
 
 """
+    with_list_order(f, h, on)
+
+`f()` with `COV_OPT_LIST_ORDER_HORIZON` (11) at 1 on `h` (a `MultiHandle`: on every shard) when `on`, so that the
+horizon calls accept a store whose area depends on the list order (non-dyadic weights); the previous value is put back
+afterwards, also when `f` throws. `on = false` leaves the option as it is.
+"""
+function with_list_order(f, h::Handle, on::Bool)
+    on || return f()
+    prev = Ref{Int64}(0)
+    check(h, ccall((:cov_get_option, LIB), Cint, (Ptr{Cvoid}, Cint, Ref{Int64}), h.ptr, 11, prev))
+    check(h, ccall((:cov_set_option, LIB), Cint, (Ptr{Cvoid}, Cint, Int64), h.ptr, 11, 1))
+    try
+        return f()
+    finally
+        ccall((:cov_set_option, LIB), Cint, (Ptr{Cvoid}, Cint, Int64), h.ptr, 11, prev[])
+    end
+end
+with_list_order(f, m, on::Bool) = foldr((s, g) -> () -> with_list_order(g, s, on), m.shards; init = f)()
+
+"""
     run_horizon(h, x_start; T, S = 1, spread = 3.0, N_iter = 100, granularity = 1.0, seed = 0,
                 boxes = zeros(Float64, 4, 0), h_focus = 15.0, h_max = 30.0)
 
@@ -302,14 +322,17 @@ current swarm, S solves (from the swarm and S - 1 perturbations of it) and the b
 winner, evaluations, feasible solves, entries removed; `step_ms` the device time of every timestep.
 """
 function run_horizon(h::Handle, x_start::Vector{Float64}; T, S = 1, spread = 3.0, N_iter = 100, granularity = 1.0,
-                     seed = 0, boxes::Matrix{Float64} = zeros(Float64, 4, 0), h_focus = 15.0, h_max = 30.0)
+                     seed = 0, boxes::Matrix{Float64} = zeros(Float64, 4, 0), h_focus = 15.0, h_max = 30.0,
+                     list_order = false)
     n = length(x_start); K = size(boxes, 2)
     X = zeros(Float64, n, T); obj = zeros(Float64, T); stats = zeros(Int64, 4, T); ms = zeros(Float64, T)
-    GC.@preserve x_start boxes X obj stats ms check(h, ccall((:cov_run_horizon, LIB), Cint,
-        (Ptr{Cvoid}, Ptr{Float64}, Int64, Int64, Float64, Int64, Float64, UInt64, Ptr{Float64}, Int64, Float64,
-         Float64, Ptr{Float64}, Ptr{Float64}, Ptr{Int64}, Ptr{Float64}),
-        h.ptr, x_start, T, S, spread, N_iter, granularity, seed, K == 0 ? C_NULL : pointer(boxes), K, h_focus, h_max,
-        X, obj, stats, ms))
+    with_list_order(h, list_order) do
+        GC.@preserve x_start boxes X obj stats ms check(h, ccall((:cov_run_horizon, LIB), Cint,
+            (Ptr{Cvoid}, Ptr{Float64}, Int64, Int64, Float64, Int64, Float64, UInt64, Ptr{Float64}, Int64, Float64,
+             Float64, Ptr{Float64}, Ptr{Float64}, Ptr{Int64}, Ptr{Float64}),
+            h.ptr, x_start, T, S, spread, N_iter, granularity, seed, K == 0 ? C_NULL : pointer(boxes), K, h_focus, h_max,
+            X, obj, stats, ms))
+    end
     return X, obj, stats, ms
 end
 
@@ -326,7 +349,7 @@ from each cell (0: none).
 function run_horizon_points(h::Handle, x_start::Vector{Float64}, appends::Vector{Matrix{Float64}}; S = 1,
                             spread = 3.0, N_iter = 100, granularity = 1.0, seed = 0,
                             boxes::Matrix{Float64} = zeros(Float64, 4, 0), h_focus = 15.0, h_max = 30.0, nx = 100,
-                            ny = 100)
+                            ny = 100, list_order = false)
     T = length(appends); n = length(x_start); K = size(boxes, 2)
     offsets = zeros(Int64, T + 1)
     for t in 1:T
@@ -335,11 +358,13 @@ function run_horizon_points(h::Handle, x_start::Vector{Float64}, appends::Vector
     pts = T == 0 ? zeros(Float64, 5, 0) : reduce(hcat, appends)  # column p = the 5-tuple of entry p
     last = zeros(Cint, nx * ny)
     X = zeros(Float64, n, T); obj = zeros(Float64, T); stats = zeros(Int64, 5, T); ms = zeros(Float64, T)
-    GC.@preserve x_start boxes pts offsets X obj stats ms last check(h, ccall((:cov_run_horizon_points, LIB), Cint,
-        (Ptr{Cvoid}, Ptr{Float64}, Int64, Int64, Float64, Int64, Float64, UInt64, Ptr{Float64}, Int64, Float64,
-         Float64, Ptr{Float64}, Ptr{Int64}, Ptr{Float64}, Ptr{Float64}, Ptr{Int64}, Ptr{Float64}, Ptr{Cint}),
-        h.ptr, x_start, T, S, spread, N_iter, granularity, seed, K == 0 ? C_NULL : pointer(boxes), K, h_focus, h_max,
-        offsets[end] == 0 ? C_NULL : pointer(pts), offsets, X, obj, stats, ms, last))
+    with_list_order(h, list_order) do
+        GC.@preserve x_start boxes pts offsets X obj stats ms last check(h, ccall((:cov_run_horizon_points, LIB), Cint,
+            (Ptr{Cvoid}, Ptr{Float64}, Int64, Int64, Float64, Int64, Float64, UInt64, Ptr{Float64}, Int64, Float64,
+             Float64, Ptr{Float64}, Ptr{Int64}, Ptr{Float64}, Ptr{Float64}, Ptr{Int64}, Ptr{Float64}, Ptr{Cint}),
+            h.ptr, x_start, T, S, spread, N_iter, granularity, seed, K == 0 ? C_NULL : pointer(boxes), K, h_focus, h_max,
+            offsets[end] == 0 ? C_NULL : pointer(pts), offsets, X, obj, stats, ms, last))
+    end
     return X, obj, stats, ms, last
 end
 
@@ -380,15 +405,17 @@ lattice set through this binding (`set_points!`, `set_grid_full!` or `fire_init!
 """
 function run_horizon_ensemble(h::Handle, x_starts::Matrix{Float64}; T, S = 1, spread = 3.0, N_iter = 100,
                               granularity = 1.0, seed = 0, boxes::Matrix{Float64} = zeros(Float64, 4, 0),
-                              h_focus = 15.0, h_max = 30.0, want_cells = false)
+                              h_focus = 15.0, h_max = 30.0, want_cells = false, list_order = false)
     n, E = size(x_starts); K = size(boxes, 2)
     X = zeros(Float64, n, T, E); obj = zeros(Float64, T, E); stats = zeros(Int64, 4, T, E); ms = zeros(Float64, T)
     cells = want_cells ? zeros(UInt8, lattice_cells(h), E) : nothing
-    GC.@preserve x_starts boxes X obj stats ms cells check(h, ccall((:cov_run_horizon_ensemble, LIB), Cint,
-        (Ptr{Cvoid}, Ptr{Float64}, Int64, Int64, Int64, Float64, Int64, Float64, UInt64, Ptr{Float64}, Int64, Float64,
-         Float64, Ptr{Float64}, Ptr{Float64}, Ptr{Int64}, Ptr{Float64}, Ptr{UInt8}),
-        h.ptr, x_starts, E, T, S, spread, N_iter, granularity, seed, K == 0 ? C_NULL : pointer(boxes), K, h_focus,
-        h_max, X, obj, stats, ms, want_cells ? pointer(cells) : C_NULL))
+    with_list_order(h, list_order) do
+        GC.@preserve x_starts boxes X obj stats ms cells check(h, ccall((:cov_run_horizon_ensemble, LIB), Cint,
+            (Ptr{Cvoid}, Ptr{Float64}, Int64, Int64, Int64, Float64, Int64, Float64, UInt64, Ptr{Float64}, Int64, Float64,
+             Float64, Ptr{Float64}, Ptr{Float64}, Ptr{Int64}, Ptr{Float64}, Ptr{UInt8}),
+            h.ptr, x_starts, E, T, S, spread, N_iter, granularity, seed, K == 0 ? C_NULL : pointer(boxes), K, h_focus,
+            h_max, X, obj, stats, ms, want_cells ? pointer(cells) : C_NULL))
+    end
     return X, obj, stats, ms, cells
 end
 
@@ -447,20 +474,22 @@ function run_horizon_points_ensemble(h::Handle, x_starts::Matrix{Float64}, sched
                                      list_of::Vector{Int64} = zeros(Int64, size(x_starts, 2)), S = 1, spread = 3.0,
                                      N_iter = 100, granularity = 1.0, seed = 0,
                                      boxes::Matrix{Float64} = zeros(Float64, 4, 0), h_focus = 15.0, h_max = 30.0,
-                                     want_cells = false, want_last_removed = false)
+                                     want_cells = false, want_last_removed = false, list_order = false)
     n, E = size(x_starts); K = size(boxes, 2)
     T, L, pts, offsets = fire_schedules(schedules)
     X = zeros(Float64, n, T, E); obj = zeros(Float64, T, E); stats = zeros(Int64, 5, T, E); ms = zeros(Float64, T)
     cells = want_cells ? zeros(UInt8, lattice_cells(h), E) : nothing
     last = want_last_removed ? zeros(Cint, lattice_cells(h), E) : nothing
-    GC.@preserve x_starts boxes pts offsets list_of X obj stats ms cells last check(h,
-        ccall((:cov_run_horizon_points_ensemble, LIB), Cint,
-        (Ptr{Cvoid}, Ptr{Float64}, Int64, Int64, Int64, Float64, Int64, Float64, UInt64, Ptr{Float64}, Int64, Float64,
-         Float64, Ptr{Float64}, Ptr{Int64}, Int64, Ptr{Int64}, Ptr{Float64}, Ptr{Float64}, Ptr{Int64}, Ptr{Float64},
-         Ptr{UInt8}, Ptr{Cint}),
-        h.ptr, x_starts, E, T, S, spread, N_iter, granularity, seed, K == 0 ? C_NULL : pointer(boxes), K, h_focus,
-        h_max, offsets[end] == 0 ? C_NULL : pointer(pts), offsets, L, list_of, X, obj, stats, ms,
-        want_cells ? pointer(cells) : C_NULL, want_last_removed ? pointer(last) : C_NULL))
+    with_list_order(h, list_order) do
+        GC.@preserve x_starts boxes pts offsets list_of X obj stats ms cells last check(h,
+            ccall((:cov_run_horizon_points_ensemble, LIB), Cint,
+            (Ptr{Cvoid}, Ptr{Float64}, Int64, Int64, Int64, Float64, Int64, Float64, UInt64, Ptr{Float64}, Int64, Float64,
+             Float64, Ptr{Float64}, Ptr{Int64}, Int64, Ptr{Int64}, Ptr{Float64}, Ptr{Float64}, Ptr{Int64}, Ptr{Float64},
+             Ptr{UInt8}, Ptr{Cint}),
+            h.ptr, x_starts, E, T, S, spread, N_iter, granularity, seed, K == 0 ? C_NULL : pointer(boxes), K, h_focus,
+            h_max, offsets[end] == 0 ? C_NULL : pointer(pts), offsets, L, list_of, X, obj, stats, ms,
+            want_cells ? pointer(cells) : C_NULL, want_last_removed ? pointer(last) : C_NULL))
+    end
     return X, obj, stats, ms, cells, last
 end
 
@@ -534,7 +563,7 @@ stats, cells)`.
 """
 function multi_run_horizon_ensemble(m::MultiHandle, x_starts::Matrix{Float64}; T, S = 1, spread = 3.0, N_iter = 100,
                                     granularity = 1.0, seed = 0, boxes::Matrix{Float64} = zeros(Float64, 4, 0),
-                                    h_focus = 15.0, h_max = 30.0, want_cells = false)
+                                    h_focus = 15.0, h_max = 30.0, want_cells = false, list_order = false)
     n, E = size(x_starts); K = size(boxes, 2)
     X = zeros(Float64, n, T, E); obj = zeros(Float64, T, E); stats = zeros(Int64, 4, T, E)
     cells = nothing
@@ -543,11 +572,13 @@ function multi_run_horizon_ensemble(m::MultiHandle, x_starts::Matrix{Float64}; T
         all(s -> lattice_cells(s) == nc, m.shards) || throw(CovError(-2, "the shards hold different lattices"))
         cells = zeros(UInt8, nc, E)
     end
-    GC.@preserve x_starts boxes X obj stats cells check(m, ccall((:cov_multi_run_horizon_ensemble, LIB), Cint,
-        (Ptr{Cvoid}, Ptr{Float64}, Int64, Int64, Int64, Float64, Int64, Float64, UInt64, Ptr{Float64}, Int64, Float64,
-         Float64, Ptr{Float64}, Ptr{Float64}, Ptr{Int64}, Ptr{UInt8}),
-        m.ptr, x_starts, E, T, S, spread, N_iter, granularity, seed, K == 0 ? C_NULL : pointer(boxes), K, h_focus,
-        h_max, X, obj, stats, want_cells ? pointer(cells) : C_NULL))
+    with_list_order(m, list_order) do
+        GC.@preserve x_starts boxes X obj stats cells check(m, ccall((:cov_multi_run_horizon_ensemble, LIB), Cint,
+            (Ptr{Cvoid}, Ptr{Float64}, Int64, Int64, Int64, Float64, Int64, Float64, UInt64, Ptr{Float64}, Int64, Float64,
+             Float64, Ptr{Float64}, Ptr{Float64}, Ptr{Int64}, Ptr{UInt8}),
+            m.ptr, x_starts, E, T, S, spread, N_iter, granularity, seed, K == 0 ? C_NULL : pointer(boxes), K, h_focus,
+            h_max, X, obj, stats, want_cells ? pointer(cells) : C_NULL))
+    end
     return X, obj, stats, cells
 end
 
@@ -603,7 +634,7 @@ function multi_run_horizon_points_ensemble(m::MultiHandle, x_starts::Matrix{Floa
                                            list_of::Vector{Int64} = zeros(Int64, size(x_starts, 2)), S = 1,
                                            spread = 3.0, N_iter = 100, granularity = 1.0, seed = 0,
                                            boxes::Matrix{Float64} = zeros(Float64, 4, 0), h_focus = 15.0, h_max = 30.0,
-                                           want_cells = false, want_last_removed = false)
+                                           want_cells = false, want_last_removed = false, list_order = false)
     n, E = size(x_starts); K = size(boxes, 2)
     T, L, pts, offsets = fire_schedules(schedules)
     X = zeros(Float64, n, T, E); obj = zeros(Float64, T, E); stats = zeros(Int64, 5, T, E)
@@ -614,14 +645,16 @@ function multi_run_horizon_points_ensemble(m::MultiHandle, x_starts::Matrix{Floa
         cells = want_cells ? zeros(UInt8, nc, E) : nothing
         last = want_last_removed ? zeros(Cint, nc, E) : nothing
     end
-    GC.@preserve x_starts boxes pts offsets list_of X obj stats cells last check(m,
-        ccall((:cov_multi_run_horizon_points_ensemble, LIB), Cint,
-        (Ptr{Cvoid}, Ptr{Float64}, Int64, Int64, Int64, Float64, Int64, Float64, UInt64, Ptr{Float64}, Int64, Float64,
-         Float64, Ptr{Float64}, Ptr{Int64}, Int64, Ptr{Int64}, Ptr{Float64}, Ptr{Float64}, Ptr{Int64}, Ptr{UInt8},
-         Ptr{Cint}),
-        m.ptr, x_starts, E, T, S, spread, N_iter, granularity, seed, K == 0 ? C_NULL : pointer(boxes), K, h_focus,
-        h_max, offsets[end] == 0 ? C_NULL : pointer(pts), offsets, L, list_of, X, obj, stats,
-        want_cells ? pointer(cells) : C_NULL, want_last_removed ? pointer(last) : C_NULL))
+    with_list_order(m, list_order) do
+        GC.@preserve x_starts boxes pts offsets list_of X obj stats cells last check(m,
+            ccall((:cov_multi_run_horizon_points_ensemble, LIB), Cint,
+            (Ptr{Cvoid}, Ptr{Float64}, Int64, Int64, Int64, Float64, Int64, Float64, UInt64, Ptr{Float64}, Int64, Float64,
+             Float64, Ptr{Float64}, Ptr{Int64}, Int64, Ptr{Int64}, Ptr{Float64}, Ptr{Float64}, Ptr{Int64}, Ptr{UInt8},
+             Ptr{Cint}),
+            m.ptr, x_starts, E, T, S, spread, N_iter, granularity, seed, K == 0 ? C_NULL : pointer(boxes), K, h_focus,
+            h_max, offsets[end] == 0 ? C_NULL : pointer(pts), offsets, L, list_of, X, obj, stats,
+            want_cells ? pointer(cells) : C_NULL, want_last_removed ? pointer(last) : C_NULL))
+    end
     return X, obj, stats, cells, last
 end
 
