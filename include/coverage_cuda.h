@@ -42,7 +42,7 @@ extern "C" {
                                 cov_run_horizon_ensemble, cov_multi_run_horizon_ensemble;
                                 cov_run_horizon_fire_ensemble, cov_multi_run_horizon_fire_ensemble;
                                 cov_run_horizon_points_ensemble, cov_multi_run_horizon_points_ensemble;
-                                COV_OPT_LIST_ORDER_HORIZON */
+                                COV_OPT_LIST_ORDER_HORIZON; cov_run_horizon_region (the grid-free horizon) */
 
 #if defined(__GNUC__)
 #define COV_API __attribute__((visibility("default")))
@@ -544,6 +544,34 @@ COV_API int cov_eval_region_batch(cov_handle *h, const double *X, int64_t B, dou
 COV_API int cov_mads_solve_batch_region(cov_handle *h, const double *X0, int64_t S, int64_t n_iter,
                                         double granularity, uint64_t seed, double *X_out, double *obj_out,
                                         int64_t *stats);
+
+/* The receding horizon on the region objective (FullSimulation.run_simulation_region): cov_run_horizon's loop with
+ * the covered set in place of the cell store, all enqueued before ONE synchronise at the end.  Arguments are
+ * cov_run_horizon's.  Needs cov_set_region and cov_set_params with prev_xyR (cons3 on); no cell store is touched.
+ * Let C be the region's covered set (its M0 discs with R > 0) and cur = x_start.  For t = 1 .. T:
+ *  1. cur's discs with R > 0 are appended to C in UAV order (FullSimulation's vstack(covered, swarm), filtered as
+ *     cov_set_region filters), and the arcs of C's boundary inside the domain are recomputed as cov_set_region does;
+ *  2.-6. cov_run_horizon's steps 2 to 6 (the r_max rule, cons3's previous swarm := cur, the S starts, the solves keyed
+ *     seed + (t - 1) S + k, the winner), the solves minimising the region objective as cov_mads_solve_batch_region;
+ *  7. obj_out[t-1] (nullable) = the region objective of cur without the barrier, on step t's C and r_max.
+ * stats (nullable): T x 4 [winner k, evaluations summed over the S solves, solves that found a feasible point, arcs
+ * K_t of C's boundary at step t (at most 2048)]; step_ms (nullable): T device times, as cov_run_horizon's.  Five kernel
+ * launches per timestep (cov_launch_count).  Afterwards the region holds C with its M0 + appended discs and their
+ * arcs, and the parameters are step T's (r_max, previous swarm), exactly as the sequence cov_set_region,
+ * cov_set_params, cov_mads_solve_batch_region, cov_eval_region_batch leaves them, and every value above equals what
+ * that sequence gives, bit for bit.  T == 0 does nothing.
+ * Refused before anything is enqueued, changing nothing, in this order: COV_ERR_STATE without a region or parameters;
+ * COV_ERR_LIMIT for N > 64; COV_ERR_STATE with cons3 off; COV_ERR_LIMIT when M0 + T N > 512 (discs with R <= 0 count,
+ * since how many go is known on the device only); cov_run_horizon's COV_ERR_INVALID checks; COV_ERR_INVALID for a
+ * non-finite value in x_start.
+ * Found inside the loop: when C's boundary has more than 2048 arcs at step t, or a swarm holds a non-finite value,
+ * every later step does nothing and the call returns COV_ERR_LIMIT (the arcs) or COV_ERR_INVALID (the value) with a
+ * message naming t -- the timestep at which the sequence's cov_set_region fails with the same code.  The region and
+ * the parameters are then as before the call (C is built in buffers of the call, the parameters copied back). */
+COV_API int cov_run_horizon_region(cov_handle *h, const double *x_start, int64_t T, int64_t S, double spread,
+                                   int64_t n_iter, double granularity, uint64_t seed,
+                                   const double *boxes, int64_t n_boxes, double h_focus, double h_max,
+                                   double *X_out, double *obj_out, int64_t *stats, double *step_ms);
 
 /* ---- streams, memory, timing (so hosts without a CUDA binding can keep data resident) ------ */
 COV_API int cov_sync(cov_handle *h);

@@ -174,6 +174,48 @@ def _run_horizon(cells, pre, cons_ext, N, r_max, p, steps, S, spread, t_half, d_
     return inputs, [x.copy() for x in X], [float(ms) / 1e3 for ms in step_ms], [float(v) for v in objs]
 
 
+def run_simulation_region(cells, starting_circles, cons_ext, N, r_max, params: SimulationParameters,
+                          Nt_sim: int | None = None, starts: int = 1, spread: float = 3.0, covered_pb: list | None = None):
+    """run_simulation(objective="region") with S = starts solves per timestep, the whole horizon on the device in one
+    cov_run_horizon_region call (CoverageEngine.run_horizon_region): the domain is the cell lattice's rectangle, the
+    covered set starts empty and every timestep appends the current swarm's discs to it.  Static environment, with
+    constraints that all fuse.  Returns run_simulation's 4-tuple (runtime_data_MADS: the device time of each timestep)
+    and leaves the caller's r_max as the host loop does; covered_pb (if given) receives the covered set (M x 3 rows
+    x, y, R) each timestep's objective was built on.  cells is only read."""
+    from .mads import _flatten_constraints
+    p = params
+    if p.environment_type != "static":
+        raise ValueError("the region objective has no dynamic form: its points are not cells")
+    boxes = _boxes(p)
+    if not len(boxes):
+        raise ValueError("starts= needs at least one high-interest rectangle")
+    t_half = math.tan(p.FOV / 2)
+    pre = np.ascontiguousarray(starting_circles if not hasattr(starting_circles[0], "x")
+                               else ACC.make_MADS(starting_circles), dtype=np.float64)
+    r_max = np.ascontiguousarray(r_max, dtype=np.float64)
+    steps = p.Nt_sim if Nt_sim is None else Nt_sim
+    pl = cells.points_of_interest
+    region = (0.0, 0.0, pl.nx * pl.dx, pl.ny * pl.dy)
+    obj = TDM_STATIC_opt.createRegionObjective(region, None, N, r_max.copy())
+    try:
+        cons = _flatten_constraints([cons_ext, create_cons3(pre, p.FOV, p.d_lim * np.ones(N))])
+        if obj.native_batch_solver(cons) is None:
+            raise ValueError("starts= needs constraints that all fuse into the objective's launch")
+        _, eng = obj._engine()  # the empty region and the parameters of timestep 1's solves (cons3 from pre) set
+        X, objs, _, step_ms = eng.run_horizon_region(pre, steps, S=int(starts), spread=spread, n_iter=p.N_iter,
+                                                     granularity=1.0, seed=0 if p.seed is None else p.seed,
+                                                     boxes=boxes, h_focus=H_FOCUS, h_max=p.h_max)
+    finally:
+        obj.close()
+    inputs = [pre.copy()] + [X[t].copy() for t in range(steps - 1)]
+    if covered_pb is not None:  # timestep t's objective: the swarms of timesteps 1 .. t before their solves
+        for t in range(1, steps + 1):
+            covered_pb.append(np.concatenate([x.reshape(3, N).T for x in inputs[:t]]))
+    for t in range(2, steps + 1):  # the caller's r_max as the host loop leaves it
+        apply_r_max_rule(X[t - 2], r_max, N, p, t_half)
+    return inputs, [x.copy() for x in X], [float(ms) / 1e3 for ms in step_ms], [float(v) for v in objs]
+
+
 def run_simulation_ensemble(cells, starting_swarms, cons_ext, N, r_max, params: SimulationParameters,
                             Nt_sim: int | None = None, starts: int = 1, spread: float = 3.0, list_order: bool = False):
     """run_simulation(starts=S) from E starting swarms at once, in one cov_run_horizon_ensemble call (static

@@ -94,6 +94,8 @@ SIGNATURES = {
     "cov_set_region": (_i, [_vp, _d, _d, _d, _d, _vp, _i64]),
     "cov_eval_region_batch": (_i, [_vp, _vp, _i64, _vp, _vp, _vp, C.c_int32, _pd, _pi64]),
     "cov_mads_solve_batch_region": (_i, [_vp, _vp, _i64, _i64, _d, C.c_uint64, _vp, _vp, _vp]),
+    "cov_run_horizon_region": (_i, [_vp, _vp, _i64, _i64, _d, _i64, _d, C.c_uint64, _vp, _i64, _d, _d, _vp, _vp, _vp,
+                                    _vp]),
     "cov_sync": (_i, [_vp]),
     "cov_stream": (_vp, [_vp]),
     "cov_set_stream": (_i, [_vp, _vp]),

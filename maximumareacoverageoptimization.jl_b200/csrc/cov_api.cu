@@ -2061,6 +2061,17 @@ struct HorizonAppend {
     int64_t first_step = 0;
 };
 
+// The arguments every horizon call takes (the last of cov_run_horizon's checks).
+static int check_horizon_args(cov_handle *h, const char *who, const double *x_start, int64_t T, int64_t S, double spread,
+                              int64_t n_iter, double granularity, const double *boxes, int64_t n_boxes,
+                              const double *X_out)
+{
+    if (T < 0 || S < 1 || n_iter < 0 || (T > 0 && (!x_start || !X_out)) || !std::isfinite(spread) || spread < 0 ||
+        !(granularity >= 0) || n_boxes < 0 || (n_boxes > 0 && !boxes))
+        return fail(h, COV_ERR_INVALID, std::string(who) + ": bad arguments");
+    return COV_OK;
+}
+
 // The arguments and store every horizon call needs (cov_run_horizon's checks, in its order).  list_ok: the call can
 // replay the list-order sum (not the automaton), which it does when COV_OPT_LIST_ORDER_HORIZON is 1.
 static int check_horizon(cov_handle *h, const char *who, const double *x_start, int64_t T, int64_t S, double spread,
@@ -2072,10 +2083,7 @@ static int check_horizon(cov_handle *h, const char *who, const double *x_start, 
         return fail(h, COV_ERR_STATE, std::string(who) + ": the parameters have no previous swarm (cons3 is off)");
     if (!h->area_exact && !(list_ok && h->list_order_horizon))
         return fail(h, COV_ERR_STATE, std::string(who) + ": the store's area depends on the list order (area_exact == 0)");
-    if (T < 0 || S < 1 || n_iter < 0 || (T > 0 && (!x_start || !X_out)) || !std::isfinite(spread) || spread < 0 ||
-        !(granularity >= 0) || n_boxes < 0 || (n_boxes > 0 && !boxes))
-        return fail(h, COV_ERR_INVALID, std::string(who) + ": bad arguments");
-    return COV_OK;
+    return check_horizon_args(h, who, x_start, T, S, spread, n_iter, granularity, boxes, n_boxes, X_out);
 }
 
 // The envelope's plane set: for class k, planes for bits 0 .. floor(log2(max_mult[k])), where max_mult[k] bounds the
@@ -2971,6 +2979,178 @@ extern "C" int cov_mads_solve_batch_region(cov_handle *h, const double *X0, int6
     DeviceGuard dg(h->device);
     OK(check_region(h, "cov_mads_solve_batch_region"));
     return mads_solve_batch(h, true, X0, S, n_iter, granularity, seed, X_out, obj_out, stats);
+}
+
+// cov_run_horizon's loop on the region objective (DESIGN.md 18), all enqueued before one synchronise.  Per timestep
+// five launches: the covered set's step (launch_cover_arcs), horizon_start_kernel, the S solves (launch_cover_mads),
+// horizon_commit_kernel (its thresholds go to scratch: nothing reads them) and the objective of the winner
+// (launch_cover_eval).  The covered set grows in a buffer of the call; the handle gets it only when every timestep
+// passed, and otherwise its parameters are copied back from the snapshot taken when the call started.
+extern "C" int cov_run_horizon_region(cov_handle *h, const double *x_start, int64_t T, int64_t S, double spread,
+                                      int64_t n_iter, double granularity, uint64_t seed, const double *boxes,
+                                      int64_t n_boxes, double h_focus, double h_max, double *X_out, double *obj_out,
+                                      int64_t *stats, double *step_ms)
+{
+    const char *who = "cov_run_horizon_region";
+    if (!h) return fail(nullptr, COV_ERR_INVALID, "NULL handle");
+    DeviceGuard dg(h->device);
+    OK(check_region(h, who));
+    if (!h->o.use_cons3)
+        return fail(h, COV_ERR_STATE, std::string(who) + ": the parameters have no previous swarm (cons3 is off)");
+    OK(check_mads_limits(h, who, nullptr));
+    const int N = h->o.N, n = 3 * N, M0 = h->region.M;
+    if (T > 0 && T > (kRegionMaxCovered - M0) / N) // discs with R <= 0 count: how many go is known on the device only
+        return fail(h, COV_ERR_LIMIT, std::string(who) + ": M0 + T N = " + std::to_string(M0) + " + " +
+                                          std::to_string(T) + " x " + std::to_string(N) + " covered discs exceed the " +
+                                          std::to_string(kRegionMaxCovered) + " of the kernels' shared-memory plan");
+    OK(check_horizon_args(h, who, x_start, T, S, spread, n_iter, granularity, boxes, n_boxes, X_out));
+    if (T == 0) return COV_OK;
+    for (int q = 0; q < n; ++q)
+        if (!std::isfinite(x_start[q])) return fail(h, COV_ERR_INVALID, std::string(who) + ": x_start is not finite");
+    const int pitch = M0 + (int)T * N;
+    // in: [pow10 | x_start: n | boxes: 4 n_boxes | ctl: 4 ints | the solves' inputs]; out: [the solves' outputs |
+    // X_out: T n | obj_out: T | stats: T x 4 | the parameters at the call: 5N | thresholds: n | covered discs: 3 pitch]
+    const size_t tn = (size_t)T * n, o_x = kPow10Bytes, o_box = o_x + (size_t)n * 8;
+    const size_t o_ctl = o_box + (size_t)n_boxes * 32, o_X0 = o_ctl + 16;
+    const size_t o_par = tn * 8 + (size_t)T * 8 + (size_t)T * 32, o_xyT = o_par + (size_t)5 * N * 8;
+    const size_t o_disc = o_xyT + (size_t)n * 8, dev_bytes = o_disc + (size_t)3 * pitch * 8;
+    std::vector<unsigned char> hin(o_X0);
+    MadsArgs a;
+    OK(mads_buffers(h, o_X0, S, n, dev_bytes, hin, a));
+    memcpy(hin.data() + o_x, x_start, (size_t)n * 8);
+    if (n_boxes) memcpy(hin.data() + o_box, boxes, (size_t)n_boxes * 32);
+    const int ctl0[4] = {M0, h->region.K, 0, 0};
+    memcpy(hin.data() + o_ctl, ctl0, sizeof(ctl0));
+    OK(ensure_pinned(h, &h->h_out, &h->h_out_cap, o_par + sizeof(ctl0)));
+    DevBuf dd, da; // the region's discs and arcs after the call, swapped in on success as cov_set_region does
+    auto release = [&] {
+        if (dd.p) cudaFree(dd.p);
+        if (da.p) cudaFree(da.p);
+    };
+    int rc = ensure(h, dd, (size_t)3 * pitch * 8);
+    if (rc == COV_OK) rc = ensure(h, da, (size_t)kRegionMaxArcs * sizeof(RegionArc));
+    if (rc != COV_OK) {
+        release();
+        return rc;
+    }
+    unsigned char *din = (unsigned char *)h->mads_in.p;
+    const double *d_x0 = (const double *)(din + o_x);
+    double *d_Xo = (double *)(a.stats + 4 * S), *d_oo = d_Xo + tn;
+    long long *d_st = (long long *)(d_oo + T);
+    unsigned char *dres = (unsigned char *)d_Xo;
+    double *params = (double *)h->params.p, *backup = (double *)(dres + o_par), *xyT = (double *)(dres + o_xyT);
+    const RegionDesc &r = h->region;
+    const CoverSet cs{r.x_lo, r.y_lo, r.x_hi, r.y_hi, (double *)(dres + o_disc), (RegionArc *)da.p, pitch,
+                      (int *)(din + o_ctl)};
+    a.n_iter = n_iter;
+    a.granularity = granularity;
+    a.ordered = 0;
+    HorizonStep hs{};
+    hs.N = N;
+    hs.n_boxes = (int)n_boxes;
+    hs.S = S;
+    hs.E = 1;
+    hs.spread = spread;
+    hs.granularity = granularity;
+    hs.seed = seed;
+    hs.pow10 = a.pow10;
+    hs.boxes = (const double *)(din + o_box);
+    hs.h_focus = h_focus;
+    hs.h_max = h_max;
+    hs.tan_half_fov = h->o.tan_half_fov;
+    std::vector<cudaEvent_t> ev;
+    if (step_ms)
+        for (int64_t t = 0; t <= T; ++t) ev.push_back(get_event(h));
+
+    cudaError_t e = cudaMemcpyAsync(din, hin.data(), o_X0, cudaMemcpyHostToDevice, h->stream);
+    const char *what = "upload";
+    bool saved = false; // the parameters' snapshot is enqueued
+    if (e == cudaSuccess) {
+        what = "parameters";
+        e = cudaMemcpyAsync(backup, params, (size_t)5 * N * 8, cudaMemcpyDeviceToDevice, h->stream);
+        saved = e == cudaSuccess;
+    }
+    if (e == cudaSuccess && M0 > 0) // the handle's discs at the call's pitch
+        e = cudaMemcpy2DAsync(cs.discs, (size_t)pitch * 8, r.discs, (size_t)M0 * 8, (size_t)M0 * 8, 3,
+                              cudaMemcpyDeviceToDevice, h->stream), what = "covered discs";
+    for (int64_t t = 1; t <= T && e == cudaSuccess && rc == COV_OK; ++t) {
+        const double *cur = t == 1 ? d_x0 : d_Xo + (size_t)(t - 2) * n;
+        double *next = d_Xo + (size_t)(t - 1) * n;
+        long long *row = d_st + 4 * (t - 1);
+        if (step_ms && (e = cudaEventRecord(ev[(size_t)t - 1], h->stream)) != cudaSuccess) break;
+        what = "covered set";
+        if ((e = launch_cover_arcs(cs, cur, N, t, row, h->stream)) != cudaSuccess) break;
+        hs.t = t;
+        what = "horizon_start";
+        if ((e = launch_horizon_start(hs, cur, params, (double *)a.X0, (double *)a.a0, (int *)a.b0, h->stream)) !=
+            cudaSuccess)
+            break;
+        a.seed = seed + (uint64_t)(t - 1) * (uint64_t)S;
+        unsigned long long *counter = nullptr;
+        if ((rc = take_counter(h, &counter)) != COV_OK) break;
+        what = "MADS kernel";
+        if ((e = launch_cover_mads(cs, h->o, h->cfg, a, counter, h->stream)) != cudaSuccess) break;
+        what = "horizon_commit";
+        if ((e = launch_horizon_commit(S, N, a.X_out, a.obj_out, a.stats, next, row, xyT, h->stream)) != cudaSuccess)
+            break;
+        what = "objective";
+        if ((e = launch_cover_eval(cs, h->o, next, d_oo + (t - 1), h->stream)) != cudaSuccess) break;
+        h->launches += 5;
+    }
+    if (e == cudaSuccess && rc == COV_OK && step_ms) e = cudaEventRecord(ev[(size_t)T], h->stream), what = "event";
+    unsigned char *hres = (unsigned char *)h->h_out;
+    if (e == cudaSuccess && rc == COV_OK)
+        e = cudaMemcpyAsync(hres, d_Xo, o_par, cudaMemcpyDeviceToHost, h->stream), what = "download";
+    if (e == cudaSuccess && rc == COV_OK)
+        e = cudaMemcpyAsync(hres + o_par, cs.ctl, sizeof(ctl0), cudaMemcpyDeviceToHost, h->stream);
+    if (e == cudaSuccess && rc == COV_OK) e = cudaStreamSynchronize(h->stream), what = "synchronise";
+    const int *ctl = (const int *)(hres + o_par); // M_T, K_T, failure, its timestep
+    if (e == cudaSuccess && rc == COV_OK && ctl[2] == kCoverBadDisc)
+        rc = fail(h, COV_ERR_INVALID, std::string(who) + ": timestep " + std::to_string(ctl[3]) +
+                                          ": a disc of the swarm is not finite");
+    else if (e == cudaSuccess && rc == COV_OK && ctl[2] == kCoverManyArcs)
+        rc = fail(h, COV_ERR_LIMIT, std::string(who) + ": timestep " + std::to_string(ctl[3]) +
+                                        ": the covered discs' boundary has " + std::to_string(ctl[1]) +
+                                        " arcs inside the domain, more than the " + std::to_string(kRegionMaxArcs) +
+                                        " of the kernels' shared-memory plan");
+    // success: the final discs at their own pitch, cov_set_region's layout
+    if (e == cudaSuccess && rc == COV_OK && ctl[0] > 0)
+        e = cudaMemcpy2DAsync(dd.p, (size_t)ctl[0] * 8, cs.discs, (size_t)pitch * 8, (size_t)ctl[0] * 8, 3,
+                              cudaMemcpyDeviceToDevice, h->stream), what = "covered discs";
+    if (e != cudaSuccess || rc != COV_OK) { // the region and the parameters as before the call
+        if (rc == COV_OK)
+            rc = e == cudaErrorInvalidConfiguration
+                     ? fail(h, COV_ERR_LIMIT, std::string(who) + ": one warp of the solver does not fit the shared memory")
+                     : fail_cuda(h, e, (std::string(who) + ": " + what).c_str());
+        const std::string msg = h->err;
+        if (saved) {
+            (void)cudaMemcpyAsync(params, backup, (size_t)5 * N * 8, cudaMemcpyDeviceToDevice, h->stream);
+            (void)cudaStreamSynchronize(h->stream);
+            (void)cudaGetLastError();
+        }
+        release();
+        for (cudaEvent_t x : ev) h->ev_pool.push_back(x);
+        h->err = msg;
+        return rc;
+    }
+    std::swap(h->region_discs, dd);
+    std::swap(h->region_arcs, da);
+    release(); // the earlier region's buffers
+    h->region = RegionDesc{r.x_lo, r.y_lo, r.x_hi, r.y_hi, ctl[0], ctl[1], (const double *)h->region_discs.p,
+                           (const RegionArc *)h->region_arcs.p};
+    const double *hX = (const double *)hres, *hobj = hX + tn;
+    const int64_t *hst = (const int64_t *)(hobj + T);
+    memcpy(X_out, hX, tn * 8);
+    if (obj_out) memcpy(obj_out, hobj, (size_t)T * 8);
+    if (stats) memcpy(stats, hst, (size_t)T * 32);
+    for (int64_t t = 0; step_ms && t < T && rc == COV_OK; ++t) {
+        float ms = 0;
+        if ((e = cudaEventElapsedTime(&ms, ev[(size_t)t], ev[(size_t)t + 1])) != cudaSuccess)
+            rc = fail_cuda(h, e, (std::string(who) + ": cudaEventElapsedTime").c_str());
+        step_ms[t] = ms;
+    }
+    for (cudaEvent_t x : ev) h->ev_pool.push_back(x);
+    return rc;
 }
 
 // ------------------------------------------------------------------------------------------

@@ -141,6 +141,28 @@ cudaError_t launch_region_eval(const RegionDesc &r, const ObjParams &o, const La
 cudaError_t launch_mads_region(const RegionDesc &r, const ObjParams &o, const LaunchCfg &cfg, const MadsArgs &a,
                                unsigned long long *counter, cudaStream_t stream);
 
+// ---- cov_run_horizon_region (cov_region.cu, cov_mads.cu): the covered set grows on the device ----
+// The discs sit at a fixed pitch (the call's M0 + T N), so appending never moves them; M and K live in ctl, because
+// the R <= 0 filter and the arc count are known only on the device.  Once ctl[2] is set every kernel below returns at
+// once, touching nothing.
+constexpr int kCoverBadDisc = 1, kCoverManyArcs = 2; // ctl[2]
+struct CoverSet {
+    double x_lo, y_lo, x_hi, y_hi;
+    double *discs;   // [x_1..x_pitch | y | R]: the first ctl[0] of each are the covered discs
+    RegionArc *arcs; // the arcs of their boundary (capacity kRegionMaxArcs)
+    int pitch;
+    int *ctl;        // {M, K, failure (0: none), the timestep that failed}
+};
+// Step 1 of timestep t: cur's discs with R > 0 appended, the arcs recomputed, K to stats_row[3].
+cudaError_t launch_cover_arcs(const CoverSet &c, const double *cur, int N, long long t, long long *stats_row,
+                              cudaStream_t s);
+// cov_mads_solve_batch_region's solves on the covered set as ctl gives it, with the shared-memory plan of pitch discs
+// and kRegionMaxArcs arcs (cudaErrorInvalidConfiguration when even that plan's one warp does not fit).
+cudaError_t launch_cover_mads(const CoverSet &c, const ObjParams &o, const LaunchCfg &cfg, const MadsArgs &a,
+                              unsigned long long *counter, cudaStream_t stream);
+// The region objective without the barrier of one swarm x (device, 3N) to *obj (device).
+cudaError_t launch_cover_eval(const CoverSet &c, const ObjParams &o, const double *x, double *obj, cudaStream_t s);
+
 // ---- cell-store kernels (cov_grid_kernels.cu) ----
 // stats[0] = entries, stats[1] = cells, stats[2 + k] = OR of the multiplicities of class k
 cudaError_t launch_grid_stats(const unsigned char *mult, const unsigned char *cls, long long ncell,

@@ -540,6 +540,48 @@ cudaError_t launch_mads_region(const RegionDesc &r, const ObjParams &o, const La
     return cudaGetLastError();
 }
 
+// region_solve_kernel on cov_run_horizon_region's covered set: M and K read from c.ctl, the discs staged from their
+// pitch.  The shared-memory plan is the call's worst case (c.pitch discs, kRegionMaxArcs arcs), fixed for every
+// timestep; a candidate's area does not depend on the lists' capacity or on the warps per CTA, so the solves give
+// region_solve_kernel's bits.
+__global__ void __launch_bounds__(kRegionThreads, kRegionCtas)
+cover_solve_kernel(const __grid_constant__ CoverSet c, const __grid_constant__ ObjParams o,
+                   const __grid_constant__ MadsArgs a, unsigned long long *counter)
+{
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    if (c.ctl[2]) return; // the same word for every thread: the whole grid returns
+    const int N = o.N, n = 3 * N, warp = threadIdx.x >> 5;
+    unsigned char *rbase = smem_raw + mads_state_bytes(n);
+    const RegionDesc r{c.x_lo, c.y_lo, c.x_hi, c.y_hi, 0, 0, c.discs, c.arcs};
+    const RegionView v = cover_stage(r, c.pitch, c.ctl[0], min(c.ctl[1], kRegionMaxArcs), rbase);
+    unsigned char *wbase = rbase + region_smem_bytes(c.pitch, kRegionMaxArcs) + (size_t)warp * region_warp_bytes(N, c.pitch);
+    double *stage = reinterpret_cast<double *>(wbase);
+    double *ia = reinterpret_cast<double *>(wbase + round_up(3 * N * 8, 16)), *ib = ia + region_list_cap(N, c.pitch);
+    __syncthreads();
+    mads_solves(a, n, smem_raw, stage, counter, [&](unsigned long long k) { return a.seed + k; },
+                [&](const double *p) { // region_objective with the extreme barrier, as region_solve_kernel
+        const CandScalars cs = candidate_prologue<false>(GridDesc{}, o, p, nullptr, false);
+        if (!cs.feasible) return __longlong_as_double(0x7ff0000000000000ll);
+        const double obj = objective_from_area(region_area(v, p, N, ia, ib), cs.violation, o);
+        return (obj == obj) ? obj : __longlong_as_double(0x7ff0000000000000ll);
+    });
+}
+
+cudaError_t launch_cover_mads(const CoverSet &c, const ObjParams &o, const LaunchCfg &cfg, const MadsArgs &a,
+                              unsigned long long *counter, cudaStream_t stream)
+{
+    if (a.S <= 0) return cudaSuccess;
+    int warps = 0, smem = 0;
+    if (o.N > kRegionMaxUavs ||
+        !region_plan(o.N, c.pitch, kRegionMaxArcs, mads_state_bytes(3 * o.N), cfg.max_smem_optin - 1024 /* the kernel's static shared memory */, &warps, &smem))
+        return cudaErrorInvalidConfiguration;
+    int grid = 0;
+    cudaError_t err = persistent_grid(cover_solve_kernel, warps * 32, smem, a.S, cfg, &grid);
+    if (err != cudaSuccess) return err;
+    cover_solve_kernel<<<grid, warps * 32, smem, stream>>>(c, o, a, counter);
+    return cudaGetLastError();
+}
+
 // ---- the horizons on a list-order store (launch_list_mads, launch_list_eval) ----
 // Scenario e's list at timestep w.t (ListWalk): the base list, then its schedule's entries up to the timestep, each
 // live iff no removal since its append reached its cell.  The walk skips dead entries, so the sum is the one over the

@@ -64,6 +64,21 @@ __device__ __forceinline__ RegionView region_stage(const RegionDesc &r, unsigned
     return RegionView{d, d + r.M, d + 2 * r.M, arcs, r.M, r.K, r.x_lo, r.y_lo, r.x_hi, r.y_hi};
 }
 
+// region_stage for cov_run_horizon_region's covered set: M discs held at pitch `pitch` (r.discs: [x | y | R], each
+// pitch doubles) and K arcs at r.arcs, both counts read on the device.  The shared-memory layout is region_stage's.
+__device__ __forceinline__ RegionView cover_stage(const RegionDesc &r, int pitch, int M, int K, unsigned char *smem)
+{
+    double *d = reinterpret_cast<double *>(smem);
+    RegionArc *arcs = reinterpret_cast<RegionArc *>(smem + 3 * M * 8);
+    for (int t = threadIdx.x; t < M; t += blockDim.x) {
+        d[t] = r.discs[t];
+        d[M + t] = r.discs[pitch + t];
+        d[2 * M + t] = r.discs[2 * pitch + t];
+    }
+    for (int t = threadIdx.x; t < K; t += blockDim.x) arcs[t] = r.arcs[t];
+    return RegionView{d, d + M, d + 2 * M, arcs, M, K, r.x_lo, r.y_lo, r.x_hi, r.y_hi};
+}
+
 // 1/2 integral of (x dy - y dx) over the arc [t1, t2] of the circle (cx, cy, R), counter-clockwise.
 __device__ __forceinline__ double arc_term(double R, double cx, double cy, double t1, double t2)
 {
@@ -187,6 +202,48 @@ __device__ __forceinline__ void for_each_exposed(const double *ia, const double 
         }
         fn(has, pos, nxt);
     }
+}
+
+// The arcs of every covered circle m of r (r.M discs; r.arcs / r.K unused) that lie inside the domain and inside no
+// other covered disc, in circle order and, per circle, in list order of their starts, by one warp; ia / ib: the warp's
+// list, region_list_cap(0, M) doubles each.  Writes at most cap arcs to out and the count of all of them to *count
+// (lane 0); every lane returns that count.
+__device__ __forceinline__ int covered_arcs(const RegionView &v, double *ia, double *ib, RegionArc *out, int cap,
+                                            int *count)
+{
+    const int M = v.M;
+    const uint32_t lane = lane_id();
+    int K = 0;
+    for (int m = 0; m < M; ++m) {
+        const double cx = v.cx[m], cy = v.cy[m], R = v.cr[m];
+        int n = 0;
+        bool whole = false;
+        for (int j0 = 0; j0 < M + 4 && !whole; j0 += 32) {
+            const int j = j0 + (int)lane;
+            int rel = 0;
+            double phi = 0.0, alpha = 0.0;
+            if (j < M) {
+                if (j != m) rel = circle_vs_disc(cx, cy, R, v.cx[j], v.cy[j], v.cr[j], m < j, phi, alpha);
+            } else if (j < M + 4) {
+                rel = circle_vs_edge(v, j - M, cx, cy, R, phi, alpha);
+            }
+            whole = __any_sync(0xffffffffu, rel == 2);
+            double a0 = 0, b0 = 0, a1 = 0, b1 = 0;
+            const int k = rel == 1 ? wrap_interval(phi, alpha, a0, b0, a1, b1) : 0;
+            n = warp_append(ia, ib, n, k, a0, b0, a1, b1);
+        }
+        __syncwarp();
+        if (!whole)
+            for_each_exposed(ia, ib, n, 0.0, kTwoPi, [&](bool has, double pos, double nxt) {
+                const uint32_t bal = __ballot_sync(0xffffffffu, has);
+                const int at = K + __popc(bal & ((1u << lane) - 1u));
+                if (has && at < cap) out[at] = RegionArc{pos, nxt, m, 0};
+                K += __popc(bal);
+            });
+        __syncwarp();
+    }
+    if (lane == 0) *count = K;
+    return K;
 }
 
 // A(x) of the candidate in `st` (3N doubles, shared memory, visible to the warp), by one warp; ia / ib: the warp's

@@ -530,7 +530,7 @@ class CoverageEngine:
         return out + tuple(a for a, want in ((cells, want_cells), (last, want_last_removed)) if want)
 
     def _horizon(self, fn, x_start, T, cols, S, spread, n_iter, granularity, seed, boxes, h_focus, h_max, source,
-                 tail=()):
+                 tail=(), names=("winner", "evaluations", "feasible", "removed", "appended")):
         x_start = _f64(x_start).ravel()
         if self.N is None or x_start.size != 3 * self.N:
             raise ValueError("x_start must have 3N entries")
@@ -544,8 +544,7 @@ class CoverageEngine:
         self._check(fn(self._h, _ptr(x_start), T, int(S), float(spread), int(n_iter), float(granularity),
                        int(seed) & (2**64 - 1), _ptr(B) if len(B) else None, len(B), float(h_focus), float(h_max),
                        *source, _ptr(X), _ptr(obj), _ptr(st), _ptr(ms), *tail))
-        names = ("winner", "evaluations", "feasible", "removed", "appended")[:cols]
-        return X, obj, {name: st[:, q].copy() for q, name in enumerate(names)}, ms
+        return X, obj, {name: st[:, q].copy() for q, name in enumerate(names[:cols])}, ms
 
     # ---- grid-free static objective ----
     def set_region(self, x_lo: float, y_lo: float, x_hi: float, y_hi: float, covered=None):
@@ -555,6 +554,19 @@ class CoverageEngine:
         xyR = np.ascontiguousarray(C3.T).ravel()  # [x_1..x_M, y_1..y_M, R_1..R_M]
         self._check(lib.cov_set_region(self._h, float(x_lo), float(y_lo), float(x_hi), float(y_hi),
                                        _ptr(xyR) if len(C3) else None, len(C3)))
+
+    def run_horizon_region(self, x_start, T: int, S: int = 1, spread: float = 3.0, n_iter: int = 100,
+                           granularity: float = 1.0, seed: int = 0, boxes=None, h_focus: float = 15.0,
+                           h_max: float = 30.0):
+        """run_horizon on the grid-free static objective (cov_run_horizon_region): per timestep the current swarm's
+        discs with R > 0 join the region's covered set, then the r_max rule, cons3 from the current swarm and S
+        mads_solve_batch_region solves, the best one as the next swarm.  Needs set_region and set_params with
+        prev_xyR.  Returns (X (T, 3N), obj (T,), stats, step_ms (T,)) with stats a dict of int64 arrays: winner,
+        evaluations, feasible, arcs (of the covered set's boundary at each timestep).  The covered set, its arcs and the
+        parameters of the last timestep stay set on the engine; a call that raises leaves the region and the parameters
+        as they were."""
+        return self._horizon(lib.cov_run_horizon_region, x_start, T, 4, S, spread, n_iter, granularity, seed, boxes,
+                             h_focus, h_max, (), names=("winner", "evaluations", "feasible", "arcs"))
 
     def eval_region_batch(self, X, want_area=True, want_feasible=True, best=False, barrier: bool = True):
         """cov_eval_region_batch: dict(obj, area, feasible) for every row of X (B, 3N), with best=True also

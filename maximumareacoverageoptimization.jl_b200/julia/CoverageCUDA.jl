@@ -693,6 +693,29 @@ function mads_solve_batch_region(h::Handle, X0::Matrix{Float64}; N_iter = 100, g
 end
 
 """
+    run_horizon_region(h, x_start; T, S = 1, spread = 3.0, N_iter = 100, granularity = 1.0, seed = 0,
+                       boxes = zeros(Float64, 4, 0), h_focus = 15.0, h_max = 30.0)
+
+`run_horizon` on the region objective (`cov_run_horizon_region`): per timestep the current swarm's discs with R > 0
+join the region's covered set, then the r_max rule, cons3 from the current swarm, S `mads_solve_batch_region` solves
+and the best as the next swarm. Needs `set_region!` and `set_params!` with a previous swarm. Returns
+`(X, objectives, stats, step_ms)`: `X` 3N x T, `stats` 4 x T with rows winner, evaluations, feasible solves, arcs of
+the covered set's boundary.
+"""
+function run_horizon_region(h::Handle, x_start::Vector{Float64}; T, S = 1, spread = 3.0, N_iter = 100,
+                            granularity = 1.0, seed = 0, boxes::Matrix{Float64} = zeros(Float64, 4, 0), h_focus = 15.0,
+                            h_max = 30.0)
+    n = length(x_start); K = size(boxes, 2)
+    X = zeros(Float64, n, T); obj = zeros(Float64, T); stats = zeros(Int64, 4, T); ms = zeros(Float64, T)
+    GC.@preserve x_start boxes X obj stats ms check(h, ccall((:cov_run_horizon_region, LIB), Cint,
+        (Ptr{Cvoid}, Ptr{Float64}, Int64, Int64, Float64, Int64, Float64, UInt64, Ptr{Float64}, Int64, Float64,
+         Float64, Ptr{Float64}, Ptr{Float64}, Ptr{Int64}, Ptr{Float64}),
+        h.ptr, x_start, T, S, spread, N_iter, granularity, seed, K == 0 ? C_NULL : pointer(boxes), K, h_focus, h_max,
+        X, obj, stats, ms))
+    return X, obj, stats, ms
+end
+
+"""
     createObjective(cells, N, r_max; handle = Handle())
 
 Same signature and value as the reference's `TDM_STATIC_opt.createObjective` (src/TDM_STATIC_opt.jl:82):
